@@ -5,6 +5,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...     # the reference arm: the CPU oracle on all host threads
+    python bench.py ... --dump-outputs DIR   # also write the last timed step's tau and qdd (a fixed sample) to DIR
 
 One step = one batched RNEA pass (BASELINE.json configs[1]) + one batched forward-dynamics pass (configs[2]) over
 2^24 synthetic FR3 states per GPU, device-resident SoA, sampled on the device by the counter-based generator of
@@ -45,6 +46,8 @@ FP64_STATIC = {"rb_rnea_kernel": 804, "rb_fd_kernel": 1299}
 FP64_FALLBACK = {"rb_rnea_kernel": 126, "rb_fd_kernel": 126}
 FP64_INSTR = {k: FP64_STATIC[k] - FP64_FALLBACK[k] for k in FP64_STATIC}
 FP64_LANES_PER_SM = 64
+# --dump-outputs: states written per array, chosen once by a fixed seed so that two builds compare output for output
+DUMP_STATES, DUMP_SEED = 1 << 18, 0x5EED00D0
 
 
 def profiled(kernel):
@@ -279,6 +282,18 @@ def fp64_roofline(kernel, ms, units, instr_per_unit, flops_executed_per_unit, al
     return d
 
 
+def dump_outputs(out_dir, arrays):
+    """Writes each [n, B] float64 device array as out_dir/<name>.npy.  Where B > DUMP_STATES only the columns of a fixed,
+    seeded sample of DUMP_STATES state indices (increasing) are written: 2 x 7 x 2^18 doubles = 29 MB for the FR3 step."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name, x in arrays.items():
+        if x.shape[1] > DUMP_STATES:
+            idx = np.sort(np.random.default_rng(DUMP_SEED).choice(x.shape[1], DUMP_STATES, replace=False))
+            x = x.index_select(1, torch.from_numpy(idx).to(x.device))
+        np.save(os.path.join(out_dir, name + ".npy"), x.cpu().numpy())
+
+
 def run_ours(args, rank, local_rank, world):
     import torch
     import torch.distributed as dist
@@ -340,6 +355,8 @@ def run_ours(args, rank, local_rank, world):
     clocks = sampler.stop()
     launches = mb.launch_count - launches0
     mb.sync()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"tau": tau, "qdd": qdd})
     total_ms = t_start.elapsed_time(t_end)
     # FP64 roofline denominator: DFMA probe on the same GPU in the same run, run for about as long as the timed
     # region (a burst of a few ms keeps 1965 MHz; seconds of FP64 work pull ~1 kW and settle near 1.7 GHz under
@@ -590,7 +607,14 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-chain32", action="store_true", help="skip the configs.chain32 leg")
     ap.add_argument("--chain32-states", type=int, default=1 << 26, help="states of the chain32 leg, split over the GPUs (BASELINE configs[4]: 64M)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write DIR/tau.npy and DIR/qdd.npy: the last step's RNEA and forward-dynamics "
+                         "results, float64 [n, S], S = a fixed seeded sample of 2^18 states (all if fewer); rank 0's states")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

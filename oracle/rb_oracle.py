@@ -14,6 +14,7 @@ from __future__ import annotations
 import ctypes as C
 import os
 import subprocess
+import tempfile
 import xml.etree.ElementTree as ET
 from dataclasses import dataclass
 
@@ -87,11 +88,16 @@ def parse_urdf(path) -> ModelArrays:
 
 
 # --------------------------------------------------------------------------- library
-def build(fast: bool = False) -> str:
-    """Compile the oracle with the committed recipe (oracle/Makefile); returns the .so path."""
-    target = "librb_oracle_fast.so" if fast else "librb_oracle.so"
-    subprocess.run(["make", "-s", "-C", _HERE, target], check=True)
-    return os.path.join(_HERE, target)
+def build(fast: bool = False, out_dir: str | None = None) -> str:
+    """Compile the oracle with the committed recipe (oracle/Makefile); returns the .so path.  The -march=native
+    build (`fast`) goes to `out_dir`, which the caller creates afresh: it is specific to this host, and the tree it
+    would otherwise land in may be read-only."""
+    if not fast:
+        subprocess.run(["make", "-s", "-C", _HERE, "librb_oracle.so"], check=True)
+        return os.path.join(_HERE, "librb_oracle.so")
+    path = os.path.join(out_dir, "librb_oracle_fast.so")
+    subprocess.run(["make", "-s", "-C", _HERE, "FAST_SO=" + path, path], check=True)
+    return path
 
 
 class _MB(C.Structure):
@@ -110,8 +116,11 @@ class Oracle:
     """One loaded model.  All arrays float64; batch layout 'soa' = [n][B], 'aos' = [B][n]."""
 
     def __init__(self, model: ModelArrays, fast: bool = False):
-        path = build(fast)
-        lib = C.CDLL(path)
+        if fast:
+            with tempfile.TemporaryDirectory(prefix="rb_oracle_") as d:
+                lib = C.CDLL(build(True, d))         # stays loaded after its directory is gone
+        else:
+            lib = C.CDLL(build())
         self.lib = lib
         self.model = model
         self.n = model.n

@@ -1,6 +1,5 @@
 """CPU tests of the oracle itself (no GPU): what pins the oracle, since the reference pins nothing (SURVEY.md 4, 8c)."""
 import ctypes as C
-import os
 
 import numpy as np
 import pytest
@@ -27,12 +26,13 @@ def test_urdf_pairing_matches_survey_table(oracle_fr3):
     np.testing.assert_array_equal(m.effort, [87, 87, 87, 87, 12, 12, 12])
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/assets/fr3.urdf"), reason="reference checkout absent")
 def test_dynamics_only_urdf_equals_reference_urdf():
-    a, b = parse_urdf("/root/reference/assets/fr3.urdf"), parse_urdf(FR3)
+    """assets/fr3.urdf loads to exactly the model the reference's robot description gives (stored in
+    tests/golden/fr3_reference_model.json)."""
+    a, b = load_golden("fr3_reference_model.json"), parse_urdf(FR3)
     for k in ("axis", "xyz", "rpy", "mass", "com", "inertia6", "lower", "upper", "velocity", "effort"):
-        np.testing.assert_array_equal(getattr(a, k), getattr(b, k))
-    assert a.names == b.names
+        np.testing.assert_array_equal(np.array(a[k]), getattr(b, k))
+    assert a["names"] == b.names
 
 
 def test_survey_known_answers(oracle_fr3):
