@@ -57,6 +57,11 @@ struct DevBuf {
     void release() { if (p) cudaFree(p); p = nullptr; bytes = 0; }
 };
 
+// One entry point of an engine, bound when the engine is created: the launcher, its parameter block, and whether its
+// kernels work in engine-owned scratch (RbOps::shared_scratch).
+template <class Fn>
+struct Bound { Fn fn = nullptr; const void* param = nullptr; bool shared = false; };
+
 }  // namespace
 
 // One host thread per device of a multi-device engine: runs the slice of a host batch that its device owns.
@@ -112,11 +117,13 @@ struct RbGpu {
     int device = 0;
     int sm_count = 0;
     RbHostModel model;
-    const RbOps* ops = nullptr;
+    const RbOps* ops = nullptr;           // the primary family
     std::vector<unsigned char> param;     // host image of the kernel-parameter block `ops` expects
     std::vector<double> flat;             // the model rows as uploaded (rb_model.h layout)
-    const RbOps* ops2 = nullptr;          // fallback table for entries `ops` leaves null (run-time-n family)
-    std::vector<unsigned char> param2;
+    std::vector<unsigned char> param_n;   // parameter block of the fallback table (run-time-n family) if `ops` leaves entries null
+    // bound by bind_entries; the optional entries (rnea_aos, fd_aos, rnea_fd, rnea_f32, fd_f32) are the primary family's alone
+    Bound<decltype(RbOps::rnea)> rnea; Bound<decltype(RbOps::fd)> fd; Bound<decltype(RbOps::crba)> crba;
+    Bound<decltype(RbOps::fwd_kin)> fwd_kin; Bound<decltype(RbOps::jac)> jac; Bound<decltype(RbOps::rollout)> rollout;
     size_t hpk_states = 0;
     RbJitParam jit{};                     // run-time compiled kernels (jit-specialised family); lib == nullptr if unused
     std::string family_note;              // why this family was chosen (e.g. the JIT fallback reason)
@@ -149,20 +156,26 @@ struct Multibody {
     std::mutex mu;
 };
 
-// Table / parameter block serving one entry point: the primary family, or the fallback where it has no kernel.
-#define RB_TABLE(g, fn) ((g)->ops->fn ? (g)->ops : (g)->ops2)
-#define RB_PARAM(g, fn) ((g)->ops->fn ? (const void*)(g)->param.data() : (const void*)(g)->param2.data())
-
 namespace {
 
 // Kernel families that work in engine-owned scratch (RbOps::shared_scratch) must not overlap with each other
 // across streams: every such launch waits for the previous one's event and records its own.
 struct ScratchOrder {
     RbGpu* g; cudaStream_t st; bool on;
-    ScratchOrder(RbGpu* g_, const RbOps* t, cudaStream_t st_);
-    ScratchOrder(RbGpu* g_, bool shared, cudaStream_t st_);
-    ~ScratchOrder();
+    ScratchOrder(RbGpu* g_, bool shared, cudaStream_t st_) : g(g_), st(st_), on(shared) {
+        if (on) { g->mu_scratch.lock(); cudaStreamWaitEvent(st, g->ev_scratch, 0); }
+    }
+    ~ScratchOrder() {
+        if (on) { cudaEventRecord(g->ev_scratch, st); g->mu_scratch.unlock(); }
+    }
 };
+
+// Runs a bound entry on stream `st` (every RbOps launcher takes the stream last), ordered by ScratchOrder.
+template <class Fn, class... A>
+cudaError_t launch(RbGpu* g, const Bound<Fn>& e, cudaStream_t st, A... a) {
+    ScratchOrder so(g, e.shared, st);
+    return e.fn(e.param, a..., st);
+}
 
 struct DeviceGuard {
     int prev = -1; bool ok = true;
@@ -173,20 +186,10 @@ struct DeviceGuard {
     ~DeviceGuard() { if (prev >= 0) cudaSetDevice(prev); }
 };
 
-// Sets up the run-time-n family (model rows + scratch + H chunk on the device) as table `ops`/`param`.
-ScratchOrder::ScratchOrder(RbGpu* g_, const RbOps* t, cudaStream_t st_) : g(g_), st(st_), on(t->shared_scratch) {
-    if (on) { g->mu_scratch.lock(); cudaStreamWaitEvent(st, g->ev_scratch, 0); }
-}
-ScratchOrder::ScratchOrder(RbGpu* g_, bool shared, cudaStream_t st_) : g(g_), st(st_), on(shared) {
-    if (on) { g->mu_scratch.lock(); cudaStreamWaitEvent(st, g->ev_scratch, 0); }
-}
-ScratchOrder::~ScratchOrder() {
-    if (on) { cudaEventRecord(g->ev_scratch, st); g->mu_scratch.unlock(); }
-}
-
-int setup_generic_n(RbGpu* g, const std::vector<double>& flat, const RbOps** ops, std::vector<unsigned char>* param) {
+// Sets up the run-time-n family (model rows + scratch + H chunk on the device); `param` receives its parameter block.
+int setup_generic_n(RbGpu* g, std::vector<unsigned char>* param) {
     const int n = g->model.n;
-    *ops = rb_ops_generic_n();
+    const std::vector<double>& flat = g->flat;
     RB_CUDA(cudaMalloc((void**)&g->d_model, flat.size() * sizeof(double)));
     RB_CUDA(cudaMemcpy(g->d_model, flat.data(), flat.size() * sizeof(double), cudaMemcpyHostToDevice));
     // persistent grid: 8 blocks of RB_BLOCK threads per SM; scratch sized for the largest user (rollout)
@@ -206,106 +209,117 @@ int setup_generic_n(RbGpu* g, const std::vector<double>& flat, const RbOps** ops
     }
     RbNParam P{g->d_model, n, g->scratch.p, g->scratch_threads, slots, g->hpk.p, g->hpk_states, tree ? 1 : 0};
     param->assign(sizeof(P), 0);
-    if ((*ops)->param_bytes != sizeof(P)) return fail(RB_ERR_ARG, "internal: RbNParam size mismatch");
+    if (rb_ops_generic_n()->param_bytes != sizeof(P)) return fail(RB_ERR_ARG, "internal: RbNParam size mismatch");
     memcpy(param->data(), &P, sizeof(P));
     return RB_OK;
 }
 
-// Chooses the kernel family for the uploaded chain.  `ops` may leave entries null (long-chain families serve
-// rnea / fd / crba only); those calls go to the fallback table `ops2` (always the run-time-n family).
+// Compiles (or reads from the disk cache) and loads the run-time specialised kernels of the chain and installs them as
+// the primary family: rb_jit_compile builds the full set up to RB_JIT_MAX_N joints ("jit-specialised") and the long-chain
+// set beyond ("jit-long").  On failure returns the status with the reason in `log`; the caller decides whether it is fatal.
+int install_jit(RbGpu* g, std::string& log) {
+    RbJitImage img;
+    int rc = rb_jit_compile(g->model, img, log);
+    if (rc == RB_OK) { std::string err; rc = rb_jit_load(img, g->model.n, g->jit, err); if (rc != RB_OK) log = err; }
+    if (rc != RB_OK) return rc;
+    g->ops = g->model.n > RB_JIT_MAX_N ? rb_ops_jit_long() : rb_ops_jit();
+    g->param.assign(sizeof(RbJitParam), 0);
+    memcpy(g->param.data(), &g->jit, sizeof(RbJitParam));
+    g->family_note = std::string(g->model.serial ? "" : "kinematic tree: ") + (img.from_cache ? "kernels from the disk cache" : "kernels compiled with NVRTC");
+    return RB_OK;
+}
+
+// Chooses the primary kernel family for the uploaded chain ($RIGIDBODY_B200_VARIANT forces one, $RIGIDBODY_B200_JIT=0
+// keeps `auto` off the run-time compiler).  The families are tried top to bottom; the first that fits serves.
 int pick_ops(RbGpu* g) {
     const char* force = getenv("RIGIDBODY_B200_VARIANT");
+    const char* jit_env = getenv("RIGIDBODY_B200_JIT");
     const std::string want = force ? force : "auto";
+    const bool any = want == "auto", jit_on = !(jit_env && std::string(jit_env) == "0");
     const int n = g->model.n;
     g->flat = rb_model_flat(g->model);
     const std::vector<double>& flat = g->flat;
+    const std::string too_long = "RIGIDBODY_B200_VARIANT=jit-specialised needs a chain of at most " + std::to_string(RB_JIT_MAX_N) + " joints";
+    std::string log;
     if (!g->model.serial) {
         // kinematic trees (parent[i] != i-1): run-time specialised kernels up to RB_JIT_MAX_N joints (the unrolled templates follow
         // the compile-time parent table, rb_dyn_tree.cuh), the run-time-n family otherwise
-        if (want != "auto" && want != "generic-n" && want != "jit-specialised")
+        if (!any && want != "generic-n" && want != "jit-specialised")
             return fail(RB_ERR_UNSUPPORTED, "RIGIDBODY_B200_VARIANT=" + want + " serves serial chains only; trees run on jit-specialised or generic-n");
-        const char* jit_env = getenv("RIGIDBODY_B200_JIT");
-        const bool jit_on = !(jit_env && std::string(jit_env) == "0");
-        if (want != "generic-n" && (jit_on || want == "jit-specialised") && n <= RB_JIT_MAX_N) {
-            RbJitImage img; std::string log;
-            int rc = rb_jit_compile(g->model, img, log);
-            if (rc == RB_OK) { std::string err; rc = rb_jit_load(img, n, g->jit, err); if (rc != RB_OK) log = err; }
-            if (rc == RB_OK) {
-                g->ops = rb_ops_jit();
-                g->param.assign(sizeof(RbJitParam), 0);
-                memcpy(g->param.data(), &g->jit, sizeof(RbJitParam));
-                g->family_note = std::string("kinematic tree: ") + (img.from_cache ? "kernels from the disk cache" : "kernels compiled with NVRTC");
-                return RB_OK;
-            }
+        if ((want == "jit-specialised" || (any && jit_on)) && n <= RB_JIT_MAX_N) {
+            const int rc = install_jit(g, log);
+            if (rc == RB_OK) return RB_OK;
             if (want == "jit-specialised") return fail(rc, "run-time specialisation failed: " + log);
         } else if (want == "jit-specialised") {
-            return fail(RB_ERR_UNSUPPORTED, "RIGIDBODY_B200_VARIANT=jit-specialised needs a chain of at most 18 joints");
+            return fail(RB_ERR_UNSUPPORTED, too_long);
         }
         g->family_note = "kinematic tree: run-time-n kernels (rbn_tree_* recursions)";
-        return setup_generic_n(g, flat, &g->ops, &g->param);
+        g->ops = rb_ops_generic_n();
+        return setup_generic_n(g, &g->param);
     }
     const bool is_fr3 = n == 7 && memcmp(flat.data(), rb_fr3_table(), sizeof(double) * RB_MODEL_DOUBLES(7)) == 0;
     const bool is_c32 = n == 32 && memcmp(flat.data(), rb_chain32_table(), sizeof(double) * RB_MODEL_DOUBLES(32)) == 0;
-    if ((want == "auto" || want == "fr3-specialised") && is_fr3) {
+    const bool jit_auto = any && jit_on && !is_c32;
+    // the compiled-in FR3 model
+    if ((any || want == "fr3-specialised") && is_fr3) {
         g->ops = rb_ops_fr3();
         g->param.assign(g->ops->param_bytes, 0);
         return RB_OK;
     }
     if (want == "fr3-specialised") return fail(RB_ERR_UNSUPPORTED, "RIGIDBODY_B200_VARIANT=fr3-specialised but the chain is not the compiled-in FR3 model");
-    // Any other short chain: compile the same templates for ITS constants at run time (NVRTC, disk-cached).
-    const char* jit_env = getenv("RIGIDBODY_B200_JIT");
-    const bool jit_on = !(jit_env && std::string(jit_env) == "0");
-    if ((want == "jit-specialised" || (want == "auto" && jit_on && !is_c32)) && n <= RB_JIT_MAX_N) {
-        RbJitImage img; std::string log;
-        int rc = rb_jit_compile(g->model, img, log);
-        if (rc == RB_OK) { std::string err; rc = rb_jit_load(img, n, g->jit, err); if (rc != RB_OK) log = err; }
-        if (rc == RB_OK) {
-            g->ops = rb_ops_jit();
-            g->param.assign(sizeof(RbJitParam), 0);
-            memcpy(g->param.data(), &g->jit, sizeof(RbJitParam));
-            g->family_note = img.from_cache ? "kernels from the disk cache" : "kernels compiled with NVRTC";
-            return RB_OK;
-        }
+    // any other short chain: the same templates compiled for ITS constants at run time (NVRTC, disk-cached)
+    if ((want == "jit-specialised" || jit_auto) && n <= RB_JIT_MAX_N) {
+        const int rc = install_jit(g, log);
+        if (rc == RB_OK) return RB_OK;
         if (want == "jit-specialised") return fail(rc, "run-time specialisation failed: " + log);
         g->family_note = "run-time specialisation unavailable (" + log.substr(0, 200) + "); using run-time-constant kernels";
     } else if (want == "jit-specialised") {
-        return fail(RB_ERR_UNSUPPORTED, "RIGIDBODY_B200_VARIANT=jit-specialised needs a chain of at most 18 joints");
+        return fail(RB_ERR_UNSUPPORTED, too_long);
     }
-    // chains of 19..32 joints: rnea / crba / fwd_kin / jac specialised at load time ("jit-long"), forward dynamics and
-    // rollouts through the run-time-n family (lane-per-joint kernels)
-    if ((want == "jit-long" || (want == "auto" && jit_on && !is_c32)) && n > RB_JIT_MAX_N && n <= RB_JIT_LONG_MAX_N) {
-        RbJitImage img; std::string log;
-        int rc = rb_jit_compile(g->model, img, log);
-        if (rc == RB_OK) { std::string err; rc = rb_jit_load(img, n, g->jit, err); if (rc != RB_OK) log = err; }
-        if (rc == RB_OK) {
-            g->ops = rb_ops_jit_long();
-            g->param.assign(sizeof(RbJitParam), 0);
-            memcpy(g->param.data(), &g->jit, sizeof(RbJitParam));
-            g->family_note = img.from_cache ? "kernels from the disk cache" : "kernels compiled with NVRTC";
-            return setup_generic_n(g, flat, &g->ops2, &g->param2);
-        }
+    // chains of 19..32 joints: rnea / crba / fwd_kin / jac specialised at load time, forward dynamics and rollouts
+    // through the fallback table (lane-per-joint kernels)
+    if ((want == "jit-long" || jit_auto) && n > RB_JIT_MAX_N && n <= RB_JIT_LONG_MAX_N) {
+        const int rc = install_jit(g, log);
+        if (rc == RB_OK) return setup_generic_n(g, &g->param_n);
         if (want == "jit-long") return fail(rc, "run-time specialisation failed: " + log);
         g->family_note = "run-time specialisation unavailable (" + log.substr(0, 200) + "); using run-time-n kernels";
     } else if (want == "jit-long") {
         return fail(RB_ERR_UNSUPPORTED, "RIGIDBODY_B200_VARIANT=jit-long serves chains of 19..32 joints");
     }
-    if ((want == "auto" || want == "generic-7") && n == 7) {
+    // any 7-joint chain, constants from the kernel-parameter bank
+    if ((any || want == "generic-7") && n == 7) {
         g->ops = rb_ops_rt7();
-        g->param.assign(g->ops->param_bytes, 0);
         if (g->ops->param_bytes != flat.size() * sizeof(double)) return fail(RB_ERR_ARG, "internal: RbModelK<7> size mismatch");
-        memcpy(g->param.data(), flat.data(), g->ops->param_bytes);
+        g->param.assign((const unsigned char*)flat.data(), (const unsigned char*)flat.data() + g->ops->param_bytes);
         return RB_OK;
     }
     if (want == "generic-7") return fail(RB_ERR_UNSUPPORTED, "RIGIDBODY_B200_VARIANT=generic-7 needs a 7-joint chain");
-    if (want != "auto" && want != "generic-n" && want != "chain32-specialised" && want != "jit-specialised" && want != "jit-long")
+    if (!any && want != "generic-n" && want != "chain32-specialised" && want != "jit-specialised" && want != "jit-long")
         return fail(RB_ERR_ARG, "unknown RIGIDBODY_B200_VARIANT '" + want + "'");
-    if ((want == "auto" || want == "chain32-specialised") && is_c32) {
+    // the compiled-in 32-joint model: rnea / crba, the rest through the fallback table
+    if ((any || want == "chain32-specialised") && is_c32) {
         g->ops = rb_ops_chain32();
         g->param.assign(g->ops->param_bytes, 0);
-        return setup_generic_n(g, flat, &g->ops2, &g->param2);
+        return setup_generic_n(g, &g->param_n);
     }
     if (want == "chain32-specialised") return fail(RB_ERR_UNSUPPORTED, "RIGIDBODY_B200_VARIANT=chain32-specialised but the chain is not the compiled-in 32-joint model");
-    return setup_generic_n(g, flat, &g->ops, &g->param);
+    g->ops = rb_ops_generic_n();
+    return setup_generic_n(g, &g->param);
+}
+
+// Binds rnea, fd, crba, fwd_kin, jac and rollout once: to the primary family where it has the entry, otherwise to the
+// fallback table, whose parameter block pick_ops set up for the families that need it.
+int bind_entries(RbGpu* g) {
+    bool ok = true;
+    auto bind = [&](auto& e, auto RbOps::*fn) {
+        const bool own = g->ops->*fn != nullptr;
+        const RbOps* t = own ? g->ops : rb_ops_generic_n();
+        e = {t->*fn, own ? g->param.data() : g->param_n.data(), t->shared_scratch};
+        ok = ok && e.fn && (own || !g->param_n.empty());
+    };
+    bind(g->rnea, &RbOps::rnea); bind(g->fd, &RbOps::fd); bind(g->crba, &RbOps::crba);
+    bind(g->fwd_kin, &RbOps::fwd_kin); bind(g->jac, &RbOps::jac); bind(g->rollout, &RbOps::rollout);
+    return ok ? RB_OK : fail(RB_ERR_ARG, std::string("internal: kernel family '") + g->ops->name + "' leaves an entry point unbound");
 }
 
 int gpu_create(const RbHostModel& model, int device, RbGpu** out) {
@@ -347,6 +361,7 @@ int gpu_create(const RbHostModel& model, int device, RbGpu** out) {
     // cost weights of multibody_rollout_cost: allocated once, here (a lazy first-call allocation would race)
     { int rcw = g->cost_w.ensure(sizeof(double) * RB_CW_ROWS * RB_MAX_N); if (rcw != RB_OK) return bail(rcw); }
     int rc = pick_ops(g);
+    if (rc == RB_OK) rc = bind_entries(g);
     if (rc != RB_OK) return bail(rc);
     if (const char* f = getenv("RIGIDBODY_B200_FUSED")) g->split_rnea_fd = std::string(f) == "0";
     *out = g;
@@ -651,8 +666,7 @@ int gpu_create_multi(const RbHostModel& model, const int* devices, int n_dev, Rb
             multibody_gpu_free(g);
             return fail(rc, msg);
         }
-    g->sm_count = g->peers[0]->sm_count;
-    g->ops = g->peers[0]->ops;
+    g->ops = g->peers[0]->ops;            // kernel_variant and family_note only: the peers run the calls
     g->family_note = g->peers[0]->family_note;
     for (int i = 0; i < n_dev; ++i) {
         RbWorker* w = new (std::nothrow) RbWorker();
@@ -815,8 +829,7 @@ extern "C" int multibody_rnea_batch(RbGpu* g, const double* q, const double* dq,
     const int n = g->model.n;
     OpDesc op{3, {q, dq, ddq}, {n, n, n}, tau, n,
               [](RbGpu* g, const double* const* in, double* out, size_t B, size_t ld, cudaStream_t st, int* status) {
-                  ScratchOrder so(g, RB_TABLE(g, rnea), st);
-                  return RB_TABLE(g, rnea)->rnea(RB_PARAM(g, rnea), in[0], in[1], in[2], out, B, ld, st);
+                  return launch(g, g->rnea, st, in[0], in[1], in[2], out, B, ld);
               },
               [](RbGpu* g, const double* const* in, double* out, size_t B, cudaStream_t st, int* status) {
                   return g->ops->rnea_aos(g->param.data(), in[0], in[1], in[2], out, B, st);
@@ -831,8 +844,7 @@ extern "C" int multibody_forward_dynamics_batch(RbGpu* g, const double* q, const
     const int n = g->model.n;
     OpDesc op{3, {q, dq, tau}, {n, n, n}, qdd, n,
               [](RbGpu* g, const double* const* in, double* out, size_t B, size_t ld, cudaStream_t st, int* status) {
-                  ScratchOrder so(g, RB_TABLE(g, fd), st);
-                  return RB_TABLE(g, fd)->fd(RB_PARAM(g, fd), in[0], in[1], in[2], out, B, ld, status, st);
+                  return launch(g, g->fd, st, in[0], in[1], in[2], out, B, ld, status);
               },
               [](RbGpu* g, const double* const* in, double* out, size_t B, cudaStream_t st, int* status) {
                   return g->ops->fd_aos(g->param.data(), in[0], in[1], in[2], out, B, status, st);
@@ -852,14 +864,10 @@ extern "C" int multibody_rnea_fd_batch(RbGpu* g, const double* q, const double* 
                   // one fused pass where the family has it (shared sin/cos, bias recursion and mass matrix)
                   if (g->ops->rnea_fd && !g->split_rnea_fd)
                       return g->ops->rnea_fd(g->param.data(), in[0], in[1], in[2], in[3], out, B, ld, status, st);
-                  {
-                      ScratchOrder so(g, RB_TABLE(g, rnea), st);
-                      cudaError_t e = RB_TABLE(g, rnea)->rnea(RB_PARAM(g, rnea), in[0], in[1], in[2], out, B, ld, st);
-                      if (e != cudaSuccess) return e;
-                  }
+                  cudaError_t e = launch(g, g->rnea, st, in[0], in[1], in[2], out, B, ld);
+                  if (e != cudaSuccess) return e;
                   g->launches += 1;
-                  ScratchOrder so(g, RB_TABLE(g, fd), st);
-                  return RB_TABLE(g, fd)->fd(RB_PARAM(g, fd), in[0], in[1], in[3], out + (size_t)n * ld, B, ld, status, st);
+                  return launch(g, g->fd, st, in[0], in[1], in[3], out + (size_t)n * ld, B, ld, status);
               }};
     return run_op(g, op, n_states, ld, layout, mem, stream, true);
 }
@@ -935,8 +943,7 @@ extern "C" int multibody_crba_batch(RbGpu* g, const double* q, double* H, size_t
     const int n = g->model.n;
     OpDesc op{1, {q, nullptr, nullptr}, {n, 0, 0}, H, n * n,
               [](RbGpu* g, const double* const* in, double* out, size_t B, size_t ld, cudaStream_t st, int* status) {
-                  ScratchOrder so(g, RB_TABLE(g, crba), st);
-                  return RB_TABLE(g, crba)->crba(RB_PARAM(g, crba), in[0], out, B, ld, st);
+                  return launch(g, g->crba, st, in[0], out, B, ld);
               }};
     return run_op(g, op, n_states, ld, layout, mem, stream, false);
 }
@@ -947,8 +954,7 @@ extern "C" int multibody_fwd_kin_batch(RbGpu* g, const double* q, double* xyz, s
     const int n = g->model.n;
     OpDesc op{1, {q, nullptr, nullptr}, {n, 0, 0}, xyz, 3,
               [](RbGpu* g, const double* const* in, double* out, size_t B, size_t ld, cudaStream_t st, int* status) {
-                  ScratchOrder so(g, RB_TABLE(g, fwd_kin), st);
-                  return RB_TABLE(g, fwd_kin)->fwd_kin(RB_PARAM(g, fwd_kin), in[0], out, B, ld, st);
+                  return launch(g, g->fwd_kin, st, in[0], out, B, ld);
               }};
     return run_op(g, op, n_states, ld, layout, mem, stream, false);
 }
@@ -959,8 +965,7 @@ extern "C" int multibody_jac_batch(RbGpu* g, const double* q, double* J, size_t 
     const int n = g->model.n;
     OpDesc op{1, {q, nullptr, nullptr}, {n, 0, 0}, J, 6 * n,
               [](RbGpu* g, const double* const* in, double* out, size_t B, size_t ld, cudaStream_t st, int* status) {
-                  ScratchOrder so(g, RB_TABLE(g, jac), st);
-                  return RB_TABLE(g, jac)->jac(RB_PARAM(g, jac), in[0], out, B, ld, st);
+                  return launch(g, g->jac, st, in[0], out, B, ld);
               }};
     return run_op(g, op, n_states, ld, layout, mem, stream, false);
 }
@@ -1014,12 +1019,12 @@ int rollout_impl(RbGpu* g, const double* q0, const double* dq0, const double* ta
                 cw[r * RB_MAX_N + i] = rows[r][i];
             }
     }
-    const bool shared = cost != nullptr || RB_TABLE(g, rollout)->shared_scratch;
+    const bool shared = cost != nullptr || g->rollout.shared;
     if (mem == RB_MEM_DEVICE && layout == RB_LAYOUT_SOA) {
         ScratchOrder so(g, shared, st);
         if (cost) RB_CUDA(cudaMemcpyAsync(g->cost_w.p, cw, sizeof cw, cudaMemcpyHostToDevice, st));
-        cudaError_t e = RB_TABLE(g, rollout)->rollout(RB_PARAM(g, rollout), q0, dq0, tau, dt, horizon, q_traj, dq_traj, q_final, dq_final,
-                                        n_traj, ld, g->d_status, cost ? g->cost_w.p : nullptr, cost, st);
+        cudaError_t e = g->rollout.fn(g->rollout.param, q0, dq0, tau, dt, horizon, q_traj, dq_traj, q_final, dq_final,
+                                      n_traj, ld, g->d_status, cost ? g->cost_w.p : nullptr, cost, st);
         g->launches += 1;
         if (e != cudaSuccess) return fail_cuda(e, "rollout launch");
         return RB_OK;
@@ -1068,10 +1073,10 @@ int rollout_impl(RbGpu* g, const double* q0, const double* dq0, const double* ta
     {
         ScratchOrder so(g, shared, st);
         if (cost) RB_CUDA(cudaMemcpyAsync(g->cost_w.p, cw, sizeof cw, cudaMemcpyHostToDevice, st));
-        e = RB_TABLE(g, rollout)->rollout(RB_PARAM(g, rollout), d_in, d_in + one, d_in + 2 * one, dt, horizon,
-                                    q_traj ? d_qt : nullptr, dq_traj ? d_dqt : nullptr, q_final ? d_qf : nullptr,
-                                    dq_final ? d_dqf : nullptr, B, B, d_stat, cost ? g->cost_w.p : nullptr,
-                                    cost ? d_cost : nullptr, st);
+        e = g->rollout.fn(g->rollout.param, d_in, d_in + one, d_in + 2 * one, dt, horizon,
+                          q_traj ? d_qt : nullptr, dq_traj ? d_dqt : nullptr, q_final ? d_qf : nullptr,
+                          dq_final ? d_dqf : nullptr, B, B, d_stat, cost ? g->cost_w.p : nullptr,
+                          cost ? d_cost : nullptr, st);
     }
     g->launches += 1;
     if (e != cudaSuccess) return fail_cuda(e, "rollout launch");

@@ -89,6 +89,8 @@ const char* const kLongExprs[RB_JIT_KERNELS] = {
     "rb_long_rnea_kernel<CtModel<TabJit>>", nullptr, nullptr, nullptr,
     "rb_long_crba_kernel<CtModel<TabJit>>", "rb_fwd_kin_kernel<CtModel<TabJit>>",
     "rb_jac_kernel<CtModel<TabJit>>",       nullptr, nullptr, nullptr, nullptr};
+// the AoS variants stage 3 arrays of RB_BLOCK states through dynamic shared memory
+size_t aos_smem(int n) { return (size_t)3 * RB_BLOCK * n * sizeof(double); }
 const char* const kOptions[] = {"--gpu-architecture=sm_100a", "-std=c++17", "-lineinfo", "-default-device", "-DRB_DEVICE_ONLY=1"};
 
 uint64_t fnv1a(uint64_t h, const void* data, size_t n) {
@@ -258,11 +260,9 @@ int rb_jit_load(const RbJitImage& img, int n, RbJitParam& out, std::string& err)
         if (e != cudaSuccess) { err = std::string("cudaLibraryGetKernel(") + img.lowered[k] + "): " + cudaGetErrorString(e); cudaLibraryUnload(lib); out.lib = nullptr; return RB_ERR_CUDA; }
         out.k[k] = kern;
     }
-    // the AoS variants stage 3 arrays of RB_BLOCK states through dynamic shared memory
-    const int aos_smem = 3 * RB_BLOCK * n * (int)sizeof(double);
-    if (aos_smem > 48 * 1024)
+    if (aos_smem(n) > 48 * 1024)
         for (int k : {RB_JK_RNEA_AOS, RB_JK_FD_AOS})
-            if (out.k[k]) cudaFuncSetAttribute((const void*)out.k[k], cudaFuncAttributeMaxDynamicSharedMemorySize, aos_smem);
+            if (out.k[k]) cudaFuncSetAttribute((const void*)out.k[k], cudaFuncAttributeMaxDynamicSharedMemorySize, (int)aos_smem(n));
     return RB_OK;
 }
 
@@ -273,88 +273,72 @@ void rb_jit_unload(RbJitParam& p) {
 
 // ---- launchers: same grids / blocks / shared memory as RbLaunch<M> in rb_kernels.cuh ---------------------------------
 namespace {
-unsigned jgrid(size_t B, int block) { return (unsigned)((B + block - 1) / block); }
-
-cudaError_t j_rnea(const void* param, const double* q, const double* dq, const double* ddq, double* tau, size_t B, size_t ld, cudaStream_t st) {
-    const RbJitParam* P = (const RbJitParam*)param;
+// Launches kernel `k` of the chain's image over B states in blocks of `block` threads.  The kernel takes the (empty)
+// model parameter, then `a` in order: each must have the exact type of its kernel parameter (size_t B and ld, not int).
+template <class... A>
+cudaError_t jlaunch(const void* param, int k, int block, size_t smem, size_t B, cudaStream_t st, A... a) {
     if (B == 0) return cudaSuccess;
     RbEmptyParam ep{0};
-    void* args[] = {&ep, &q, &dq, &ddq, &tau, &B, &ld};
-    return cudaLaunchKernel((const void*)P->k[RB_JK_RNEA], dim3(jgrid(B, RB_BLOCK)), dim3(RB_BLOCK), args, 0, st);
+    void* args[] = {&ep, &a...};
+    return cudaLaunchKernel((const void*)((const RbJitParam*)param)->k[k], dim3((unsigned)((B + block - 1) / block)), dim3(block),
+                            args, smem, st);
 }
-cudaError_t j_rnea_aos(const void* param, const double* q, const double* dq, const double* ddq, double* tau, size_t B, cudaStream_t st) {
-    const RbJitParam* P = (const RbJitParam*)param;
-    if (B == 0) return cudaSuccess;
-    RbEmptyParam ep{0}; size_t ld = 0;
-    void* args[] = {&ep, &q, &dq, &ddq, &tau, &B, &ld};
-    return cudaLaunchKernel((const void*)P->k[RB_JK_RNEA_AOS], dim3(jgrid(B, RB_BLOCK)), dim3(RB_BLOCK), args,
-                            (size_t)3 * RB_BLOCK * P->n * sizeof(double), st);
+cudaError_t j_rnea(const void* p, const double* q, const double* dq, const double* ddq, double* tau, size_t B, size_t ld, cudaStream_t st) {
+    return jlaunch(p, RB_JK_RNEA, RB_BLOCK, 0, B, st, q, dq, ddq, tau, B, ld);
 }
-cudaError_t j_fd(const void* param, const double* q, const double* dq, const double* tau, double* qdd, size_t B, size_t ld, int* status, cudaStream_t st) {
-    const RbJitParam* P = (const RbJitParam*)param;
-    if (B == 0) return cudaSuccess;
-    RbEmptyParam ep{0};
-    void* args[] = {&ep, &q, &dq, &tau, &qdd, &B, &ld, &status};
-    return cudaLaunchKernel((const void*)P->k[RB_JK_FD], dim3(jgrid(B, RB_BLOCK)), dim3(RB_BLOCK), args, 0, st);
+cudaError_t j_rnea_aos(const void* p, const double* q, const double* dq, const double* ddq, double* tau, size_t B, cudaStream_t st) {
+    return jlaunch(p, RB_JK_RNEA_AOS, RB_BLOCK, aos_smem(((const RbJitParam*)p)->n), B, st, q, dq, ddq, tau, B, (size_t)0);
 }
-cudaError_t j_fd_aos(const void* param, const double* q, const double* dq, const double* tau, double* qdd, size_t B, int* status, cudaStream_t st) {
-    const RbJitParam* P = (const RbJitParam*)param;
-    if (B == 0) return cudaSuccess;
-    RbEmptyParam ep{0}; size_t ld = 0;
-    void* args[] = {&ep, &q, &dq, &tau, &qdd, &B, &ld, &status};
-    return cudaLaunchKernel((const void*)P->k[RB_JK_FD_AOS], dim3(jgrid(B, RB_BLOCK)), dim3(RB_BLOCK), args,
-                            (size_t)3 * RB_BLOCK * P->n * sizeof(double), st);
+cudaError_t j_fd(const void* p, const double* q, const double* dq, const double* tau, double* qdd, size_t B, size_t ld, int* status, cudaStream_t st) {
+    return jlaunch(p, RB_JK_FD, RB_BLOCK, 0, B, st, q, dq, tau, qdd, B, ld, status);
 }
-cudaError_t j_q_only(const RbJitParam* P, int which, const double* q, double* out, size_t B, size_t ld, cudaStream_t st) {
-    if (B == 0) return cudaSuccess;
-    RbEmptyParam ep{0};
-    void* args[] = {&ep, &q, &out, &B, &ld};
-    return cudaLaunchKernel((const void*)P->k[which], dim3(jgrid(B, RB_BLOCK)), dim3(RB_BLOCK), args, 0, st);
+cudaError_t j_fd_aos(const void* p, const double* q, const double* dq, const double* tau, double* qdd, size_t B, int* status, cudaStream_t st) {
+    return jlaunch(p, RB_JK_FD_AOS, RB_BLOCK, aos_smem(((const RbJitParam*)p)->n), B, st, q, dq, tau, qdd, B, (size_t)0, status);
 }
-cudaError_t j_crba(const void* param, const double* q, double* H, size_t B, size_t ld, cudaStream_t st) { return j_q_only((const RbJitParam*)param, RB_JK_CRBA, q, H, B, ld, st); }
-cudaError_t j_fk(const void* param, const double* q, double* x, size_t B, size_t ld, cudaStream_t st) { return j_q_only((const RbJitParam*)param, RB_JK_FK, q, x, B, ld, st); }
-cudaError_t j_jac(const void* param, const double* q, double* J, size_t B, size_t ld, cudaStream_t st) { return j_q_only((const RbJitParam*)param, RB_JK_JAC, q, J, B, ld, st); }
-cudaError_t j_rollout(const void* param, const double* q0, const double* dq0, const double* tau, double dt, int horizon,
+cudaError_t j_crba(const void* p, const double* q, double* H, size_t B, size_t ld, cudaStream_t st) {
+    return jlaunch(p, RB_JK_CRBA, RB_BLOCK, 0, B, st, q, H, B, ld);
+}
+cudaError_t j_fk(const void* p, const double* q, double* x, size_t B, size_t ld, cudaStream_t st) {
+    return jlaunch(p, RB_JK_FK, RB_BLOCK, 0, B, st, q, x, B, ld);
+}
+cudaError_t j_jac(const void* p, const double* q, double* J, size_t B, size_t ld, cudaStream_t st) {
+    return jlaunch(p, RB_JK_JAC, RB_BLOCK, 0, B, st, q, J, B, ld);
+}
+cudaError_t j_rollout(const void* p, const double* q0, const double* dq0, const double* tau, double dt, int horizon,
                       double* q_traj, double* dq_traj, double* q_fin, double* dq_fin, size_t B, size_t ld, int* status,
                       const double* cost_w, double* cost, cudaStream_t st) {
-    const RbJitParam* P = (const RbJitParam*)param;
-    if (B == 0) return cudaSuccess;
-    RbEmptyParam ep{0};
-    void* args[] = {&ep, &q0, &dq0, &tau, &dt, &horizon, &q_traj, &dq_traj, &q_fin, &dq_fin, &B, &ld, &status, &cost_w, &cost};
-    return cudaLaunchKernel((const void*)P->k[RB_JK_ROLLOUT], dim3(jgrid(B, RB_RO_BLOCK)), dim3(RB_RO_BLOCK), args, 0, st);
+    return jlaunch(p, RB_JK_ROLLOUT, RB_RO_BLOCK, 0, B, st, q0, dq0, tau, dt, horizon, q_traj, dq_traj, q_fin, dq_fin, B, ld,
+                   status, cost_w, cost);
 }
-cudaError_t j_rnea_f32(const void* param, const float* q, const float* dq, const float* ddq, float* tau, size_t B, size_t ld, cudaStream_t st) {
-    const RbJitParam* P = (const RbJitParam*)param;
-    if (B == 0) return cudaSuccess;
-    RbEmptyParam ep{0};
-    void* args[] = {&ep, &q, &dq, &ddq, &tau, &B, &ld};
-    return cudaLaunchKernel((const void*)P->k[RB_JK_RNEA_F32], dim3(jgrid(B, RB_BLOCK)), dim3(RB_BLOCK), args, 0, st);
+cudaError_t j_rnea_f32(const void* p, const float* q, const float* dq, const float* ddq, float* tau, size_t B, size_t ld, cudaStream_t st) {
+    return jlaunch(p, RB_JK_RNEA_F32, RB_BLOCK, 0, B, st, q, dq, ddq, tau, B, ld);
 }
-cudaError_t j_fd_f32(const void* param, const float* q, const float* dq, const float* tau, float* qdd, size_t B, size_t ld, int* status, cudaStream_t st) {
-    const RbJitParam* P = (const RbJitParam*)param;
-    if (B == 0) return cudaSuccess;
-    RbEmptyParam ep{0};
-    void* args[] = {&ep, &q, &dq, &tau, &qdd, &B, &ld, &status};
-    return cudaLaunchKernel((const void*)P->k[RB_JK_FD_F32], dim3(jgrid(B, RB_BLOCK)), dim3(RB_BLOCK), args, 0, st);
+cudaError_t j_fd_f32(const void* p, const float* q, const float* dq, const float* tau, float* qdd, size_t B, size_t ld, int* status, cudaStream_t st) {
+    return jlaunch(p, RB_JK_FD_F32, RB_BLOCK, 0, B, st, q, dq, tau, qdd, B, ld, status);
 }
-cudaError_t j_rnea_fd(const void* param, const double* q, const double* dq, const double* ddq, const double* tau_in, double* out,
+cudaError_t j_rnea_fd(const void* p, const double* q, const double* dq, const double* ddq, const double* tau_in, double* out,
                       size_t B, size_t ld, int* status, cudaStream_t st) {
-    const RbJitParam* P = (const RbJitParam*)param;
-    if (B == 0) return cudaSuccess;
-    RbEmptyParam ep{0};
-    void* args[] = {&ep, &q, &dq, &ddq, &tau_in, &out, &B, &ld, &status};
-    return cudaLaunchKernel((const void*)P->k[RB_JK_RNEA_FD], dim3(jgrid(B, RB_BLOCK)), dim3(RB_BLOCK), args, 0, st);
+    return jlaunch(p, RB_JK_RNEA_FD, RB_BLOCK, 0, B, st, q, dq, ddq, tau_in, out, B, ld, status);
 }
 }  // namespace
 
 const RbOps* rb_ops_jit_long() {
-    static const RbOps ops = {"jit-long", 0, sizeof(RbJitParam), false, &j_rnea, nullptr, nullptr, nullptr,
-                              &j_crba, &j_fk, &j_jac, nullptr, nullptr, nullptr};
+    static const RbOps ops = [] {
+        RbOps o{};
+        o.name = "jit-long"; o.param_bytes = sizeof(RbJitParam);
+        o.rnea = &j_rnea; o.crba = &j_crba; o.fwd_kin = &j_fk; o.jac = &j_jac;
+        return o;
+    }();
     return &ops;
 }
 
 const RbOps* rb_ops_jit() {
-    static const RbOps ops = {"jit-specialised", 0, sizeof(RbJitParam), false, &j_rnea, &j_fd, &j_rnea_aos, &j_fd_aos,
-                              &j_crba, &j_fk, &j_jac, &j_rollout, &j_rnea_f32, &j_fd_f32, &j_rnea_fd};
+    static const RbOps ops = [] {
+        RbOps o{};
+        o.name = "jit-specialised"; o.param_bytes = sizeof(RbJitParam);
+        o.rnea = &j_rnea; o.fd = &j_fd; o.rnea_aos = &j_rnea_aos; o.fd_aos = &j_fd_aos; o.crba = &j_crba; o.fwd_kin = &j_fk;
+        o.jac = &j_jac; o.rollout = &j_rollout; o.rnea_f32 = &j_rnea_f32; o.fd_f32 = &j_fd_f32; o.rnea_fd = &j_rnea_fd;
+        return o;
+    }();
     return &ops;
 }

@@ -57,7 +57,6 @@ typedef unsigned long uintptr_t;
 #ifndef RB_DEVICE_ONLY
 struct RbOps {
     const char* name;
-    int n;                 // joints this table serves (0 = any, run-time n)
     size_t param_bytes;    // bytes of model parameter the launchers expect behind `param`
     bool shared_scratch;   // kernels work in engine-owned scratch: launches must be ordered across streams
     cudaError_t (*rnea)(const void* param, const double* q, const double* dq, const double* ddq, double* tau,
@@ -82,8 +81,7 @@ struct RbOps {
     cudaError_t (*fd_f32)(const void* param, const float* q, const float* dq, const float* tau, float* qdd,
                           size_t B, size_t ld, int* status, cudaStream_t st);
     // optional: tau = rnea(q, dq, ddq) and qdd = fd(q, dq, tau_in) in ONE pass over SoA batches, out = [2n][ld]
-    // (null = the API issues the rnea and fd launches back to back).  Keep this entry last: the positional
-    // initialisers of the partial tables leave it null.
+    // (null = the API issues the rnea and fd launches back to back)
     cudaError_t (*rnea_fd)(const void* param, const double* q, const double* dq, const double* ddq, const double* tau_in,
                            double* out, size_t B, size_t ld, int* status, cudaStream_t st);
 };
@@ -495,10 +493,9 @@ struct RbLaunch {
     template <class M32 = void>
     static RbOps ops(const char* name) {
         RbOps o{};
-        o.name = name; o.n = M::N; o.param_bytes = sizeof(P); o.shared_scratch = false;
+        o.name = name; o.param_bytes = sizeof(P);
         o.rnea = &rnea; o.fd = &fd; o.rnea_aos = &rnea_aos; o.fd_aos = &fd_aos;
-        o.crba = &crba; o.fwd_kin = &fwd_kin; o.jac = &jac; o.rollout = &rollout;
-        o.rnea_f32 = nullptr; o.fd_f32 = nullptr; o.rnea_fd = &rnea_fd;
+        o.crba = &crba; o.fwd_kin = &fwd_kin; o.jac = &jac; o.rollout = &rollout; o.rnea_fd = &rnea_fd;
         if constexpr (!std::is_void<M32>::value) { o.rnea_f32 = &rnea_f32<M32>; o.fd_f32 = &fd_f32<M32>; }
         return o;
     }

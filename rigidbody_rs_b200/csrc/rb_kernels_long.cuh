@@ -73,9 +73,8 @@ struct RbLaunchLong {
     // fd / fwd_kin / jac / rollout are served by the run-time-n family (null here = use the fallback table).
     static RbOps ops(const char* name) {
         RbOps o{};
-        o.name = name; o.n = M::N; o.param_bytes = sizeof(MP); o.shared_scratch = false;
-        o.rnea = &rnea; o.fd = nullptr; o.rnea_aos = nullptr; o.fd_aos = nullptr; o.crba = &crba; o.fwd_kin = nullptr; o.jac = nullptr; o.rollout = nullptr;
-        o.rnea_f32 = nullptr; o.fd_f32 = nullptr;
+        o.name = name; o.param_bytes = sizeof(MP);
+        o.rnea = &rnea; o.crba = &crba;
         return o;
     }
 };

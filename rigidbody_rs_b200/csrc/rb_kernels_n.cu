@@ -485,7 +485,12 @@ cudaError_t n_rollout(const void* param, const double* q0, const double* dq0, co
 }  // namespace
 
 const RbOps* rb_ops_generic_n() {
-    static const RbOps ops = {"generic-n", 0, sizeof(RbNParam), true, &n_rnea, &n_fd, nullptr, nullptr, &n_crba, &n_fk, &n_jac, &n_rollout, nullptr, nullptr};
+    static const RbOps ops = [] {
+        RbOps o{};
+        o.name = "generic-n"; o.param_bytes = sizeof(RbNParam); o.shared_scratch = true;
+        o.rnea = &n_rnea; o.fd = &n_fd; o.crba = &n_crba; o.fwd_kin = &n_fk; o.jac = &n_jac; o.rollout = &n_rollout;
+        return o;
+    }();
     return &ops;
 }
 
