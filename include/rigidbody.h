@@ -276,6 +276,27 @@ int multibody_rollout_cost(RbGpu* g, const double* q0, const double* dq0, const 
                            const RbQuadCost* weights, double* cost, double* q_final, double* dq_final,
                            size_t n_traj, size_t ld, RbLayout layout, RbMem mem, void* stream);
 
+/* Gradients of rollouts, for gradient-based MPC and trajectory optimisation: one adjoint pass backwards through the
+ * rollout (one thread per trajectory, O(n) per step), serial chains of at most 12 joints (RB_ERR_UNSUPPORTED otherwise,
+ * and for kinematic trees), fp64.  They are the gradients of the exact-arithmetic rollout map evaluated at the computed
+ * states, not of its rounded floating-point evaluation.  Layouts, ld, host/device memory, horizon == 0, multi-device
+ * handles and status reporting as multibody_rollout; a trajectory that meets a non-SPD mass matrix gets NaN gradients.
+ * Reverse-mode (vector-Jacobian) product of multibody_rollout.  q_traj / dq_traj: what multibody_rollout returned for
+ * these q0, dq0, tau, dt (the states the pass linearises about; not re-checked).  g_*: upstream gradients shaped like the
+ * matching rollout outputs, each may be NULL (= 0).  grad_tau shaped like tau, grad_q0 / grad_dq0 like q0; each may be NULL.
+ * With horizon == 0 tau and the trajectory are not read, grad_q0 = g_q_final and grad_dq0 = g_dq_final. */
+int multibody_rollout_vjp(RbGpu* g, const double* q0, const double* dq0, const double* tau, double dt, int horizon,
+                          const double* q_traj, const double* dq_traj,
+                          const double* g_q_traj, const double* g_dq_traj, const double* g_q_final, const double* g_dq_final,
+                          double* grad_tau, double* grad_q0, double* grad_dq0,
+                          size_t n_traj, size_t ld, RbLayout layout, RbMem mem, void* stream);
+/* multibody_rollout_cost plus its gradient: cost bit-identical to multibody_rollout_cost on the same engine, and
+ * d cost / d tau, d cost / d q0, d cost / d dq0 (each may be NULL).  Device calls take a workspace of at most 1 GiB per
+ * chunk of trajectories in stream order on `stream` (cudaMallocAsync). */
+int multibody_rollout_cost_grad(RbGpu* g, const double* q0, const double* dq0, const double* tau, double dt, int horizon,
+                                const RbQuadCost* weights, double* cost, double* grad_tau, double* grad_q0, double* grad_dq0,
+                                size_t n_traj, size_t ld, RbLayout layout, RbMem mem, void* stream);
+
 /* ---- device-side helpers (bench / tests) --------------------------------------------------- */
 /* Fill a device SOA array [n][ld] with the counter-based sampler of SURVEY.md 8d:
  * value(joint i, state s) = fma(hi[i]-lo[i], u, lo[i]),  u = top 53 bits of

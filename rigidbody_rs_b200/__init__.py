@@ -327,29 +327,8 @@ class Multibody:
         """Semi-implicit Euler rollout through forward dynamics (SURVEY.md a14).
         soa: q0, dq0 [n, B], tau [H, n, B];  aos: q0, dq0 [B, n], tau [H, B, n].
         Returns (q_traj, dq_traj) shaped like tau, and/or (q_final, dq_final) shaped like q0."""
-        a_q, a_dq, a_tau = _Arg(q0, "q0"), _Arg(dq0, "dq0"), _Arg(tau, "tau")
+        a_q, a_dq, a_tau, B, H, lay, new = self._rollout_args(q0, dq0, tau, layout, "rollout")
         cuda = a_q.cuda
-        if a_dq.cuda != cuda or a_tau.cuda != cuda:
-            raise ValueError("all arrays of one call must live in the same place")
-        n = self.n
-        if layout == "soa":
-            B = a_q.shape[1]; H = a_tau.shape[0]
-            ok = a_q.shape == (n, B) and a_dq.shape == (n, B) and a_tau.shape == (H, n, B)
-            lay = RB_LAYOUT_SOA
-        elif layout == "aos":
-            B = a_q.shape[0]; H = a_tau.shape[0]
-            ok = a_q.shape == (B, n) and a_dq.shape == (B, n) and a_tau.shape == (H, B, n)
-            lay = RB_LAYOUT_AOS
-        else:
-            raise ValueError("layout must be 'soa' or 'aos'")
-        if not ok:
-            raise ValueError("rollout: inconsistent shapes")
-
-        def new(shape):
-            if cuda:
-                import torch
-                return _Arg(torch.empty(shape, dtype=torch.float64, device=a_q.device), "out")
-            return _Arg(np.empty(shape, dtype=np.float64), "out")
 
         qt = new(a_tau.shape) if trajectory else None
         dqt = new(a_tau.shape) if trajectory else None
@@ -370,34 +349,9 @@ class Multibody:
                      layout="soa", final=False):
         """Fused rollout + quadratic running/terminal cost (one scalar per trajectory; include/rigidbody.h
         multibody_rollout_cost).  Shapes as `rollout`; weights are length-n vectors (None = zeros)."""
-        a_q, a_dq, a_tau = _Arg(q0, "q0"), _Arg(dq0, "dq0"), _Arg(tau, "tau")
+        a_q, a_dq, a_tau, B, H, lay, new = self._rollout_args(q0, dq0, tau, layout, "rollout_cost")
         cuda = a_q.cuda
-        if a_dq.cuda != cuda or a_tau.cuda != cuda:
-            raise ValueError("all arrays of one call must live in the same place")
-        n = self.n
-        if layout == "soa":
-            B = a_q.shape[1]; H = a_tau.shape[0]
-            ok = a_q.shape == (n, B) and a_dq.shape == (n, B) and a_tau.shape == (H, n, B); lay = RB_LAYOUT_SOA
-        elif layout == "aos":
-            B = a_q.shape[0]; H = a_tau.shape[0]
-            ok = a_q.shape == (B, n) and a_dq.shape == (B, n) and a_tau.shape == (H, B, n); lay = RB_LAYOUT_AOS
-        else:
-            raise ValueError("layout must be 'soa' or 'aos'")
-        if not ok:
-            raise ValueError("rollout_cost: inconsistent shapes")
-        qc = _lib.RbQuadCost()
-        keep = []
-        for name, v in (("q_ref", q_ref), ("w_q", w_q), ("w_dq", w_dq), ("w_tau", w_tau), ("w_q_final", w_q_final), ("w_dq_final", w_dq_final)):
-            if v is not None:
-                a = np.ascontiguousarray(np.broadcast_to(v, (n,)), dtype=np.float64); keep.append(a)
-                setattr(qc, name, a.ctypes.data_as(C.POINTER(C.c_double)))
-
-        def new(shape):
-            if cuda:
-                import torch
-                return _Arg(torch.empty(shape, dtype=torch.float64, device=a_q.device), "out")
-            return _Arg(np.empty(shape, dtype=np.float64), "out")
-
+        qc, keep = self._quad_cost(q_ref, w_q, w_dq, w_tau, w_q_final, w_dq_final)
         cost = new((B,))
         qf = new(a_q.shape) if final else None
         dqf = new(a_q.shape) if final else None
@@ -406,6 +360,88 @@ class Multibody:
                                          ptr(qf), ptr(dqf), B, 0, lay, RB_MEM_DEVICE if cuda else RB_MEM_HOST,
                                          self._stream(cuda, a_q)))
         return (cost.arr, qf.arr, dqf.arr) if final else cost.arr
+
+    def rollout_cost_grad(self, q0, dq0, tau, dt, q_ref=None, w_q=None, w_dq=None, w_tau=None, w_q_final=None, w_dq_final=None,
+                          layout="soa"):
+        """`rollout_cost` and its gradient (include/rigidbody.h multibody_rollout_cost_grad): returns (cost, grad_tau,
+        grad_q0, grad_dq0), the cost bit for bit `rollout_cost`'s, grad_tau shaped like tau, grad_q0 / grad_dq0 like q0.
+        Serial chains of at most 12 joints."""
+        a_q, a_dq, a_tau, B, H, lay, new = self._rollout_args(q0, dq0, tau, layout, "rollout_cost_grad")
+        cuda = a_q.cuda
+        qc, keep = self._quad_cost(q_ref, w_q, w_dq, w_tau, w_q_final, w_dq_final)
+        cost, gt, gq, gdq = new((B,)), new(a_tau.shape), new(a_q.shape), new(a_q.shape)
+        check(lib.multibody_rollout_cost_grad(self._h, C.c_void_p(a_q.ptr), C.c_void_p(a_dq.ptr), C.c_void_p(a_tau.ptr), float(dt), int(H),
+                                              C.byref(qc), C.c_void_p(cost.ptr), C.c_void_p(gt.ptr), C.c_void_p(gq.ptr), C.c_void_p(gdq.ptr),
+                                              B, 0, lay, RB_MEM_DEVICE if cuda else RB_MEM_HOST, self._stream(cuda, a_q)))
+        return cost.arr, gt.arr, gq.arr, gdq.arr
+
+    def rollout_vjp(self, q0, dq0, tau, dt, q_traj, dq_traj, g_q_traj=None, g_dq_traj=None, g_q_final=None, g_dq_final=None,
+                    layout="soa"):
+        """Vector-Jacobian product of `rollout` (include/rigidbody.h multibody_rollout_vjp): given the trajectory `rollout`
+        returned for these inputs and upstream gradients of (q_traj, dq_traj, q_final, dq_final) (None = zero), returns
+        (grad_tau, grad_q0, grad_dq0).  Serial chains of at most 12 joints."""
+        a_q, a_dq, a_tau, B, H, lay, new = self._rollout_args(q0, dq0, tau, layout, "rollout_vjp")
+        cuda = a_q.cuda
+
+        def arg(x, name, shape):
+            if x is None:
+                return None
+            a = _Arg(x, name)
+            if a.shape != shape or a.cuda != cuda:
+                raise ValueError(f"rollout_vjp: {name} must have shape {shape} and live with q0")
+            return a
+        ins = [arg(q_traj, "q_traj", a_tau.shape), arg(dq_traj, "dq_traj", a_tau.shape), arg(g_q_traj, "g_q_traj", a_tau.shape),
+               arg(g_dq_traj, "g_dq_traj", a_tau.shape), arg(g_q_final, "g_q_final", a_q.shape), arg(g_dq_final, "g_dq_final", a_q.shape)]
+        gt, gq, gdq = new(a_tau.shape), new(a_q.shape), new(a_q.shape)
+        ptr = lambda a: C.c_void_p(a.ptr) if a is not None else None
+        check(lib.multibody_rollout_vjp(self._h, ptr(a_q), ptr(a_dq), ptr(a_tau), float(dt), int(H), *[ptr(a) for a in ins],
+                                        ptr(gt), ptr(gq), ptr(gdq), B, 0, lay, RB_MEM_DEVICE if cuda else RB_MEM_HOST,
+                                        self._stream(cuda, a_q)))
+        return gt.arr, gq.arr, gdq.arr
+
+    def rollout_autograd(self, q0, dq0, tau, dt):
+        """`rollout` as a differentiable torch function: q0, dq0 [n, B] and tau [H, n, B] are CUDA float64 tensors (layout
+        'soa'); returns (q_traj, dq_traj) [H, n, B], whose backward pass is `rollout_vjp` on the current stream."""
+        return _rollout_function().apply(self, q0, dq0, tau, float(dt))
+
+    # ---- argument plumbing of the rollout entries
+    def _rollout_args(self, q0, dq0, tau, layout, what):
+        """Checks (q0, dq0, tau) against `layout`; returns their _Args, B, H, the layout code and an allocator of outputs
+        that live with them."""
+        a_q, a_dq, a_tau = _Arg(q0, "q0"), _Arg(dq0, "dq0"), _Arg(tau, "tau")
+        cuda = a_q.cuda
+        if a_dq.cuda != cuda or a_tau.cuda != cuda:
+            raise ValueError("all arrays of one call must live in the same place")
+        n = self.n
+        if layout == "soa":
+            B = a_q.shape[1]; H = a_tau.shape[0]
+            ok = a_q.shape == (n, B) and a_dq.shape == (n, B) and a_tau.shape == (H, n, B)
+            lay = RB_LAYOUT_SOA
+        elif layout == "aos":
+            B = a_q.shape[0]; H = a_tau.shape[0]
+            ok = a_q.shape == (B, n) and a_dq.shape == (B, n) and a_tau.shape == (H, B, n)
+            lay = RB_LAYOUT_AOS
+        else:
+            raise ValueError("layout must be 'soa' or 'aos'")
+        if not ok:
+            raise ValueError(f"{what}: inconsistent shapes")
+
+        def new(shape):
+            if cuda:
+                import torch
+                return _Arg(torch.empty(shape, dtype=torch.float64, device=a_q.device), "out")
+            return _Arg(np.empty(shape, dtype=np.float64), "out")
+        return a_q, a_dq, a_tau, B, H, lay, new
+
+    def _quad_cost(self, q_ref=None, w_q=None, w_dq=None, w_tau=None, w_q_final=None, w_dq_final=None):
+        """An RbQuadCost over length-n weight vectors (None = zeros) and the arrays it points into (keep them alive)."""
+        qc = _lib.RbQuadCost()
+        keep = []
+        for name, v in (("q_ref", q_ref), ("w_q", w_q), ("w_dq", w_dq), ("w_tau", w_tau), ("w_q_final", w_q_final), ("w_dq_final", w_dq_final)):
+            if v is not None:
+                a = np.ascontiguousarray(np.broadcast_to(v, (self.n,)), dtype=np.float64); keep.append(a)
+                setattr(qc, name, a.ctypes.data_as(C.POINTER(C.c_double)))
+        return qc, keep
 
     # ---- device-side sampler (bench / tests)
     def fill(self, out, seed, field, lo, hi, first_index=0):
@@ -419,3 +455,35 @@ class Multibody:
         check(lib.multibody_gpu_fill(self._h, C.c_void_p(o.ptr), int(seed), int(field), dp(lo), dp(hi),
                                      int(first_index), o.shape[1], o.shape[1], self._stream(True, o)))
         return out
+
+
+_ROLLOUT_FN = None
+
+
+def _rollout_function():
+    """The torch.autograd.Function behind Multibody.rollout_autograd (built on first use: torch stays a lazy import)."""
+    global _ROLLOUT_FN
+    if _ROLLOUT_FN is None:
+        import torch
+
+        class RolloutFunction(torch.autograd.Function):
+            @staticmethod
+            def forward(ctx, mb, q0, dq0, tau, dt):
+                for name, t in (("q0", q0), ("dq0", dq0), ("tau", tau)):
+                    if not (_is_torch(t) and t.is_cuda and t.dtype == torch.float64):
+                        raise TypeError(f"rollout_autograd: {name} must be a CUDA float64 tensor")
+                q0, dq0, tau = q0.contiguous(), dq0.contiguous(), tau.contiguous()
+                qt, dqt = mb.rollout(q0, dq0, tau, dt)
+                ctx.mb, ctx.dt = mb, dt
+                ctx.save_for_backward(q0, dq0, tau, qt, dqt)
+                return qt, dqt
+
+            @staticmethod
+            def backward(ctx, g_qt, g_dqt):
+                q0, dq0, tau, qt, dqt = ctx.saved_tensors
+                c = lambda g: None if g is None else g.contiguous()
+                gt, gq, gdq = ctx.mb.rollout_vjp(q0, dq0, tau, ctx.dt, qt, dqt, c(g_qt), c(g_dqt))
+                return None, gq, gdq, gt, None
+
+        _ROLLOUT_FN = RolloutFunction
+    return _ROLLOUT_FN

@@ -72,6 +72,8 @@ PROTOTYPES = {
     "multibody_jac_batch": (_i, [_vp, _vp, _vp, _sz, _sz, _i, _i, _vp]),
     "multibody_rollout": (_i, [_vp, _vp, _vp, _vp, C.c_double, _i, _vp, _vp, _vp, _vp, _sz, _sz, _i, _i, _vp]),
     "multibody_rollout_cost": (_i, [_vp, _vp, _vp, _vp, C.c_double, _i, C.POINTER(RbQuadCost), _vp, _vp, _vp, _sz, _sz, _i, _i, _vp]),
+    "multibody_rollout_vjp": (_i, [_vp, _vp, _vp, _vp, C.c_double, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _sz, _i, _i, _vp]),
+    "multibody_rollout_cost_grad": (_i, [_vp, _vp, _vp, _vp, C.c_double, _i, C.POINTER(RbQuadCost), _vp, _vp, _vp, _vp, _sz, _sz, _i, _i, _vp]),
     "multibody_gpu_fill": (_i, [_vp, _vp, _u64, C.c_uint32, _dp, _dp, _sz, _sz, _sz, _vp]),
     "multibody_gpu_sync": (_i, [_vp]),
     "multibody_gpu_status": (_i, [_vp]),

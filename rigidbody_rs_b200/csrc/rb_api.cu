@@ -971,8 +971,131 @@ extern "C" int multibody_jac_batch(RbGpu* g, const double* q, double* J, size_t 
 }
 
 namespace {
-// `aos_stride`: elements between consecutive steps of the AoS arrays tau / q_traj / dq_traj (0 = n_traj * n, a dense
-// [H][n_traj][n] array; a multi-device engine passes the stride of the whole batch when it hands out slices).
+// Host and/or AoS arguments of the rollout entries, moved through the engine's staging buffers as SoA with ld = n_traj.
+// An input or output is `arrays` consecutive state arrays (n doubles per trajectory each: q0 is one, tau `horizon`),
+// or, `plain`, one vector of n_traj doubles (the cost).  A NULL pointer is neither copied nor handed on.
+struct StagedIn { const double* p; size_t arrays; };
+struct StagedOut { double* p; size_t arrays; bool plain; };
+using StagedRun = std::function<int(const double* const* d_in, double* const* d_out, int* d_stat)>;
+
+// Brings `ins` in, calls run() on the staged copies (SoA, ld = n_traj; NULL where the caller passed NULL), brings `outs`
+// back, and drains the stream.  `aos_stride`: elements between consecutive steps of the caller's AoS arrays (0 = n_traj * n,
+// a dense [H][n_traj][n] array; a multi-device engine passes the stride of the whole batch when it hands out slices).
+// Takes g->mu; a host call owns status word 1 and reports it.
+int run_staged(RbGpu* g, const std::vector<StagedIn>& ins, const std::vector<StagedOut>& outs, size_t n_traj, size_t ld,
+               RbLayout layout, RbMem mem, size_t aos_stride, cudaStream_t st, const StagedRun& run) {
+    std::lock_guard<std::mutex> lk(g->mu);
+    int* const d_stat = g->d_status + (mem == RB_MEM_HOST ? 1 : 0);
+    if (mem == RB_MEM_HOST) RB_CUDA(cudaMemsetAsync(d_stat, 0, sizeof(int), st));
+    auto staged = [&]() -> int {
+    const int n = g->model.n;
+    const size_t B = n_traj, one = (size_t)n * B;
+    const bool aos = layout == RB_LAYOUT_AOS, host = mem == RB_MEM_HOST;
+    const size_t src_step = aos ? (aos_stride ? aos_stride : one) : (size_t)n * ld;    // caller's distance between steps
+    size_t in_arrays = 0, out_arrays = 0, out_plain = 0;
+    for (const StagedIn& a : ins) in_arrays += a.arrays;
+    for (const StagedOut& a : outs) (a.plain ? out_plain : out_arrays) += a.arrays;
+    // in[0]: the inputs in order      out[0]: the outputs in order      tmp[0]: AoS landing zone
+    int rc = g->in[0].ensure(in_arrays * one * sizeof(double)); if (rc) return rc;
+    rc = g->out[0].ensure((out_arrays * one + out_plain * B) * sizeof(double)); if (rc) return rc;
+    if (aos) { rc = g->tmp[0].ensure(std::max(in_arrays, out_arrays) * one * sizeof(double)); if (rc) return rc; }
+    double* d_tmp = g->tmp[0].p;
+    auto bring_in = [&](const double* src, double* dst, size_t arrays) -> int {
+        // `arrays` consecutive state arrays
+        for (size_t a = 0; a < arrays; ++a) {
+            const double* s_a = src + a * src_step;
+            double* d_a = dst + a * one;
+            if (!aos) {
+                RB_CUDA(cudaMemcpy2DAsync(d_a, B * sizeof(double), s_a, ld * sizeof(double), B * sizeof(double), (size_t)n,
+                                          host ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice, st));
+            } else {
+                const double* a_src = s_a;
+                if (host) {
+                    double* land = d_tmp + a * one;
+                    RB_CUDA(cudaMemcpyAsync(land, s_a, one * sizeof(double), cudaMemcpyHostToDevice, st));
+                    a_src = land;
+                }
+                cudaError_t e = rb_launch_aos_to_soa(a_src, d_a, n, B, B, st);
+                g->launches += 1;
+                if (e != cudaSuccess) return fail_cuda(e, "aos_to_soa launch");
+            }
+        }
+        return RB_OK;
+    };
+    std::vector<const double*> d_in(ins.size());
+    double* d = g->in[0].p;
+    for (size_t k = 0; k < ins.size(); ++k) {
+        d_in[k] = ins[k].p ? d : nullptr;
+        if (ins[k].p) { rc = bring_in(ins[k].p, d, ins[k].arrays); if (rc) return rc; }
+        d += ins[k].arrays * one;
+    }
+    std::vector<double*> d_out(outs.size());
+    d = g->out[0].p;
+    for (size_t k = 0; k < outs.size(); ++k) {
+        d_out[k] = outs[k].p ? d : nullptr;
+        d += outs[k].arrays * (outs[k].plain ? B : one);
+    }
+    rc = run(d_in.data(), d_out.data(), d_stat); if (rc) return rc;
+    auto bring_out = [&](const double* src, double* dst, size_t arrays) -> int {
+        if (!dst) return RB_OK;
+        for (size_t a = 0; a < arrays; ++a) {
+            const double* s_a = src + a * one;
+            double* d_a = dst + a * src_step;
+            if (!aos) {
+                RB_CUDA(cudaMemcpy2DAsync(d_a, ld * sizeof(double), s_a, B * sizeof(double), B * sizeof(double), (size_t)n,
+                                          host ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice, st));
+            } else {
+                double* a_dst = host ? d_tmp + a * one : d_a;
+                cudaError_t e2 = rb_launch_soa_to_aos(s_a, a_dst, n, B, B, st);
+                g->launches += 1;
+                if (e2 != cudaSuccess) return fail_cuda(e2, "soa_to_aos launch");
+                if (host) RB_CUDA(cudaMemcpyAsync(d_a, a_dst, one * sizeof(double), cudaMemcpyDeviceToHost, st));
+            }
+        }
+        return RB_OK;
+    };
+    d = g->out[0].p;
+    bool first = true;
+    for (size_t k = 0; k < outs.size(); ++k) {
+        const StagedOut& o = outs[k];
+        if (o.plain) {
+            if (o.p) RB_CUDA(cudaMemcpyAsync(o.p, d, B * sizeof(double), host ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice, st));
+            d += o.arrays * B;
+            continue;
+        }
+        // the AoS landing zone is reused per output array group, so drain between groups
+        if (!first && aos && host) RB_CUDA(cudaStreamSynchronize(st));
+        first = false;
+        rc = bring_out(d, o.p, o.arrays); if (rc) return rc;
+        d += o.arrays * one;
+    }
+    // everything above went through engine-owned staging: drain before another call may reuse it
+    RB_CUDA(cudaStreamSynchronize(st));
+    return RB_OK;
+    };
+    const int rc_staged = staged();
+    if (rc_staged != RB_OK) {       // copies already queued must not outlive the call
+        const std::string keep = g_err;
+        cudaStreamSynchronize(st);
+        if (mem == RB_MEM_HOST) drain_host_pipeline(g);
+        g_err = keep;
+        return rc_staged;
+    }
+    return mem == RB_MEM_HOST ? fetch_status(g, 1) : RB_OK;     // still under g->mu
+}
+
+// Checks the weights of an RbQuadCost and packs them into the layout of the engine's cost-weight block (RB_CW_* rows).
+int pack_cost_weights(int n, const RbQuadCost* w, double (&cw)[RB_CW_ROWS * RB_MAX_N]) {
+    memset(cw, 0, sizeof cw);
+    const double* rows[RB_CW_ROWS] = {w->q_ref, w->w_q, w->w_dq, w->w_tau, w->w_q_final, w->w_dq_final};
+    for (int r = 0; r < RB_CW_ROWS; ++r)
+        if (rows[r]) for (int i = 0; i < n; ++i) {
+            if (!std::isfinite(rows[r][i]) || (r != RB_CW_QREF && rows[r][i] < 0.0)) return fail(RB_ERR_ARG, "cost weights must be finite and non-negative");
+            cw[r * RB_MAX_N + i] = rows[r][i];
+        }
+    return RB_OK;
+}
+
 int rollout_impl(RbGpu* g, const double* q0, const double* dq0, const double* tau, double dt, int horizon,
                  double* q_traj, double* dq_traj, double* q_final, double* dq_final, const RbQuadCost* w, double* cost,
                  size_t n_traj, size_t ld, RbLayout layout, RbMem mem, void* stream, size_t aos_stride = 0) {
@@ -1010,15 +1133,7 @@ int rollout_impl(RbGpu* g, const double* q0, const double* dq0, const double* ta
     cudaStream_t st = mem == RB_MEM_DEVICE ? (cudaStream_t)stream : g->stream;
     // cost weights -> the engine's device block (shared by all cost rollouts, hence ordered like scratch)
     double cw[RB_CW_ROWS * RB_MAX_N];
-    if (cost) {
-        memset(cw, 0, sizeof cw);
-        const double* rows[RB_CW_ROWS] = {w->q_ref, w->w_q, w->w_dq, w->w_tau, w->w_q_final, w->w_dq_final};
-        for (int r = 0; r < RB_CW_ROWS; ++r)
-            if (rows[r]) for (int i = 0; i < n; ++i) {
-                if (!std::isfinite(rows[r][i]) || (r != RB_CW_QREF && rows[r][i] < 0.0)) return fail(RB_ERR_ARG, "cost weights must be finite and non-negative");
-                cw[r * RB_MAX_N + i] = rows[r][i];
-            }
-    }
+    if (cost) { const int rc = pack_cost_weights(n, w, cw); if (rc != RB_OK) return rc; }
     const bool shared = cost != nullptr || g->rollout.shared;
     if (mem == RB_MEM_DEVICE && layout == RB_LAYOUT_SOA) {
         ScratchOrder so(g, shared, st);
@@ -1030,96 +1145,139 @@ int rollout_impl(RbGpu* g, const double* q0, const double* dq0, const double* ta
         return RB_OK;
     }
     // Host pointers and/or AoS: stage everything on the device as SoA with ld = n_traj, run once, bring results back.
-    std::lock_guard<std::mutex> lk(g->mu);
-    int* const d_stat = g->d_status + (mem == RB_MEM_HOST ? 1 : 0);
-    if (mem == RB_MEM_HOST) RB_CUDA(cudaMemsetAsync(d_stat, 0, sizeof(int), st));
-    auto staged = [&]() -> int {
-    const size_t B = n_traj, one = (size_t)n * B, H = (size_t)horizon;
-    const bool aos = layout == RB_LAYOUT_AOS, host = mem == RB_MEM_HOST;
-    const size_t src_step = aos ? (aos_stride ? aos_stride : one) : (size_t)n * ld;    // caller's distance between steps
-    // in[0]: q0 | dq0 | tau[H]      out[0]: q_traj[H] | dq_traj[H] | q_fin | dq_fin      tmp[0]: AoS landing zone
-    int rc = g->in[0].ensure((2 + H) * one * sizeof(double)); if (rc) return rc;
-    rc = g->out[0].ensure(((2 * H + 2) * one + B) * sizeof(double)); if (rc) return rc;      // ... | cost[B]
-    if (aos) { rc = g->tmp[0].ensure(std::max<size_t>(2 + H, 2 * H + 2) * one * sizeof(double)); if (rc) return rc; }
-    double* d_in = g->in[0].p; double* d_out = g->out[0].p; double* d_tmp = g->tmp[0].p;
-    auto bring_in = [&](const double* src, double* dst, size_t arrays) -> int {
-        // `arrays` consecutive state arrays
-        for (size_t a = 0; a < arrays; ++a) {
-            const double* s_a = src + a * src_step;
-            double* d_a = dst + a * one;
-            if (!aos) {
-                RB_CUDA(cudaMemcpy2DAsync(d_a, B * sizeof(double), s_a, ld * sizeof(double), B * sizeof(double), (size_t)n,
-                                          host ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice, st));
-            } else {
-                const double* a_src = s_a;
-                if (host) {
-                    double* land = d_tmp + a * one;
-                    RB_CUDA(cudaMemcpyAsync(land, s_a, one * sizeof(double), cudaMemcpyHostToDevice, st));
-                    a_src = land;
-                }
-                cudaError_t e = rb_launch_aos_to_soa(a_src, d_a, n, B, B, st);
-                g->launches += 1;
-                if (e != cudaSuccess) return fail_cuda(e, "aos_to_soa launch");
-            }
+    const size_t H = (size_t)horizon;
+    return run_staged(g, {{q0, 1}, {dq0, 1}, {tau, H}}, {{q_traj, H, false}, {dq_traj, H, false}, {q_final, 1, false}, {dq_final, 1, false}, {cost, 1, true}},
+                      n_traj, ld, layout, mem, aos_stride, st, [&](const double* const* in, double* const* out, int* d_stat) -> int {
+        cudaError_t e;
+        {
+            ScratchOrder so(g, shared, st);
+            if (cost) RB_CUDA(cudaMemcpyAsync(g->cost_w.p, cw, sizeof cw, cudaMemcpyHostToDevice, st));
+            e = g->rollout.fn(g->rollout.param, in[0], in[1], in[2], dt, horizon, out[0], out[1], out[2], out[3], n_traj, n_traj, d_stat,
+                              cost ? g->cost_w.p : nullptr, out[4], st);
         }
+        g->launches += 1;
+        if (e != cudaSuccess) return fail_cuda(e, "rollout launch");
         return RB_OK;
-    };
-    rc = bring_in(q0, d_in, 1); if (rc) return rc;
-    rc = bring_in(dq0, d_in + one, 1); if (rc) return rc;
-    rc = bring_in(tau, d_in + 2 * one, H); if (rc) return rc;
-    double* d_qt = d_out; double* d_dqt = d_out + H * one; double* d_qf = d_out + 2 * H * one; double* d_dqf = d_qf + one;
-    double* d_cost = d_dqf + one;
-    cudaError_t e;
-    {
-        ScratchOrder so(g, shared, st);
-        if (cost) RB_CUDA(cudaMemcpyAsync(g->cost_w.p, cw, sizeof cw, cudaMemcpyHostToDevice, st));
-        e = g->rollout.fn(g->rollout.param, d_in, d_in + one, d_in + 2 * one, dt, horizon,
-                          q_traj ? d_qt : nullptr, dq_traj ? d_dqt : nullptr, q_final ? d_qf : nullptr,
-                          dq_final ? d_dqf : nullptr, B, B, d_stat, cost ? g->cost_w.p : nullptr,
-                          cost ? d_cost : nullptr, st);
+    });
+}
+// Arguments of multibody_rollout_vjp (q_traj .. g_dqf) and multibody_rollout_cost_grad (w, cost).
+struct GradArgs {
+    const double *q0, *dq0, *tau; double dt; int horizon;
+    const double *q_traj, *dq_traj, *g_q, *g_dq, *g_qf, *g_dqf;
+    const RbQuadCost* w; double* cost;
+    double *grad_tau, *grad_q0, *grad_dq0;
+};
+
+// The trajectory workspace of one chunk of a cost-gradient call, 2 H n doubles per trajectory, stays within this.
+constexpr size_t kGradWorkspace = (size_t)1 << 30;
+
+// Both gradient entries on device SoA arrays with leading dimension ld, asynchronous on st.  The cost gradient runs the
+// engine's rollout launcher (so that its cost is multibody_rollout_cost's, bit for bit) into a stream-ordered workspace,
+// then the adjoint over the stored trajectory, chunk by chunk; the weight upload and every launch sit in one ScratchOrder
+// region because the weight block is shared by all cost rollouts on the engine.
+int grad_device(RbGpu* g, const GradArgs& a, const double* cw, size_t B, size_t ld, cudaStream_t st, int* d_stat) {
+    const int n = g->model.n;
+    RbAdjointArgs ad{a.q0, a.dq0, a.tau, a.q_traj, a.dq_traj, ld, a.g_q, a.g_dq, a.g_qf, a.g_dqf, nullptr,
+                     a.grad_tau, a.grad_q0, a.grad_dq0, a.dt, a.horizon};
+    if (!a.cost) {
+        cudaError_t e = rb_launch_rollout_adjoint(n, g->flat.data(), ad, B, ld, d_stat, st);
+        g->launches += 1;
+        return e == cudaSuccess ? RB_OK : fail_cuda(e, "rollout adjoint launch");
     }
-    g->launches += 1;
-    if (e != cudaSuccess) return fail_cuda(e, "rollout launch");
-    auto bring_out = [&](const double* src, double* dst, size_t arrays) -> int {
-        if (!dst) return RB_OK;
-        for (size_t a = 0; a < arrays; ++a) {
-            const double* s_a = src + a * one;
-            double* d_a = dst + a * src_step;
-            if (!aos) {
-                RB_CUDA(cudaMemcpy2DAsync(d_a, ld * sizeof(double), s_a, B * sizeof(double), B * sizeof(double), (size_t)n,
-                                          host ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice, st));
-            } else {
-                double* a_dst = host ? d_tmp + a * one : d_a;
-                cudaError_t e2 = rb_launch_soa_to_aos(s_a, a_dst, n, B, B, st);
-                g->launches += 1;
-                if (e2 != cudaSuccess) return fail_cuda(e2, "soa_to_aos launch");
-                if (host) RB_CUDA(cudaMemcpyAsync(d_a, a_dst, one * sizeof(double), cudaMemcpyDeviceToHost, st));
-            }
+    ScratchOrder so(g, true, st);
+    RB_CUDA(cudaMemcpyAsync(g->cost_w.p, cw, sizeof(double) * RB_CW_ROWS * RB_MAX_N, cudaMemcpyHostToDevice, st));
+    ad.cost_w = g->cost_w.p;
+    const size_t H = (size_t)a.horizon, nn = (size_t)n;
+    // A rollout writes its trajectory with the leading dimension of its inputs: a chunk whose inputs are not already a
+    // dense [n][chunk] block (a cut batch, a padded ld) gets a dense copy of them next to its trajectory.
+    const bool whole = H == 0 || (ld == B && 2 * H * nn * B * sizeof(double) <= kGradWorkspace);
+    const size_t per_traj = (whole ? 2 * H : 3 * H + 2) * nn * sizeof(double);
+    size_t chunk = whole ? B : kGradWorkspace / per_traj;
+    if (!whole) chunk = std::max<size_t>(1, std::min(B, chunk >= 32 ? chunk / 32 * 32 : chunk));
+    double* ws = nullptr;
+    if (H > 0) RB_CUDA(cudaMallocAsync((void**)&ws, per_traj * chunk, st));
+    int rc = RB_OK;
+    for (size_t lo = 0; lo < B && rc == RB_OK; lo += chunk) {
+        const size_t cnt = std::min(chunk, B - lo);
+        const size_t lw = whole ? ld : cnt;                   // leading dimension of the rollout (and of the trajectory)
+        double* qt = ws; double* dqt = ws ? ws + H * nn * cnt : nullptr;
+        const double *rq0 = a.q0 + lo, *rdq0 = a.dq0 + lo, *rtau = a.tau ? a.tau + lo : nullptr;
+        cudaError_t e = cudaSuccess;
+        if (!whole) {
+            double* in = ws + 2 * H * nn * cnt;
+            e = cudaMemcpy2DAsync(in, cnt * sizeof(double), rq0, ld * sizeof(double), cnt * sizeof(double), nn, cudaMemcpyDeviceToDevice, st);
+            if (e == cudaSuccess)
+                e = cudaMemcpy2DAsync(in + nn * cnt, cnt * sizeof(double), rdq0, ld * sizeof(double), cnt * sizeof(double), nn, cudaMemcpyDeviceToDevice, st);
+            if (e == cudaSuccess)
+                e = cudaMemcpy2DAsync(in + 2 * nn * cnt, cnt * sizeof(double), rtau, ld * sizeof(double), cnt * sizeof(double), H * nn, cudaMemcpyDeviceToDevice, st);
+            if (e != cudaSuccess) { rc = fail_cuda(e, "cudaMemcpy2DAsync(gradient workspace)"); break; }
+            rq0 = in; rdq0 = in + nn * cnt; rtau = in + 2 * nn * cnt;
         }
-        return RB_OK;
-    };
-    // the AoS landing zone is reused per output array group, so drain between groups
-    rc = bring_out(d_qt, q_traj, H); if (rc) return rc;
-    if (aos && host) RB_CUDA(cudaStreamSynchronize(st));
-    rc = bring_out(d_dqt, dq_traj, H); if (rc) return rc;
-    if (aos && host) RB_CUDA(cudaStreamSynchronize(st));
-    rc = bring_out(d_qf, q_final, 1); if (rc) return rc;
-    if (aos && host) RB_CUDA(cudaStreamSynchronize(st));
-    rc = bring_out(d_dqf, dq_final, 1); if (rc) return rc;
-    if (cost) RB_CUDA(cudaMemcpyAsync(cost, d_cost, B * sizeof(double), host ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice, st));
-    // everything above went through engine-owned staging: drain before another call may reuse it
-    RB_CUDA(cudaStreamSynchronize(st));
-    return RB_OK;
-    };
-    const int rc_staged = staged();
-    if (rc_staged != RB_OK) {       // copies already queued must not outlive the call
-        const std::string keep = g_err;
-        cudaStreamSynchronize(st);
-        if (mem == RB_MEM_HOST) drain_host_pipeline(g);
-        g_err = keep;
-        return rc_staged;
+        e = g->rollout.fn(g->rollout.param, rq0, rdq0, rtau, a.dt, a.horizon, qt, dqt, nullptr, nullptr, cnt, lw, d_stat,
+                          g->cost_w.p, a.cost + lo, st);
+        g->launches += 1;
+        if (e != cudaSuccess) { rc = fail_cuda(e, "rollout launch"); break; }
+        RbAdjointArgs c = ad;
+        c.q0 = a.q0 + lo; c.dq0 = a.dq0 + lo; c.tau = a.tau ? a.tau + lo : nullptr;
+        c.q_traj = qt; c.dq_traj = dqt; c.ld_traj = lw;
+        c.grad_tau = a.grad_tau ? a.grad_tau + lo : nullptr;
+        c.grad_q0 = a.grad_q0 ? a.grad_q0 + lo : nullptr;
+        c.grad_dq0 = a.grad_dq0 ? a.grad_dq0 + lo : nullptr;
+        e = rb_launch_rollout_adjoint(n, g->flat.data(), c, cnt, ld, d_stat, st);
+        g->launches += 1;
+        if (e != cudaSuccess) rc = fail_cuda(e, "rollout adjoint launch");
     }
-    return mem == RB_MEM_HOST ? fetch_status(g, 1) : RB_OK;     // still under g->mu
+    if (ws) { cudaError_t e = cudaFreeAsync(ws, st); if (e != cudaSuccess && rc == RB_OK) rc = fail_cuda(e, "cudaFreeAsync(gradient workspace)"); }
+    return rc;
+}
+
+int grad_impl(RbGpu* g, const GradArgs& a, size_t n_traj, size_t ld, RbLayout layout, RbMem mem, void* stream, size_t aos_stride = 0) {
+    if (!g) return fail(RB_ERR_NULL, "engine handle is NULL");
+    if (g->model.n > RB_DERIV_MAX_N || !g->model.serial)
+        return fail(RB_ERR_UNSUPPORTED, "rollout gradients use the forward-dynamics derivative kernels, which serve serial chains of at most 12 joints");
+    if (layout != RB_LAYOUT_SOA && layout != RB_LAYOUT_AOS) return fail(RB_ERR_ARG, "bad layout");
+    if (!g->peers.empty()) {
+        if (mem != RB_MEM_HOST) return fail(mem == RB_MEM_DEVICE ? RB_ERR_UNSUPPORTED : RB_ERR_ARG, mem == RB_MEM_DEVICE ? kMultiDeviceOnly : "bad mem");
+        if (n_traj == 0) return RB_OK;
+        const bool aos = layout == RB_LAYOUT_AOS;
+        const size_t n = (size_t)g->model.n;
+        if (!aos) { if (ld == 0) ld = n_traj; if (ld < n_traj) return fail(RB_ERR_ARG, "ld < n_traj"); }
+        return run_on_peers(g, [&](size_t i) -> int {
+            size_t lo, hi; slice_bounds(n_traj, g->peers.size(), i, &lo, &hi);
+            if (hi == lo) return RB_OK;
+            const size_t o = lo * (aos ? n : 1);              // offset of trajectory lo inside one state array
+            auto at = [&](const double* p) { return p ? p + o : nullptr; };
+            auto atw = [&](double* p) { return p ? p + o : nullptr; };
+            GradArgs s = a;
+            s.q0 = at(a.q0); s.dq0 = at(a.dq0); s.tau = at(a.tau); s.q_traj = at(a.q_traj); s.dq_traj = at(a.dq_traj);
+            s.g_q = at(a.g_q); s.g_dq = at(a.g_dq); s.g_qf = at(a.g_qf); s.g_dqf = at(a.g_dqf);
+            s.cost = a.cost ? a.cost + lo : nullptr;
+            s.grad_tau = atw(a.grad_tau); s.grad_q0 = atw(a.grad_q0); s.grad_dq0 = atw(a.grad_dq0);
+            return grad_impl(g->peers[i], s, hi - lo, ld, layout, mem, nullptr, aos ? n_traj * n : 0);
+        });
+    }
+    if (mem != RB_MEM_HOST && mem != RB_MEM_DEVICE) return fail(RB_ERR_ARG, "bad mem");
+    if (a.horizon < 0) return fail(RB_ERR_ARG, "horizon < 0");
+    if (!std::isfinite(a.dt)) return fail(RB_ERR_ARG, "dt must be finite");
+    if (n_traj == 0) return RB_OK;
+    const bool cost = a.w != nullptr;
+    const size_t H = (size_t)a.horizon;
+    if (!a.q0 || !a.dq0 || (H > 0 && (!a.tau || (!cost && (!a.q_traj || !a.dq_traj))))) return fail(RB_ERR_NULL, "input pointer is NULL");
+    if (layout == RB_LAYOUT_SOA) { if (ld == 0) ld = n_traj; if (ld < n_traj) return fail(RB_ERR_ARG, "ld < n_traj"); }
+    double cw[RB_CW_ROWS * RB_MAX_N];
+    if (cost) { const int rc = pack_cost_weights(g->model.n, a.w, cw); if (rc != RB_OK) return rc; }
+    if (!cost && !a.grad_tau && !a.grad_q0 && !a.grad_dq0) return RB_OK;
+    DeviceGuard dg(g->device);
+    if (!dg.ok) return fail(RB_ERR_CUDA, "cudaSetDevice failed");
+    cudaStream_t st = mem == RB_MEM_DEVICE ? (cudaStream_t)stream : g->stream;
+    if (mem == RB_MEM_DEVICE && layout == RB_LAYOUT_SOA) return grad_device(g, a, cw, n_traj, ld, st, g->d_status);
+    // Host pointers and/or AoS: staged like the rollout; the staged call then runs as a device SoA call with ld = n_traj.
+    return run_staged(g, {{a.q0, 1}, {a.dq0, 1}, {a.tau, H}, {a.q_traj, H}, {a.dq_traj, H}, {a.g_q, H}, {a.g_dq, H}, {a.g_qf, 1}, {a.g_dqf, 1}},
+                      {{a.grad_tau, H, false}, {a.grad_q0, 1, false}, {a.grad_dq0, 1, false}, {a.cost, 1, true}},
+                      n_traj, ld, layout, mem, aos_stride, st, [&](const double* const* in, double* const* out, int* d_stat) -> int {
+        const GradArgs s{in[0], in[1], in[2], a.dt, a.horizon, in[3], in[4], in[5], in[6], in[7], in[8], a.w, out[3], out[0], out[1], out[2]};
+        return grad_device(g, s, cw, n_traj, n_traj, st, d_stat);
+    });
 }
 }  // namespace
 
@@ -1134,6 +1292,26 @@ extern "C" int multibody_rollout_cost(RbGpu* g, const double* q0, const double* 
                                       size_t n_traj, size_t ld, RbLayout layout, RbMem mem, void* stream) {
     if (!cost) return fail(RB_ERR_NULL, "cost output pointer is NULL");
     return rollout_impl(g, q0, dq0, tau, dt, horizon, nullptr, nullptr, q_final, dq_final, weights, cost, n_traj, ld, layout, mem, stream);
+}
+
+extern "C" int multibody_rollout_vjp(RbGpu* g, const double* q0, const double* dq0, const double* tau, double dt, int horizon,
+                                     const double* q_traj, const double* dq_traj,
+                                     const double* g_q_traj, const double* g_dq_traj, const double* g_q_final, const double* g_dq_final,
+                                     double* grad_tau, double* grad_q0, double* grad_dq0,
+                                     size_t n_traj, size_t ld, RbLayout layout, RbMem mem, void* stream) {
+    const GradArgs a{q0, dq0, tau, dt, horizon, q_traj, dq_traj, g_q_traj, g_dq_traj, g_q_final, g_dq_final, nullptr, nullptr,
+                     grad_tau, grad_q0, grad_dq0};
+    return grad_impl(g, a, n_traj, ld, layout, mem, stream);
+}
+
+extern "C" int multibody_rollout_cost_grad(RbGpu* g, const double* q0, const double* dq0, const double* tau, double dt, int horizon,
+                                           const RbQuadCost* weights, double* cost, double* grad_tau, double* grad_q0, double* grad_dq0,
+                                           size_t n_traj, size_t ld, RbLayout layout, RbMem mem, void* stream) {
+    if (!weights) return fail(RB_ERR_NULL, "cost weights are NULL");
+    if (!cost) return fail(RB_ERR_NULL, "cost output pointer is NULL");
+    const GradArgs a{q0, dq0, tau, dt, horizon, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, weights, cost,
+                     grad_tau, grad_q0, grad_dq0};
+    return grad_impl(g, a, n_traj, ld, layout, mem, stream);
 }
 
 // ===================================================================== helpers

@@ -115,19 +115,11 @@ RB_DI void rb_screw_cols(const double (&R)[3][3], const double (&P)[3], const do
     for (int k = 0; k < 6; ++k) da[k] += t6[k];
 }
 
-// put(blk, r, c, v): blk 0 = d tau_r / d q_c, blk 1 = d tau_r / d dq_c.
-// Real loops over the joints (model rows from the constant bank by index), and no per-joint arrays: a thread cannot
-// hold N screws and column vectors next to the composites -- the first, fully unrolled version did and spilled 4 KB
-// per thread through L2 to HBM (5x the algorithmic write traffic).  Instead, for every pair (i, j < i) the inward
-// sweep walks a copy of (pose, v, a) back from link i to link j and rebuilds s_j, dv_j, da0_j there: ~160 FP64
-// instructions per pair, all in registers.  sn, cs, dq, ddq are indexed at run time (thread-local memory, L1).
-template <int N, class Put>
-RB_DI void rb_rnea_derivatives(const RbModelK<N>& p, const double* sn, const double* cs, const double* dq, const double* ddq,
-                               Put&& put) {
-    double R[3][3] = {{1.0, 0.0, 0.0}, {0.0, 1.0, 0.0}, {0.0, 0.0, 1.0}}, P[3] = {0.0, 0.0, 0.0};
-    double v[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
-    double a[6] = {0.0, 0.0, 0.0, p.g[0], p.g[1], p.g[2]};
-    // ---- outward: world pose, velocity and acceleration of the last link
+// ---- the two sweeps both routines below share
+// Outward: world pose (R, P), velocity v and acceleration a of the last link; screw(i, s_i) sees every joint's screw.
+template <int N, class Screw>
+RB_DI void rb_deriv_outward(const RbModelK<N>& p, const double* sn, const double* cs, const double* dq, const double* ddq,
+                            double (&R)[3][3], double (&P)[3], double (&v)[6], double (&a)[6], Screw&& screw) {
 #pragma unroll 1
     for (int i = 0; i < N; ++i) {
         rb_pose_out(p.jt[i], sn[i], cs[i], R, P);
@@ -141,76 +133,112 @@ RB_DI void rb_rnea_derivatives(const RbModelK<N>& p, const double* sn, const dou
         rb_mcross(v, s6, dv);                                // v_i x s_i
 #pragma unroll
         for (int k = 0; k < 6; ++k) a[k] = fma(s6[k], ddqi, fma(dv[k], dqi, a[k]));
+        screw(i, s6);
     }
+}
+
+// Composites of links i..N-1 (^c above): inertia I^c (its mass is the model constant mc), inertia rate Idot^c,
+// momentum h^c and wrench F^c, all about the world origin.
+struct RbDerivComposites {
+    double Hc[3], Ic[6], dHc[3], dIc[6], hc[6], Fc[6];
+};
+
+// Inward step at link i (pose R, P, velocity v, acceleration a): adds the link to the composites, then forms the
+// per-joint vectors s_i, dv_i, da0_i (rb_screw_cols) and A_i, B_i, G_i, G'_i (the d/d dq counterpart of G_i).
+RB_DI void rb_deriv_inward(const RbJointK& Jt, const double (&R)[3][3], const double (&P)[3], const double (&v)[6],
+                           const double (&a)[6], RbDerivComposites& C, double (&sI)[6], double (&dvI)[6], double (&daI)[6],
+                           double (&A)[6], double (&Bv)[6], double (&G)[6], double (&Gp)[6]) {
+    {   // link i about the world origin
+        const double m = Jt.m;
+        double hw[3], T[3][3], Hm[3], IO[6];
+#pragma unroll
+        for (int r = 0; r < 3; ++r) {
+            hw[r] = fma(R[r][0], Jt.h[0], fma(R[r][1], Jt.h[1], R[r][2] * Jt.h[2]));
+            T[r][0] = fma(R[r][0], Jt.I[0], fma(R[r][1], Jt.I[1], R[r][2] * Jt.I[2]));
+            T[r][1] = fma(R[r][0], Jt.I[1], fma(R[r][1], Jt.I[3], R[r][2] * Jt.I[4]));
+            T[r][2] = fma(R[r][0], Jt.I[2], fma(R[r][1], Jt.I[4], R[r][2] * Jt.I[5]));
+        }
+        double u[3];
+#pragma unroll
+        for (int r = 0; r < 3; ++r) { Hm[r] = fma(m, P[r], hw[r]); u[r] = fma(0.5 * m, P[r], hw[r]); }
+        const double pu2 = 2.0 * fma(P[0], u[0], fma(P[1], u[1], P[2] * u[2]));
+        auto rr = [&](int x, int y) { return fma(T[x][0], R[y][0], fma(T[x][1], R[y][1], T[x][2] * R[y][2])); };
+        IO[0] = rr(0, 0) - 2.0 * P[0] * u[0] + pu2;
+        IO[1] = rr(0, 1) - fma(P[0], u[1], u[0] * P[1]);
+        IO[2] = rr(0, 2) - fma(P[0], u[2], u[0] * P[2]);
+        IO[3] = rr(1, 1) - 2.0 * P[1] * u[1] + pu2;
+        IO[4] = rr(1, 2) - fma(P[1], u[2], u[1] * P[2]);
+        IO[5] = rr(2, 2) - 2.0 * P[2] * u[2] + pu2;
+        // momentum, wrench, inertia rate of the link; accumulate the composites
+        double h6[6], f6[6];
+        rb_wimul<false>(m, Hm, IO, v, h6);
+        rb_wimul<false>(m, Hm, IO, a, f6);
+        rb_fcross<true>(v, h6, f6);
+        const double w[3] = {v[0], v[1], v[2]}, vo[3] = {v[3], v[4], v[5]};
+        double dH[3] = {m * vo[0], m * vo[1], m * vo[2]};
+        rb_cross3_acc(w, Hm, dH);
+        // d IO = [w]x IO + ([w]x IO)^T + 2 (H . vo) Id - vo H^T - H vo^T
+        const double c0[3] = {IO[0], IO[1], IO[2]}, c1[3] = {IO[1], IO[3], IO[4]}, c2[3] = {IO[2], IO[4], IO[5]};
+        double W0[3], W1[3], W2[3];                          // columns of [w]x IO
+        rb_cross3(w, c0, W0); rb_cross3(w, c1, W1); rb_cross3(w, c2, W2);
+        const double hv2 = 2.0 * fma(Hm[0], vo[0], fma(Hm[1], vo[1], Hm[2] * vo[2]));
+        C.dIc[0] += 2.0 * W0[0] + hv2 - 2.0 * vo[0] * Hm[0];
+        C.dIc[1] += W1[0] + W0[1] - fma(vo[0], Hm[1], Hm[0] * vo[1]);
+        C.dIc[2] += W2[0] + W0[2] - fma(vo[0], Hm[2], Hm[0] * vo[2]);
+        C.dIc[3] += 2.0 * W1[1] + hv2 - 2.0 * vo[1] * Hm[1];
+        C.dIc[4] += W2[1] + W1[2] - fma(vo[1], Hm[2], Hm[1] * vo[2]);
+        C.dIc[5] += 2.0 * W2[2] + hv2 - 2.0 * vo[2] * Hm[2];
+#pragma unroll
+        for (int k = 0; k < 3; ++k) { C.Hc[k] += Hm[k]; C.dHc[k] += dH[k]; }
+#pragma unroll
+        for (int k = 0; k < 6; ++k) { C.Ic[k] += IO[k]; C.hc[k] += h6[k]; C.Fc[k] += f6[k]; }
+    }
+    const double mc = Jt.mc;
+    rb_screw_cols(R, P, v, a, sI, dvI, daI);
+    double dv2[6], sh[6];
+    rb_wimul<false>(mc, C.Hc, C.Ic, sI, A);
+    rb_wimul<false>(0.0, C.dHc, C.dIc, sI, Bv);              // Idot^c s
+    rb_fcross<false>(sI, C.hc, sh);                          // s x* h^c
+#pragma unroll
+    for (int k = 0; k < 6; ++k) { Gp[k] = Bv[k] + sh[k]; Bv[k] -= sh[k]; dv2[k] = 2.0 * dvI[k]; }
+    rb_wimul<true>(mc, C.Hc, C.Ic, dv2, Gp);
+    rb_fcross<false>(sI, C.Fc, G);
+    rb_wimul<true>(mc, C.Hc, C.Ic, daI, G);
+    rb_wimul<true>(0.0, C.dHc, C.dIc, dvI, G);
+    rb_fcross<true>(dvI, C.hc, G);
+}
+
+// One link back along the chain for (R, P, v, a), leaving link i whose screw / dv are s / dv:
+//   a <- a - s ddq_i - dv dq_i,  v <- v - s dq_i,  pose of link i -> link i-1.
+RB_DI void rb_deriv_step_back(const RbJointK& Jt, double sn, double cs, double dqi, double ddqi, const double (&s)[6],
+                              const double (&dv)[6], double (&R)[3][3], double (&P)[3], double (&v)[6], double (&a)[6]) {
+#pragma unroll
+    for (int k = 0; k < 6; ++k) {
+        a[k] = fma(-s[k], ddqi, fma(-dv[k], dqi, a[k]));
+        v[k] = fma(-s[k], dqi, v[k]);
+    }
+    rb_pose_back(Jt, sn, cs, R, P);
+}
+
+// put(blk, r, c, v): blk 0 = d tau_r / d q_c, blk 1 = d tau_r / d dq_c.
+// Real loops over the joints (model rows from the constant bank by index), and no per-joint arrays: a thread cannot
+// hold N screws and column vectors next to the composites -- the first, fully unrolled version did and spilled 4 KB
+// per thread through L2 to HBM (5x the algorithmic write traffic).  Instead, for every pair (i, j < i) the inward
+// sweep walks a copy of (pose, v, a) back from link i to link j and rebuilds s_j, dv_j, da0_j there: ~160 FP64
+// instructions per pair, all in registers.  sn, cs, dq, ddq are indexed at run time (thread-local memory, L1).
+template <int N, class Put>
+RB_DI void rb_rnea_derivatives(const RbModelK<N>& p, const double* sn, const double* cs, const double* dq, const double* ddq,
+                               Put&& put) {
+    double R[3][3] = {{1.0, 0.0, 0.0}, {0.0, 1.0, 0.0}, {0.0, 0.0, 1.0}}, P[3] = {0.0, 0.0, 0.0};
+    double v[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+    double a[6] = {0.0, 0.0, 0.0, p.g[0], p.g[1], p.g[2]};
+    rb_deriv_outward<N>(p, sn, cs, dq, ddq, R, P, v, a, [](int, const double (&)[6]) {});
     // ---- inward: composites, the per-joint vectors, and the entries
-    double Hc[3] = {0.0, 0.0, 0.0}, Ic[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};           // I^c (mass: model constant)
-    double dHc[3] = {0.0, 0.0, 0.0}, dIc[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};         // Idot^c
-    double hc[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0}, Fc[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+    RbDerivComposites C = {};
 #pragma unroll 1
     for (int i = N - 1; i >= 0; --i) {
-        const RbJointK& Jt = p.jt[i];
-        {   // link i about the world origin
-            const double m = Jt.m;
-            double hw[3], T[3][3], Hm[3], IO[6];
-#pragma unroll
-            for (int r = 0; r < 3; ++r) {
-                hw[r] = fma(R[r][0], Jt.h[0], fma(R[r][1], Jt.h[1], R[r][2] * Jt.h[2]));
-                T[r][0] = fma(R[r][0], Jt.I[0], fma(R[r][1], Jt.I[1], R[r][2] * Jt.I[2]));
-                T[r][1] = fma(R[r][0], Jt.I[1], fma(R[r][1], Jt.I[3], R[r][2] * Jt.I[4]));
-                T[r][2] = fma(R[r][0], Jt.I[2], fma(R[r][1], Jt.I[4], R[r][2] * Jt.I[5]));
-            }
-            double u[3];
-#pragma unroll
-            for (int r = 0; r < 3; ++r) { Hm[r] = fma(m, P[r], hw[r]); u[r] = fma(0.5 * m, P[r], hw[r]); }
-            const double pu2 = 2.0 * fma(P[0], u[0], fma(P[1], u[1], P[2] * u[2]));
-            auto rr = [&](int x, int y) { return fma(T[x][0], R[y][0], fma(T[x][1], R[y][1], T[x][2] * R[y][2])); };
-            IO[0] = rr(0, 0) - 2.0 * P[0] * u[0] + pu2;
-            IO[1] = rr(0, 1) - fma(P[0], u[1], u[0] * P[1]);
-            IO[2] = rr(0, 2) - fma(P[0], u[2], u[0] * P[2]);
-            IO[3] = rr(1, 1) - 2.0 * P[1] * u[1] + pu2;
-            IO[4] = rr(1, 2) - fma(P[1], u[2], u[1] * P[2]);
-            IO[5] = rr(2, 2) - 2.0 * P[2] * u[2] + pu2;
-            // momentum, wrench, inertia rate of the link; accumulate the composites
-            double h6[6], f6[6];
-            rb_wimul<false>(m, Hm, IO, v, h6);
-            rb_wimul<false>(m, Hm, IO, a, f6);
-            rb_fcross<true>(v, h6, f6);
-            const double w[3] = {v[0], v[1], v[2]}, vo[3] = {v[3], v[4], v[5]};
-            double dH[3] = {m * vo[0], m * vo[1], m * vo[2]};
-            rb_cross3_acc(w, Hm, dH);
-            // d IO = [w]x IO + ([w]x IO)^T + 2 (H . vo) Id - vo H^T - H vo^T
-            const double c0[3] = {IO[0], IO[1], IO[2]}, c1[3] = {IO[1], IO[3], IO[4]}, c2[3] = {IO[2], IO[4], IO[5]};
-            double W0[3], W1[3], W2[3];                      // columns of [w]x IO
-            rb_cross3(w, c0, W0); rb_cross3(w, c1, W1); rb_cross3(w, c2, W2);
-            const double hv2 = 2.0 * fma(Hm[0], vo[0], fma(Hm[1], vo[1], Hm[2] * vo[2]));
-            dIc[0] += 2.0 * W0[0] + hv2 - 2.0 * vo[0] * Hm[0];
-            dIc[1] += W1[0] + W0[1] - fma(vo[0], Hm[1], Hm[0] * vo[1]);
-            dIc[2] += W2[0] + W0[2] - fma(vo[0], Hm[2], Hm[0] * vo[2]);
-            dIc[3] += 2.0 * W1[1] + hv2 - 2.0 * vo[1] * Hm[1];
-            dIc[4] += W2[1] + W1[2] - fma(vo[1], Hm[2], Hm[1] * vo[2]);
-            dIc[5] += 2.0 * W2[2] + hv2 - 2.0 * vo[2] * Hm[2];
-#pragma unroll
-            for (int k = 0; k < 3; ++k) { Hc[k] += Hm[k]; dHc[k] += dH[k]; }
-#pragma unroll
-            for (int k = 0; k < 6; ++k) { Ic[k] += IO[k]; hc[k] += h6[k]; Fc[k] += f6[k]; }
-        }
-        const double mc = Jt.mc;
-        double sI[6], dvI[6], daI[6];
-        rb_screw_cols(R, P, v, a, sI, dvI, daI);
-        double A[6], Bv[6], G[6], Gp[6];
-        {
-            double dv2[6], sh[6];
-            rb_wimul<false>(mc, Hc, Ic, sI, A);
-            rb_wimul<false>(0.0, dHc, dIc, sI, Bv);          // Idot^c s
-            rb_fcross<false>(sI, hc, sh);                    // s x* h^c
-#pragma unroll
-            for (int k = 0; k < 6; ++k) { Gp[k] = Bv[k] + sh[k]; Bv[k] -= sh[k]; dv2[k] = 2.0 * dvI[k]; }
-            rb_wimul<true>(mc, Hc, Ic, dv2, Gp);
-            rb_fcross<false>(sI, Fc, G);
-            rb_wimul<true>(mc, Hc, Ic, daI, G);
-            rb_wimul<true>(0.0, dHc, dIc, dvI, G);
-            rb_fcross<true>(dvI, hc, G);
-        }
+        double sI[6], dvI[6], daI[6], A[6], Bv[6], G[6], Gp[6];
+        rb_deriv_inward(p.jt[i], R, P, v, a, C, sI, dvI, daI, A, Bv, G, Gp);
         put(0, i, i, rb_dot6(sI, G));
         put(1, i, i, rb_dot6(sI, Gp));
         // walk a copy back to every j < i:  column i above the diagonal, row i below it
@@ -221,13 +249,7 @@ RB_DI void rb_rnea_derivatives(const RbModelK<N>& p, const double* sn, const dou
         for (int k = 0; k < 6; ++k) { vt[k] = v[k]; at[k] = a[k]; }
 #pragma unroll 1
         for (int j = i - 1; j >= 0; --j) {                   // leaving link j+1, whose screw / dv are in sI / dvI
-            const double dqn = dq[j + 1], ddqn = ddq[j + 1];
-#pragma unroll
-            for (int k = 0; k < 6; ++k) {
-                at[k] = fma(-sI[k], ddqn, fma(-dvI[k], dqn, at[k]));
-                vt[k] = fma(-sI[k], dqn, vt[k]);
-            }
-            rb_pose_back(p.jt[j + 1], sn[j + 1], cs[j + 1], Rt, Pt);
+            rb_deriv_step_back(p.jt[j + 1], sn[j + 1], cs[j + 1], dq[j + 1], ddq[j + 1], sI, dvI, Rt, Pt, vt, at);
             rb_screw_cols(Rt, Pt, vt, at, sI, dvI, daI);
             put(0, j, i, rb_dot6(sI, G));
             put(1, j, i, rb_dot6(sI, Gp));
@@ -240,6 +262,41 @@ RB_DI void rb_rnea_derivatives(const RbModelK<N>& p, const double* sn, const dou
                 for (int k = 0; k < 6; ++k) { v[k] = vt[k]; a[k] = at[k]; }
             }
         }
+    }
+}
+
+// Vector-Jacobian product of inverse dynamics in O(N), SUBTRACTED from gq and gdq (the adjoints a caller accumulates):
+//   gq_j  -= (mu^T d tau / d q )_j = Sbar_j . G_j  +   da0_j . Abar_j + dv_j . Bbar_j
+//   gdq_j -= (mu^T d tau / d dq)_j = Sbar_j . G'_j + 2 dv_j . Abar_j +  s_j . Bbar_j
+//   Sbar_j = sum_{m <= j} mu_m s_m,   Abar_j = sum_{m > j} mu_m A_m,   Bbar_j = sum_{m > j} mu_m B_m
+// (the pair formulas of the header above, summed over m).  The outward sweep adds up Sbar over all joints; the inward
+// sweep carries Abar and Bbar and takes each joint's term out of Sbar after using it, so the pair walk-back of
+// rb_rnea_derivatives becomes one step back per joint.  Like sn, cs, dq, ddq and mu, gq and gdq are indexed at run
+// time (thread-local memory): a caller's adjoints do not occupy registers across the sweeps.
+template <int N>
+RB_DI void rb_rnea_vjp(const RbModelK<N>& p, const double* sn, const double* cs, const double* dq, const double* ddq,
+                       const double* mu, double* gq, double* gdq) {
+    double R[3][3] = {{1.0, 0.0, 0.0}, {0.0, 1.0, 0.0}, {0.0, 0.0, 1.0}}, P[3] = {0.0, 0.0, 0.0};
+    double v[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+    double a[6] = {0.0, 0.0, 0.0, p.g[0], p.g[1], p.g[2]};
+    double Sb[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+    rb_deriv_outward<N>(p, sn, cs, dq, ddq, R, P, v, a, [&](int i, const double (&s6)[6]) {
+        const double mi = mu[i];
+#pragma unroll
+        for (int k = 0; k < 6; ++k) Sb[k] = fma(mi, s6[k], Sb[k]);
+    });
+    RbDerivComposites C = {};
+    double Ab[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0}, Bb[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+#pragma unroll 1
+    for (int i = N - 1; i >= 0; --i) {
+        double sI[6], dvI[6], daI[6], A[6], Bv[6], G[6], Gp[6];
+        rb_deriv_inward(p.jt[i], R, P, v, a, C, sI, dvI, daI, A, Bv, G, Gp);
+        gq[i] -= rb_dot6(Sb, G) + (rb_dot6(daI, Ab) + rb_dot6(dvI, Bb));
+        gdq[i] -= rb_dot6(Sb, Gp) + fma(2.0, rb_dot6(dvI, Ab), rb_dot6(sI, Bb));
+        const double mi = mu[i];
+#pragma unroll
+        for (int k = 0; k < 6; ++k) { Ab[k] = fma(mi, A[k], Ab[k]); Bb[k] = fma(mi, Bv[k], Bb[k]); Sb[k] = fma(-mi, sI[k], Sb[k]); }
+        if (i > 0) rb_deriv_step_back(p.jt[i], sn[i], cs[i], dq[i], ddq[i], sI, dvI, R, P, v, a);
     }
 }
 
