@@ -297,6 +297,38 @@ int multibody_rollout_cost_grad(RbGpu* g, const double* q0, const double* dq0, c
                                 const RbQuadCost* weights, double* cost, double* grad_tau, double* grad_q0, double* grad_dq0,
                                 size_t n_traj, size_t ld, RbLayout layout, RbMem mem, void* stream);
 
+/* Tip-pose tracking terms for the fused rollout cost and its gradient: MPC tasks stated at the end effector.
+ * The tip frame is the frame of multibody_jac: the reference's last link frame (for a kinematic tree the last link,
+ * reached along its supporting branch).  Its origin is what multibody_fwd_kin returns.  With R(q) its orientation in
+ * the base frame and x(q) = p(q) + R(q) offset the tracked point,
+ *   cost = [every term of multibody_rollout_cost for `weights`]
+ *        + sum_{t=0}^{H-1} dt * ( sum_k w_p[k] (x_k(q_{t+1}) - p_ref[k])^2 + w_R ||R(q_{t+1}) - R_ref||_F^2 )
+ *        +                      sum_k w_p_final[k] (x_k(q_H) - p_ref[k])^2 + w_R_final ||R(q_H) - R_ref||_F^2.
+ * Weights must be finite and non-negative, offset / p_ref / R_ref finite (RB_ERR_ARG otherwise).  The target is shared
+ * by all trajectories and steps. */
+typedef struct RbTipCost {
+    const double* offset;     /* [3] tracked point in the tip frame (tool centre point); NULL = the tip frame's origin */
+    const double* p_ref;      /* [3] its target in the base frame; NULL = 0 */
+    const double* w_p;        /* [3] running weights per base-frame axis; NULL = 0 */
+    const double* w_p_final;  /* [3] terminal weights per base-frame axis; NULL = 0 */
+    const double* R_ref;      /* [9] row-major target orientation of the tip frame in the base frame; NULL = identity */
+    double w_R;               /* running weight of ||R - R_ref||_F^2 */
+    double w_R_final;         /* terminal weight of the same */
+} RbTipCost;
+/* multibody_rollout_cost with the tip terms of `tip` added.  weights == NULL: no quadratic terms; tip == NULL: exactly
+ * multibody_rollout_cost (same results, same launches).  Every chain and kernel family multibody_rollout_cost serves. */
+int multibody_rollout_tip_cost(RbGpu* g, const double* q0, const double* dq0, const double* tau, double dt, int horizon,
+                               const RbQuadCost* weights, const RbTipCost* tip, double* cost, double* q_final, double* dq_final,
+                               size_t n_traj, size_t ld, RbLayout layout, RbMem mem, void* stream);
+/* multibody_rollout_cost_grad with the tip terms: cost bit-identical to multibody_rollout_tip_cost on the same engine, and
+ * its gradient (the tip terms' part from one world-frame wrench per state projected on the joint screws, O(n) per state).
+ * weights == NULL: no quadratic terms; tip == NULL: exactly multibody_rollout_cost_grad.  Serial chains of at most 12
+ * joints (RB_ERR_UNSUPPORTED otherwise), everything else as multibody_rollout_cost_grad. */
+int multibody_rollout_tip_cost_grad(RbGpu* g, const double* q0, const double* dq0, const double* tau, double dt, int horizon,
+                                    const RbQuadCost* weights, const RbTipCost* tip, double* cost, double* grad_tau,
+                                    double* grad_q0, double* grad_dq0, size_t n_traj, size_t ld, RbLayout layout, RbMem mem,
+                                    void* stream);
+
 /* ---- device-side helpers (bench / tests) --------------------------------------------------- */
 /* Fill a device SOA array [n][ld] with the counter-based sampler of SURVEY.md 8d:
  * value(joint i, state s) = fma(hi[i]-lo[i], u, lo[i]),  u = top 53 bits of

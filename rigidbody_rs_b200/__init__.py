@@ -346,9 +346,11 @@ class Multibody:
         return tuple(res)
 
     def rollout_cost(self, q0, dq0, tau, dt, q_ref=None, w_q=None, w_dq=None, w_tau=None, w_q_final=None, w_dq_final=None,
-                     layout="soa", final=False):
+                     layout="soa", final=False, tip=None):
         """Fused rollout + quadratic running/terminal cost (one scalar per trajectory; include/rigidbody.h
-        multibody_rollout_cost).  Shapes as `rollout`; weights are length-n vectors (None = zeros)."""
+        multibody_rollout_cost).  Shapes as `rollout`; weights are length-n vectors (None = zeros).  `tip`: a mapping
+        with the keys of RbTipCost (offset, p_ref, w_p, w_p_final: 3 values; R_ref: 3x3; w_R, w_R_final: scalars;
+        missing = the struct's NULL / 0) adds the tip-pose terms (multibody_rollout_tip_cost)."""
         a_q, a_dq, a_tau, B, H, lay, new = self._rollout_args(q0, dq0, tau, layout, "rollout_cost")
         cuda = a_q.cuda
         qc, keep = self._quad_cost(q_ref, w_q, w_dq, w_tau, w_q_final, w_dq_final)
@@ -356,24 +358,40 @@ class Multibody:
         qf = new(a_q.shape) if final else None
         dqf = new(a_q.shape) if final else None
         ptr = lambda a: C.c_void_p(a.ptr) if a is not None else None
-        check(lib.multibody_rollout_cost(self._h, ptr(a_q), ptr(a_dq), ptr(a_tau), float(dt), int(H), C.byref(qc), ptr(cost),
-                                         ptr(qf), ptr(dqf), B, 0, lay, RB_MEM_DEVICE if cuda else RB_MEM_HOST,
-                                         self._stream(cuda, a_q)))
+        head = (self._h, ptr(a_q), ptr(a_dq), ptr(a_tau), float(dt), int(H), C.byref(qc))
+        tail = (ptr(cost), ptr(qf), ptr(dqf), B, 0, lay, RB_MEM_DEVICE if cuda else RB_MEM_HOST, self._stream(cuda, a_q))
+        if tip is None:
+            check(lib.multibody_rollout_cost(*head, *tail))
+        else:
+            tc, keep_tip = _tip_cost(tip)
+            check(lib.multibody_rollout_tip_cost(*head, C.byref(tc), *tail))
         return (cost.arr, qf.arr, dqf.arr) if final else cost.arr
 
     def rollout_cost_grad(self, q0, dq0, tau, dt, q_ref=None, w_q=None, w_dq=None, w_tau=None, w_q_final=None, w_dq_final=None,
-                          layout="soa"):
+                          layout="soa", tip=None):
         """`rollout_cost` and its gradient (include/rigidbody.h multibody_rollout_cost_grad): returns (cost, grad_tau,
         grad_q0, grad_dq0), the cost bit for bit `rollout_cost`'s, grad_tau shaped like tau, grad_q0 / grad_dq0 like q0.
-        Serial chains of at most 12 joints."""
+        `tip` as for `rollout_cost` (multibody_rollout_tip_cost_grad).  Serial chains of at most 12 joints."""
         a_q, a_dq, a_tau, B, H, lay, new = self._rollout_args(q0, dq0, tau, layout, "rollout_cost_grad")
         cuda = a_q.cuda
         qc, keep = self._quad_cost(q_ref, w_q, w_dq, w_tau, w_q_final, w_dq_final)
         cost, gt, gq, gdq = new((B,)), new(a_tau.shape), new(a_q.shape), new(a_q.shape)
-        check(lib.multibody_rollout_cost_grad(self._h, C.c_void_p(a_q.ptr), C.c_void_p(a_dq.ptr), C.c_void_p(a_tau.ptr), float(dt), int(H),
-                                              C.byref(qc), C.c_void_p(cost.ptr), C.c_void_p(gt.ptr), C.c_void_p(gq.ptr), C.c_void_p(gdq.ptr),
-                                              B, 0, lay, RB_MEM_DEVICE if cuda else RB_MEM_HOST, self._stream(cuda, a_q)))
+        head = (self._h, C.c_void_p(a_q.ptr), C.c_void_p(a_dq.ptr), C.c_void_p(a_tau.ptr), float(dt), int(H), C.byref(qc))
+        tail = (C.c_void_p(cost.ptr), C.c_void_p(gt.ptr), C.c_void_p(gq.ptr), C.c_void_p(gdq.ptr),
+                B, 0, lay, RB_MEM_DEVICE if cuda else RB_MEM_HOST, self._stream(cuda, a_q))
+        if tip is None:
+            check(lib.multibody_rollout_cost_grad(*head, *tail))
+        else:
+            tc, keep_tip = _tip_cost(tip)
+            check(lib.multibody_rollout_tip_cost_grad(*head, C.byref(tc), *tail))
         return cost.arr, gt.arr, gq.arr, gdq.arr
+
+    def rollout_cost_autograd(self, q0, dq0, tau, dt, tip=None, **weights):
+        """`rollout_cost` as a differentiable torch function: q0, dq0 [n, B] and tau [H, n, B] are CUDA float64 tensors
+        (layout 'soa'); returns cost [B].  The forward pass runs `rollout_cost_grad` (`rollout_cost` when no input requires
+        a gradient); the backward pass scales the stored gradients by the upstream gradient of each trajectory's cost.
+        `tip` and the weights as for `rollout_cost`."""
+        return _rollout_cost_function().apply(self, q0, dq0, tau, float(dt), tip, weights)
 
     def rollout_vjp(self, q0, dq0, tau, dt, q_traj, dq_traj, g_q_traj=None, g_dq_traj=None, g_q_final=None, g_dq_final=None,
                     layout="soa"):
@@ -457,7 +475,30 @@ class Multibody:
         return out
 
 
+_TIP_KEYS = {"offset": 3, "p_ref": 3, "w_p": 3, "w_p_final": 3, "R_ref": 9}
+
+
+def _tip_cost(tip):
+    """An RbTipCost from a mapping with its keys (missing = NULL / 0) and the arrays it points into (keep them alive)."""
+    unknown = set(tip) - set(_TIP_KEYS) - {"w_R", "w_R_final"}
+    if unknown:
+        raise ValueError(f"tip: unknown keys {sorted(unknown)}")
+    tc = _lib.RbTipCost()
+    keep = []
+    for name, size in _TIP_KEYS.items():
+        if tip.get(name) is not None:
+            a = np.ascontiguousarray(np.asarray(tip[name], dtype=np.float64).reshape(-1))
+            if a.size != size:
+                raise ValueError(f"tip: {name} must have {size} values")
+            keep.append(a)
+            setattr(tc, name, a.ctypes.data_as(C.POINTER(C.c_double)))
+    tc.w_R = float(tip.get("w_R", 0.0))
+    tc.w_R_final = float(tip.get("w_R_final", 0.0))
+    return tc, keep
+
+
 _ROLLOUT_FN = None
+_ROLLOUT_COST_FN = None
 
 
 def _rollout_function():
@@ -487,3 +528,33 @@ def _rollout_function():
 
         _ROLLOUT_FN = RolloutFunction
     return _ROLLOUT_FN
+
+
+def _rollout_cost_function():
+    """The torch.autograd.Function behind Multibody.rollout_cost_autograd (built on first use: torch stays a lazy import)."""
+    global _ROLLOUT_COST_FN
+    if _ROLLOUT_COST_FN is None:
+        import torch
+
+        class RolloutCostFunction(torch.autograd.Function):
+            @staticmethod
+            def forward(ctx, mb, q0, dq0, tau, dt, tip, weights):
+                for name, t in (("q0", q0), ("dq0", dq0), ("tau", tau)):
+                    if not (_is_torch(t) and t.is_cuda and t.dtype == torch.float64):
+                        raise TypeError(f"rollout_cost_autograd: {name} must be a CUDA float64 tensor")
+                q0, dq0, tau = q0.contiguous(), dq0.contiguous(), tau.contiguous()
+                if any(ctx.needs_input_grad[1:4]):
+                    cost, gt, gq, gdq = mb.rollout_cost_grad(q0, dq0, tau, dt, tip=tip, **weights)
+                    ctx.save_for_backward(gq, gdq, gt)
+                else:
+                    cost = mb.rollout_cost(q0, dq0, tau, dt, tip=tip, **weights)
+                return cost
+
+            @staticmethod
+            def backward(ctx, g_cost):
+                gq, gdq, gt = ctx.saved_tensors
+                g = g_cost.contiguous()
+                return None, gq * g[None, :], gdq * g[None, :], gt * g[None, None, :], None, None, None
+
+        _ROLLOUT_COST_FN = RolloutCostFunction
+    return _ROLLOUT_COST_FN

@@ -30,6 +30,10 @@ class RbQuadCost(C.Structure):
     _fields_ = [(k, _dp) for k in ("q_ref", "w_q", "w_dq", "w_tau", "w_q_final", "w_dq_final")]
 
 
+class RbTipCost(C.Structure):
+    _fields_ = [(k, _dp) for k in ("offset", "p_ref", "w_p", "w_p_final", "R_ref")] + [("w_R", C.c_double), ("w_R_final", C.c_double)]
+
+
 class RbJointLimits(C.Structure):
     _fields_ = [(k, C.c_double * RB_MAX_JOINTS) for k in ("lower", "upper", "velocity", "effort")]
 
@@ -74,6 +78,10 @@ PROTOTYPES = {
     "multibody_rollout_cost": (_i, [_vp, _vp, _vp, _vp, C.c_double, _i, C.POINTER(RbQuadCost), _vp, _vp, _vp, _sz, _sz, _i, _i, _vp]),
     "multibody_rollout_vjp": (_i, [_vp, _vp, _vp, _vp, C.c_double, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _sz, _i, _i, _vp]),
     "multibody_rollout_cost_grad": (_i, [_vp, _vp, _vp, _vp, C.c_double, _i, C.POINTER(RbQuadCost), _vp, _vp, _vp, _vp, _sz, _sz, _i, _i, _vp]),
+    "multibody_rollout_tip_cost": (_i, [_vp, _vp, _vp, _vp, C.c_double, _i, C.POINTER(RbQuadCost), C.POINTER(RbTipCost), _vp, _vp, _vp,
+                                        _sz, _sz, _i, _i, _vp]),
+    "multibody_rollout_tip_cost_grad": (_i, [_vp, _vp, _vp, _vp, C.c_double, _i, C.POINTER(RbQuadCost), C.POINTER(RbTipCost), _vp, _vp,
+                                             _vp, _vp, _sz, _sz, _i, _i, _vp]),
     "multibody_gpu_fill": (_i, [_vp, _vp, _u64, C.c_uint32, _dp, _dp, _sz, _sz, _sz, _vp]),
     "multibody_gpu_sync": (_i, [_vp]),
     "multibody_gpu_status": (_i, [_vp]),

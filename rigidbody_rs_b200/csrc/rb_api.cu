@@ -124,6 +124,7 @@ struct RbGpu {
     // bound by bind_entries; the optional entries (rnea_aos, fd_aos, rnea_fd, rnea_f32, fd_f32) are the primary family's alone
     Bound<decltype(RbOps::rnea)> rnea; Bound<decltype(RbOps::fd)> fd; Bound<decltype(RbOps::crba)> crba;
     Bound<decltype(RbOps::fwd_kin)> fwd_kin; Bound<decltype(RbOps::jac)> jac; Bound<decltype(RbOps::rollout)> rollout;
+    Bound<decltype(RbOps::rollout_tip)> rollout_tip;
     size_t hpk_states = 0;
     RbJitParam jit{};                     // run-time compiled kernels (jit-specialised family); lib == nullptr if unused
     std::string family_note;              // why this family was chosen (e.g. the JIT fallback reason)
@@ -131,7 +132,7 @@ struct RbGpu {
     double* d_model = nullptr;            // generic-n: model rows on the device
     DevBuf scratch;                       // generic-n: per-thread strided scratch
     DevBuf hpk;                           // generic-n: packed H of one chunk of states (forward dynamics)
-    DevBuf cost_w;                        // rollout cost weights (RB_CW_ROWS x RB_MAX_N doubles), engine-owned: ordered like scratch
+    DevBuf cost_w;                        // rollout cost weights (RB_CW_ROWS_TIP x RB_MAX_N doubles), engine-owned: ordered like scratch
     size_t scratch_threads = 0;
     cudaStream_t stream = nullptr, s_h2d = nullptr, s_d2h = nullptr;
     cudaEvent_t ev_h2d[kSlots] = {}, ev_comp[kSlots] = {}, ev_d2h[kSlots] = {};
@@ -307,7 +308,7 @@ int pick_ops(RbGpu* g) {
     return setup_generic_n(g, &g->param);
 }
 
-// Binds rnea, fd, crba, fwd_kin, jac and rollout once: to the primary family where it has the entry, otherwise to the
+// Binds rnea, fd, crba, fwd_kin, jac, rollout and rollout_tip once: to the primary family where it has the entry, otherwise to the
 // fallback table, whose parameter block pick_ops set up for the families that need it.
 int bind_entries(RbGpu* g) {
     bool ok = true;
@@ -319,6 +320,7 @@ int bind_entries(RbGpu* g) {
     };
     bind(g->rnea, &RbOps::rnea); bind(g->fd, &RbOps::fd); bind(g->crba, &RbOps::crba);
     bind(g->fwd_kin, &RbOps::fwd_kin); bind(g->jac, &RbOps::jac); bind(g->rollout, &RbOps::rollout);
+    bind(g->rollout_tip, &RbOps::rollout_tip);
     return ok ? RB_OK : fail(RB_ERR_ARG, std::string("internal: kernel family '") + g->ops->name + "' leaves an entry point unbound");
 }
 
@@ -359,7 +361,7 @@ int gpu_create(const RbHostModel& model, int device, RbGpu** out) {
     if ((e = cudaMallocHost((void**)&g->h_status, 2 * sizeof(int))) != cudaSuccess) return bail(fail_cuda(e, "cudaMallocHost(status)"));
     g->h_status[0] = g->h_status[1] = 0;
     // cost weights of multibody_rollout_cost: allocated once, here (a lazy first-call allocation would race)
-    { int rcw = g->cost_w.ensure(sizeof(double) * RB_CW_ROWS * RB_MAX_N); if (rcw != RB_OK) return bail(rcw); }
+    { int rcw = g->cost_w.ensure(sizeof(double) * RB_CW_ROWS_TIP * RB_MAX_N); if (rcw != RB_OK) return bail(rcw); }
     int rc = pick_ops(g);
     if (rc == RB_OK) rc = bind_entries(g);
     if (rc != RB_OK) return bail(rc);
@@ -1085,8 +1087,8 @@ int run_staged(RbGpu* g, const std::vector<StagedIn>& ins, const std::vector<Sta
 }
 
 // Checks the weights of an RbQuadCost and packs them into the layout of the engine's cost-weight block (RB_CW_* rows).
-int pack_cost_weights(int n, const RbQuadCost* w, double (&cw)[RB_CW_ROWS * RB_MAX_N]) {
-    memset(cw, 0, sizeof cw);
+int pack_cost_weights(int n, const RbQuadCost* w, double* cw) {
+    memset(cw, 0, sizeof(double) * RB_CW_ROWS * RB_MAX_N);
     const double* rows[RB_CW_ROWS] = {w->q_ref, w->w_q, w->w_dq, w->w_tau, w->w_q_final, w->w_dq_final};
     for (int r = 0; r < RB_CW_ROWS; ++r)
         if (rows[r]) for (int i = 0; i < n; ++i) {
@@ -1096,9 +1098,46 @@ int pack_cost_weights(int n, const RbQuadCost* w, double (&cw)[RB_CW_ROWS * RB_M
     return RB_OK;
 }
 
+// The whole cost-weight block of a cost call: the RB_CW_* rows, and the RB_CW_TIP row when tip terms are on.
+struct CostBlock {
+    double w[RB_CW_ROWS_TIP * RB_MAX_N];
+    bool tip;
+    size_t bytes() const { return sizeof(double) * (tip ? RB_CW_ROWS_TIP : RB_CW_ROWS) * RB_MAX_N; }
+};
+
+// Checks the terms of an RbTipCost and packs them into row RB_CW_TIP (RB_TW_* entries).  `on` = some weight is not
+// zero; a tip cost whose weights are all zero adds nothing, and the call runs as one without tip terms.
+int pack_tip_weights(const RbTipCost* t, double* row, bool* on) {
+    memset(row, 0, sizeof(double) * RB_MAX_N);
+    *on = false;
+    if (!t) return RB_OK;
+    const struct { const double* v; int at, len; bool weight; } parts[] = {
+        {t->offset, RB_TW_OFFSET, 3, false}, {t->p_ref, RB_TW_PREF, 3, false}, {t->w_p, RB_TW_WP, 3, true},
+        {t->w_p_final, RB_TW_WPF, 3, true}, {t->R_ref, RB_TW_RREF, 9, false}, {&t->w_R, RB_TW_WR, 1, true},
+        {&t->w_R_final, RB_TW_WRF, 1, true}};
+    for (const auto& pt : parts) {
+        if (!pt.v) continue;
+        for (int k = 0; k < pt.len; ++k) {
+            const double v = pt.v[k];
+            if (!std::isfinite(v) || (pt.weight && v < 0.0)) return fail(RB_ERR_ARG, "tip cost terms must be finite and its weights non-negative");
+            row[pt.at + k] = v;
+            if (pt.weight && v != 0.0) *on = true;
+        }
+    }
+    if (!t->R_ref) row[RB_TW_RREF] = row[RB_TW_RREF + 4] = row[RB_TW_RREF + 8] = 1.0;
+    return RB_OK;
+}
+
+// Checks and packs both parts of a cost call's weights.
+int pack_cost_block(int n, const RbQuadCost* w, const RbTipCost* tip, CostBlock& cb) {
+    const int rc = pack_cost_weights(n, w, cb.w);
+    if (rc != RB_OK) return rc;
+    return pack_tip_weights(tip, cb.w + RB_CW_TIP * RB_MAX_N, &cb.tip);
+}
+
 int rollout_impl(RbGpu* g, const double* q0, const double* dq0, const double* tau, double dt, int horizon,
-                 double* q_traj, double* dq_traj, double* q_final, double* dq_final, const RbQuadCost* w, double* cost,
-                 size_t n_traj, size_t ld, RbLayout layout, RbMem mem, void* stream, size_t aos_stride = 0) {
+                 double* q_traj, double* dq_traj, double* q_final, double* dq_final, const RbQuadCost* w, const RbTipCost* tip,
+                 double* cost, size_t n_traj, size_t ld, RbLayout layout, RbMem mem, void* stream, size_t aos_stride = 0) {
     if (!g) return fail(RB_ERR_NULL, "engine handle is NULL");
     if (!g->peers.empty()) {
         if (layout != RB_LAYOUT_SOA && layout != RB_LAYOUT_AOS) return fail(RB_ERR_ARG, "bad layout");
@@ -1114,7 +1153,7 @@ int rollout_impl(RbGpu* g, const double* q0, const double* dq0, const double* ta
             auto at = [&](const double* p) { return p ? p + o : nullptr; };
             auto atw = [&](double* p) { return p ? p + o : nullptr; };
             return rollout_impl(g->peers[i], at(q0), at(dq0), at(tau), dt, horizon, atw(q_traj), atw(dq_traj), atw(q_final), atw(dq_final),
-                                w, cost ? cost + lo : nullptr, hi - lo, ld, layout, mem, nullptr, aos ? n_traj * n : 0);
+                                w, tip, cost ? cost + lo : nullptr, hi - lo, ld, layout, mem, nullptr, aos ? n_traj * n : 0);
         });
     }
     if (layout != RB_LAYOUT_SOA && layout != RB_LAYOUT_AOS) return fail(RB_ERR_ARG, "bad layout");
@@ -1132,14 +1171,16 @@ int rollout_impl(RbGpu* g, const double* q0, const double* dq0, const double* ta
     if (!dg.ok) return fail(RB_ERR_CUDA, "cudaSetDevice failed");
     cudaStream_t st = mem == RB_MEM_DEVICE ? (cudaStream_t)stream : g->stream;
     // cost weights -> the engine's device block (shared by all cost rollouts, hence ordered like scratch)
-    double cw[RB_CW_ROWS * RB_MAX_N];
-    if (cost) { const int rc = pack_cost_weights(n, w, cw); if (rc != RB_OK) return rc; }
-    const bool shared = cost != nullptr || g->rollout.shared;
+    CostBlock cb;
+    cb.tip = false;
+    if (cost) { const int rc = pack_cost_block(n, w, tip, cb); if (rc != RB_OK) return rc; }
+    const auto& ro = cb.tip ? g->rollout_tip : g->rollout;
+    const bool shared = cost != nullptr || ro.shared;
     if (mem == RB_MEM_DEVICE && layout == RB_LAYOUT_SOA) {
         ScratchOrder so(g, shared, st);
-        if (cost) RB_CUDA(cudaMemcpyAsync(g->cost_w.p, cw, sizeof cw, cudaMemcpyHostToDevice, st));
-        cudaError_t e = g->rollout.fn(g->rollout.param, q0, dq0, tau, dt, horizon, q_traj, dq_traj, q_final, dq_final,
-                                      n_traj, ld, g->d_status, cost ? g->cost_w.p : nullptr, cost, st);
+        if (cost) RB_CUDA(cudaMemcpyAsync(g->cost_w.p, cb.w, cb.bytes(), cudaMemcpyHostToDevice, st));
+        cudaError_t e = ro.fn(ro.param, q0, dq0, tau, dt, horizon, q_traj, dq_traj, q_final, dq_final,
+                              n_traj, ld, g->d_status, cost ? g->cost_w.p : nullptr, cost, st);
         g->launches += 1;
         if (e != cudaSuccess) return fail_cuda(e, "rollout launch");
         return RB_OK;
@@ -1151,9 +1192,9 @@ int rollout_impl(RbGpu* g, const double* q0, const double* dq0, const double* ta
         cudaError_t e;
         {
             ScratchOrder so(g, shared, st);
-            if (cost) RB_CUDA(cudaMemcpyAsync(g->cost_w.p, cw, sizeof cw, cudaMemcpyHostToDevice, st));
-            e = g->rollout.fn(g->rollout.param, in[0], in[1], in[2], dt, horizon, out[0], out[1], out[2], out[3], n_traj, n_traj, d_stat,
-                              cost ? g->cost_w.p : nullptr, out[4], st);
+            if (cost) RB_CUDA(cudaMemcpyAsync(g->cost_w.p, cb.w, cb.bytes(), cudaMemcpyHostToDevice, st));
+            e = ro.fn(ro.param, in[0], in[1], in[2], dt, horizon, out[0], out[1], out[2], out[3], n_traj, n_traj, d_stat,
+                      cost ? g->cost_w.p : nullptr, out[4], st);
         }
         g->launches += 1;
         if (e != cudaSuccess) return fail_cuda(e, "rollout launch");
@@ -1166,6 +1207,7 @@ struct GradArgs {
     const double *q_traj, *dq_traj, *g_q, *g_dq, *g_qf, *g_dqf;
     const RbQuadCost* w; double* cost;
     double *grad_tau, *grad_q0, *grad_dq0;
+    const RbTipCost* tip = nullptr;       // multibody_rollout_tip_cost_grad
 };
 
 // The trajectory workspace of one chunk of a cost-gradient call, 2 H n doubles per trajectory, stays within this.
@@ -1175,7 +1217,7 @@ constexpr size_t kGradWorkspace = (size_t)1 << 30;
 // engine's rollout launcher (so that its cost is multibody_rollout_cost's, bit for bit) into a stream-ordered workspace,
 // then the adjoint over the stored trajectory, chunk by chunk; the weight upload and every launch sit in one ScratchOrder
 // region because the weight block is shared by all cost rollouts on the engine.
-int grad_device(RbGpu* g, const GradArgs& a, const double* cw, size_t B, size_t ld, cudaStream_t st, int* d_stat) {
+int grad_device(RbGpu* g, const GradArgs& a, const CostBlock& cb, size_t B, size_t ld, cudaStream_t st, int* d_stat) {
     const int n = g->model.n;
     RbAdjointArgs ad{a.q0, a.dq0, a.tau, a.q_traj, a.dq_traj, ld, a.g_q, a.g_dq, a.g_qf, a.g_dqf, nullptr,
                      a.grad_tau, a.grad_q0, a.grad_dq0, a.dt, a.horizon};
@@ -1185,8 +1227,10 @@ int grad_device(RbGpu* g, const GradArgs& a, const double* cw, size_t B, size_t 
         return e == cudaSuccess ? RB_OK : fail_cuda(e, "rollout adjoint launch");
     }
     ScratchOrder so(g, true, st);
-    RB_CUDA(cudaMemcpyAsync(g->cost_w.p, cw, sizeof(double) * RB_CW_ROWS * RB_MAX_N, cudaMemcpyHostToDevice, st));
+    RB_CUDA(cudaMemcpyAsync(g->cost_w.p, cb.w, cb.bytes(), cudaMemcpyHostToDevice, st));
     ad.cost_w = g->cost_w.p;
+    ad.tip = cb.tip;
+    const auto& ro = cb.tip ? g->rollout_tip : g->rollout;
     const size_t H = (size_t)a.horizon, nn = (size_t)n;
     // A rollout writes its trajectory with the leading dimension of its inputs: a chunk whose inputs are not already a
     // dense [n][chunk] block (a cut batch, a padded ld) gets a dense copy of them next to its trajectory.
@@ -1213,8 +1257,7 @@ int grad_device(RbGpu* g, const GradArgs& a, const double* cw, size_t B, size_t 
             if (e != cudaSuccess) { rc = fail_cuda(e, "cudaMemcpy2DAsync(gradient workspace)"); break; }
             rq0 = in; rdq0 = in + nn * cnt; rtau = in + 2 * nn * cnt;
         }
-        e = g->rollout.fn(g->rollout.param, rq0, rdq0, rtau, a.dt, a.horizon, qt, dqt, nullptr, nullptr, cnt, lw, d_stat,
-                          g->cost_w.p, a.cost + lo, st);
+        e = ro.fn(ro.param, rq0, rdq0, rtau, a.dt, a.horizon, qt, dqt, nullptr, nullptr, cnt, lw, d_stat, g->cost_w.p, a.cost + lo, st);
         g->launches += 1;
         if (e != cudaSuccess) { rc = fail_cuda(e, "rollout launch"); break; }
         RbAdjointArgs c = ad;
@@ -1264,19 +1307,20 @@ int grad_impl(RbGpu* g, const GradArgs& a, size_t n_traj, size_t ld, RbLayout la
     const size_t H = (size_t)a.horizon;
     if (!a.q0 || !a.dq0 || (H > 0 && (!a.tau || (!cost && (!a.q_traj || !a.dq_traj))))) return fail(RB_ERR_NULL, "input pointer is NULL");
     if (layout == RB_LAYOUT_SOA) { if (ld == 0) ld = n_traj; if (ld < n_traj) return fail(RB_ERR_ARG, "ld < n_traj"); }
-    double cw[RB_CW_ROWS * RB_MAX_N];
-    if (cost) { const int rc = pack_cost_weights(g->model.n, a.w, cw); if (rc != RB_OK) return rc; }
+    CostBlock cb;
+    cb.tip = false;
+    if (cost) { const int rc = pack_cost_block(g->model.n, a.w, a.tip, cb); if (rc != RB_OK) return rc; }
     if (!cost && !a.grad_tau && !a.grad_q0 && !a.grad_dq0) return RB_OK;
     DeviceGuard dg(g->device);
     if (!dg.ok) return fail(RB_ERR_CUDA, "cudaSetDevice failed");
     cudaStream_t st = mem == RB_MEM_DEVICE ? (cudaStream_t)stream : g->stream;
-    if (mem == RB_MEM_DEVICE && layout == RB_LAYOUT_SOA) return grad_device(g, a, cw, n_traj, ld, st, g->d_status);
+    if (mem == RB_MEM_DEVICE && layout == RB_LAYOUT_SOA) return grad_device(g, a, cb, n_traj, ld, st, g->d_status);
     // Host pointers and/or AoS: staged like the rollout; the staged call then runs as a device SoA call with ld = n_traj.
     return run_staged(g, {{a.q0, 1}, {a.dq0, 1}, {a.tau, H}, {a.q_traj, H}, {a.dq_traj, H}, {a.g_q, H}, {a.g_dq, H}, {a.g_qf, 1}, {a.g_dqf, 1}},
                       {{a.grad_tau, H, false}, {a.grad_q0, 1, false}, {a.grad_dq0, 1, false}, {a.cost, 1, true}},
                       n_traj, ld, layout, mem, aos_stride, st, [&](const double* const* in, double* const* out, int* d_stat) -> int {
-        const GradArgs s{in[0], in[1], in[2], a.dt, a.horizon, in[3], in[4], in[5], in[6], in[7], in[8], a.w, out[3], out[0], out[1], out[2]};
-        return grad_device(g, s, cw, n_traj, n_traj, st, d_stat);
+        const GradArgs s{in[0], in[1], in[2], a.dt, a.horizon, in[3], in[4], in[5], in[6], in[7], in[8], a.w, out[3], out[0], out[1], out[2], a.tip};
+        return grad_device(g, s, cb, n_traj, n_traj, st, d_stat);
     });
 }
 }  // namespace
@@ -1284,14 +1328,23 @@ int grad_impl(RbGpu* g, const GradArgs& a, size_t n_traj, size_t ld, RbLayout la
 extern "C" int multibody_rollout(RbGpu* g, const double* q0, const double* dq0, const double* tau, double dt, int horizon,
                                  double* q_traj, double* dq_traj, double* q_final, double* dq_final,
                                  size_t n_traj, size_t ld, RbLayout layout, RbMem mem, void* stream) {
-    return rollout_impl(g, q0, dq0, tau, dt, horizon, q_traj, dq_traj, q_final, dq_final, nullptr, nullptr, n_traj, ld, layout, mem, stream);
+    return rollout_impl(g, q0, dq0, tau, dt, horizon, q_traj, dq_traj, q_final, dq_final, nullptr, nullptr, nullptr, n_traj, ld, layout, mem, stream);
 }
 
 extern "C" int multibody_rollout_cost(RbGpu* g, const double* q0, const double* dq0, const double* tau, double dt, int horizon,
                                       const RbQuadCost* weights, double* cost, double* q_final, double* dq_final,
                                       size_t n_traj, size_t ld, RbLayout layout, RbMem mem, void* stream) {
     if (!cost) return fail(RB_ERR_NULL, "cost output pointer is NULL");
-    return rollout_impl(g, q0, dq0, tau, dt, horizon, nullptr, nullptr, q_final, dq_final, weights, cost, n_traj, ld, layout, mem, stream);
+    return rollout_impl(g, q0, dq0, tau, dt, horizon, nullptr, nullptr, q_final, dq_final, weights, nullptr, cost, n_traj, ld, layout, mem, stream);
+}
+
+extern "C" int multibody_rollout_tip_cost(RbGpu* g, const double* q0, const double* dq0, const double* tau, double dt, int horizon,
+                                          const RbQuadCost* weights, const RbTipCost* tip, double* cost, double* q_final, double* dq_final,
+                                          size_t n_traj, size_t ld, RbLayout layout, RbMem mem, void* stream) {
+    if (!cost) return fail(RB_ERR_NULL, "cost output pointer is NULL");
+    const RbQuadCost none{};
+    return rollout_impl(g, q0, dq0, tau, dt, horizon, nullptr, nullptr, q_final, dq_final, weights ? weights : &none, tip, cost,
+                        n_traj, ld, layout, mem, stream);
 }
 
 extern "C" int multibody_rollout_vjp(RbGpu* g, const double* q0, const double* dq0, const double* tau, double dt, int horizon,
@@ -1311,6 +1364,17 @@ extern "C" int multibody_rollout_cost_grad(RbGpu* g, const double* q0, const dou
     if (!cost) return fail(RB_ERR_NULL, "cost output pointer is NULL");
     const GradArgs a{q0, dq0, tau, dt, horizon, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, weights, cost,
                      grad_tau, grad_q0, grad_dq0};
+    return grad_impl(g, a, n_traj, ld, layout, mem, stream);
+}
+
+extern "C" int multibody_rollout_tip_cost_grad(RbGpu* g, const double* q0, const double* dq0, const double* tau, double dt, int horizon,
+                                               const RbQuadCost* weights, const RbTipCost* tip, double* cost, double* grad_tau,
+                                               double* grad_q0, double* grad_dq0, size_t n_traj, size_t ld, RbLayout layout, RbMem mem,
+                                               void* stream) {
+    if (!cost) return fail(RB_ERR_NULL, "cost output pointer is NULL");
+    const RbQuadCost none{};
+    const GradArgs a{q0, dq0, tau, dt, horizon, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, weights ? weights : &none, cost,
+                     grad_tau, grad_q0, grad_dq0, tip};
     return grad_impl(g, a, n_traj, ld, layout, mem, stream);
 }
 

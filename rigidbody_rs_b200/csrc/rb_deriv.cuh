@@ -265,6 +265,59 @@ RB_DI void rb_rnea_derivatives(const RbModelK<N>& p, const double* sn, const dou
     }
 }
 
+// ---- tip-pose cost terms (RbTipCost) of a state whose last link has the world pose (Rl, P)
+// With R = Rl tip (the tip frame), x = P + R offset, e = x - p_ref, the terms a (running) and b (terminal) times
+//   sum_k W_k e_k^2 + w ||R - R_ref||_F^2,   W = a w_p + b w_p_final,  w = a w_R + b w_R_final,
+// change with joint j's angle at the rate s_j . (n ; f) for the joint's world screw s_j = (z_j ; P_j x z_j) and the world
+// wrench (moment about the origin ; force)
+//   f = 2 W e,   n = x x f + 2 w sum_k R_ref[:,k] x R[:,k]
+// (dx = z_j x (x - P_j) dq_j,  dR = [z_j]x R dq_j,  ||R - R_ref||^2 = 6 - 2 tr(R_ref^T R)).  No Jacobian is formed.
+RB_DI void rb_tip_wrench(const double (&Rl)[3][3], const double (&P)[3], const double* tip, const double* __restrict__ tw,
+                         double a, double b, double (&w)[6]) {
+    auto c = [&](int k) { return __ldg(tw + k); };
+    double R[3][3], x[3], f[3], nm[3];
+#pragma unroll
+    for (int r = 0; r < 3; ++r)
+#pragma unroll
+        for (int k = 0; k < 3; ++k) R[r][k] = fma(Rl[r][2], tip[6 + k], fma(Rl[r][1], tip[3 + k], Rl[r][0] * tip[k]));
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        x[k] = fma(R[k][2], c(RB_TW_OFFSET + 2), fma(R[k][1], c(RB_TW_OFFSET + 1), fma(R[k][0], c(RB_TW_OFFSET), P[k])));
+        const double W = fma(b, c(RB_TW_WPF + k), a * c(RB_TW_WP + k));
+        f[k] = 2.0 * (W * (x[k] - c(RB_TW_PREF + k)));
+    }
+    rb_cross3(x, f, nm);
+    const double wr2 = 2.0 * fma(b, c(RB_TW_WRF), a * c(RB_TW_WR));
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        const double rr[3] = {c(RB_TW_RREF + k), c(RB_TW_RREF + 3 + k), c(RB_TW_RREF + 6 + k)}, rk[3] = {R[0][k], R[1][k], R[2][k]};
+        double t[3];
+        rb_cross3(rr, rk, t);
+#pragma unroll
+        for (int r = 0; r < 3; ++r) nm[r] = fma(wr2, t[r], nm[r]);
+    }
+    w[0] = nm[0]; w[1] = nm[1]; w[2] = nm[2]; w[3] = f[0]; w[4] = f[1]; w[5] = f[2];
+}
+
+// gq[j] += the derivative of those terms (a running, b terminal) at one state, one sweep out (pose of the last link) and
+// one back (the screws).
+template <int N>
+RB_DI void rb_tip_grad(const RbModelK<N>& p, const double* sn, const double* cs, const double* tw, double a, double b, double* gq) {
+    double R[3][3] = {{1.0, 0.0, 0.0}, {0.0, 1.0, 0.0}, {0.0, 0.0, 1.0}}, P[3] = {0.0, 0.0, 0.0};
+#pragma unroll 1
+    for (int i = 0; i < N; ++i) rb_pose_out(p.jt[i], sn[i], cs[i], R, P);
+    double w[6];
+    rb_tip_wrench(R, P, p.tip, tw, a, b, w);
+#pragma unroll 1
+    for (int i = N - 1; i >= 0; --i) {
+        const double z[3] = {R[0][2], R[1][2], R[2][2]};
+        double pz[3];
+        rb_cross3(P, z, pz);
+        gq[i] += fma(z[0], w[0], fma(z[1], w[1], fma(z[2], w[2], fma(pz[0], w[3], fma(pz[1], w[4], pz[2] * w[5])))));
+        if (i > 0) rb_pose_back(p.jt[i], sn[i], cs[i], R, P);
+    }
+}
+
 // Vector-Jacobian product of inverse dynamics in O(N), SUBTRACTED from gq and gdq (the adjoints a caller accumulates):
 //   gq_j  -= (mu^T d tau / d q )_j = Sbar_j . G_j  +   da0_j . Abar_j + dv_j . Bbar_j
 //   gdq_j -= (mu^T d tau / d dq)_j = Sbar_j . G'_j + 2 dv_j . Abar_j +  s_j . Bbar_j
@@ -273,9 +326,11 @@ RB_DI void rb_rnea_derivatives(const RbModelK<N>& p, const double* sn, const dou
 // sweep carries Abar and Bbar and takes each joint's term out of Sbar after using it, so the pair walk-back of
 // rb_rnea_derivatives becomes one step back per joint.  Like sn, cs, dq, ddq and mu, gq and gdq are indexed at run
 // time (thread-local memory): a caller's adjoints do not occupy registers across the sweeps.
-template <int N>
+// TIP with tip_a != 0 also ADDS the running tip-pose terms' derivative (rb_tip_wrench, weight tip_a, row tw) at this
+// state to gq: the wrench from the outward sweep's last-link pose, projected on each screw the inward sweep forms.
+template <int N, bool TIP = false>
 RB_DI void rb_rnea_vjp(const RbModelK<N>& p, const double* sn, const double* cs, const double* dq, const double* ddq,
-                       const double* mu, double* gq, double* gdq) {
+                       const double* mu, double* gq, double* gdq, const double* tw = nullptr, double tip_a = 0.0) {
     double R[3][3] = {{1.0, 0.0, 0.0}, {0.0, 1.0, 0.0}, {0.0, 0.0, 1.0}}, P[3] = {0.0, 0.0, 0.0};
     double v[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
     double a[6] = {0.0, 0.0, 0.0, p.g[0], p.g[1], p.g[2]};
@@ -285,6 +340,12 @@ RB_DI void rb_rnea_vjp(const RbModelK<N>& p, const double* sn, const double* cs,
 #pragma unroll
         for (int k = 0; k < 6; ++k) Sb[k] = fma(mi, s6[k], Sb[k]);
     });
+    double wt[6];
+    bool tip = false;
+    if constexpr (TIP) {
+        tip = tip_a != 0.0;
+        if (tip) rb_tip_wrench(R, P, p.tip, tw, tip_a, 0.0, wt);
+    }
     RbDerivComposites C = {};
     double Ab[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0}, Bb[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
 #pragma unroll 1
@@ -292,6 +353,7 @@ RB_DI void rb_rnea_vjp(const RbModelK<N>& p, const double* sn, const double* cs,
         double sI[6], dvI[6], daI[6], A[6], Bv[6], G[6], Gp[6];
         rb_deriv_inward(p.jt[i], R, P, v, a, C, sI, dvI, daI, A, Bv, G, Gp);
         gq[i] -= rb_dot6(Sb, G) + (rb_dot6(daI, Ab) + rb_dot6(dvI, Bb));
+        if constexpr (TIP) { if (tip) gq[i] += rb_dot6(sI, wt); }
         gdq[i] -= rb_dot6(Sb, Gp) + fma(2.0, rb_dot6(dvI, Ab), rb_dot6(sI, Bb));
         const double mi = mu[i];
 #pragma unroll

@@ -77,6 +77,7 @@ struct RtModel {
     template <int K> static constexpr int gcls() { return RB_GEN; }
     template <int K> static RB_DI Real g(const Param& p) { return (Real)p.g[K]; }
     template <int K> static RB_DI Real tip(const Param& p) { return (Real)p.tip[K]; }
+    template <int K> static constexpr int tipcls() { return RB_GEN; }
     static constexpr bool kTree = false;     // run-time constants: serial chains only
     template <int I> static constexpr int parent() { return I - 1; }
 };
@@ -103,6 +104,7 @@ struct CtModel {
     template <int K> static constexpr int gcls() { return rb_classify(Tab::G[K]); }
     template <int K> static RB_DI Real g(const Param&) { constexpr Real v = (Real)Tab::G[K]; return v; }
     template <int K> static RB_DI Real tip(const Param&) { constexpr Real v = (Real)Tab::TIP[K]; return v; }
+    template <int K> static constexpr int tipcls() { return rb_classify(Tab::TIP[K]); }
     // parent link of joint I (slot 23 of the row); a table whose joints do not all hang off their predecessor is a
     // kinematic tree and takes the rb_*_tree forms (rb_dyn_tree.cuh)
     template <int I> static constexpr int parent() { return (int)Tab::T[I][23]; }
@@ -696,3 +698,75 @@ RB_DI void rb_jac(const typename M::Param& p, const RB_R (&s)[M::N], const RB_R 
 }
 
 #include "rb_dyn_tree.cuh"
+
+// ------------------------------------------------------------------ tip pose (tip-pose cost terms of rollouts)
+// Orientation R of the tip frame in the base frame (the frame of rb_jac: the reference's last link frame, tip rotation
+// included) and its origin pos (rb_fwd_kin's result, the same operations).  Composed tip -> base along the supporting
+// branch (the whole chain for serial chains): A <- R_p Rz A; the last joint's factor starts from the identity and the
+// tip rotation is applied at the end, so the exact 0 and +-1 of the fixed rotations drop out of every product.
+template <class M>
+RB_DI void rb_tip_pose(const typename M::Param& p, const RB_R (&s)[M::N], const RB_R (&c)[M::N], RB_R (&R)[3][3], RB_R (&pos)[3]) {
+    constexpr int N = M::N;
+    RB_R A[3][3];
+    pos[0] = 0.0; pos[1] = 0.0; pos[2] = 0.0;
+    rb_for_anc<M, N - 1>([&](auto ic) {
+        constexpr int I = decltype(ic)::value;
+        const RB_R y0 = fma(c[I], pos[0], -(s[I] * pos[1])), y1 = fma(s[I], pos[0], c[I] * pos[1]), y2 = pos[2];
+        pos[0] = k_dot3_acc<KC(I, RB_F_R, 0), KC(I, RB_F_R, 1), KC(I, RB_F_R, 2)>(KV(I, RB_F_T, 0), KV(I, RB_F_R, 0), KV(I, RB_F_R, 1), KV(I, RB_F_R, 2), y0, y1, y2);
+        pos[1] = k_dot3_acc<KC(I, RB_F_R, 3), KC(I, RB_F_R, 4), KC(I, RB_F_R, 5)>(KV(I, RB_F_T, 1), KV(I, RB_F_R, 3), KV(I, RB_F_R, 4), KV(I, RB_F_R, 5), y0, y1, y2);
+        pos[2] = k_dot3_acc<KC(I, RB_F_R, 6), KC(I, RB_F_R, 7), KC(I, RB_F_R, 8)>(KV(I, RB_F_T, 2), KV(I, RB_F_R, 6), KV(I, RB_F_R, 7), KV(I, RB_F_R, 8), y0, y1, y2);
+        if constexpr (I == N - 1) {
+            // A = R_p Rz(q): columns (c r0 + s r1, c r1 - s r0, r2) of R_p's rows r
+            rb_for_up<0, 3>([&](auto rc) {
+                constexpr int r = decltype(rc)::value;
+                A[r][0] = k_dot3<KC(I, RB_F_R, 3 * r), KC(I, RB_F_R, 3 * r + 1), RB_ZERO>(KV(I, RB_F_R, 3 * r), KV(I, RB_F_R, 3 * r + 1), RB_R(0), c[I], s[I], RB_R(0));
+                A[r][1] = k_dot3<KC(I, RB_F_R, 3 * r + 1), KC(I, RB_F_R, 3 * r), RB_ZERO>(KV(I, RB_F_R, 3 * r + 1), KV(I, RB_F_R, 3 * r), RB_R(0), c[I], -s[I], RB_R(0));
+                A[r][2] = KV(I, RB_F_R, 3 * r + 2);
+            });
+        } else {
+            RB_R B[3][3];
+#pragma unroll
+            for (int k = 0; k < 3; ++k) {
+                B[0][k] = fma(c[I], A[0][k], -(s[I] * A[1][k]));
+                B[1][k] = fma(s[I], A[0][k], c[I] * A[1][k]);
+                B[2][k] = A[2][k];
+            }
+#pragma unroll
+            for (int k = 0; k < 3; ++k) {
+                A[0][k] = k_dot3<KC(I, RB_F_R, 0), KC(I, RB_F_R, 1), KC(I, RB_F_R, 2)>(KV(I, RB_F_R, 0), KV(I, RB_F_R, 1), KV(I, RB_F_R, 2), B[0][k], B[1][k], B[2][k]);
+                A[1][k] = k_dot3<KC(I, RB_F_R, 3), KC(I, RB_F_R, 4), KC(I, RB_F_R, 5)>(KV(I, RB_F_R, 3), KV(I, RB_F_R, 4), KV(I, RB_F_R, 5), B[0][k], B[1][k], B[2][k]);
+                A[2][k] = k_dot3<KC(I, RB_F_R, 6), KC(I, RB_F_R, 7), KC(I, RB_F_R, 8)>(KV(I, RB_F_R, 6), KV(I, RB_F_R, 7), KV(I, RB_F_R, 8), B[0][k], B[1][k], B[2][k]);
+            }
+        }
+    });
+    // R = A tip
+    rb_for_up<0, 3>([&](auto kc) {
+        constexpr int k = decltype(kc)::value;
+        constexpr int T0 = M::template tipcls<k>(), T1 = M::template tipcls<3 + k>(), T2 = M::template tipcls<6 + k>();
+#pragma unroll
+        for (int r = 0; r < 3; ++r)
+            R[r][k] = k_dot3<T0, T1, T2>(M::template tip<k>(p), M::template tip<3 + k>(p), M::template tip<6 + k>(p), A[r][0], A[r][1], A[r][2]);
+    });
+}
+
+// The tip-pose terms of RbTipCost at one state whose tip pose is (R, pos); tw = their row of the cost-weight block
+// (RB_TW_* entries).  With x = pos + R offset and e = x - p_ref:
+//   run = sum_k w_p[k] e_k^2 + w_R ||R - R_ref||_F^2,   fin = the same with w_p_final, w_R_final.
+RB_DI void rb_tip_terms(const double (&R)[3][3], const double (&pos)[3], const double* __restrict__ tw, double& run, double& fin) {
+    auto w = [&](int k) { return __ldg(tw + k); };
+    double ep = 0.0, epf = 0.0, dR = 0.0;
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        const double x = fma(R[k][2], w(RB_TW_OFFSET + 2), fma(R[k][1], w(RB_TW_OFFSET + 1), fma(R[k][0], w(RB_TW_OFFSET), pos[k])));
+        const double e = x - w(RB_TW_PREF + k);
+        ep = fma(w(RB_TW_WP + k) * e, e, ep);
+        epf = fma(w(RB_TW_WPF + k) * e, e, epf);
+#pragma unroll
+        for (int j = 0; j < 3; ++j) {
+            const double d = R[k][j] - w(RB_TW_RREF + 3 * k + j);
+            dR = fma(d, d, dR);
+        }
+    }
+    run = fma(w(RB_TW_WR), dR, ep);
+    fin = fma(w(RB_TW_WRF), dR, epf);
+}

@@ -313,3 +313,34 @@ RB_DI bool rbn_ldlt_solve(int n, const RbScratch& Hs, const RbScratch& x, const 
     }
     return ok;
 }
+
+// Tip frame in the base frame (rb_tip_pose with run-time n): A <- R_p Rz(q_i) A, r <- R_p Rz(q_i) r + t_i from the last
+// link down its supporting branch, starting from A = the model's tip rotation `tip` and r = 0.  sincos(i, &s, &c) gives
+// joint i's sin/cos; col(i, A, r) sees the pose of the tip in frame i before joint i's step (the Jacobian's column i).
+template <class SinCos, class Col>
+RB_DI void rbn_tip_pose(const RbJointK* jt, const double* tip, int n, SinCos&& sincos_i, Col&& col, double (&A)[3][3],
+                        double (&r)[3]) {
+#pragma unroll
+    for (int k = 0; k < 3; ++k) { A[k][0] = tip[3 * k]; A[k][1] = tip[3 * k + 1]; A[k][2] = tip[3 * k + 2]; r[k] = 0.0; }
+    for (int i = n - 1; i >= 0; i = (int)jt[i].parent) {
+        const RbJointK& j = jt[i];
+        col(i, A, r);
+        double sn, cs;
+        sincos_i(i, &sn, &cs);
+        double Bm[3][3], y[3];
+#pragma unroll
+        for (int k = 0; k < 3; ++k) {
+            Bm[0][k] = fma(cs, A[0][k], -(sn * A[1][k]));
+            Bm[1][k] = fma(sn, A[0][k], cs * A[1][k]);
+            Bm[2][k] = A[2][k];
+        }
+        y[0] = fma(cs, r[0], -(sn * r[1])); y[1] = fma(sn, r[0], cs * r[1]); y[2] = r[2];
+#pragma unroll
+        for (int a = 0; a < 3; ++a) {
+#pragma unroll
+            for (int k = 0; k < 3; ++k)
+                A[a][k] = fma(j.R[3 * a + 2], Bm[2][k], fma(j.R[3 * a + 1], Bm[1][k], j.R[3 * a] * Bm[0][k]));
+            r[a] = fma(j.R[3 * a + 2], y[2], fma(j.R[3 * a + 1], y[1], fma(j.R[3 * a], y[0], j.t[a])));
+        }
+    }
+}

@@ -74,6 +74,10 @@ struct RbOps {
     cudaError_t (*rollout)(const void* param, const double* q0, const double* dq0, const double* tau, double dt,
                            int horizon, double* q_traj, double* dq_traj, double* q_fin, double* dq_fin,
                            size_t B, size_t ld, int* status, const double* cost_w, double* cost, cudaStream_t st);
+    // the same rollout with the tip-pose terms of RbTipCost added to the cost (cost_w carries the RB_CW_TIP row)
+    cudaError_t (*rollout_tip)(const void* param, const double* q0, const double* dq0, const double* tau, double dt,
+                               int horizon, double* q_traj, double* dq_traj, double* q_fin, double* dq_fin,
+                               size_t B, size_t ld, int* status, const double* cost_w, double* cost, cudaStream_t st);
     // optional fp32 mode (BASELINE.json: "an optional fp32 mode is held to a stated 1e-4 tolerance"): the same kernels
     // instantiated with Real = float, device-resident SoA batches only (null = family has no fp32 kernels)
     cudaError_t (*rnea_f32)(const void* param, const float* q, const float* dq, const float* ddq, float* tau,
@@ -306,11 +310,17 @@ rb_jac_kernel(const __grid_constant__ typename M::Param p, const RB_R* __restric
 
 // MPC rollout (SURVEY.md a14): the trajectory's (q, dq) stay in registers for the whole horizon; per step the
 // kernel reads tau[t] (n doubles) and writes the new (q, dq) (2n doubles).
+// TIP adds the tip-pose terms of RbTipCost (row RB_CW_TIP of cost_w).  The pose of q_t needs sin/cos of q_t, which step t
+// computes for forward dynamics anyway: the running term of q_t is added at the top of step t (t >= 1) from that step's
+// sin/cos, and only q_H takes one more sin/cos after the last step (running and terminal term from one pose).  Computing
+// the pose of q_{t+1} right after the integration would pay a second sin/cos of every joint per step instead.
 #ifndef RB_MINB_ROLLOUT
 #define RB_MINB_ROLLOUT 2   // measured on B200 (profiles/r1_kbench_rollout.jsonl): 255 regs, 2 blocks per SM is fastest
 #endif
 // Rows of the cost-weight block a rollout may carry: cost_w[row * RB_MAX_N + joint] (see RbQuadCost in rigidbody.h).
 enum : int { RB_CW_QREF = 0, RB_CW_Q, RB_CW_DQ, RB_CW_TAU, RB_CW_QF, RB_CW_DQF, RB_CW_ROWS };
+// ... and behind them the tip-pose terms of RbTipCost (RB_TW_* entries of one row, rb_model.h)
+enum : int { RB_CW_TIP = RB_CW_ROWS, RB_CW_ROWS_TIP };
 #ifndef RB_ROLLOUT_WS
 #define RB_ROLLOUT_WS 0
 #endif
@@ -321,7 +331,7 @@ enum : int { RB_CW_QREF = 0, RB_CW_Q, RB_CW_DQ, RB_CW_TAU, RB_CW_QF, RB_CW_DQF, 
 #ifndef RB_RO_MINB
 #define RB_RO_MINB (RB_MINB_ROLLOUT * (128 / RB_RO_BLOCK))
 #endif
-template <class M>
+template <class M, bool TIP = false>
 __global__ void __launch_bounds__(RB_RO_BLOCK, RB_RO_MINB)
 rb_rollout_kernel(const __grid_constant__ typename M::Param p, const RB_R* __restrict__ q0, const RB_R* __restrict__ dq0,
                   const RB_R* __restrict__ tau, RB_R dt, int horizon, RB_R* __restrict__ q_traj,
@@ -344,6 +354,14 @@ rb_rollout_kernel(const __grid_constant__ typename M::Param p, const RB_R* __res
         // prefetch the next step's torques so the load latency hides behind this step's arithmetic
         if (t + 1 < horizon) rb_load<N>(tau + (size_t)(t + 1) * step, ld, s, un);
         rb_sincos_all<N>(q, sn, cs);
+        if constexpr (TIP) {
+            if (t > 0) {                               // running tip terms of q_t
+                RB_R R[3][3], pos[3], run, fin;
+                rb_tip_pose<M>(p, sn, cs, R, pos);
+                rb_tip_terms(R, pos, cost_w + RB_CW_TIP * RB_MAX_N, run, fin);
+                J = fma(dt, run, J);
+            }
+        }
         ok = rb_forward_dynamics<M>(p, sn, cs, dq, u, qdd) && ok;
 #pragma unroll
         for (int i = 0; i < N; ++i) {
@@ -374,6 +392,14 @@ rb_rollout_kernel(const __grid_constant__ typename M::Param p, const RB_R* __res
             const RB_R e = q[i] - __ldg(cost_w + RB_CW_QREF * RB_MAX_N + i);
             J = fma(__ldg(cost_w + RB_CW_QF * RB_MAX_N + i) * e, e, J);
             J = fma(__ldg(cost_w + RB_CW_DQF * RB_MAX_N + i) * dq[i], dq[i], J);
+        }
+        if constexpr (TIP) {                           // q_H: its running term (horizon > 0) and the terminal term
+            RB_R sn[N], cs[N], R[3][3], pos[3], run, fin;
+            rb_sincos_all<N>(q, sn, cs);
+            rb_tip_pose<M>(p, sn, cs, R, pos);
+            rb_tip_terms(R, pos, cost_w + RB_CW_TIP * RB_MAX_N, run, fin);
+            if (horizon > 0) J = fma(dt, run, J);
+            J += fin;
         }
         __stcs(cost + s, ok ? J : rb_nan<RB_R>());
     }
@@ -475,6 +501,14 @@ struct RbLaunch {
             *(const P*)param, q0, dq0, tau, dt, horizon, q_traj, dq_traj, q_fin, dq_fin, B, ld, status, cost_w, cost);
         return cudaGetLastError();
     }
+    static cudaError_t rollout_tip(const void* param, const double* q0, const double* dq0, const double* tau, double dt,
+                                   int horizon, double* q_traj, double* dq_traj, double* q_fin, double* dq_fin,
+                                   size_t B, size_t ld, int* status, const double* cost_w, double* cost, cudaStream_t st) {
+        if (B == 0) return cudaSuccess;
+        rb_rollout_kernel<M, true><<<(unsigned)((B + RB_RO_BLOCK - 1) / RB_RO_BLOCK), RB_RO_BLOCK, 0, st>>>(
+            *(const P*)param, q0, dq0, tau, dt, horizon, q_traj, dq_traj, q_fin, dq_fin, B, ld, status, cost_w, cost);
+        return cudaGetLastError();
+    }
     // M32 = the same policy with Real = float (fp32 mode)
     template <class M32>
     static cudaError_t rnea_f32(const void* param, const float* q, const float* dq, const float* ddq, float* tau,
@@ -495,7 +529,8 @@ struct RbLaunch {
         RbOps o{};
         o.name = name; o.param_bytes = sizeof(P);
         o.rnea = &rnea; o.fd = &fd; o.rnea_aos = &rnea_aos; o.fd_aos = &fd_aos;
-        o.crba = &crba; o.fwd_kin = &fwd_kin; o.jac = &jac; o.rollout = &rollout; o.rnea_fd = &rnea_fd;
+        o.crba = &crba; o.fwd_kin = &fwd_kin; o.jac = &jac; o.rollout = &rollout; o.rollout_tip = &rollout_tip;
+        o.rnea_fd = &rnea_fd;
         if constexpr (!std::is_void<M32>::value) { o.rnea_f32 = &rnea_f32<M32>; o.fd_f32 = &fd_f32<M32>; }
         return o;
     }

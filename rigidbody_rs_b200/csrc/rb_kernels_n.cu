@@ -211,59 +211,51 @@ rbn_fk_jac_kernel(RbNParam P, const double* __restrict__ q, double* __restrict__
     const int n = P.n;
     const RbJointK* jt = reinterpret_cast<const RbJointK*>(P.model);
     for (size_t s = tid; s < B; s += nthr) {
-        const double* tip = P.model + (size_t)n * 24 + 3;
-        double A[3][3] = {{tip[0], tip[1], tip[2]}, {tip[3], tip[4], tip[5]}, {tip[6], tip[7], tip[8]}};
-        double r[3] = {0.0, 0.0, 0.0};
+        double A[3][3], r[3];
         if (Jout && P.tree)                              // joints that do not support the tip (last link): zero columns
             for (int k = 0; k < 6 * n; ++k) __stcs(Jout + (size_t)k * ld + s, 0.0);
-        for (int i = n - 1; i >= 0; i = (int)jt[i].parent) {
-            const RbJointK& j = jt[i];
-            if (Jout) {
+        rbn_tip_pose(jt, P.model + (size_t)n * 24 + 3, n,
+                     [&](int i, double* sn, double* cs) { sincos(__ldcs(q + (size_t)i * ld + s), sn, cs); },
+                     [&](int i, const double (&A)[3][3], const double (&r)[3]) {
+                         if (!Jout) return;
 #pragma unroll
-                for (int k = 0; k < 3; ++k) {
-                    __stcs(Jout + (size_t)(k + 6 * i) * ld + s, fma(A[1][k], r[0], -(A[0][k] * r[1])));
-                    __stcs(Jout + (size_t)(3 + k + 6 * i) * ld + s, A[2][k]);
-                }
-            }
-            double sn, cs;
-            sincos(__ldcs(q + (size_t)i * ld + s), &sn, &cs);
-            double Bm[3][3], y[3];
-#pragma unroll
-            for (int k = 0; k < 3; ++k) {
-                Bm[0][k] = fma(cs, A[0][k], -(sn * A[1][k]));
-                Bm[1][k] = fma(sn, A[0][k], cs * A[1][k]);
-                Bm[2][k] = A[2][k];
-            }
-            y[0] = fma(cs, r[0], -(sn * r[1])); y[1] = fma(sn, r[0], cs * r[1]); y[2] = r[2];
-#pragma unroll
-            for (int a = 0; a < 3; ++a) {
-#pragma unroll
-                for (int k = 0; k < 3; ++k)
-                    A[a][k] = fma(j.R[3 * a + 2], Bm[2][k], fma(j.R[3 * a + 1], Bm[1][k], j.R[3 * a] * Bm[0][k]));
-                r[a] = fma(j.R[3 * a + 2], y[2], fma(j.R[3 * a + 1], y[1], fma(j.R[3 * a], y[0], j.t[a])));
-            }
-        }
+                         for (int k = 0; k < 3; ++k) {
+                             __stcs(Jout + (size_t)(k + 6 * i) * ld + s, fma(A[1][k], r[0], -(A[0][k] * r[1])));
+                             __stcs(Jout + (size_t)(3 + k + 6 * i) * ld + s, A[2][k]);
+                         }
+                     }, A, r);
         if (xyz) {
             __stcs(xyz + s, r[0]); __stcs(xyz + ld + s, r[1]); __stcs(xyz + 2 * ld + s, r[2]);
         }
     }
 }
 
+// Running and terminal tip-pose terms (rb_tip_terms) of a state whose sin/cos sincos_i gives, with the run-time-n tip pose.
+template <class SinCos>
+RB_DI void rbn_tip_terms(const RbNParam& P, SinCos&& sincos_i, const double* tw, double& run, double& fin) {
+    double R[3][3], x[3];
+    rbn_tip_pose(reinterpret_cast<const RbJointK*>(P.model), P.model + (size_t)P.n * 24 + 3, P.n, sincos_i,
+                 [](int, const double (&)[3][3], const double (&)[3]) {}, R, x);
+    rb_tip_terms(R, x, tw, run, fin);
+}
+
 // scratch slots: [0,2n) sincos, [2n,8n) f, (trees: [8n,20n) link motions / composites,) then n*n H, n rhs/x, n dinv,
-// 2n carried (q, dq).  The per-step solve
+// 2n carried (q, dq).  tip != 0 adds the tip-pose terms of RbTipCost (row RB_CW_TIP of cost_w), each running term of
+// q_t from the sin/cos step t computes for q_t, as rb_rollout_kernel does.  The per-step solve
 // still factorises H in the per-thread global scratch (slow for long chains; rollouts of long chains are not a
 // BASELINE.json configuration).
 __global__ void __launch_bounds__(RB_BLOCK)
 rbn_rollout_kernel(RbNParam P, const double* __restrict__ q0, const double* __restrict__ dq0, const double* __restrict__ tau,
                    double dt, int horizon, double* __restrict__ q_traj, double* __restrict__ dq_traj,
                    double* __restrict__ q_fin, double* __restrict__ dq_fin, size_t B, size_t ld, int* __restrict__ status,
-                   const double* __restrict__ cost_w, double* __restrict__ cost) {
+                   const double* __restrict__ cost_w, double* __restrict__ cost, int tip) {
     const size_t tid = (size_t)blockIdx.x * RB_BLOCK + threadIdx.x;
     const size_t nthr = (size_t)gridDim.x * RB_BLOCK;
     const int n = P.n;
     const RbJointK* jt = reinterpret_cast<const RbJointK*>(P.model);
     const double* g = P.model + (size_t)n * 24;
     RbScratch sc{P.scratch + tid, P.threads};
+    auto sc_sincos = [&](int i, double* sn, double* cs) { *sn = sc[i]; *cs = sc[n + i]; };
     const int o = P.tree ? 20 * n : 8 * n;           // trees keep 12n link motions / 9n composites at [8n, 20n)
     RbScratch va{P.scratch + tid + (size_t)(8 * n) * P.threads, P.threads};
     RbScratch Hs{P.scratch + tid + (size_t)o * P.threads, P.threads};
@@ -282,6 +274,11 @@ rbn_rollout_kernel(RbNParam P, const double* __restrict__ q0, const double* __re
                 double sn, cs;
                 sincos(qs[i], &sn, &cs);
                 sc[i] = sn; sc[n + i] = cs;
+            }
+            if (tip && t > 0) {                          // running tip terms of q_t
+                double run, fin;
+                rbn_tip_terms(P, sc_sincos, cost_w + RB_CW_TIP * RB_MAX_N, run, fin);
+                J = fma(dt, run, J);
             }
             if (P.tree) rbn_tree_rnea(jt, g, n, sc, va, dqs.base, nullptr, dqs.stride, x);
             else rbn_rnea(jt, g, n, sc, dqs.base, nullptr, dqs.stride, x);
@@ -314,6 +311,12 @@ rbn_rollout_kernel(RbNParam P, const double* __restrict__ q0, const double* __re
                 J = fma(cost_w[RB_CW_QF * RB_MAX_N + i] * e, e, J);
                 J = fma(cost_w[RB_CW_DQF * RB_MAX_N + i] * dqs[i], dqs[i], J);
             }
+            if (tip) {                                   // q_H: its running term (horizon > 0) and the terminal term
+                double run, fin;
+                rbn_tip_terms(P, [&](int i, double* sn, double* cs) { sincos(qs[i], sn, cs); }, cost_w + RB_CW_TIP * RB_MAX_N, run, fin);
+                if (horizon > 0) J = fma(dt, run, J);
+                J += fin;
+            }
             __stcs(cost + s, ok_s ? J : __longlong_as_double(0x7ff8000000000000LL));
         }
         for (int i = 0; i < n; ++i) {
@@ -327,11 +330,13 @@ rbn_rollout_kernel(RbNParam P, const double* __restrict__ q0, const double* __re
 // ---- rollout of serial chains of <= 32 joints: one forward-dynamics launch (rb_kernels_warp.cu) + one integration
 // launch per step.  The per-thread factorisation of rbn_rollout_kernel touches O(n^3) scratch words per step; here the
 // state (q, dq) and qdd of all trajectories live in three [n][B] scratch arrays between the launches.
+// tip != NULL (the model, RbNParam::model) adds the tip-pose terms of the state reached: forward dynamics runs in
+// another kernel, so the pose takes its own sin/cos of q_{t+1} here.
 __global__ void __launch_bounds__(RB_BLOCK)
 rbn_euler_kernel(int n, double dt, double* __restrict__ qc, double* __restrict__ dqc, const double* __restrict__ qdd,
                  const double* __restrict__ tau_t, double* __restrict__ q_out, double* __restrict__ dq_out, size_t B, size_t ldc,
                  size_t ld, const double* __restrict__ cost_w, double* __restrict__ cost, int first, int last,
-                 double* __restrict__ q_fin, double* __restrict__ dq_fin) {
+                 double* __restrict__ q_fin, double* __restrict__ dq_fin, const double* __restrict__ tip) {
     const size_t s = (size_t)blockIdx.x * RB_BLOCK + threadIdx.x;
     if (s >= B) return;
     double c = 0.0, term = 0.0;
@@ -356,6 +361,15 @@ rbn_euler_kernel(int n, double dt, double* __restrict__ qc, double* __restrict__
                 term = fma(cost_w[RB_CW_DQF * RB_MAX_N + i] * dqn, dqn, term);
             }
         }
+    }
+    if (tip) {
+        double R[3][3], x[3], run, fin;
+        rbn_tip_pose(reinterpret_cast<const RbJointK*>(tip), tip + (size_t)n * 24 + 3, n,
+                     [&](int i, double* sn, double* cs) { sincos(qc[(size_t)i * ldc + s], sn, cs); },
+                     [](int, const double (&)[3][3], const double (&)[3]) {}, R, x);
+        rb_tip_terms(R, x, cost_w + RB_CW_TIP * RB_MAX_N, run, fin);
+        c += run;
+        if (last) term += fin;
     }
     if (cost) {
         const double J = fma(dt, c, first ? 0.0 : cost[s]);
@@ -444,9 +458,9 @@ cudaError_t n_jac(const void* param, const double* q, double* J, size_t B, size_
     rbn_fk_jac_kernel<<<ngrid(P, B), RB_BLOCK, 0, st>>>(*P, q, nullptr, J, B, ld);
     return cudaGetLastError();
 }
-cudaError_t n_rollout(const void* param, const double* q0, const double* dq0, const double* tau, double dt, int horizon,
-                      double* q_traj, double* dq_traj, double* q_fin, double* dq_fin, size_t B, size_t ld, int* status,
-                      const double* cost_w, double* cost, cudaStream_t st) {
+cudaError_t n_rollout_any(const void* param, const double* q0, const double* dq0, const double* tau, double dt, int horizon,
+                          double* q_traj, double* dq_traj, double* q_fin, double* dq_fin, size_t B, size_t ld, int* status,
+                          const double* cost_w, double* cost, bool tip, cudaStream_t st) {
     const RbNParam* P = (const RbNParam*)param;
     if (B == 0) return cudaSuccess;
 #if RB_WARP_FD
@@ -471,7 +485,7 @@ cudaError_t n_rollout(const void* param, const double* q0, const double* dq0, co
                 rbn_euler_kernel<<<(unsigned)((cnt + RB_BLOCK - 1) / RB_BLOCK), RB_BLOCK, 0, st>>>(
                     n, dt, qc, dqc, acc, tau_t, q_traj ? q_traj + (size_t)t * step + off : nullptr,
                     dq_traj ? dq_traj + (size_t)t * step + off : nullptr, cnt, cnt, ld, cost_w, cost ? cost + off : nullptr,
-                    t == 0, t == horizon - 1, q_fin ? q_fin + off : nullptr, dq_fin ? dq_fin + off : nullptr);
+                    t == 0, t == horizon - 1, q_fin ? q_fin + off : nullptr, dq_fin ? dq_fin + off : nullptr, tip ? P->model : nullptr);
                 e = cudaGetLastError();
                 if (e != cudaSuccess) return e;
             }
@@ -479,8 +493,19 @@ cudaError_t n_rollout(const void* param, const double* q0, const double* dq0, co
         return cudaSuccess;
     }
 #endif
-    rbn_rollout_kernel<<<ngrid(P, B), RB_BLOCK, 0, st>>>(*P, q0, dq0, tau, dt, horizon, q_traj, dq_traj, q_fin, dq_fin, B, ld, status, cost_w, cost);
+    rbn_rollout_kernel<<<ngrid(P, B), RB_BLOCK, 0, st>>>(*P, q0, dq0, tau, dt, horizon, q_traj, dq_traj, q_fin, dq_fin, B, ld, status, cost_w, cost,
+                                                         tip ? 1 : 0);
     return cudaGetLastError();
+}
+cudaError_t n_rollout(const void* param, const double* q0, const double* dq0, const double* tau, double dt, int horizon,
+                      double* q_traj, double* dq_traj, double* q_fin, double* dq_fin, size_t B, size_t ld, int* status,
+                      const double* cost_w, double* cost, cudaStream_t st) {
+    return n_rollout_any(param, q0, dq0, tau, dt, horizon, q_traj, dq_traj, q_fin, dq_fin, B, ld, status, cost_w, cost, false, st);
+}
+cudaError_t n_rollout_tip(const void* param, const double* q0, const double* dq0, const double* tau, double dt, int horizon,
+                          double* q_traj, double* dq_traj, double* q_fin, double* dq_fin, size_t B, size_t ld, int* status,
+                          const double* cost_w, double* cost, cudaStream_t st) {
+    return n_rollout_any(param, q0, dq0, tau, dt, horizon, q_traj, dq_traj, q_fin, dq_fin, B, ld, status, cost_w, cost, true, st);
 }
 }  // namespace
 
@@ -489,6 +514,7 @@ const RbOps* rb_ops_generic_n() {
         RbOps o{};
         o.name = "generic-n"; o.param_bytes = sizeof(RbNParam); o.shared_scratch = true;
         o.rnea = &n_rnea; o.fd = &n_fd; o.crba = &n_crba; o.fwd_kin = &n_fk; o.jac = &n_jac; o.rollout = &n_rollout;
+        o.rollout_tip = &n_rollout_tip;
         return o;
     }();
     return &ops;

@@ -34,5 +34,10 @@ struct RbModelK {
 // Entry-class tags used by compile-time-specialised models to drop multiplications by 0 and +-1.
 enum : int { RB_GEN = 0, RB_ZERO = 1, RB_ONE = 2, RB_NEG1 = 3 };
 
+// Tip-pose cost terms of a rollout (RbTipCost in rigidbody.h), packed into one row of the engine's cost-weight block:
+// tracked point in the tip frame, its target, running / terminal weights per base axis, target orientation (row-major),
+// running / terminal orientation weights.
+enum : int { RB_TW_OFFSET = 0, RB_TW_PREF = 3, RB_TW_WP = 6, RB_TW_WPF = 9, RB_TW_RREF = 12, RB_TW_WR = 21, RB_TW_WRF = 22, RB_TW_COUNT = 23 };
+
 // Field selectors for the model policy accessors.
 enum : int { RB_F_R = 0, RB_F_T = 1, RB_F_M = 2, RB_F_H = 3, RB_F_I = 4 };

@@ -118,6 +118,13 @@ extern "C" {
     pub fn multibody_rollout_cost_grad(g: *mut RbGpu, q0: *const f64, dq0: *const f64, tau: *const f64, dt: f64, horizon: c_int,
                                        w: *const RbQuadCost, cost: *mut f64, grad_tau: *mut f64, grad_q0: *mut f64, grad_dq0: *mut f64,
                                        n_traj: usize, ld: usize, layout: RbLayout, mem: RbMem, stream: *mut c_void) -> c_int;
+    pub fn multibody_rollout_tip_cost(g: *mut RbGpu, q0: *const f64, dq0: *const f64, tau: *const f64, dt: f64, horizon: c_int,
+                                      w: *const RbQuadCost, tip: *const RbTipCost, cost: *mut f64, q_final: *mut f64, dq_final: *mut f64,
+                                      n_traj: usize, ld: usize, layout: RbLayout, mem: RbMem, stream: *mut c_void) -> c_int;
+    pub fn multibody_rollout_tip_cost_grad(g: *mut RbGpu, q0: *const f64, dq0: *const f64, tau: *const f64, dt: f64, horizon: c_int,
+                                           w: *const RbQuadCost, tip: *const RbTipCost, cost: *mut f64, grad_tau: *mut f64,
+                                           grad_q0: *mut f64, grad_dq0: *mut f64, n_traj: usize, ld: usize, layout: RbLayout, mem: RbMem,
+                                           stream: *mut c_void) -> c_int;
     // ---- device-side helpers
     pub fn multibody_gpu_fill(g: *mut RbGpu, dev_out: *mut f64, seed: u64, field: u32, lo: *const f64, hi: *const f64,
                               first_index: usize, count: usize, ld: usize, stream: *mut c_void) -> c_int;
@@ -142,6 +149,20 @@ pub struct RbQuadCost {
     pub w_tau: *const f64,
     pub w_q_final: *const f64,
     pub w_dq_final: *const f64,
+}
+
+/// Tip-pose tracking terms of `multibody_rollout_tip_cost` (include/rigidbody.h RbTipCost): host arrays of 3 values
+/// (`r_ref`: 9, row-major) and two scalar weights; a null pointer means the header's default (zeros, identity `r_ref`).
+#[repr(C)]
+#[derive(Clone, Copy)]
+pub struct RbTipCost {
+    pub offset: *const f64,
+    pub p_ref: *const f64,
+    pub w_p: *const f64,
+    pub w_p_final: *const f64,
+    pub r_ref: *const f64,
+    pub w_r: f64,
+    pub w_r_final: f64,
 }
 
 #[derive(Debug)]
@@ -344,6 +365,24 @@ impl GpuMultibody {
         check(unsafe { multibody_rollout_cost_grad(self.raw, q0.as_ptr(), dq0.as_ptr(), tau.as_ptr(), dt, horizon as c_int, w, cost.as_mut_ptr(),
                                                    grad_tau.as_mut_ptr(), grad_q0.as_mut_ptr(), grad_dq0.as_mut_ptr(), n_traj, 0, layout,
                                                    RbMem::Host, ptr::null_mut()) })
+    }
+
+    /// `rollout_cost_grad` with the tip-pose terms of `tip` added (multibody_rollout_tip_cost_grad); host slices, shapes as
+    /// `rollout_cost_grad`.  Serial chains of at most 12 joints.
+    #[allow(clippy::too_many_arguments)]
+    pub fn rollout_tip_cost_grad(&mut self, q0: &[f64], dq0: &[f64], tau: &[f64], dt: f64, horizon: usize, w: &RbQuadCost, tip: &RbTipCost,
+                                 cost: &mut [f64], grad_tau: &mut [f64], grad_q0: &mut [f64], grad_dq0: &mut [f64], n_traj: usize,
+                                 layout: RbLayout) -> Result<(), RbError> {
+        self.check_len("q0", q0.len(), self.n, n_traj)?;
+        self.check_len("dq0", dq0.len(), self.n, n_traj)?;
+        self.check_len("tau", tau.len(), self.n * horizon, n_traj)?;
+        self.check_len("cost", cost.len(), 1, n_traj)?;
+        self.check_len("grad_tau", grad_tau.len(), self.n * horizon, n_traj)?;
+        self.check_len("grad_q0", grad_q0.len(), self.n, n_traj)?;
+        self.check_len("grad_dq0", grad_dq0.len(), self.n, n_traj)?;
+        check(unsafe { multibody_rollout_tip_cost_grad(self.raw, q0.as_ptr(), dq0.as_ptr(), tau.as_ptr(), dt, horizon as c_int, w, tip,
+                                                       cost.as_mut_ptr(), grad_tau.as_mut_ptr(), grad_q0.as_mut_ptr(), grad_dq0.as_mut_ptr(),
+                                                       n_traj, 0, layout, RbMem::Host, ptr::null_mut()) })
     }
 
     /// d tau / d q and d tau / d dq (2 n*n doubles per state, block b entry r + n*c); serial chains of at most 32 joints.
