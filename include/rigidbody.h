@@ -329,6 +329,48 @@ int multibody_rollout_tip_cost_grad(RbGpu* g, const double* q0, const double* dq
                                     double* grad_q0, double* grad_dq0, size_t n_traj, size_t ld, RbLayout layout, RbMem mem,
                                     void* stream);
 
+/* Pose of the tip frame (the frame of multibody_jac) and of a tracked point in it: 12 entries per state,
+ * x = p + R offset (3) then R row-major (9).  SOA: pose[k*ld + s];  AOS: pose[12 s + k].  offset: host [3], NULL = 0
+ * (finite, RB_ERR_ARG otherwise).  Every chain, tree and kernel family (one model-agnostic kernel: the same bits under
+ * every family). */
+int multibody_tip_pose_batch(RbGpu* g, const double* q, const double* offset, double* pose,
+                             size_t n_states, size_t ld, RbLayout layout, RbMem mem, void* stream);
+
+/* Inverse kinematics of the tip frame: one damped least-squares (Levenberg-Marquardt) problem per entry, minimising the
+ * per-state tip term of RbTipCost,
+ *   F(q) = sum_k w_p[k] (x_k(q) - p*_k)^2 + w_R ||R(q) - R*||_F^2,   x = p + R offset.
+ * With W = diag(sqrt(w_p), sqrt(2 w_R) 1_3), e = (p* - x ; omega), omega = 1/2 sum_k R[:,k] x R*[:,k], and J the base-frame
+ * Jacobian of (x, orientation) (column j = (z_j x (x - P_j) ; z_j) for joints that support the tip, 0 otherwise), a step is
+ *   delta = J^T W (W J J^T W + lambda I_6)^-1 W e     (a 6x6 LDL^T; a non-positive pivot counts as a rejected trial)
+ * and the loop is
+ *   q <- clamp(q_init); lambda <- damping; for k = 0, 1, ...:
+ *     converged (pos_err <= tol_p and (w_R == 0 or rot_err <= tol_R)): iters = k, stop;   k == max_iters: iters = -1, stop;
+ *     q' <- clamp(q + delta); if F(q') < F(q): q <- q', lambda <- max(lambda / 10, 1e-12); else lambda <- min(10 lambda, 1e12).
+ * F never increases: the returned q is never worse than clamp(q_init). */
+typedef struct RbIkOptions {
+    const double* offset;   /* [3] tracked point in the tip frame (as RbTipCost); NULL = tip origin */
+    const double* w_p;      /* [3] position weights per base axis; NULL = 1, 1, 1 */
+    double w_R;             /* weight of ||R - R_target||_F^2; 0 = position only (R_target is not read, may be NULL) */
+    const double* lower;    /* [n] joint bounds, +-inf allowed; NULL = unbounded */
+    const double* upper;    /* [n] */
+    int max_iters;          /* >= 0 */
+    double tol_p;           /* position tolerance (m) */
+    double tol_R;           /* rotation-angle tolerance (rad) */
+    double damping;         /* initial Levenberg-Marquardt lambda, in [1e-12, 1e12] */
+} RbIkOptions;
+
+/* One damped least-squares problem per entry: q_init n per problem, p_target 3, R_target 9 (row-major).
+ * out: n + 3 entries per problem: q, then the position error ||x - p*||_2 over the axes with w_p[k] > 0, the rotation angle
+ * error 2 asin(min(1, ||R - R*||_F / sqrt 8)) (0 when w_R == 0), and the iterations taken (-1 = not converged).  A problem
+ * with a non-finite q_init or target gets NaN in q and both errors and -1, and the call still succeeds.  RB_ERR_ARG for a
+ * negative or non-finite weight, a NaN bound or lower > upper, max_iters < 0, a negative tolerance, damping outside
+ * [1e-12, 1e12]; RB_ERR_NULL for opt == NULL or R_target == NULL with w_R > 0.  Layouts, ld, mem, stream and multi-device
+ * slicing as every batched call.  Every chain, tree and kernel family (the same bits under every family).  Device calls
+ * take a workspace of n doubles per thread of the launch in stream order on `stream` (cudaMallocAsync). */
+int multibody_ik_batch(RbGpu* g, const double* q_init, const double* p_target, const double* R_target,
+                       const RbIkOptions* opt, double* out, size_t n_problems, size_t ld, RbLayout layout,
+                       RbMem mem, void* stream);
+
 /* ---- device-side helpers (bench / tests) --------------------------------------------------- */
 /* Fill a device SOA array [n][ld] with the counter-based sampler of SURVEY.md 8d:
  * value(joint i, state s) = fma(hi[i]-lo[i], u, lo[i]),  u = top 53 bits of

@@ -323,6 +323,77 @@ class Multibody:
             return J.reshape(n, 6).T.copy() if not _is_torch(J) else J.reshape(n, 6).T.contiguous()
         return J
 
+    def tip_pose(self, q, offset=None, layout="soa", out=None):
+        """Pose of the tip frame (the frame of `jac`) and of a tracked point `offset` (3 values in the tip frame, None = 0)
+        in the base frame (include/rigidbody.h multibody_tip_pose_batch): 12 entries per state, x = p + R offset then R
+        row-major.  soa -> [12, B]; aos -> [B, 12]; one state -> (x [3], R [3, 3])."""
+        args, cuda, single, B, lay = self._prep((q,), ("q",), layout, (self.n,))
+        o = self._out(args[0], cuda, single, B, lay, 12, out)
+        off = None if offset is None else np.ascontiguousarray(np.broadcast_to(offset, (3,)), dtype=np.float64)
+        check(lib.multibody_tip_pose_batch(self._h, C.c_void_p(args[0].ptr), None if off is None else off.ctypes.data_as(C.POINTER(C.c_double)),
+                                           C.c_void_p(o.ptr), B, 0, lay, RB_MEM_DEVICE if cuda else RB_MEM_HOST, self._stream(cuda, args[0])))
+        P = o.arr
+        return (P[:3], P[3:].reshape(3, 3)) if single else P
+
+    def ik(self, p_target, R_target=None, q_init=None, offset=None, w_p=None, w_R=None, limits=True, max_iters=100, tol_p=1e-6,
+           tol_R=1e-6, damping=1e-3, layout="soa"):
+        """Inverse kinematics of the tip frame, one damped least-squares problem per entry (include/rigidbody.h
+        multibody_ik_batch, where the algorithm is stated): finds q with tip point x(q) = p + R offset at `p_target` and,
+        when `R_target` is given, orientation R(q) at `R_target`.
+        soa: p_target [3, B], R_target [9, B] (row-major entries), q_init [n, B];  aos: [B, 3], [B, 9] or [B, 3, 3], [B, n];
+        one problem: p_target [3], R_target [3, 3].  w_R defaults to 1 with R_target and 0 without; w_p (3 values) to 1.
+        limits=True takes `limits()` (a joint whose URDF bounds are empty, lower >= upper as for continuous joints, is
+        unbounded); None = unbounded; or a (lower, upper) pair of length-n vectors.  q_init=None starts at the midpoint of
+        finite bounds, else 0.  Returns (q, info): q shaped like q_init, info rows (pos_err, rot_err, iters) shaped [3, B]
+        (soa), [B, 3] (aos) or [3]; iters = -1 marks a problem that did not converge."""
+        n = self.n
+        w_R = (0.0 if R_target is None else 1.0) if w_R is None else float(w_R)
+        if w_R > 0.0 and R_target is None:
+            raise ValueError("ik: w_R > 0 needs R_target")
+        if limits is True:
+            L = self.limits()
+            lo, hi = L["lower"].copy(), L["upper"].copy()
+            empty = ~(lo < hi)
+            lo[empty], hi[empty] = -np.inf, np.inf
+        elif limits is None:
+            lo, hi = np.full(n, -np.inf), np.full(n, np.inf)
+        else:
+            lo, hi = (np.ascontiguousarray(np.broadcast_to(np.asarray(v, dtype=np.float64), (n,))) for v in limits)
+        a_p = _Arg(p_target, "p_target")
+        single = len(a_p.shape) == 1
+        if q_init is None:
+            mid = np.where(np.isfinite(lo) & np.isfinite(hi), 0.5 * (lo + hi), 0.0)
+            B = 1 if single else (a_p.shape[1] if layout == "soa" else a_p.shape[0])
+            q0 = mid if single else (np.repeat(mid[:, None], B, 1) if layout == "soa" else np.repeat(mid[None, :], B, 0))
+            if a_p.torch:
+                import torch
+                q0 = torch.as_tensor(np.ascontiguousarray(q0), device=a_p.device)
+            q_init = q0
+        arrays, names, per = [q_init, p_target], ["q_init", "p_target"], [n, 3]
+        if w_R > 0.0:
+            R = R_target
+            if single:
+                R = R.reshape(9)
+            elif layout == "aos" and len(tuple(R.shape)) == 3:
+                R = R.reshape(R.shape[0], 9)
+            arrays.append(R); names.append("R_target"); per.append(9)
+        args, cuda, single, B, lay = self._prep(arrays, names, layout, per)
+        if cuda and args[0].device.index not in (None, self.device):
+            raise ValueError(f"tensors are on cuda:{args[0].device.index}, engine is on cuda:{self.device}")
+        o = self._out(args[0], cuda, single, B, lay, n + 3, None)
+        vec = lambda v: None if v is None else np.ascontiguousarray(np.broadcast_to(np.asarray(v, dtype=np.float64), (3,)))
+        off, wp = vec(offset), vec(w_p)
+        dp = lambda a: None if a is None else a.ctypes.data_as(C.POINTER(C.c_double))
+        opt = _lib.RbIkOptions(offset=dp(off), w_p=dp(wp), w_R=w_R, lower=dp(lo), upper=dp(hi), max_iters=int(max_iters),
+                               tol_p=float(tol_p), tol_R=float(tol_R), damping=float(damping))
+        ptr = [C.c_void_p(a.ptr) for a in args] + [None] * (3 - len(args))
+        check(lib.multibody_ik_batch(self._h, *ptr, C.byref(opt), C.c_void_p(o.ptr), B, 0, lay,
+                                     RB_MEM_DEVICE if cuda else RB_MEM_HOST, self._stream(cuda, args[0])))
+        D = o.arr
+        if single or lay == RB_LAYOUT_SOA:
+            return D[:n], D[n:]
+        return D[:, :n], D[:, n:]
+
     def rollout(self, q0, dq0, tau, dt, layout="soa", trajectory=True, final=False):
         """Semi-implicit Euler rollout through forward dynamics (SURVEY.md a14).
         soa: q0, dq0 [n, B], tau [H, n, B];  aos: q0, dq0 [B, n], tau [H, B, n].

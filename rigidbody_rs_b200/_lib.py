@@ -34,6 +34,11 @@ class RbTipCost(C.Structure):
     _fields_ = [(k, _dp) for k in ("offset", "p_ref", "w_p", "w_p_final", "R_ref")] + [("w_R", C.c_double), ("w_R_final", C.c_double)]
 
 
+class RbIkOptions(C.Structure):
+    _fields_ = [("offset", _dp), ("w_p", _dp), ("w_R", C.c_double), ("lower", _dp), ("upper", _dp), ("max_iters", C.c_int),
+                ("tol_p", C.c_double), ("tol_R", C.c_double), ("damping", C.c_double)]
+
+
 class RbJointLimits(C.Structure):
     _fields_ = [(k, C.c_double * RB_MAX_JOINTS) for k in ("lower", "upper", "velocity", "effort")]
 
@@ -82,6 +87,8 @@ PROTOTYPES = {
                                         _sz, _sz, _i, _i, _vp]),
     "multibody_rollout_tip_cost_grad": (_i, [_vp, _vp, _vp, _vp, C.c_double, _i, C.POINTER(RbQuadCost), C.POINTER(RbTipCost), _vp, _vp,
                                              _vp, _vp, _sz, _sz, _i, _i, _vp]),
+    "multibody_tip_pose_batch": (_i, [_vp, _vp, _dp, _vp, _sz, _sz, _i, _i, _vp]),
+    "multibody_ik_batch": (_i, [_vp, _vp, _vp, _vp, C.POINTER(RbIkOptions), _vp, _sz, _sz, _i, _i, _vp]),
     "multibody_gpu_fill": (_i, [_vp, _vp, _u64, C.c_uint32, _dp, _dp, _sz, _sz, _sz, _vp]),
     "multibody_gpu_sync": (_i, [_vp]),
     "multibody_gpu_status": (_i, [_vp]),

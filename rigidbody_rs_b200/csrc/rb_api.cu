@@ -129,7 +129,7 @@ struct RbGpu {
     RbJitParam jit{};                     // run-time compiled kernels (jit-specialised family); lib == nullptr if unused
     std::string family_note;              // why this family was chosen (e.g. the JIT fallback reason)
     bool split_rnea_fd = false;           // $RIGIDBODY_B200_FUSED=0: multibody_rnea_fd_batch issues the two launches instead of the fused kernel
-    double* d_model = nullptr;            // generic-n: model rows on the device
+    double* d_model = nullptr;            // model rows on the device (run-time-n family, tip pose, inverse kinematics)
     DevBuf scratch;                       // generic-n: per-thread strided scratch
     DevBuf hpk;                           // generic-n: packed H of one chunk of states (forward dynamics)
     DevBuf cost_w;                        // rollout cost weights (RB_CW_ROWS_TIP x RB_MAX_N doubles), engine-owned: ordered like scratch
@@ -365,6 +365,12 @@ int gpu_create(const RbHostModel& model, int device, RbGpu** out) {
     int rc = pick_ops(g);
     if (rc == RB_OK) rc = bind_entries(g);
     if (rc != RB_OK) return bail(rc);
+    // the tip-pose and inverse-kinematics kernels read the model rows from device memory whatever the family
+    if (!g->d_model) {
+        if ((e = cudaMalloc((void**)&g->d_model, g->flat.size() * sizeof(double))) != cudaSuccess) return bail(fail_cuda(e, "cudaMalloc(model)"));
+        if ((e = cudaMemcpy(g->d_model, g->flat.data(), g->flat.size() * sizeof(double), cudaMemcpyHostToDevice)) != cudaSuccess)
+            return bail(fail_cuda(e, "cudaMemcpy(model)"));
+    }
     if (const char* f = getenv("RIGIDBODY_B200_FUSED")) g->split_rnea_fd = std::string(f) == "0";
     *out = g;
     return RB_OK;
@@ -401,11 +407,13 @@ struct OpDesc {
     int in_per[4];               // doubles per state of each input
     double* out;
     int out_per;                 // doubles per state of the output
-    // launch on SoA device buffers with leading dimension ld
-    cudaError_t (*launch)(RbGpu* g, const double* const* in, double* out, size_t B, size_t ld, cudaStream_t st, int* status);
+    // launch on SoA device buffers with leading dimension ld; `arg` is the op's own argument block (OpDesc::arg)
+    cudaError_t (*launch)(RbGpu* g, const double* const* in, double* out, size_t B, size_t ld, cudaStream_t st, int* status,
+                          const void* arg);
     // optional: launch directly on AoS device buffers (kernel stages through shared memory); null = transpose around `launch`
     cudaError_t (*launch_aos)(RbGpu* g, const double* const* in, double* out, size_t B, cudaStream_t st, int* status) = nullptr;
     bool (*has_aos)(RbGpu* g) = nullptr;
+    const void* arg = nullptr;   // host block handed to `launch` unchanged (per-call options of the op)
 };
 
 int check_common(RbGpu* g, const OpDesc& op, size_t n_states, size_t& ld, RbLayout layout, RbMem mem) {
@@ -424,7 +432,7 @@ int check_common(RbGpu* g, const OpDesc& op, size_t n_states, size_t& ld, RbLayo
 
 int run_device(RbGpu* g, const OpDesc& op, size_t B, size_t ld, RbLayout layout, cudaStream_t st) {
     if (layout == RB_LAYOUT_SOA) {
-        cudaError_t e = op.launch(g, op.in, op.out, B, ld, st, g->d_status);
+        cudaError_t e = op.launch(g, op.in, op.out, B, ld, st, g->d_status, op.arg);
         g->launches += 1;
         if (e != cudaSuccess) return fail_cuda(e, "kernel launch");
         return RB_OK;
@@ -449,7 +457,7 @@ int run_device(RbGpu* g, const OpDesc& op, size_t B, size_t ld, RbLayout layout,
         if (e != cudaSuccess) return fail_cuda(e, "aos_to_soa launch");
         soa_in[k] = dst; off += (size_t)op.in_per[k];
     }
-    cudaError_t e = op.launch(g, soa_in, g->out[0].p, B, B, st, g->d_status);
+    cudaError_t e = op.launch(g, soa_in, g->out[0].p, B, B, st, g->d_status, op.arg);
     g->launches += 1;
     if (e != cudaSuccess) return fail_cuda(e, "kernel launch");
     e = rb_launch_soa_to_aos(g->out[0].p, op.out, op.out_per, B, B, st);
@@ -525,7 +533,7 @@ int run_host_pipeline(RbGpu* g, const OpDesc& op, size_t B, size_t ld, RbLayout 
             off = 0;
             for (int k = 0; k < op.n_in; ++k) { soa_in[k] = g->in[s].p + off * chunk; off += (size_t)op.in_per[k]; }
         }
-        cudaError_t e = op.launch(g, soa_in, g->out[s].p, cnt, cnt, g->stream, g->d_status + 1);
+        cudaError_t e = op.launch(g, soa_in, g->out[s].p, cnt, cnt, g->stream, g->d_status + 1, op.arg);
         g->launches += 1;
         if (e != cudaSuccess) return fail_cuda(e, "kernel launch");
         if (aos) {
@@ -830,7 +838,7 @@ extern "C" int multibody_rnea_batch(RbGpu* g, const double* q, const double* dq,
     if (!g) return fail(RB_ERR_NULL, "engine handle is NULL");
     const int n = g->model.n;
     OpDesc op{3, {q, dq, ddq}, {n, n, n}, tau, n,
-              [](RbGpu* g, const double* const* in, double* out, size_t B, size_t ld, cudaStream_t st, int* status) {
+              [](RbGpu* g, const double* const* in, double* out, size_t B, size_t ld, cudaStream_t st, int* status, const void*) {
                   return launch(g, g->rnea, st, in[0], in[1], in[2], out, B, ld);
               },
               [](RbGpu* g, const double* const* in, double* out, size_t B, cudaStream_t st, int* status) {
@@ -845,7 +853,7 @@ extern "C" int multibody_forward_dynamics_batch(RbGpu* g, const double* q, const
     if (!g) return fail(RB_ERR_NULL, "engine handle is NULL");
     const int n = g->model.n;
     OpDesc op{3, {q, dq, tau}, {n, n, n}, qdd, n,
-              [](RbGpu* g, const double* const* in, double* out, size_t B, size_t ld, cudaStream_t st, int* status) {
+              [](RbGpu* g, const double* const* in, double* out, size_t B, size_t ld, cudaStream_t st, int* status, const void*) {
                   return launch(g, g->fd, st, in[0], in[1], in[2], out, B, ld, status);
               },
               [](RbGpu* g, const double* const* in, double* out, size_t B, cudaStream_t st, int* status) {
@@ -861,7 +869,7 @@ extern "C" int multibody_rnea_fd_batch(RbGpu* g, const double* q, const double* 
     if (!g) return fail(RB_ERR_NULL, "engine handle is NULL");
     const int n = g->model.n;
     OpDesc op{4, {q, dq, ddq, tau_in}, {n, n, n, n}, out, 2 * n,
-              [](RbGpu* g, const double* const* in, double* out, size_t B, size_t ld, cudaStream_t st, int* status) {
+              [](RbGpu* g, const double* const* in, double* out, size_t B, size_t ld, cudaStream_t st, int* status, const void*) {
                   const int n = g->model.n;
                   // one fused pass where the family has it (shared sin/cos, bias recursion and mass matrix)
                   if (g->ops->rnea_fd && !g->split_rnea_fd)
@@ -882,7 +890,7 @@ extern "C" int multibody_rnea_derivatives_batch(RbGpu* g, const double* q, const
     if (n > RB_RNEA_DERIV_MAX_N || !g->model.serial)
         return fail(RB_ERR_UNSUPPORTED, "inverse-dynamics derivative kernels serve serial chains of at most 32 joints");
     OpDesc op{3, {q, dq, ddq}, {n, n, n}, out, 2 * n * n,
-              [](RbGpu* g, const double* const* in, double* out, size_t B, size_t ld, cudaStream_t st, int* status) {
+              [](RbGpu* g, const double* const* in, double* out, size_t B, size_t ld, cudaStream_t st, int* status, const void*) {
                   return rb_launch_rnea_deriv(g->model.n, g->flat.data(), in[0], in[1], in[2], out, B, ld, st);
               }};
     return run_op(g, op, n_states, ld, layout, mem, stream, false);
@@ -895,7 +903,7 @@ extern "C" int multibody_fd_derivatives_batch(RbGpu* g, const double* q, const d
     if (n > RB_DERIV_MAX_N || !g->model.serial)
         return fail(RB_ERR_UNSUPPORTED, "forward-dynamics derivative kernels serve serial chains of at most 12 joints");
     OpDesc op{3, {q, dq, tau}, {n, n, n}, out, 3 * n * n,
-              [](RbGpu* g, const double* const* in, double* out, size_t B, size_t ld, cudaStream_t st, int* status) {
+              [](RbGpu* g, const double* const* in, double* out, size_t B, size_t ld, cudaStream_t st, int* status, const void*) {
                   return rb_launch_fd_deriv(g->model.n, g->flat.data(), in[0], in[1], in[2], out, B, ld, status, st);
               }};
     return run_op(g, op, n_states, ld, layout, mem, stream, true);
@@ -944,7 +952,7 @@ extern "C" int multibody_crba_batch(RbGpu* g, const double* q, double* H, size_t
     if (!g) return fail(RB_ERR_NULL, "engine handle is NULL");
     const int n = g->model.n;
     OpDesc op{1, {q, nullptr, nullptr}, {n, 0, 0}, H, n * n,
-              [](RbGpu* g, const double* const* in, double* out, size_t B, size_t ld, cudaStream_t st, int* status) {
+              [](RbGpu* g, const double* const* in, double* out, size_t B, size_t ld, cudaStream_t st, int* status, const void*) {
                   return launch(g, g->crba, st, in[0], out, B, ld);
               }};
     return run_op(g, op, n_states, ld, layout, mem, stream, false);
@@ -955,7 +963,7 @@ extern "C" int multibody_fwd_kin_batch(RbGpu* g, const double* q, double* xyz, s
     if (!g) return fail(RB_ERR_NULL, "engine handle is NULL");
     const int n = g->model.n;
     OpDesc op{1, {q, nullptr, nullptr}, {n, 0, 0}, xyz, 3,
-              [](RbGpu* g, const double* const* in, double* out, size_t B, size_t ld, cudaStream_t st, int* status) {
+              [](RbGpu* g, const double* const* in, double* out, size_t B, size_t ld, cudaStream_t st, int* status, const void*) {
                   return launch(g, g->fwd_kin, st, in[0], out, B, ld);
               }};
     return run_op(g, op, n_states, ld, layout, mem, stream, false);
@@ -966,10 +974,78 @@ extern "C" int multibody_jac_batch(RbGpu* g, const double* q, double* J, size_t 
     if (!g) return fail(RB_ERR_NULL, "engine handle is NULL");
     const int n = g->model.n;
     OpDesc op{1, {q, nullptr, nullptr}, {n, 0, 0}, J, 6 * n,
-              [](RbGpu* g, const double* const* in, double* out, size_t B, size_t ld, cudaStream_t st, int* status) {
+              [](RbGpu* g, const double* const* in, double* out, size_t B, size_t ld, cudaStream_t st, int* status, const void*) {
                   return launch(g, g->jac, st, in[0], out, B, ld);
               }};
     return run_op(g, op, n_states, ld, layout, mem, stream, false);
+}
+
+// ---- tip pose and inverse kinematics of the tip frame (rb_kernels_ik.cu): one kernel for every family ----
+extern "C" int multibody_tip_pose_batch(RbGpu* g, const double* q, const double* offset, double* pose, size_t n_states, size_t ld,
+                                        RbLayout layout, RbMem mem, void* stream) {
+    if (!g) return fail(RB_ERR_NULL, "engine handle is NULL");
+    const int n = g->model.n;
+    double off[3] = {0.0, 0.0, 0.0};
+    if (offset)
+        for (int k = 0; k < 3; ++k) {
+            if (!std::isfinite(offset[k])) return fail(RB_ERR_ARG, "offset must be finite");
+            off[k] = offset[k];
+        }
+    OpDesc op{1, {q, nullptr, nullptr}, {n, 0, 0}, pose, 12,
+              [](RbGpu* g, const double* const* in, double* out, size_t B, size_t ld, cudaStream_t st, int* status, const void* arg) {
+                  return rb_launch_tip_pose(g->d_model, g->model.n, (const double*)arg, in[0], out, B, ld, st);
+              }};
+    op.arg = off;
+    return run_op(g, op, n_states, ld, layout, mem, stream, false);
+}
+
+namespace {
+// Checks an RbIkOptions and packs it into the kernel's parameter block.
+int pack_ik(const RbHostModel& m, const RbIkOptions* o, const double* R_target, RbIkParam& P) {
+    if (!o) return fail(RB_ERR_NULL, "IK options are NULL");
+    memset(&P, 0, sizeof(P));
+    const int n = m.n;
+    for (int k = 0; k < 3; ++k) {
+        P.offset[k] = o->offset ? o->offset[k] : 0.0;
+        P.w_p[k] = o->w_p ? o->w_p[k] : 1.0;
+        if (!std::isfinite(P.offset[k])) return fail(RB_ERR_ARG, "IK offset must be finite");
+        if (!std::isfinite(P.w_p[k]) || P.w_p[k] < 0.0) return fail(RB_ERR_ARG, "IK weights must be finite and non-negative");
+    }
+    if (!std::isfinite(o->w_R) || o->w_R < 0.0) return fail(RB_ERR_ARG, "IK weights must be finite and non-negative");
+    if (o->max_iters < 0) return fail(RB_ERR_ARG, "IK max_iters < 0");
+    if (!(o->tol_p >= 0.0) || !(o->tol_R >= 0.0)) return fail(RB_ERR_ARG, "IK tolerances must be non-negative");
+    if (!(o->damping >= 1e-12 && o->damping <= 1e12)) return fail(RB_ERR_ARG, "IK damping must lie in [1e-12, 1e12]");
+    if (o->w_R > 0.0 && !R_target) return fail(RB_ERR_NULL, "R_target is NULL but w_R > 0");
+    for (int i = 0; i < n; ++i) {
+        P.lower[i] = o->lower ? o->lower[i] : -INFINITY;
+        P.upper[i] = o->upper ? o->upper[i] : INFINITY;
+        if (std::isnan(P.lower[i]) || std::isnan(P.upper[i]) || P.lower[i] > P.upper[i])
+            return fail(RB_ERR_ARG, "IK bounds must not be NaN and lower <= upper");
+    }
+    P.w_R = o->w_R;
+    for (int k = 0; k < 3; ++k) { P.sw[k] = std::sqrt(P.w_p[k]); P.sw[3 + k] = std::sqrt(2.0 * P.w_R); }
+    P.tol_p = o->tol_p; P.tol_R = o->tol_R; P.damping = o->damping; P.max_iters = o->max_iters;
+    P.tree = m.serial ? 0 : 1;
+    return RB_OK;
+}
+}  // namespace
+
+extern "C" int multibody_ik_batch(RbGpu* g, const double* q_init, const double* p_target, const double* R_target,
+                                  const RbIkOptions* opt, double* out, size_t n_problems, size_t ld, RbLayout layout,
+                                  RbMem mem, void* stream) {
+    if (!g) return fail(RB_ERR_NULL, "engine handle is NULL");
+    const int n = g->model.n;
+    RbIkParam P;
+    const int rc = pack_ik(g->model, opt, R_target, P);
+    if (rc != RB_OK) return rc;
+    // w_R == 0: position only, R_target is neither read nor staged
+    OpDesc op{P.w_R > 0.0 ? 3 : 2, {q_init, p_target, R_target}, {n, 3, 9}, out, n + 3,
+              [](RbGpu* g, const double* const* in, double* out, size_t B, size_t ld, cudaStream_t st, int* status, const void* arg) {
+                  const RbIkParam& P = *(const RbIkParam*)arg;
+                  return rb_launch_ik(g->d_model, g->model.n, P, in[0], in[1], P.w_R > 0.0 ? in[2] : nullptr, out, B, ld, g->sm_count, st);
+              }};
+    op.arg = &P;
+    return run_op(g, op, n_problems, ld, layout, mem, stream, false);
 }
 
 namespace {

@@ -46,3 +46,20 @@ struct RbAdjointArgs {
 };
 cudaError_t rb_launch_rollout_adjoint(int n, const double* flat_model, const RbAdjointArgs& a, size_t B, size_t ld, int* status,
                                       cudaStream_t st);
+// Tip pose and damped least-squares inverse kinematics of the tip frame (rb_kernels_ik.cu), any chain or tree;
+// `model` = device rows in the rb_model.h layout.  Pose: [12][ld], x = p + R offset then R row-major.
+struct RbIkParam {
+    double offset[3];                  // tracked point in the tip frame
+    double w_p[3], w_R;                // objective weights
+    double sw[6];                      // diagonal of W: sqrt(w_p), sqrt(2 w_R) x 3
+    double tol_p, tol_R, damping;
+    double lower[RB_MAX_N], upper[RB_MAX_N];
+    int max_iters;
+    int tree;                          // 1 = some joints do not support the tip
+};
+cudaError_t rb_launch_tip_pose(const double* model, int n, const double* offset, const double* q, double* pose, size_t B,
+                               size_t ld, cudaStream_t st);
+// out: [n + 3][ld] = q, position error, rotation angle error, iterations (-1 = not converged).  Takes a stream-ordered
+// workspace of n doubles per thread of the grid (cudaMallocAsync on st).
+cudaError_t rb_launch_ik(const double* model, int n, const RbIkParam& P, const double* q_init, const double* p_target,
+                         const double* R_target, double* out, size_t B, size_t ld, int sm_count, cudaStream_t st);

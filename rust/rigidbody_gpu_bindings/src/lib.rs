@@ -125,6 +125,10 @@ extern "C" {
                                            w: *const RbQuadCost, tip: *const RbTipCost, cost: *mut f64, grad_tau: *mut f64,
                                            grad_q0: *mut f64, grad_dq0: *mut f64, n_traj: usize, ld: usize, layout: RbLayout, mem: RbMem,
                                            stream: *mut c_void) -> c_int;
+    pub fn multibody_tip_pose_batch(g: *mut RbGpu, q: *const f64, offset: *const f64, pose: *mut f64,
+                                    n_states: usize, ld: usize, layout: RbLayout, mem: RbMem, stream: *mut c_void) -> c_int;
+    pub fn multibody_ik_batch(g: *mut RbGpu, q_init: *const f64, p_target: *const f64, r_target: *const f64, opt: *const RbIkOptions,
+                              out: *mut f64, n_problems: usize, ld: usize, layout: RbLayout, mem: RbMem, stream: *mut c_void) -> c_int;
     // ---- device-side helpers
     pub fn multibody_gpu_fill(g: *mut RbGpu, dev_out: *mut f64, seed: u64, field: u32, lo: *const f64, hi: *const f64,
                               first_index: usize, count: usize, ld: usize, stream: *mut c_void) -> c_int;
@@ -163,6 +167,23 @@ pub struct RbTipCost {
     pub r_ref: *const f64,
     pub w_r: f64,
     pub w_r_final: f64,
+}
+
+/// Options of `multibody_ik_batch` (include/rigidbody.h RbIkOptions, where the algorithm is stated): host arrays of 3
+/// (`offset`, `w_p`) or n (`lower`, `upper`) values, a null pointer meaning the header's default (tip origin, unit weights,
+/// unbounded joints).
+#[repr(C)]
+#[derive(Clone, Copy)]
+pub struct RbIkOptions {
+    pub offset: *const f64,
+    pub w_p: *const f64,
+    pub w_r: f64,
+    pub lower: *const f64,
+    pub upper: *const f64,
+    pub max_iters: c_int,
+    pub tol_p: f64,
+    pub tol_r: f64,
+    pub damping: f64,
 }
 
 #[derive(Debug)]
@@ -383,6 +404,23 @@ impl GpuMultibody {
         check(unsafe { multibody_rollout_tip_cost_grad(self.raw, q0.as_ptr(), dq0.as_ptr(), tau.as_ptr(), dt, horizon as c_int, w, tip,
                                                        cost.as_mut_ptr(), grad_tau.as_mut_ptr(), grad_q0.as_mut_ptr(), grad_dq0.as_mut_ptr(),
                                                        n_traj, 0, layout, RbMem::Host, ptr::null_mut()) })
+    }
+
+    /// Inverse kinematics of the tip frame (multibody_ik_batch): one damped least-squares problem per entry, host slices.
+    /// `q_init` n values per problem, `p_target` 3, `r_target` 9 (row-major; may be empty when `opt.w_r == 0`), `out` n + 3:
+    /// q, position error, rotation angle error, iterations (-1 = not converged).
+    #[allow(clippy::too_many_arguments)]
+    pub fn ik(&mut self, q_init: &[f64], p_target: &[f64], r_target: &[f64], opt: &RbIkOptions, out: &mut [f64], n_problems: usize,
+              layout: RbLayout) -> Result<(), RbError> {
+        self.check_len("q_init", q_init.len(), self.n, n_problems)?;
+        self.check_len("p_target", p_target.len(), 3, n_problems)?;
+        if opt.w_r != 0.0 {
+            self.check_len("r_target", r_target.len(), 9, n_problems)?;
+        }
+        self.check_len("out", out.len(), self.n + 3, n_problems)?;
+        let r = if opt.w_r != 0.0 { r_target.as_ptr() } else { ptr::null() };
+        check(unsafe { multibody_ik_batch(self.raw, q_init.as_ptr(), p_target.as_ptr(), r, opt, out.as_mut_ptr(), n_problems, 0, layout,
+                                          RbMem::Host, ptr::null_mut()) })
     }
 
     /// d tau / d q and d tau / d dq (2 n*n doubles per state, block b entry r + n*c); serial chains of at most 32 joints.
