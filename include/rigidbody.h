@@ -371,6 +371,68 @@ int multibody_ik_batch(RbGpu* g, const double* q_init, const double* p_target, c
                        const RbIkOptions* opt, double* out, size_t n_problems, size_t ld, RbLayout layout,
                        RbMem mem, void* stream);
 
+/* ---- link poses and collision-sphere cost terms (DESIGN.md 4.11) ---------------------------------
+ * Link l is the child link of joint l; its frame is the joint frame of the descriptor / URDF (the engine re-bases a
+ * joint whose axis is not +z internally; that rotation is undone here).  The tip frame of multibody_jac and
+ * multibody_tip_pose_batch is link n-1's frame.
+ *
+ * Pose of every link: 12 entries per link per state, P_l (3) then R_l row-major (9), in the base frame.
+ * SOA: pose[(12 l + m) ld + s];  AOS: pose[12 n s + 12 l + m].  Every chain, tree and kernel family (one model-agnostic
+ * kernel: the same bits under every family). */
+int multibody_link_poses_batch(RbGpu* g, const double* q, double* pose, size_t n_states, size_t ld, RbLayout layout,
+                               RbMem mem, void* stream);
+
+#define RB_MAX_SPHERES 256
+#define RB_MAX_OBSTACLES 64
+typedef enum RbObstacleKind { RB_OBSTACLE_SPHERE = 0, RB_OBSTACLE_HALFSPACE = 1 } RbObstacleKind;
+/* Spheres fixed to the links and obstacles shared by all states.  Sphere k sits on link link[k] with centre c_k (in that
+ * link's frame) and radius r_k >= 0; its world centre is x_k = P_l + R_l c_k.  Obstacle o is
+ *   RB_OBSTACLE_SPHERE    (obstacle[4o..4o+3] = centre o, radius rho >= 0):  d_ko = ||x_k - o|| - r_k - rho,
+ *   RB_OBSTACLE_HALFSPACE (obstacle[4o..4o+3] = normal n, offset h; n is normalised on load, the free side is
+ *                          n.x >= h):                                    d_ko = n.x_k - h - r_k.
+ * With margin m >= 0 the penalty of a pair is phi(d) = max(0, m - d)^2 (C^1), and Phi(q) = sum_k sum_o phi(d_ko).
+ * A rollout cost gains  sum_{t=1}^{H} dt w Phi(q_t) + w_final Phi(q_H).
+ * Gradient: dPhi/dq_j = s_j . sum_{l supported by j} w_l, s_j = (z_j ; P_j x z_j) the joint's world screw and
+ * w_l = sum_{k on l} (x_k x g_k ; g_k) the link's world wrench, g_k = sum_o -2 max(0, m - d_ko) u_ko, where
+ * u_ko = (x_k - o) / ||x_k - o|| (u = 0 when x_k = o exactly) or n for a half-space.
+ * RB_ERR_NULL for a NULL array behind a non-zero count; RB_ERR_ARG for a count below 0 or above its cap, link outside
+ * [0, n), a non-finite centre / obstacle entry, a negative radius, an unknown kind, a zero half-space normal, or a
+ * negative or non-finite margin or weight. */
+typedef struct RbCollisionCost {
+    int32_t n_spheres;
+    const int32_t* link;      /* [S] link of each sphere */
+    const double* center;     /* [3S] centre in the link's frame */
+    const double* radius;     /* [S] */
+    int32_t n_obstacles;
+    const int32_t* kind;      /* [O] RbObstacleKind */
+    const double* obstacle;   /* [4O] (o, rho) or (n, h) */
+    double margin;            /* m */
+    double w;                 /* running weight */
+    double w_final;           /* terminal weight */
+} RbCollisionCost;
+
+/* Per state: min_{k,o} d_ko, then Phi(q) (unweighted; w / w_final are checked but not used).  2 entries per state, SOA
+ * out[m ld + s], AOS out[2 s + m].  At least one sphere and one obstacle (RB_ERR_ARG otherwise).  Every chain, tree and
+ * kernel family. */
+int multibody_sphere_distance_batch(RbGpu* g, const double* q, const RbCollisionCost* col, double* out, size_t n_states,
+                                    size_t ld, RbLayout layout, RbMem mem, void* stream);
+/* multibody_rollout_tip_cost with the collision terms of `col` added.  col == NULL, or one with no sphere, no obstacle or
+ * w = w_final = 0: exactly multibody_rollout_tip_cost (same results, same launches).  Every chain and kernel family
+ * multibody_rollout_tip_cost serves. */
+int multibody_rollout_collision_cost(RbGpu* g, const double* q0, const double* dq0, const double* tau, double dt, int horizon,
+                                     const RbQuadCost* weights, const RbTipCost* tip, const RbCollisionCost* col, double* cost,
+                                     double* q_final, double* dq_final, size_t n_traj, size_t ld, RbLayout layout, RbMem mem,
+                                     void* stream);
+/* multibody_rollout_tip_cost_grad with the collision terms: cost bit-identical to multibody_rollout_collision_cost on the
+ * same engine, and its gradient (one world wrench per link per state projected on the joint screws, O(n + S O) per state).
+ * col NULL or inactive: exactly multibody_rollout_tip_cost_grad.  Serial chains of at most 12 joints (RB_ERR_UNSUPPORTED
+ * otherwise). */
+int multibody_rollout_collision_cost_grad(RbGpu* g, const double* q0, const double* dq0, const double* tau, double dt,
+                                          int horizon, const RbQuadCost* weights, const RbTipCost* tip,
+                                          const RbCollisionCost* col, double* cost, double* grad_tau, double* grad_q0,
+                                          double* grad_dq0, size_t n_traj, size_t ld, RbLayout layout, RbMem mem,
+                                          void* stream);
+
 /* ---- device-side helpers (bench / tests) --------------------------------------------------- */
 /* Fill a device SOA array [n][ld] with the counter-based sampler of SURVEY.md 8d:
  * value(joint i, state s) = fma(hi[i]-lo[i], u, lo[i]),  u = top 53 bits of

@@ -335,6 +335,31 @@ class Multibody:
         P = o.arr
         return (P[:3], P[3:].reshape(3, 3)) if single else P
 
+    def link_poses(self, q, layout="soa", out=None):
+        """Pose of every link's frame (the descriptor / URDF joint frame of joint l's child link) in the base frame
+        (include/rigidbody.h multibody_link_poses_batch): 12 entries per link per state, P_l then R_l row-major, link-major.
+        soa -> [12 n, B]; aos -> [B, 12 n]; one state -> (P [n, 3], R [n, 3, 3])."""
+        n = self.n
+        P = self._call(lib.multibody_link_poses_batch, (q,), ("q",), (n,), 12 * n, layout, out)
+        if len(P.shape) == 1:
+            P = P.reshape(n, 12)
+            return P[:, :3], P[:, 3:].reshape(n, 3, 3)
+        return P
+
+    def sphere_distance(self, q, collision, layout="soa", out=None):
+        """Per state min_{k,o} d_ko and the unweighted penalty Phi(q) of a collision model (include/rigidbody.h
+        multibody_sphere_distance_batch).  `collision` as for `rollout_cost`.  soa -> [2, B]; aos -> [B, 2]; one state ->
+        (min d, Phi)."""
+        args, cuda, single, B, lay = self._prep((q,), ("q",), layout, (self.n,))
+        o = self._out(args[0], cuda, single, B, lay, 2, out)
+        if cuda and args[0].device.index not in (None, self.device):
+            raise ValueError(f"tensors are on cuda:{args[0].device.index}, engine is on cuda:{self.device}")
+        cc, keep = _collision_cost(collision)
+        check(lib.multibody_sphere_distance_batch(self._h, C.c_void_p(args[0].ptr), C.byref(cc), C.c_void_p(o.ptr), B, 0, lay,
+                                                  RB_MEM_DEVICE if cuda else RB_MEM_HOST, self._stream(cuda, args[0])))
+        D = o.arr
+        return (float(D[0]), float(D[1])) if single else D
+
     def ik(self, p_target, R_target=None, q_init=None, offset=None, w_p=None, w_R=None, limits=True, max_iters=100, tol_p=1e-6,
            tol_R=1e-6, damping=1e-3, layout="soa"):
         """Inverse kinematics of the tip frame, one damped least-squares problem per entry (include/rigidbody.h
@@ -417,11 +442,13 @@ class Multibody:
         return tuple(res)
 
     def rollout_cost(self, q0, dq0, tau, dt, q_ref=None, w_q=None, w_dq=None, w_tau=None, w_q_final=None, w_dq_final=None,
-                     layout="soa", final=False, tip=None):
+                     layout="soa", final=False, tip=None, collision=None):
         """Fused rollout + quadratic running/terminal cost (one scalar per trajectory; include/rigidbody.h
         multibody_rollout_cost).  Shapes as `rollout`; weights are length-n vectors (None = zeros).  `tip`: a mapping
         with the keys of RbTipCost (offset, p_ref, w_p, w_p_final: 3 values; R_ref: 3x3; w_R, w_R_final: scalars;
-        missing = the struct's NULL / 0) adds the tip-pose terms (multibody_rollout_tip_cost)."""
+        missing = the struct's NULL / 0) adds the tip-pose terms (multibody_rollout_tip_cost).  `collision`: a mapping with
+        the keys of RbCollisionCost (link [S], center [S, 3], radius [S], kind [O] of "sphere" / "halfspace", obstacle [O, 4],
+        margin, w, w_final) adds the collision-sphere terms (multibody_rollout_collision_cost)."""
         a_q, a_dq, a_tau, B, H, lay, new = self._rollout_args(q0, dq0, tau, layout, "rollout_cost")
         cuda = a_q.cuda
         qc, keep = self._quad_cost(q_ref, w_q, w_dq, w_tau, w_q_final, w_dq_final)
@@ -431,7 +458,11 @@ class Multibody:
         ptr = lambda a: C.c_void_p(a.ptr) if a is not None else None
         head = (self._h, ptr(a_q), ptr(a_dq), ptr(a_tau), float(dt), int(H), C.byref(qc))
         tail = (ptr(cost), ptr(qf), ptr(dqf), B, 0, lay, RB_MEM_DEVICE if cuda else RB_MEM_HOST, self._stream(cuda, a_q))
-        if tip is None:
+        if collision is not None:
+            tc, keep_tip = _tip_cost(tip or {})
+            cc, keep_col = _collision_cost(collision)
+            check(lib.multibody_rollout_collision_cost(*head, C.byref(tc), C.byref(cc), *tail))
+        elif tip is None:
             check(lib.multibody_rollout_cost(*head, *tail))
         else:
             tc, keep_tip = _tip_cost(tip)
@@ -439,10 +470,11 @@ class Multibody:
         return (cost.arr, qf.arr, dqf.arr) if final else cost.arr
 
     def rollout_cost_grad(self, q0, dq0, tau, dt, q_ref=None, w_q=None, w_dq=None, w_tau=None, w_q_final=None, w_dq_final=None,
-                          layout="soa", tip=None):
+                          layout="soa", tip=None, collision=None):
         """`rollout_cost` and its gradient (include/rigidbody.h multibody_rollout_cost_grad): returns (cost, grad_tau,
         grad_q0, grad_dq0), the cost bit for bit `rollout_cost`'s, grad_tau shaped like tau, grad_q0 / grad_dq0 like q0.
-        `tip` as for `rollout_cost` (multibody_rollout_tip_cost_grad).  Serial chains of at most 12 joints."""
+        `tip` and `collision` as for `rollout_cost` (multibody_rollout_tip_cost_grad,
+        multibody_rollout_collision_cost_grad).  Serial chains of at most 12 joints."""
         a_q, a_dq, a_tau, B, H, lay, new = self._rollout_args(q0, dq0, tau, layout, "rollout_cost_grad")
         cuda = a_q.cuda
         qc, keep = self._quad_cost(q_ref, w_q, w_dq, w_tau, w_q_final, w_dq_final)
@@ -450,19 +482,23 @@ class Multibody:
         head = (self._h, C.c_void_p(a_q.ptr), C.c_void_p(a_dq.ptr), C.c_void_p(a_tau.ptr), float(dt), int(H), C.byref(qc))
         tail = (C.c_void_p(cost.ptr), C.c_void_p(gt.ptr), C.c_void_p(gq.ptr), C.c_void_p(gdq.ptr),
                 B, 0, lay, RB_MEM_DEVICE if cuda else RB_MEM_HOST, self._stream(cuda, a_q))
-        if tip is None:
+        if collision is not None:
+            tc, keep_tip = _tip_cost(tip or {})
+            cc, keep_col = _collision_cost(collision)
+            check(lib.multibody_rollout_collision_cost_grad(*head, C.byref(tc), C.byref(cc), *tail))
+        elif tip is None:
             check(lib.multibody_rollout_cost_grad(*head, *tail))
         else:
             tc, keep_tip = _tip_cost(tip)
             check(lib.multibody_rollout_tip_cost_grad(*head, C.byref(tc), *tail))
         return cost.arr, gt.arr, gq.arr, gdq.arr
 
-    def rollout_cost_autograd(self, q0, dq0, tau, dt, tip=None, **weights):
+    def rollout_cost_autograd(self, q0, dq0, tau, dt, tip=None, collision=None, **weights):
         """`rollout_cost` as a differentiable torch function: q0, dq0 [n, B] and tau [H, n, B] are CUDA float64 tensors
         (layout 'soa'); returns cost [B].  The forward pass runs `rollout_cost_grad` (`rollout_cost` when no input requires
         a gradient); the backward pass scales the stored gradients by the upstream gradient of each trajectory's cost.
-        `tip` and the weights as for `rollout_cost`."""
-        return _rollout_cost_function().apply(self, q0, dq0, tau, float(dt), tip, weights)
+        `tip`, `collision` and the weights as for `rollout_cost`."""
+        return _rollout_cost_function().apply(self, q0, dq0, tau, float(dt), tip, collision, weights)
 
     def rollout_vjp(self, q0, dq0, tau, dt, q_traj, dq_traj, g_q_traj=None, g_dq_traj=None, g_q_final=None, g_dq_final=None,
                     layout="soa"):
@@ -568,6 +604,39 @@ def _tip_cost(tip):
     return tc, keep
 
 
+_COLLISION_KINDS = {"sphere": _lib.RB_OBSTACLE_SPHERE, "halfspace": _lib.RB_OBSTACLE_HALFSPACE}
+
+
+def _collision_cost(col):
+    """An RbCollisionCost from a mapping with its keys (link, center [S, 3], radius, kind of "sphere" / "halfspace",
+    obstacle [O, 4], margin, w, w_final; missing = empty / 0) and the arrays it points into (keep them alive).  The values
+    themselves are checked by the library."""
+    unknown = set(col) - {"link", "center", "radius", "kind", "obstacle", "margin", "w", "w_final"}
+    if unknown:
+        raise ValueError(f"collision: unknown keys {sorted(unknown)}")
+    link = np.ascontiguousarray(np.asarray(col.get("link", ()), dtype=np.int32).reshape(-1))
+    S = link.size
+    center = np.ascontiguousarray(np.asarray(col.get("center", np.zeros((S, 3))), dtype=np.float64).reshape(-1))
+    radius = np.ascontiguousarray(np.asarray(col.get("radius", np.zeros(S)), dtype=np.float64).reshape(-1))
+    if center.size != 3 * S or radius.size != S:
+        raise ValueError("collision: center must be [S, 3] and radius [S] for the S entries of link")
+    kinds = [k if isinstance(k, (int, np.integer)) else _COLLISION_KINDS.get(k, -1) for k in col.get("kind", ())]
+    kind = np.ascontiguousarray(np.asarray(kinds, dtype=np.int32).reshape(-1))
+    O = kind.size
+    obstacle = np.ascontiguousarray(np.asarray(col.get("obstacle", np.zeros((O, 4))), dtype=np.float64).reshape(-1))
+    if obstacle.size != 4 * O:
+        raise ValueError("collision: obstacle must be [O, 4] for the O entries of kind")
+    cc = _lib.RbCollisionCost()
+    cc.n_spheres, cc.n_obstacles = S, O
+    ip = lambda a: a.ctypes.data_as(C.POINTER(C.c_int32))
+    dp = lambda a: a.ctypes.data_as(C.POINTER(C.c_double))
+    cc.link, cc.center, cc.radius, cc.kind, cc.obstacle = ip(link), dp(center), dp(radius), ip(kind), dp(obstacle)
+    cc.margin = float(col.get("margin", 0.0))
+    cc.w = float(col.get("w", 0.0))
+    cc.w_final = float(col.get("w_final", 0.0))
+    return cc, [link, center, radius, kind, obstacle]
+
+
 _ROLLOUT_FN = None
 _ROLLOUT_COST_FN = None
 
@@ -609,23 +678,23 @@ def _rollout_cost_function():
 
         class RolloutCostFunction(torch.autograd.Function):
             @staticmethod
-            def forward(ctx, mb, q0, dq0, tau, dt, tip, weights):
+            def forward(ctx, mb, q0, dq0, tau, dt, tip, collision, weights):
                 for name, t in (("q0", q0), ("dq0", dq0), ("tau", tau)):
                     if not (_is_torch(t) and t.is_cuda and t.dtype == torch.float64):
                         raise TypeError(f"rollout_cost_autograd: {name} must be a CUDA float64 tensor")
                 q0, dq0, tau = q0.contiguous(), dq0.contiguous(), tau.contiguous()
                 if any(ctx.needs_input_grad[1:4]):
-                    cost, gt, gq, gdq = mb.rollout_cost_grad(q0, dq0, tau, dt, tip=tip, **weights)
+                    cost, gt, gq, gdq = mb.rollout_cost_grad(q0, dq0, tau, dt, tip=tip, collision=collision, **weights)
                     ctx.save_for_backward(gq, gdq, gt)
                 else:
-                    cost = mb.rollout_cost(q0, dq0, tau, dt, tip=tip, **weights)
+                    cost = mb.rollout_cost(q0, dq0, tau, dt, tip=tip, collision=collision, **weights)
                 return cost
 
             @staticmethod
             def backward(ctx, g_cost):
                 gq, gdq, gt = ctx.saved_tensors
                 g = g_cost.contiguous()
-                return None, gq * g[None, :], gdq * g[None, :], gt * g[None, None, :], None, None, None
+                return None, gq * g[None, :], gdq * g[None, :], gt * g[None, None, :], None, None, None, None
 
         _ROLLOUT_COST_FN = RolloutCostFunction
     return _ROLLOUT_COST_FN

@@ -124,7 +124,7 @@ struct RbGpu {
     // bound by bind_entries; the optional entries (rnea_aos, fd_aos, rnea_fd, rnea_f32, fd_f32) are the primary family's alone
     Bound<decltype(RbOps::rnea)> rnea; Bound<decltype(RbOps::fd)> fd; Bound<decltype(RbOps::crba)> crba;
     Bound<decltype(RbOps::fwd_kin)> fwd_kin; Bound<decltype(RbOps::jac)> jac; Bound<decltype(RbOps::rollout)> rollout;
-    Bound<decltype(RbOps::rollout_tip)> rollout_tip;
+    Bound<decltype(RbOps::rollout_tip)> rollout_tip; Bound<decltype(RbOps::rollout_col)> rollout_col;
     size_t hpk_states = 0;
     RbJitParam jit{};                     // run-time compiled kernels (jit-specialised family); lib == nullptr if unused
     std::string family_note;              // why this family was chosen (e.g. the JIT fallback reason)
@@ -132,7 +132,8 @@ struct RbGpu {
     double* d_model = nullptr;            // model rows on the device (run-time-n family, tip pose, inverse kinematics)
     DevBuf scratch;                       // generic-n: per-thread strided scratch
     DevBuf hpk;                           // generic-n: packed H of one chunk of states (forward dynamics)
-    DevBuf cost_w;                        // rollout cost weights (RB_CW_ROWS_TIP x RB_MAX_N doubles), engine-owned: ordered like scratch
+    DevBuf cost_w;                        // rollout cost weights (RB_CW_DOUBLES_COL doubles: rows, then the collision block), engine-owned: ordered like scratch
+    DevBuf link_rot;                      // [n][9] Q_l^T of every link (RbHostModel::link_rot), for link poses in descriptor frames
     size_t scratch_threads = 0;
     cudaStream_t stream = nullptr, s_h2d = nullptr, s_d2h = nullptr;
     cudaEvent_t ev_h2d[kSlots] = {}, ev_comp[kSlots] = {}, ev_d2h[kSlots] = {};
@@ -308,7 +309,7 @@ int pick_ops(RbGpu* g) {
     return setup_generic_n(g, &g->param);
 }
 
-// Binds rnea, fd, crba, fwd_kin, jac, rollout and rollout_tip once: to the primary family where it has the entry, otherwise to the
+// Binds rnea, fd, crba, fwd_kin, jac, rollout, rollout_tip and rollout_col once: to the primary family where it has the entry, otherwise to the
 // fallback table, whose parameter block pick_ops set up for the families that need it.
 int bind_entries(RbGpu* g) {
     bool ok = true;
@@ -320,7 +321,7 @@ int bind_entries(RbGpu* g) {
     };
     bind(g->rnea, &RbOps::rnea); bind(g->fd, &RbOps::fd); bind(g->crba, &RbOps::crba);
     bind(g->fwd_kin, &RbOps::fwd_kin); bind(g->jac, &RbOps::jac); bind(g->rollout, &RbOps::rollout);
-    bind(g->rollout_tip, &RbOps::rollout_tip);
+    bind(g->rollout_tip, &RbOps::rollout_tip); bind(g->rollout_col, &RbOps::rollout_col);
     return ok ? RB_OK : fail(RB_ERR_ARG, std::string("internal: kernel family '") + g->ops->name + "' leaves an entry point unbound");
 }
 
@@ -361,7 +362,14 @@ int gpu_create(const RbHostModel& model, int device, RbGpu** out) {
     if ((e = cudaMallocHost((void**)&g->h_status, 2 * sizeof(int))) != cudaSuccess) return bail(fail_cuda(e, "cudaMallocHost(status)"));
     g->h_status[0] = g->h_status[1] = 0;
     // cost weights of multibody_rollout_cost: allocated once, here (a lazy first-call allocation would race)
-    { int rcw = g->cost_w.ensure(sizeof(double) * RB_CW_ROWS_TIP * RB_MAX_N); if (rcw != RB_OK) return bail(rcw); }
+    { int rcw = g->cost_w.ensure(sizeof(double) * RB_CW_DOUBLES_COL); if (rcw != RB_OK) return bail(rcw); }
+    {
+        const size_t bytes = sizeof(double) * g->model.link_rot.size();
+        int rcl = g->link_rot.ensure(bytes);
+        if (rcl != RB_OK) return bail(rcl);
+        if ((e = cudaMemcpy(g->link_rot.p, g->model.link_rot.data(), bytes, cudaMemcpyHostToDevice)) != cudaSuccess)
+            return bail(fail_cuda(e, "cudaMemcpy(link rotations)"));
+    }
     int rc = pick_ops(g);
     if (rc == RB_OK) rc = bind_entries(g);
     if (rc != RB_OK) return bail(rc);
@@ -745,6 +753,7 @@ extern "C" void multibody_gpu_free(RbGpu* g) {
     g->scratch.release();
     g->hpk.release();
     g->cost_w.release();
+    g->link_rot.release();
     rb_jit_unload(g->jit);
     if (g->d_model) cudaFree(g->d_model);
     if (g->d_status) cudaFree(g->d_status);
@@ -1000,6 +1009,107 @@ extern "C" int multibody_tip_pose_batch(RbGpu* g, const double* q, const double*
 }
 
 namespace {
+static_assert(RB_CL_MAX_SPHERES == RB_MAX_SPHERES && RB_CL_MAX_OBSTACLES == RB_MAX_OBSTACLES, "collision block caps");
+
+// Checks an RbCollisionCost and packs it into the collision block (RB_CL_* entries): sphere centres rotated into the
+// engines' re-based link frames (c -> Q_l^T c) and stably grouped by link, sphere obstacles before half-spaces, normals
+// normalised.  `on` = the terms can add something (some sphere, some obstacle, some weight not zero).
+int pack_collision(const RbHostModel& m, const RbCollisionCost* c, double* blk, bool* on) {
+    *on = false;
+    if (!c) return RB_OK;
+    if (c->n_spheres < 0 || c->n_spheres > RB_MAX_SPHERES) return fail(RB_ERR_ARG, "n_spheres must lie in [0, RB_MAX_SPHERES]");
+    if (c->n_obstacles < 0 || c->n_obstacles > RB_MAX_OBSTACLES) return fail(RB_ERR_ARG, "n_obstacles must lie in [0, RB_MAX_OBSTACLES]");
+    const int S = c->n_spheres, O = c->n_obstacles, n = m.n;
+    if (S > 0 && (!c->link || !c->center || !c->radius)) return fail(RB_ERR_NULL, "collision sphere arrays are NULL");
+    if (O > 0 && (!c->kind || !c->obstacle)) return fail(RB_ERR_NULL, "collision obstacle arrays are NULL");
+    for (double v : {c->margin, c->w, c->w_final})
+        if (!std::isfinite(v) || v < 0.0) return fail(RB_ERR_ARG, "collision margin and weights must be finite and non-negative");
+    memset(blk, 0, sizeof(double) * RB_CL_COUNT);
+    blk[RB_CL_MARGIN] = c->margin; blk[RB_CL_W] = c->w; blk[RB_CL_WF] = c->w_final;
+    int count[RB_MAX_N + 1] = {};
+    for (int k = 0; k < S; ++k) {
+        if (c->link[k] < 0 || c->link[k] >= n) return fail(RB_ERR_ARG, "collision sphere link outside [0, n)");
+        for (int a = 0; a < 3; ++a) if (!std::isfinite(c->center[3 * k + a])) return fail(RB_ERR_ARG, "collision sphere centres must be finite");
+        if (!std::isfinite(c->radius[k]) || c->radius[k] < 0.0) return fail(RB_ERR_ARG, "collision sphere radii must be finite and non-negative");
+        count[c->link[k] + 1] += 1;
+    }
+    for (int l = 0; l < n; ++l) count[l + 1] += count[l];
+    for (int l = 0; l <= n; ++l) blk[RB_CL_TAB + l] = count[l];
+    for (int k = 0; k < S; ++k) {                             // stable: spheres of one link keep their order
+        const int l = c->link[k];
+        double* sp = blk + RB_CL_SPH + 4 * count[l]++;
+        const double* Qt = &m.link_rot[9 * (size_t)l];
+        for (int a = 0; a < 3; ++a)
+            sp[a] = Qt[3 * a] * c->center[3 * k] + Qt[3 * a + 1] * c->center[3 * k + 1] + Qt[3 * a + 2] * c->center[3 * k + 2];
+        sp[3] = c->radius[k];
+    }
+    int nos = 0, noh = 0;
+    for (int o = 0; o < O; ++o) {
+        const double* ob = c->obstacle + 4 * o;
+        for (int a = 0; a < 4; ++a) if (!std::isfinite(ob[a])) return fail(RB_ERR_ARG, "collision obstacles must be finite");
+        if (c->kind[o] == RB_OBSTACLE_SPHERE) {
+            if (ob[3] < 0.0) return fail(RB_ERR_ARG, "collision obstacle radii must be non-negative");
+            nos += 1;
+        } else if (c->kind[o] == RB_OBSTACLE_HALFSPACE) {
+            if (!(std::sqrt(ob[0] * ob[0] + ob[1] * ob[1] + ob[2] * ob[2]) > 0.0)) return fail(RB_ERR_ARG, "half-space normals must not be zero");
+            noh += 1;
+        } else {
+            return fail(RB_ERR_ARG, "unknown collision obstacle kind");
+        }
+    }
+    int at_s = 0, at_h = nos;
+    for (int o = 0; o < O; ++o) {
+        const double* ob = c->obstacle + 4 * o;
+        double* d = blk + RB_CL_OBS + 4 * (c->kind[o] == RB_OBSTACLE_SPHERE ? at_s++ : at_h++);
+        if (c->kind[o] == RB_OBSTACLE_SPHERE) {
+            for (int a = 0; a < 4; ++a) d[a] = ob[a];
+        } else {
+            const double len = std::sqrt(ob[0] * ob[0] + ob[1] * ob[1] + ob[2] * ob[2]);
+            for (int a = 0; a < 3; ++a) d[a] = ob[a] / len;
+            d[3] = ob[3];
+        }
+    }
+    blk[RB_CL_NOS] = nos; blk[RB_CL_NOH] = noh;
+    *on = S > 0 && O > 0 && (c->w > 0.0 || c->w_final > 0.0);
+    return RB_OK;
+}
+}  // namespace
+
+extern "C" int multibody_link_poses_batch(RbGpu* g, const double* q, double* pose, size_t n_states, size_t ld, RbLayout layout,
+                                          RbMem mem, void* stream) {
+    if (!g) return fail(RB_ERR_NULL, "engine handle is NULL");
+    const int n = g->model.n;
+    OpDesc op{1, {q, nullptr, nullptr}, {n, 0, 0}, pose, 12 * n,
+              [](RbGpu* g, const double* const* in, double* out, size_t B, size_t ld, cudaStream_t st, int* status, const void*) {
+                  return rb_launch_link_poses(g->d_model, (const double*)g->link_rot.p, g->model.n, in[0], out, B, ld, st);
+              }};
+    return run_op(g, op, n_states, ld, layout, mem, stream, false);
+}
+
+extern "C" int multibody_sphere_distance_batch(RbGpu* g, const double* q, const RbCollisionCost* col, double* out, size_t n_states,
+                                               size_t ld, RbLayout layout, RbMem mem, void* stream) {
+    if (!g) return fail(RB_ERR_NULL, "engine handle is NULL");
+    if (!col) return fail(RB_ERR_NULL, "collision terms are NULL");
+    const int n = g->model.n;
+    std::vector<double> blk(RB_CL_COUNT);
+    bool on;
+    const int rc = pack_collision(g->model, col, blk.data(), &on);
+    if (rc != RB_OK) return rc;
+    if (col->n_spheres == 0 || col->n_obstacles == 0) return fail(RB_ERR_ARG, "sphere distances need at least one sphere and one obstacle");
+    // the block goes to the engine's cost-weight buffer, shared by every cost call: ordered like scratch
+    OpDesc op{1, {q, nullptr, nullptr}, {n, 0, 0}, out, 2,
+              [](RbGpu* g, const double* const* in, double* out, size_t B, size_t ld, cudaStream_t st, int* status, const void* arg) {
+                  ScratchOrder so(g, true, st);
+                  double* d = (double*)g->cost_w.p + RB_CW_COL;
+                  cudaError_t e = cudaMemcpyAsync(d, arg, sizeof(double) * RB_CL_COUNT, cudaMemcpyHostToDevice, st);
+                  if (e != cudaSuccess) return e;
+                  return rb_launch_sphere_distance(g->d_model, g->model.n, d, in[0], out, B, ld, st);
+              }};
+    op.arg = blk.data();
+    return run_op(g, op, n_states, ld, layout, mem, stream, false);
+}
+
+namespace {
 // Checks an RbIkOptions and packs it into the kernel's parameter block.
 int pack_ik(const RbHostModel& m, const RbIkOptions* o, const double* R_target, RbIkParam& P) {
     if (!o) return fail(RB_ERR_NULL, "IK options are NULL");
@@ -1174,11 +1284,12 @@ int pack_cost_weights(int n, const RbQuadCost* w, double* cw) {
     return RB_OK;
 }
 
-// The whole cost-weight block of a cost call: the RB_CW_* rows, and the RB_CW_TIP row when tip terms are on.
+// The whole cost-weight block of a cost call: the RB_CW_* rows, the RB_CW_TIP row when tip terms are on, and the
+// collision block (at RB_CW_COL) when collision terms are on.
 struct CostBlock {
-    double w[RB_CW_ROWS_TIP * RB_MAX_N];
-    bool tip;
-    size_t bytes() const { return sizeof(double) * (tip ? RB_CW_ROWS_TIP : RB_CW_ROWS) * RB_MAX_N; }
+    double w[RB_CW_DOUBLES_COL];
+    bool tip, col;
+    size_t bytes() const { return sizeof(double) * (col ? RB_CW_DOUBLES_COL : (tip ? RB_CW_ROWS_TIP : RB_CW_ROWS) * RB_MAX_N); }
 };
 
 // Checks the terms of an RbTipCost and packs them into row RB_CW_TIP (RB_TW_* entries).  `on` = some weight is not
@@ -1204,16 +1315,19 @@ int pack_tip_weights(const RbTipCost* t, double* row, bool* on) {
     return RB_OK;
 }
 
-// Checks and packs both parts of a cost call's weights.
-int pack_cost_block(int n, const RbQuadCost* w, const RbTipCost* tip, CostBlock& cb) {
-    const int rc = pack_cost_weights(n, w, cb.w);
-    if (rc != RB_OK) return rc;
-    return pack_tip_weights(tip, cb.w + RB_CW_TIP * RB_MAX_N, &cb.tip);
+// Checks and packs every part of a cost call's weights.  Collision terms run in the kernels that carry the tip terms
+// too: with collision terms on, the tip row is uploaded whatever its weights.
+int pack_cost_block(const RbHostModel& m, const RbQuadCost* w, const RbTipCost* tip, const RbCollisionCost* col, CostBlock& cb) {
+    int rc = pack_cost_weights(m.n, w, cb.w);
+    if (rc == RB_OK) rc = pack_tip_weights(tip, cb.w + RB_CW_TIP * RB_MAX_N, &cb.tip);
+    if (rc == RB_OK) rc = pack_collision(m, col, cb.w + RB_CW_COL, &cb.col);
+    return rc;
 }
 
 int rollout_impl(RbGpu* g, const double* q0, const double* dq0, const double* tau, double dt, int horizon,
                  double* q_traj, double* dq_traj, double* q_final, double* dq_final, const RbQuadCost* w, const RbTipCost* tip,
-                 double* cost, size_t n_traj, size_t ld, RbLayout layout, RbMem mem, void* stream, size_t aos_stride = 0) {
+                 const RbCollisionCost* col, double* cost, size_t n_traj, size_t ld, RbLayout layout, RbMem mem, void* stream,
+                 size_t aos_stride = 0) {
     if (!g) return fail(RB_ERR_NULL, "engine handle is NULL");
     if (!g->peers.empty()) {
         if (layout != RB_LAYOUT_SOA && layout != RB_LAYOUT_AOS) return fail(RB_ERR_ARG, "bad layout");
@@ -1229,7 +1343,7 @@ int rollout_impl(RbGpu* g, const double* q0, const double* dq0, const double* ta
             auto at = [&](const double* p) { return p ? p + o : nullptr; };
             auto atw = [&](double* p) { return p ? p + o : nullptr; };
             return rollout_impl(g->peers[i], at(q0), at(dq0), at(tau), dt, horizon, atw(q_traj), atw(dq_traj), atw(q_final), atw(dq_final),
-                                w, tip, cost ? cost + lo : nullptr, hi - lo, ld, layout, mem, nullptr, aos ? n_traj * n : 0);
+                                w, tip, col, cost ? cost + lo : nullptr, hi - lo, ld, layout, mem, nullptr, aos ? n_traj * n : 0);
         });
     }
     if (layout != RB_LAYOUT_SOA && layout != RB_LAYOUT_AOS) return fail(RB_ERR_ARG, "bad layout");
@@ -1248,9 +1362,9 @@ int rollout_impl(RbGpu* g, const double* q0, const double* dq0, const double* ta
     cudaStream_t st = mem == RB_MEM_DEVICE ? (cudaStream_t)stream : g->stream;
     // cost weights -> the engine's device block (shared by all cost rollouts, hence ordered like scratch)
     CostBlock cb;
-    cb.tip = false;
-    if (cost) { const int rc = pack_cost_block(n, w, tip, cb); if (rc != RB_OK) return rc; }
-    const auto& ro = cb.tip ? g->rollout_tip : g->rollout;
+    cb.tip = cb.col = false;
+    if (cost) { const int rc = pack_cost_block(g->model, w, tip, col, cb); if (rc != RB_OK) return rc; }
+    const auto& ro = cb.col ? g->rollout_col : cb.tip ? g->rollout_tip : g->rollout;
     const bool shared = cost != nullptr || ro.shared;
     if (mem == RB_MEM_DEVICE && layout == RB_LAYOUT_SOA) {
         ScratchOrder so(g, shared, st);
@@ -1284,6 +1398,7 @@ struct GradArgs {
     const RbQuadCost* w; double* cost;
     double *grad_tau, *grad_q0, *grad_dq0;
     const RbTipCost* tip = nullptr;       // multibody_rollout_tip_cost_grad
+    const RbCollisionCost* col = nullptr; // multibody_rollout_collision_cost_grad
 };
 
 // The trajectory workspace of one chunk of a cost-gradient call, 2 H n doubles per trajectory, stays within this.
@@ -1305,8 +1420,9 @@ int grad_device(RbGpu* g, const GradArgs& a, const CostBlock& cb, size_t B, size
     ScratchOrder so(g, true, st);
     RB_CUDA(cudaMemcpyAsync(g->cost_w.p, cb.w, cb.bytes(), cudaMemcpyHostToDevice, st));
     ad.cost_w = g->cost_w.p;
-    ad.tip = cb.tip;
-    const auto& ro = cb.tip ? g->rollout_tip : g->rollout;
+    ad.tip = cb.tip || cb.col;
+    ad.col = cb.col;
+    const auto& ro = cb.col ? g->rollout_col : cb.tip ? g->rollout_tip : g->rollout;
     const size_t H = (size_t)a.horizon, nn = (size_t)n;
     // A rollout writes its trajectory with the leading dimension of its inputs: a chunk whose inputs are not already a
     // dense [n][chunk] block (a cut batch, a padded ld) gets a dense copy of them next to its trajectory.
@@ -1384,8 +1500,8 @@ int grad_impl(RbGpu* g, const GradArgs& a, size_t n_traj, size_t ld, RbLayout la
     if (!a.q0 || !a.dq0 || (H > 0 && (!a.tau || (!cost && (!a.q_traj || !a.dq_traj))))) return fail(RB_ERR_NULL, "input pointer is NULL");
     if (layout == RB_LAYOUT_SOA) { if (ld == 0) ld = n_traj; if (ld < n_traj) return fail(RB_ERR_ARG, "ld < n_traj"); }
     CostBlock cb;
-    cb.tip = false;
-    if (cost) { const int rc = pack_cost_block(g->model.n, a.w, a.tip, cb); if (rc != RB_OK) return rc; }
+    cb.tip = cb.col = false;
+    if (cost) { const int rc = pack_cost_block(g->model, a.w, a.tip, a.col, cb); if (rc != RB_OK) return rc; }
     if (!cost && !a.grad_tau && !a.grad_q0 && !a.grad_dq0) return RB_OK;
     DeviceGuard dg(g->device);
     if (!dg.ok) return fail(RB_ERR_CUDA, "cudaSetDevice failed");
@@ -1395,7 +1511,7 @@ int grad_impl(RbGpu* g, const GradArgs& a, size_t n_traj, size_t ld, RbLayout la
     return run_staged(g, {{a.q0, 1}, {a.dq0, 1}, {a.tau, H}, {a.q_traj, H}, {a.dq_traj, H}, {a.g_q, H}, {a.g_dq, H}, {a.g_qf, 1}, {a.g_dqf, 1}},
                       {{a.grad_tau, H, false}, {a.grad_q0, 1, false}, {a.grad_dq0, 1, false}, {a.cost, 1, true}},
                       n_traj, ld, layout, mem, aos_stride, st, [&](const double* const* in, double* const* out, int* d_stat) -> int {
-        const GradArgs s{in[0], in[1], in[2], a.dt, a.horizon, in[3], in[4], in[5], in[6], in[7], in[8], a.w, out[3], out[0], out[1], out[2], a.tip};
+        const GradArgs s{in[0], in[1], in[2], a.dt, a.horizon, in[3], in[4], in[5], in[6], in[7], in[8], a.w, out[3], out[0], out[1], out[2], a.tip, a.col};
         return grad_device(g, s, cb, n_traj, n_traj, st, d_stat);
     });
 }
@@ -1404,14 +1520,16 @@ int grad_impl(RbGpu* g, const GradArgs& a, size_t n_traj, size_t ld, RbLayout la
 extern "C" int multibody_rollout(RbGpu* g, const double* q0, const double* dq0, const double* tau, double dt, int horizon,
                                  double* q_traj, double* dq_traj, double* q_final, double* dq_final,
                                  size_t n_traj, size_t ld, RbLayout layout, RbMem mem, void* stream) {
-    return rollout_impl(g, q0, dq0, tau, dt, horizon, q_traj, dq_traj, q_final, dq_final, nullptr, nullptr, nullptr, n_traj, ld, layout, mem, stream);
+    return rollout_impl(g, q0, dq0, tau, dt, horizon, q_traj, dq_traj, q_final, dq_final, nullptr, nullptr, nullptr, nullptr, n_traj, ld,
+                        layout, mem, stream);
 }
 
 extern "C" int multibody_rollout_cost(RbGpu* g, const double* q0, const double* dq0, const double* tau, double dt, int horizon,
                                       const RbQuadCost* weights, double* cost, double* q_final, double* dq_final,
                                       size_t n_traj, size_t ld, RbLayout layout, RbMem mem, void* stream) {
     if (!cost) return fail(RB_ERR_NULL, "cost output pointer is NULL");
-    return rollout_impl(g, q0, dq0, tau, dt, horizon, nullptr, nullptr, q_final, dq_final, weights, nullptr, cost, n_traj, ld, layout, mem, stream);
+    return rollout_impl(g, q0, dq0, tau, dt, horizon, nullptr, nullptr, q_final, dq_final, weights, nullptr, nullptr, cost, n_traj, ld,
+                        layout, mem, stream);
 }
 
 extern "C" int multibody_rollout_tip_cost(RbGpu* g, const double* q0, const double* dq0, const double* tau, double dt, int horizon,
@@ -1419,7 +1537,17 @@ extern "C" int multibody_rollout_tip_cost(RbGpu* g, const double* q0, const doub
                                           size_t n_traj, size_t ld, RbLayout layout, RbMem mem, void* stream) {
     if (!cost) return fail(RB_ERR_NULL, "cost output pointer is NULL");
     const RbQuadCost none{};
-    return rollout_impl(g, q0, dq0, tau, dt, horizon, nullptr, nullptr, q_final, dq_final, weights ? weights : &none, tip, cost,
+    return rollout_impl(g, q0, dq0, tau, dt, horizon, nullptr, nullptr, q_final, dq_final, weights ? weights : &none, tip, nullptr, cost,
+                        n_traj, ld, layout, mem, stream);
+}
+
+extern "C" int multibody_rollout_collision_cost(RbGpu* g, const double* q0, const double* dq0, const double* tau, double dt, int horizon,
+                                                const RbQuadCost* weights, const RbTipCost* tip, const RbCollisionCost* col, double* cost,
+                                                double* q_final, double* dq_final, size_t n_traj, size_t ld, RbLayout layout, RbMem mem,
+                                                void* stream) {
+    if (!cost) return fail(RB_ERR_NULL, "cost output pointer is NULL");
+    const RbQuadCost none{};
+    return rollout_impl(g, q0, dq0, tau, dt, horizon, nullptr, nullptr, q_final, dq_final, weights ? weights : &none, tip, col, cost,
                         n_traj, ld, layout, mem, stream);
 }
 
@@ -1451,6 +1579,18 @@ extern "C" int multibody_rollout_tip_cost_grad(RbGpu* g, const double* q0, const
     const RbQuadCost none{};
     const GradArgs a{q0, dq0, tau, dt, horizon, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, weights ? weights : &none, cost,
                      grad_tau, grad_q0, grad_dq0, tip};
+    return grad_impl(g, a, n_traj, ld, layout, mem, stream);
+}
+
+extern "C" int multibody_rollout_collision_cost_grad(RbGpu* g, const double* q0, const double* dq0, const double* tau, double dt,
+                                                     int horizon, const RbQuadCost* weights, const RbTipCost* tip,
+                                                     const RbCollisionCost* col, double* cost, double* grad_tau, double* grad_q0,
+                                                     double* grad_dq0, size_t n_traj, size_t ld, RbLayout layout, RbMem mem,
+                                                     void* stream) {
+    if (!cost) return fail(RB_ERR_NULL, "cost output pointer is NULL");
+    const RbQuadCost none{};
+    const GradArgs a{q0, dq0, tau, dt, horizon, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, weights ? weights : &none, cost,
+                     grad_tau, grad_q0, grad_dq0, tip, col};
     return grad_impl(g, a, n_traj, ld, layout, mem, stream);
 }
 

@@ -318,6 +318,73 @@ RB_DI void rb_tip_grad(const RbModelK<N>& p, const double* sn, const double* cs,
     }
 }
 
+// ---- collision-sphere cost terms (RbCollisionCost) of link l at its world pose (R, P); col = the collision block
+// W += a (x_k x g_k ; g_k) summed over the link's spheres, g_k = sum_o -2 max(0, m - d_ko) u_ko the gradient of the
+// penalty in the sphere's world centre x_k (u = (x - o) / ||x - o||, 0 when x = o; n for a half-space).  Summed over the
+// links a joint supports and dotted with its screw, this is dPhi/dq_j (the same wrench projection as rb_tip_wrench).
+RB_DI void rb_col_wrench(const double (&R)[3][3], const double (&P)[3], const double* __restrict__ col, int l, double a,
+                         double (&W)[6]) {
+    auto c = [&](int k) { return __ldg(col + k); };
+    const int b = (int)c(RB_CL_TAB + l), e = (int)c(RB_CL_TAB + l + 1), nos = (int)c(RB_CL_NOS), noh = (int)c(RB_CL_NOH);
+    const double m = c(RB_CL_MARGIN);
+#pragma unroll 1
+    for (int k = b; k < e; ++k) {
+        const double* sp = col + RB_CL_SPH + 4 * k;
+        const double c0 = __ldg(sp), c1 = __ldg(sp + 1), c2 = __ldg(sp + 2), r = __ldg(sp + 3);
+        double x[3], g[3] = {0.0, 0.0, 0.0};
+#pragma unroll
+        for (int i = 0; i < 3; ++i) x[i] = fma(R[i][2], c2, fma(R[i][1], c1, fma(R[i][0], c0, P[i])));
+#pragma unroll 1
+        for (int o = 0; o < nos; ++o) {
+            const double* ob = col + RB_CL_OBS + 4 * o;
+            const double d0 = x[0] - __ldg(ob), d1 = x[1] - __ldg(ob + 1), d2 = x[2] - __ldg(ob + 2);
+            const double reach = r + __ldg(ob + 3) + m, dd = fma(d0, d0, fma(d1, d1, d2 * d2));
+            if (dd < reach * reach && dd > 0.0) {
+                const double nrm = sqrt(dd), f = -2.0 * (reach - nrm) / nrm;
+                g[0] = fma(f, d0, g[0]); g[1] = fma(f, d1, g[1]); g[2] = fma(f, d2, g[2]);
+            }
+        }
+#pragma unroll 1
+        for (int o = nos; o < nos + noh; ++o) {
+            const double* ob = col + RB_CL_OBS + 4 * o;
+            const double n0 = __ldg(ob), n1 = __ldg(ob + 1), n2 = __ldg(ob + 2);
+            const double pen = (m + __ldg(ob + 3) + r) - fma(n0, x[0], fma(n1, x[1], n2 * x[2]));
+            if (pen > 0.0) {
+                const double f = -2.0 * pen;
+                g[0] = fma(f, n0, g[0]); g[1] = fma(f, n1, g[1]); g[2] = fma(f, n2, g[2]);
+            }
+        }
+#pragma unroll
+        for (int i = 0; i < 3; ++i) g[i] *= a;
+        double mo[3];
+        rb_cross3(x, g, mo);
+#pragma unroll
+        for (int i = 0; i < 3; ++i) { W[i] += mo[i]; W[3 + i] += g[i]; }
+    }
+}
+
+// gq[j] += the derivative of the tip-pose terms (rb_tip_grad's) and of a Phi(q) at one state: one sweep out, and one
+// back that adds each link's collision wrench to a running wrench and projects it on the joint's screw.
+template <int N>
+RB_DI void rb_col_grad(const RbModelK<N>& p, const double* sn, const double* cs, const double* tw, const double* col, double a,
+                       double b, double* gq) {
+    double R[3][3] = {{1.0, 0.0, 0.0}, {0.0, 1.0, 0.0}, {0.0, 0.0, 1.0}}, P[3] = {0.0, 0.0, 0.0};
+#pragma unroll 1
+    for (int i = 0; i < N; ++i) rb_pose_out(p.jt[i], sn[i], cs[i], R, P);
+    double w[6];
+    rb_tip_wrench(R, P, p.tip, tw, a, b, w);
+    const double wc = fma(b, __ldg(col + RB_CL_WF), a * __ldg(col + RB_CL_W));
+#pragma unroll 1
+    for (int i = N - 1; i >= 0; --i) {
+        rb_col_wrench(R, P, col, i, wc, w);
+        const double z[3] = {R[0][2], R[1][2], R[2][2]};
+        double pz[3];
+        rb_cross3(P, z, pz);
+        gq[i] += fma(z[0], w[0], fma(z[1], w[1], fma(z[2], w[2], fma(pz[0], w[3], fma(pz[1], w[4], pz[2] * w[5])))));
+        if (i > 0) rb_pose_back(p.jt[i], sn[i], cs[i], R, P);
+    }
+}
+
 // Vector-Jacobian product of inverse dynamics in O(N), SUBTRACTED from gq and gdq (the adjoints a caller accumulates):
 //   gq_j  -= (mu^T d tau / d q )_j = Sbar_j . G_j  +   da0_j . Abar_j + dv_j . Bbar_j
 //   gdq_j -= (mu^T d tau / d dq)_j = Sbar_j . G'_j + 2 dv_j . Abar_j +  s_j . Bbar_j
@@ -328,9 +395,13 @@ RB_DI void rb_tip_grad(const RbModelK<N>& p, const double* sn, const double* cs,
 // time (thread-local memory): a caller's adjoints do not occupy registers across the sweeps.
 // TIP with tip_a != 0 also ADDS the running tip-pose terms' derivative (rb_tip_wrench, weight tip_a, row tw) at this
 // state to gq: the wrench from the outward sweep's last-link pose, projected on each screw the inward sweep forms.
-template <int N, bool TIP = false>
+// COL (with TIP) adds the collision terms' derivative as well (weight tip_a times the block's running weight, block col):
+// the inward sweep adds each link's collision wrench (rb_col_wrench, from the link pose it holds) to the tip wrench, and
+// the running sum is what each screw is projected on.
+template <int N, bool TIP = false, bool COL = false>
 RB_DI void rb_rnea_vjp(const RbModelK<N>& p, const double* sn, const double* cs, const double* dq, const double* ddq,
-                       const double* mu, double* gq, double* gdq, const double* tw = nullptr, double tip_a = 0.0) {
+                       const double* mu, double* gq, double* gdq, const double* tw = nullptr, double tip_a = 0.0,
+                       const double* col = nullptr) {
     double R[3][3] = {{1.0, 0.0, 0.0}, {0.0, 1.0, 0.0}, {0.0, 0.0, 1.0}}, P[3] = {0.0, 0.0, 0.0};
     double v[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
     double a[6] = {0.0, 0.0, 0.0, p.g[0], p.g[1], p.g[2]};
@@ -346,6 +417,14 @@ RB_DI void rb_rnea_vjp(const RbModelK<N>& p, const double* sn, const double* cs,
         tip = tip_a != 0.0;
         if (tip) rb_tip_wrench(R, P, p.tip, tw, tip_a, 0.0, wt);
     }
+    double wc = 0.0;
+    if constexpr (COL) {
+        wc = tip_a * __ldg(col + RB_CL_W);
+        if (!tip) {
+#pragma unroll
+            for (int k = 0; k < 6; ++k) wt[k] = 0.0;
+        }
+    }
     RbDerivComposites C = {};
     double Ab[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0}, Bb[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
 #pragma unroll 1
@@ -353,7 +432,10 @@ RB_DI void rb_rnea_vjp(const RbModelK<N>& p, const double* sn, const double* cs,
         double sI[6], dvI[6], daI[6], A[6], Bv[6], G[6], Gp[6];
         rb_deriv_inward(p.jt[i], R, P, v, a, C, sI, dvI, daI, A, Bv, G, Gp);
         gq[i] -= rb_dot6(Sb, G) + (rb_dot6(daI, Ab) + rb_dot6(dvI, Bb));
-        if constexpr (TIP) { if (tip) gq[i] += rb_dot6(sI, wt); }
+        if constexpr (COL) {
+            if (wc != 0.0) rb_col_wrench(R, P, col, i, wc, wt);
+            gq[i] += rb_dot6(sI, wt);
+        } else if constexpr (TIP) { if (tip) gq[i] += rb_dot6(sI, wt); }
         gdq[i] -= rb_dot6(Sb, Gp) + fma(2.0, rb_dot6(dvI, Ab), rb_dot6(sI, Bb));
         const double mi = mu[i];
 #pragma unroll

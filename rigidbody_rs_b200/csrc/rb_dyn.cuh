@@ -770,3 +770,70 @@ RB_DI void rb_tip_terms(const double (&R)[3][3], const double (&pos)[3], const d
     run = fma(w(RB_TW_WR), dR, ep);
     fin = fma(w(RB_TW_WRF), dR, epf);
 }
+
+// ------------------------------------------------------------------ collision spheres (RbCollisionCost)
+// Penalty sum_k sum_o max(0, m - d_ko)^2 of the spheres of link l at the link's world pose (R, P) in the engine frame;
+// col = the collision block (RB_CL_* entries).  A sphere pair takes its square root only within reach,
+// ||x - o||^2 < (r + rho + m)^2, where m - d = (r + rho + m) - ||x - o||.
+RB_DI double rb_col_link(const double (&R)[3][3], const double (&P)[3], const double* __restrict__ col, int l) {
+    auto c = [&](int k) { return __ldg(col + k); };
+    const int b = (int)c(RB_CL_TAB + l), e = (int)c(RB_CL_TAB + l + 1), nos = (int)c(RB_CL_NOS), noh = (int)c(RB_CL_NOH);
+    const double m = c(RB_CL_MARGIN);
+    double phi = 0.0;
+#pragma unroll 1
+    for (int k = b; k < e; ++k) {
+        const double* sp = col + RB_CL_SPH + 4 * k;
+        const double c0 = __ldg(sp), c1 = __ldg(sp + 1), c2 = __ldg(sp + 2), r = __ldg(sp + 3);
+        double x[3];
+#pragma unroll
+        for (int a = 0; a < 3; ++a) x[a] = fma(R[a][2], c2, fma(R[a][1], c1, fma(R[a][0], c0, P[a])));
+#pragma unroll 1
+        for (int o = 0; o < nos; ++o) {
+            const double* ob = col + RB_CL_OBS + 4 * o;
+            const double d0 = x[0] - __ldg(ob), d1 = x[1] - __ldg(ob + 1), d2 = x[2] - __ldg(ob + 2);
+            const double reach = r + __ldg(ob + 3) + m, dd = fma(d0, d0, fma(d1, d1, d2 * d2));
+            if (dd < reach * reach) { const double pen = reach - sqrt(dd); phi = fma(pen, pen, phi); }
+        }
+#pragma unroll 1
+        for (int o = nos; o < nos + noh; ++o) {
+            const double* ob = col + RB_CL_OBS + 4 * o;
+            const double pen = (m + __ldg(ob + 3) + r) - fma(__ldg(ob), x[0], fma(__ldg(ob + 1), x[1], __ldg(ob + 2) * x[2]));
+            if (pen > 0.0) phi = fma(pen, pen, phi);
+        }
+    }
+    return phi;
+}
+
+// Phi(q) of every link (rb_col_link), the link poses composed base -> tip along the compile-time parent table:
+// R_I = R_parent R_p Rz(q_I), P_I = P_parent + R_parent t_I.  A serial chain keeps only the previous link's pose live.
+template <class M>
+RB_DI double rb_col_phi(const typename M::Param& p, const RB_R (&s)[M::N], const RB_R (&c)[M::N], const double* __restrict__ col) {
+    constexpr int N = M::N;
+    RB_R Rs[N][3][3], Ps[N][3];
+    double phi = 0.0;
+    rb_for_up<0, N>([&](auto ic) {
+        constexpr int I = decltype(ic)::value;
+        constexpr int A = M::template parent<I>();
+        RB_R T[3][3];                                  // R_parent R_p
+        rb_for_up<0, 3>([&](auto rc) {
+            constexpr int r = decltype(rc)::value;
+            if constexpr (A < 0) {
+                T[r][0] = KV(I, RB_F_R, 3 * r); T[r][1] = KV(I, RB_F_R, 3 * r + 1); T[r][2] = KV(I, RB_F_R, 3 * r + 2);
+                Ps[I][r] = KV(I, RB_F_T, r);
+            } else {
+                rb_for_up<0, 3>([&](auto kc) {
+                    constexpr int k = decltype(kc)::value;
+                    T[r][k] = k_dot3<KC(I, RB_F_R, k), KC(I, RB_F_R, 3 + k), KC(I, RB_F_R, 6 + k)>(
+                        KV(I, RB_F_R, k), KV(I, RB_F_R, 3 + k), KV(I, RB_F_R, 6 + k), Rs[A][r][0], Rs[A][r][1], Rs[A][r][2]);
+                });
+                Ps[I][r] = k_dot3_acc<KC(I, RB_F_T, 0), KC(I, RB_F_T, 1), KC(I, RB_F_T, 2)>(
+                    Ps[A][r], KV(I, RB_F_T, 0), KV(I, RB_F_T, 1), KV(I, RB_F_T, 2), Rs[A][r][0], Rs[A][r][1], Rs[A][r][2]);
+            }
+            Rs[I][r][0] = fma(c[I], T[r][0], s[I] * T[r][1]);
+            Rs[I][r][1] = fma(c[I], T[r][1], -(s[I] * T[r][0]));
+            Rs[I][r][2] = T[r][2];
+        });
+        phi += rb_col_link(Rs[I], Ps[I], col, I);
+    });
+    return phi;
+}

@@ -344,3 +344,62 @@ RB_DI void rbn_tip_pose(const RbJointK* jt, const double* tip, int n, SinCos&& s
         }
     }
 }
+
+// World pose (R, P) of every link in the engine frame, base -> tip: f(l, R, P) for l = 0..n-1.  A link that hangs off
+// its predecessor extends the running pose, P <- P + R t_l, R <- R R_p Rz(q_l); the first link of a branch (trees) is
+// composed from the base along its ancestors instead, (R, P) <- X_i (R, P) as rbn_tip_pose does.  sincos(i, &s, &c)
+// gives joint i's sin/cos.
+template <class SinCos, class F>
+RB_DI void rbn_link_walk(const RbJointK* jt, int n, SinCos&& sincos_i, F&& f) {
+    double R[3][3] = {{1.0, 0.0, 0.0}, {0.0, 1.0, 0.0}, {0.0, 0.0, 1.0}}, P[3] = {0.0, 0.0, 0.0};
+    for (int l = 0; l < n; ++l) {
+        const int par = (int)jt[l].parent;
+        if (par == l - 1) {
+            const RbJointK& j = jt[l];
+            double sn, cs;
+            sincos_i(l, &sn, &cs);
+#pragma unroll
+            for (int r = 0; r < 3; ++r) {
+                P[r] = fma(R[r][0], j.t[0], fma(R[r][1], j.t[1], fma(R[r][2], j.t[2], P[r])));
+                const double t0 = fma(R[r][0], j.R[0], fma(R[r][1], j.R[3], R[r][2] * j.R[6]));
+                const double t1 = fma(R[r][0], j.R[1], fma(R[r][1], j.R[4], R[r][2] * j.R[7]));
+                const double t2 = fma(R[r][0], j.R[2], fma(R[r][1], j.R[5], R[r][2] * j.R[8]));
+                R[r][0] = fma(cs, t0, sn * t1);
+                R[r][1] = fma(cs, t1, -(sn * t0));
+                R[r][2] = t2;
+            }
+        } else {
+#pragma unroll
+            for (int k = 0; k < 3; ++k) { R[k][0] = k == 0; R[k][1] = k == 1; R[k][2] = k == 2; P[k] = 0.0; }
+            for (int i = l; i >= 0; i = (int)jt[i].parent) {
+                const RbJointK& j = jt[i];
+                double sn, cs;
+                sincos_i(i, &sn, &cs);
+                double Bm[3][3], y[3];
+#pragma unroll
+                for (int k = 0; k < 3; ++k) {
+                    Bm[0][k] = fma(cs, R[0][k], -(sn * R[1][k]));
+                    Bm[1][k] = fma(sn, R[0][k], cs * R[1][k]);
+                    Bm[2][k] = R[2][k];
+                }
+                y[0] = fma(cs, P[0], -(sn * P[1])); y[1] = fma(sn, P[0], cs * P[1]); y[2] = P[2];
+#pragma unroll
+                for (int a = 0; a < 3; ++a) {
+#pragma unroll
+                    for (int k = 0; k < 3; ++k)
+                        R[a][k] = fma(j.R[3 * a + 2], Bm[2][k], fma(j.R[3 * a + 1], Bm[1][k], j.R[3 * a] * Bm[0][k]));
+                    P[a] = fma(j.R[3 * a + 2], y[2], fma(j.R[3 * a + 1], y[1], fma(j.R[3 * a], y[0], j.t[a])));
+                }
+            }
+        }
+        f(l, R, P);
+    }
+}
+
+// Phi(q) of RbCollisionCost (rb_col_link over every link of rbn_link_walk); col = the collision block.
+template <class SinCos>
+RB_DI double rbn_col_phi(const RbJointK* jt, int n, SinCos&& sincos_i, const double* col) {
+    double phi = 0.0;
+    rbn_link_walk(jt, n, sincos_i, [&](int l, const double (&R)[3][3], const double (&P)[3]) { phi += rb_col_link(R, P, col, l); });
+    return phi;
+}

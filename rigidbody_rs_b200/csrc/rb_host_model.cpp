@@ -232,8 +232,12 @@ int build_model(const std::vector<RawJoint>& raw, RbHostModel& out, std::string&
         memcpy(&Qs[i * 9], Q, sizeof Q);
         Qid[i] = identity;
     }
-    mat3_t(&Qs[(raw.size() - 1) * 9], out.tip);      // the original last frame seen from the re-based one
-    for (int e = 0; e < 9; ++e) out.tip[e] = snap(out.tip[e]);
+    out.link_rot.assign(raw.size() * 9, 0.0);       // the original frames seen from the re-based ones
+    for (size_t i = 0; i < raw.size(); ++i) {
+        mat3_t(&Qs[i * 9], &out.link_rot[i * 9]);
+        for (int e = 0; e < 9; ++e) out.link_rot[i * 9 + e] = snap(out.link_rot[i * 9 + e]);
+    }
+    memcpy(out.tip, &out.link_rot[(raw.size() - 1) * 9], sizeof out.tip);
     out.n = (int)raw.size();
     finish_model(out);
     return RB_OK;

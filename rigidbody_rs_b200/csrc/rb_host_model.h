@@ -23,6 +23,8 @@ struct RbHostModel {
     std::vector<RbJointK> jt;
     double g[3] = {0.0, 0.0, 9.81};          // multibody.rs:118
     double tip[9] = {1, 0, 0, 0, 1, 0, 0, 0, 1};
+    // n x 9, row-major: link l's descriptor (URDF) frame seen from its re-based engine frame, Q_l^T; tip is link n-1's
+    std::vector<double> link_rot;
     bool serial = true;                      // every joint hangs off the previous one (the reference's only case)
     RbJointLimits lim{};
     std::vector<std::string> names;

@@ -82,13 +82,14 @@ const char* const kKernelExprs[RB_JIT_KERNELS] = {
     "rb_crba_kernel<CtModel<TabJit>>",        "rb_fwd_kin_kernel<CtModel<TabJit>>",
     "rb_jac_kernel<CtModel<TabJit>>",         "rb_rollout_kernel<CtModel<TabJit>>",
     "rb_rnea_kernel<CtModel<TabJit, float>, false>", "rb_fd_kernel<CtModel<TabJit, float>, false>",
-    "rb_rnea_fd_kernel<CtModel<TabJit>>",    "rb_rollout_kernel<CtModel<TabJit>, true>"};
+    "rb_rnea_fd_kernel<CtModel<TabJit>>",    "rb_rollout_kernel<CtModel<TabJit>, true>",
+    "rb_rollout_kernel<CtModel<TabJit>, true, true>"};
 // chains of RB_JIT_MAX_N+1 .. RB_JIT_LONG_MAX_N joints: the long-chain layouts of rb_kernels_long.cuh for rnea / crba
 // (no n x n array in the thread), the plain kernels for fwd_kin / jac, nothing else
 const char* const kLongExprs[RB_JIT_KERNELS] = {
     "rb_long_rnea_kernel<CtModel<TabJit>>", nullptr, nullptr, nullptr,
     "rb_long_crba_kernel<CtModel<TabJit>>", "rb_fwd_kin_kernel<CtModel<TabJit>>",
-    "rb_jac_kernel<CtModel<TabJit>>",       nullptr, nullptr, nullptr, nullptr, nullptr};
+    "rb_jac_kernel<CtModel<TabJit>>",       nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
 // the AoS variants stage 3 arrays of RB_BLOCK states through dynamic shared memory
 size_t aos_smem(int n) { return (size_t)3 * RB_BLOCK * n * sizeof(double); }
 const char* const kOptions[] = {"--gpu-architecture=sm_100a", "-std=c++17", "-lineinfo", "-default-device", "-DRB_DEVICE_ONLY=1"};
@@ -316,6 +317,12 @@ cudaError_t j_rollout_tip(const void* p, const double* q0, const double* dq0, co
     return jlaunch(p, RB_JK_ROLLOUT_TIP, RB_RO_BLOCK, 0, B, st, q0, dq0, tau, dt, horizon, q_traj, dq_traj, q_fin, dq_fin, B, ld,
                    status, cost_w, cost);
 }
+cudaError_t j_rollout_col(const void* p, const double* q0, const double* dq0, const double* tau, double dt, int horizon,
+                          double* q_traj, double* dq_traj, double* q_fin, double* dq_fin, size_t B, size_t ld, int* status,
+                          const double* cost_w, double* cost, cudaStream_t st) {
+    return jlaunch(p, RB_JK_ROLLOUT_COL, RB_RO_BLOCK, 0, B, st, q0, dq0, tau, dt, horizon, q_traj, dq_traj, q_fin, dq_fin, B, ld,
+                   status, cost_w, cost);
+}
 cudaError_t j_rnea_f32(const void* p, const float* q, const float* dq, const float* ddq, float* tau, size_t B, size_t ld, cudaStream_t st) {
     return jlaunch(p, RB_JK_RNEA_F32, RB_BLOCK, 0, B, st, q, dq, ddq, tau, B, ld);
 }
@@ -343,7 +350,7 @@ const RbOps* rb_ops_jit() {
         RbOps o{};
         o.name = "jit-specialised"; o.param_bytes = sizeof(RbJitParam);
         o.rnea = &j_rnea; o.fd = &j_fd; o.rnea_aos = &j_rnea_aos; o.fd_aos = &j_fd_aos; o.crba = &j_crba; o.fwd_kin = &j_fk;
-        o.jac = &j_jac; o.rollout = &j_rollout; o.rollout_tip = &j_rollout_tip; o.rnea_f32 = &j_rnea_f32; o.fd_f32 = &j_fd_f32; o.rnea_fd = &j_rnea_fd;
+        o.jac = &j_jac; o.rollout = &j_rollout; o.rollout_tip = &j_rollout_tip; o.rollout_col = &j_rollout_col; o.rnea_f32 = &j_rnea_f32; o.fd_f32 = &j_fd_f32; o.rnea_fd = &j_rnea_fd;
         return o;
     }();
     return &ops;

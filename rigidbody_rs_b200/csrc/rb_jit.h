@@ -6,9 +6,10 @@
 
 #define RB_JIT_MAX_N 18        // longest chain the register-resident unrolled kernels are compiled for (FD falls off a cliff at 20)
 #define RB_JIT_LONG_MAX_N 32   // 19..32 joints: only rnea / crba / fwd_kin / jac are compiled ("jit-long"); the rest falls through
-#define RB_JIT_KERNELS 12
+#define RB_JIT_KERNELS 13
 enum : int { RB_JK_RNEA = 0, RB_JK_RNEA_AOS, RB_JK_FD, RB_JK_FD_AOS, RB_JK_CRBA, RB_JK_FK, RB_JK_JAC, RB_JK_ROLLOUT,
-             RB_JK_RNEA_F32, RB_JK_FD_F32, RB_JK_RNEA_FD, RB_JK_ROLLOUT_TIP };
+             RB_JK_RNEA_F32, RB_JK_FD_F32, RB_JK_RNEA_FD, RB_JK_ROLLOUT_TIP,
+             RB_JK_ROLLOUT_COL };
 
 struct RbJitImage {             // what the compiler produces / the disk cache holds
     std::vector<char> cubin;

@@ -78,6 +78,10 @@ struct RbOps {
     cudaError_t (*rollout_tip)(const void* param, const double* q0, const double* dq0, const double* tau, double dt,
                                int horizon, double* q_traj, double* dq_traj, double* q_fin, double* dq_fin,
                                size_t B, size_t ld, int* status, const double* cost_w, double* cost, cudaStream_t st);
+    // ... with the collision-sphere terms of RbCollisionCost added as well (cost_w carries the tip row and the block at RB_CW_COL)
+    cudaError_t (*rollout_col)(const void* param, const double* q0, const double* dq0, const double* tau, double dt,
+                               int horizon, double* q_traj, double* dq_traj, double* q_fin, double* dq_fin,
+                               size_t B, size_t ld, int* status, const double* cost_w, double* cost, cudaStream_t st);
     // optional fp32 mode (BASELINE.json: "an optional fp32 mode is held to a stated 1e-4 tolerance"): the same kernels
     // instantiated with Real = float, device-resident SoA batches only (null = family has no fp32 kernels)
     cudaError_t (*rnea_f32)(const void* param, const float* q, const float* dq, const float* ddq, float* tau,
@@ -314,6 +318,9 @@ rb_jac_kernel(const __grid_constant__ typename M::Param p, const RB_R* __restric
 // computes for forward dynamics anyway: the running term of q_t is added at the top of step t (t >= 1) from that step's
 // sin/cos, and only q_H takes one more sin/cos after the last step (running and terminal term from one pose).  Computing
 // the pose of q_{t+1} right after the integration would pay a second sin/cos of every joint per step instead.
+// COL (with TIP) adds the collision-sphere terms of RbCollisionCost (the block at cost_w + RB_CW_COL, RB_CL_* entries) on
+// the same schedule: dt w Phi(q_t) at the top of step t >= 1 from that step's sin/cos, and dt w Phi(q_H) + w_final Phi(q_H)
+// after the last step.  Without collision terms the caller runs the TIP kernel (same bits as the tip-cost call).
 #ifndef RB_MINB_ROLLOUT
 #define RB_MINB_ROLLOUT 2   // measured on B200 (profiles/r1_kbench_rollout.jsonl): 255 regs, 2 blocks per SM is fastest
 #endif
@@ -321,6 +328,8 @@ rb_jac_kernel(const __grid_constant__ typename M::Param p, const RB_R* __restric
 enum : int { RB_CW_QREF = 0, RB_CW_Q, RB_CW_DQ, RB_CW_TAU, RB_CW_QF, RB_CW_DQF, RB_CW_ROWS };
 // ... and behind them the tip-pose terms of RbTipCost (RB_TW_* entries of one row, rb_model.h)
 enum : int { RB_CW_TIP = RB_CW_ROWS, RB_CW_ROWS_TIP };
+// ... and behind those rows the collision block (RB_CL_* entries, rb_model.h): offset and size in doubles
+enum : int { RB_CW_COL = RB_CW_ROWS_TIP * RB_MAX_N, RB_CW_DOUBLES_COL = RB_CW_COL + RB_CL_COUNT };
 #ifndef RB_ROLLOUT_WS
 #define RB_ROLLOUT_WS 0
 #endif
@@ -331,7 +340,7 @@ enum : int { RB_CW_TIP = RB_CW_ROWS, RB_CW_ROWS_TIP };
 #ifndef RB_RO_MINB
 #define RB_RO_MINB (RB_MINB_ROLLOUT * (128 / RB_RO_BLOCK))
 #endif
-template <class M, bool TIP = false>
+template <class M, bool TIP = false, bool COL = false>
 __global__ void __launch_bounds__(RB_RO_BLOCK, RB_RO_MINB)
 rb_rollout_kernel(const __grid_constant__ typename M::Param p, const RB_R* __restrict__ q0, const RB_R* __restrict__ dq0,
                   const RB_R* __restrict__ tau, RB_R dt, int horizon, RB_R* __restrict__ q_traj,
@@ -360,6 +369,7 @@ rb_rollout_kernel(const __grid_constant__ typename M::Param p, const RB_R* __res
                 rb_tip_pose<M>(p, sn, cs, R, pos);
                 rb_tip_terms(R, pos, cost_w + RB_CW_TIP * RB_MAX_N, run, fin);
                 J = fma(dt, run, J);
+                if constexpr (COL) J = fma(dt, __ldg(cost_w + RB_CW_COL + RB_CL_W) * rb_col_phi<M>(p, sn, cs, cost_w + RB_CW_COL), J);
             }
         }
         ok = rb_forward_dynamics<M>(p, sn, cs, dq, u, qdd) && ok;
@@ -400,6 +410,11 @@ rb_rollout_kernel(const __grid_constant__ typename M::Param p, const RB_R* __res
             rb_tip_terms(R, pos, cost_w + RB_CW_TIP * RB_MAX_N, run, fin);
             if (horizon > 0) J = fma(dt, run, J);
             J += fin;
+            if constexpr (COL) {                       // the same for the collision terms
+                const RB_R phi = rb_col_phi<M>(p, sn, cs, cost_w + RB_CW_COL);
+                if (horizon > 0) J = fma(dt, __ldg(cost_w + RB_CW_COL + RB_CL_W) * phi, J);
+                J = fma(__ldg(cost_w + RB_CW_COL + RB_CL_WF), phi, J);
+            }
         }
         __stcs(cost + s, ok ? J : rb_nan<RB_R>());
     }
@@ -509,6 +524,14 @@ struct RbLaunch {
             *(const P*)param, q0, dq0, tau, dt, horizon, q_traj, dq_traj, q_fin, dq_fin, B, ld, status, cost_w, cost);
         return cudaGetLastError();
     }
+    static cudaError_t rollout_col(const void* param, const double* q0, const double* dq0, const double* tau, double dt,
+                                   int horizon, double* q_traj, double* dq_traj, double* q_fin, double* dq_fin,
+                                   size_t B, size_t ld, int* status, const double* cost_w, double* cost, cudaStream_t st) {
+        if (B == 0) return cudaSuccess;
+        rb_rollout_kernel<M, true, true><<<(unsigned)((B + RB_RO_BLOCK - 1) / RB_RO_BLOCK), RB_RO_BLOCK, 0, st>>>(
+            *(const P*)param, q0, dq0, tau, dt, horizon, q_traj, dq_traj, q_fin, dq_fin, B, ld, status, cost_w, cost);
+        return cudaGetLastError();
+    }
     // M32 = the same policy with Real = float (fp32 mode)
     template <class M32>
     static cudaError_t rnea_f32(const void* param, const float* q, const float* dq, const float* ddq, float* tau,
@@ -530,6 +553,7 @@ struct RbLaunch {
         o.name = name; o.param_bytes = sizeof(P);
         o.rnea = &rnea; o.fd = &fd; o.rnea_aos = &rnea_aos; o.fd_aos = &fd_aos;
         o.crba = &crba; o.fwd_kin = &fwd_kin; o.jac = &jac; o.rollout = &rollout; o.rollout_tip = &rollout_tip;
+        o.rollout_col = &rollout_col;
         o.rnea_fd = &rnea_fd;
         if constexpr (!std::is_void<M32>::value) { o.rnea_f32 = &rnea_f32<M32>; o.fd_f32 = &fd_f32<M32>; }
         return o;

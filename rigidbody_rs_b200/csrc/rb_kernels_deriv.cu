@@ -82,11 +82,13 @@ rb_fd_deriv_kernel(const __grid_constant__ RbModelK<N> p, const double* __restri
 // TIP (with QUAD): also the tip-pose terms of RbTipCost (row RB_CW_TIP of cost_w): the adjoint of each stored state q_t,
 // t >= 1, gains dt times their running gradient, added inside rb_rnea_vjp from the step's own sin/cos; q_H gains the
 // running and terminal gradient from one more sin/cos (rb_tip_grad).
+// COL (with TIP): also the collision-sphere terms of RbCollisionCost (the block at cost_w + RB_CW_COL), the same way: per
+// link wrenches summed in rb_rnea_vjp's inward sweep, and rb_col_grad for q_H.
 // These are gradients of the exact-arithmetic map evaluated at the computed states, not of the rounded fma-Euler map.
 // One LDL^T of H(q_t) per step serves both solves: qdd_t (operation for operation rb_forward_dynamics) and mu.
 // The trajectory (q_traj, dq_traj) has its own leading dimension ld_traj; everything else uses ld.  A trajectory that
 // meets a non-SPD mass matrix sets the status bit and gets NaN in every gradient.
-template <int N, bool QUAD, bool TIP = false>
+template <int N, bool QUAD, bool TIP = false, bool COL = false>
 __global__ void __launch_bounds__(RB_BLOCK, RB_MINB_ADJOINT)
 rb_rollout_adjoint_kernel(const __grid_constant__ RbModelK<N> p, const double* __restrict__ q0, const double* __restrict__ dq0,
                           const double* __restrict__ tau, const double* __restrict__ q_traj, const double* __restrict__ dq_traj,
@@ -120,7 +122,11 @@ rb_rollout_adjoint_kernel(const __grid_constant__ RbModelK<N> p, const double* _
                 adq[i] = fma(2.0 * dt, w(RB_CW_DQ, i) * xd[i], adq[i]);
             }
         }
-        if constexpr (TIP) {
+        if constexpr (COL) {
+            double sn[N], cs[N];
+            rb_sincos_all<N>(x, sn, cs);
+            rb_col_grad<N>(p, sn, cs, cost_w + RB_CW_TIP * RB_MAX_N, cost_w + RB_CW_COL, horizon > 0 ? dt : 0.0, 1.0, aq);
+        } else if constexpr (TIP) {
             double sn[N], cs[N];
             rb_sincos_all<N>(x, sn, cs);
             rb_tip_grad<N>(p, sn, cs, cost_w + RB_CW_TIP * RB_MAX_N, horizon > 0 ? dt : 0.0, 1.0, aq);
@@ -170,7 +176,9 @@ rb_rollout_adjoint_kernel(const __grid_constant__ RbModelK<N> p, const double* _
                 __stcs(grad_tau + (size_t)t * step + (size_t)i * ld + s, gt);
             }
         }
-        if constexpr (TIP) rb_rnea_vjp<N, true>(p, sn, cs, xd, qdd, mu, aq, adq, cost_w + RB_CW_TIP * RB_MAX_N, t > 0 ? dt : 0.0);
+        if constexpr (COL) rb_rnea_vjp<N, true, true>(p, sn, cs, xd, qdd, mu, aq, adq, cost_w + RB_CW_TIP * RB_MAX_N, t > 0 ? dt : 0.0,
+                                                      cost_w + RB_CW_COL);
+        else if constexpr (TIP) rb_rnea_vjp<N, true>(p, sn, cs, xd, qdd, mu, aq, adq, cost_w + RB_CW_TIP * RB_MAX_N, t > 0 ? dt : 0.0);
         else rb_rnea_vjp<N>(p, sn, cs, xd, qdd, mu, aq, adq);             // a_q -= (d tau/d q)^T mu,  a_dq = b - (d tau/d dq)^T mu
         if (t > 0) {                                          // upstream gradients of the state before step t
             if constexpr (QUAD) {
@@ -224,7 +232,11 @@ template <int N>
 cudaError_t launch_adjoint(const double* flat, const RbAdjointArgs& a, size_t B, size_t ld, int* status, cudaStream_t st) {
     RbModelK<N> p;
     memcpy(&p, flat, sizeof(p));
-    if (a.cost_w && a.tip)
+    if (a.cost_w && a.col)
+        rb_rollout_adjoint_kernel<N, true, true, true><<<dgrid(B), RB_BLOCK, 0, st>>>(p, a.q0, a.dq0, a.tau, a.q_traj, a.dq_traj, a.ld_traj, nullptr,
+                                                                                      nullptr, nullptr, nullptr, a.cost_w, a.grad_tau, a.grad_q0,
+                                                                                      a.grad_dq0, a.dt, a.horizon, B, ld, status);
+    else if (a.cost_w && a.tip)
         rb_rollout_adjoint_kernel<N, true, true><<<dgrid(B), RB_BLOCK, 0, st>>>(p, a.q0, a.dq0, a.tau, a.q_traj, a.dq_traj, a.ld_traj, nullptr, nullptr,
                                                                                 nullptr, nullptr, a.cost_w, a.grad_tau, a.grad_q0, a.grad_dq0,
                                                                                 a.dt, a.horizon, B, ld, status);

@@ -1,6 +1,7 @@
 // rb_kernels_ik.cu -- batched tip pose and damped least-squares inverse kinematics of the tip frame
-// (multibody_tip_pose_batch, multibody_ik_batch).  Model-agnostic: both kernels run the run-time-n loop kinematics of
-// rb_dyn_n.cuh (rbn_tip_pose) on the model rows in device memory, so every kernel family gives the same bits.
+// (multibody_tip_pose_batch, multibody_ik_batch), link poses and sphere distances (multibody_link_poses_batch,
+// multibody_sphere_distance_batch).  Model-agnostic: the kernels run the run-time-n loop kinematics of rb_dyn_n.cuh
+// (rbn_tip_pose, rbn_link_walk) on the model rows in device memory, so every kernel family gives the same bits.
 #include "rb_kernels.cuh"
 #include "rb_dyn_n.cuh"
 #include "rb_util.cuh"
@@ -80,6 +81,70 @@ rbn_tip_pose_kernel(const double* __restrict__ model, int n, double o0, double o
         __stcs(pose + (size_t)k * ld + s, fma(R[k][2], off[2], fma(R[k][1], off[1], fma(R[k][0], off[0], r[k]))));
 #pragma unroll
     for (int k = 0; k < 9; ++k) __stcs(pose + (size_t)(3 + k) * ld + s, R[k / 3][k % 3]);
+}
+
+// Link l's descriptor frame: P_l, and R_l = R_engine,l Q_l^T (link_rot row l = Q_l^T, row-major).
+__global__ void __launch_bounds__(RB_BLOCK)
+rbn_link_poses_kernel(const double* __restrict__ model, const double* __restrict__ link_rot, int n, const double* __restrict__ q,
+                      double* __restrict__ pose, size_t B, size_t ld) {
+    const size_t s = (size_t)blockIdx.x * RB_BLOCK + threadIdx.x;
+    if (s >= B) return;
+    rbn_link_walk(reinterpret_cast<const RbJointK*>(model), n,
+                  [&](int i, double* sn, double* cs) { sincos(__ldg(q + (size_t)i * ld + s), sn, cs); },
+                  [&](int l, const double (&R)[3][3], const double (&P)[3]) {
+                      double* o = pose + (size_t)(12 * l) * ld + s;
+                      const double* Qt = link_rot + 9 * l;
+#pragma unroll
+                      for (int k = 0; k < 3; ++k) __stcs(o + (size_t)k * ld, P[k]);
+#pragma unroll
+                      for (int a = 0; a < 3; ++a)
+#pragma unroll
+                          for (int k = 0; k < 3; ++k)
+                              __stcs(o + (size_t)(3 + 3 * a + k) * ld,
+                                     fma(R[a][2], __ldg(Qt + 6 + k), fma(R[a][1], __ldg(Qt + 3 + k), R[a][0] * __ldg(Qt + k))));
+                  });
+}
+
+// min_{k,o} d_ko and Phi(q) of the collision block col (RB_CL_* entries): every pair's distance, with the penalty formed
+// as rb_col_link forms it.
+__global__ void __launch_bounds__(RB_BLOCK)
+rbn_sphere_distance_kernel(const double* __restrict__ model, int n, const double* __restrict__ col, const double* __restrict__ q,
+                           double* __restrict__ out, size_t B, size_t ld) {
+    const size_t s = (size_t)blockIdx.x * RB_BLOCK + threadIdx.x;
+    if (s >= B) return;
+    const int nos = (int)__ldg(col + RB_CL_NOS), noh = (int)__ldg(col + RB_CL_NOH);
+    const double m = __ldg(col + RB_CL_MARGIN);
+    double dmin = INFINITY, phi = 0.0;
+    rbn_link_walk(reinterpret_cast<const RbJointK*>(model), n,
+                  [&](int i, double* sn, double* cs) { sincos(__ldg(q + (size_t)i * ld + s), sn, cs); },
+                  [&](int l, const double (&R)[3][3], const double (&P)[3]) {
+                      const int b = (int)__ldg(col + RB_CL_TAB + l), e = (int)__ldg(col + RB_CL_TAB + l + 1);
+                      for (int k = b; k < e; ++k) {
+                          const double* sp = col + RB_CL_SPH + 4 * k;
+                          const double c0 = __ldg(sp), c1 = __ldg(sp + 1), c2 = __ldg(sp + 2), r = __ldg(sp + 3);
+                          double x[3];
+#pragma unroll
+                          for (int a = 0; a < 3; ++a) x[a] = fma(R[a][2], c2, fma(R[a][1], c1, fma(R[a][0], c0, P[a])));
+                          for (int o = 0; o < nos + noh; ++o) {
+                              const double* ob = col + RB_CL_OBS + 4 * o;
+                              double d, pen;
+                              if (o < nos) {
+                                  const double d0 = x[0] - __ldg(ob), d1 = x[1] - __ldg(ob + 1), d2 = x[2] - __ldg(ob + 2);
+                                  const double nrm = sqrt(fma(d0, d0, fma(d1, d1, d2 * d2)));
+                                  d = nrm - r - __ldg(ob + 3);
+                                  pen = (r + __ldg(ob + 3) + m) - nrm;
+                              } else {
+                                  const double h = fma(__ldg(ob), x[0], fma(__ldg(ob + 1), x[1], __ldg(ob + 2) * x[2]));
+                                  d = h - __ldg(ob + 3) - r;
+                                  pen = (m + __ldg(ob + 3) + r) - h;
+                              }
+                              dmin = fmin(dmin, d);
+                              if (pen > 0.0) phi = fma(pen, pen, phi);
+                          }
+                      }
+                  });
+    __stcs(out + s, dmin);
+    __stcs(out + ld + s, phi);
 }
 
 // One thread per problem, grid-stride.  q lives in the output rows, the trial q' in `ws` (n doubles per thread,
@@ -243,6 +308,20 @@ cudaError_t rb_launch_tip_pose(const double* model, int n, const double* offset,
                                size_t ld, cudaStream_t st) {
     if (B == 0) return cudaSuccess;
     rbn_tip_pose_kernel<<<(unsigned)((B + RB_BLOCK - 1) / RB_BLOCK), RB_BLOCK, 0, st>>>(model, n, offset[0], offset[1], offset[2], q, pose, B, ld);
+    return cudaGetLastError();
+}
+
+cudaError_t rb_launch_link_poses(const double* model, const double* link_rot, int n, const double* q, double* pose, size_t B,
+                                 size_t ld, cudaStream_t st) {
+    if (B == 0) return cudaSuccess;
+    rbn_link_poses_kernel<<<(unsigned)((B + RB_BLOCK - 1) / RB_BLOCK), RB_BLOCK, 0, st>>>(model, link_rot, n, q, pose, B, ld);
+    return cudaGetLastError();
+}
+
+cudaError_t rb_launch_sphere_distance(const double* model, int n, const double* col, const double* q, double* out, size_t B,
+                                      size_t ld, cudaStream_t st) {
+    if (B == 0) return cudaSuccess;
+    rbn_sphere_distance_kernel<<<(unsigned)((B + RB_BLOCK - 1) / RB_BLOCK), RB_BLOCK, 0, st>>>(model, n, col, q, out, B, ld);
     return cudaGetLastError();
 }
 

@@ -241,9 +241,11 @@ RB_DI void rbn_tip_terms(const RbNParam& P, SinCos&& sincos_i, const double* tw,
 
 // scratch slots: [0,2n) sincos, [2n,8n) f, (trees: [8n,20n) link motions / composites,) then n*n H, n rhs/x, n dinv,
 // 2n carried (q, dq).  tip != 0 adds the tip-pose terms of RbTipCost (row RB_CW_TIP of cost_w), each running term of
-// q_t from the sin/cos step t computes for q_t, as rb_rollout_kernel does.  The per-step solve
+// q_t from the sin/cos step t computes for q_t, as rb_rollout_kernel does; COL (with tip) adds the collision-sphere
+// terms of RbCollisionCost (the block at cost_w + RB_CW_COL) on the same schedule.  The per-step solve
 // still factorises H in the per-thread global scratch (slow for long chains; rollouts of long chains are not a
 // BASELINE.json configuration).
+template <bool COL = false>
 __global__ void __launch_bounds__(RB_BLOCK)
 rbn_rollout_kernel(RbNParam P, const double* __restrict__ q0, const double* __restrict__ dq0, const double* __restrict__ tau,
                    double dt, int horizon, double* __restrict__ q_traj, double* __restrict__ dq_traj,
@@ -279,6 +281,7 @@ rbn_rollout_kernel(RbNParam P, const double* __restrict__ q0, const double* __re
                 double run, fin;
                 rbn_tip_terms(P, sc_sincos, cost_w + RB_CW_TIP * RB_MAX_N, run, fin);
                 J = fma(dt, run, J);
+                if constexpr (COL) J = fma(dt, cost_w[RB_CW_COL + RB_CL_W] * rbn_col_phi(jt, n, sc_sincos, cost_w + RB_CW_COL), J);
             }
             if (P.tree) rbn_tree_rnea(jt, g, n, sc, va, dqs.base, nullptr, dqs.stride, x);
             else rbn_rnea(jt, g, n, sc, dqs.base, nullptr, dqs.stride, x);
@@ -316,6 +319,11 @@ rbn_rollout_kernel(RbNParam P, const double* __restrict__ q0, const double* __re
                 rbn_tip_terms(P, [&](int i, double* sn, double* cs) { sincos(qs[i], sn, cs); }, cost_w + RB_CW_TIP * RB_MAX_N, run, fin);
                 if (horizon > 0) J = fma(dt, run, J);
                 J += fin;
+                if constexpr (COL) {
+                    const double phi = rbn_col_phi(jt, n, [&](int i, double* sn, double* cs) { sincos(qs[i], sn, cs); }, cost_w + RB_CW_COL);
+                    if (horizon > 0) J = fma(dt, cost_w[RB_CW_COL + RB_CL_W] * phi, J);
+                    J = fma(cost_w[RB_CW_COL + RB_CL_WF], phi, J);
+                }
             }
             __stcs(cost + s, ok_s ? J : __longlong_as_double(0x7ff8000000000000LL));
         }
@@ -331,7 +339,8 @@ rbn_rollout_kernel(RbNParam P, const double* __restrict__ q0, const double* __re
 // launch per step.  The per-thread factorisation of rbn_rollout_kernel touches O(n^3) scratch words per step; here the
 // state (q, dq) and qdd of all trajectories live in three [n][B] scratch arrays between the launches.
 // tip != NULL (the model, RbNParam::model) adds the tip-pose terms of the state reached: forward dynamics runs in
-// another kernel, so the pose takes its own sin/cos of q_{t+1} here.
+// another kernel, so the pose takes its own sin/cos of q_{t+1} here.  COL (with tip) adds the collision-sphere terms the same way.
+template <bool COL = false>
 __global__ void __launch_bounds__(RB_BLOCK)
 rbn_euler_kernel(int n, double dt, double* __restrict__ qc, double* __restrict__ dqc, const double* __restrict__ qdd,
                  const double* __restrict__ tau_t, double* __restrict__ q_out, double* __restrict__ dq_out, size_t B, size_t ldc,
@@ -370,6 +379,13 @@ rbn_euler_kernel(int n, double dt, double* __restrict__ qc, double* __restrict__
         rb_tip_terms(R, x, cost_w + RB_CW_TIP * RB_MAX_N, run, fin);
         c += run;
         if (last) term += fin;
+        if constexpr (COL) {
+            const double* col = cost_w + RB_CW_COL;
+            const double phi = rbn_col_phi(reinterpret_cast<const RbJointK*>(tip), n,
+                                           [&](int i, double* sn, double* cs) { sincos(qc[(size_t)i * ldc + s], sn, cs); }, col);
+            c = fma(col[RB_CL_W], phi, c);
+            if (last) term = fma(col[RB_CL_WF], phi, term);
+        }
     }
     if (cost) {
         const double J = fma(dt, c, first ? 0.0 : cost[s]);
@@ -460,7 +476,7 @@ cudaError_t n_jac(const void* param, const double* q, double* J, size_t B, size_
 }
 cudaError_t n_rollout_any(const void* param, const double* q0, const double* dq0, const double* tau, double dt, int horizon,
                           double* q_traj, double* dq_traj, double* q_fin, double* dq_fin, size_t B, size_t ld, int* status,
-                          const double* cost_w, double* cost, bool tip, cudaStream_t st) {
+                          const double* cost_w, double* cost, bool tip, bool col, cudaStream_t st) {
     const RbNParam* P = (const RbNParam*)param;
     if (B == 0) return cudaSuccess;
 #if RB_WARP_FD
@@ -482,7 +498,7 @@ cudaError_t n_rollout_any(const void* param, const double* q0, const double* dq0
                 if (e != cudaSuccess) return e;
                 e = rb_launch_warp_fd(P->model, n, qc, dqc, tc, acc, cnt, cnt, status, st);
                 if (e != cudaSuccess) return e;
-                rbn_euler_kernel<<<(unsigned)((cnt + RB_BLOCK - 1) / RB_BLOCK), RB_BLOCK, 0, st>>>(
+                (col ? rbn_euler_kernel<true> : rbn_euler_kernel<false>)<<<(unsigned)((cnt + RB_BLOCK - 1) / RB_BLOCK), RB_BLOCK, 0, st>>>(
                     n, dt, qc, dqc, acc, tau_t, q_traj ? q_traj + (size_t)t * step + off : nullptr,
                     dq_traj ? dq_traj + (size_t)t * step + off : nullptr, cnt, cnt, ld, cost_w, cost ? cost + off : nullptr,
                     t == 0, t == horizon - 1, q_fin ? q_fin + off : nullptr, dq_fin ? dq_fin + off : nullptr, tip ? P->model : nullptr);
@@ -493,19 +509,24 @@ cudaError_t n_rollout_any(const void* param, const double* q0, const double* dq0
         return cudaSuccess;
     }
 #endif
-    rbn_rollout_kernel<<<ngrid(P, B), RB_BLOCK, 0, st>>>(*P, q0, dq0, tau, dt, horizon, q_traj, dq_traj, q_fin, dq_fin, B, ld, status, cost_w, cost,
-                                                         tip ? 1 : 0);
+    (col ? rbn_rollout_kernel<true> : rbn_rollout_kernel<false>)<<<ngrid(P, B), RB_BLOCK, 0, st>>>(
+        *P, q0, dq0, tau, dt, horizon, q_traj, dq_traj, q_fin, dq_fin, B, ld, status, cost_w, cost, tip ? 1 : 0);
     return cudaGetLastError();
 }
 cudaError_t n_rollout(const void* param, const double* q0, const double* dq0, const double* tau, double dt, int horizon,
                       double* q_traj, double* dq_traj, double* q_fin, double* dq_fin, size_t B, size_t ld, int* status,
                       const double* cost_w, double* cost, cudaStream_t st) {
-    return n_rollout_any(param, q0, dq0, tau, dt, horizon, q_traj, dq_traj, q_fin, dq_fin, B, ld, status, cost_w, cost, false, st);
+    return n_rollout_any(param, q0, dq0, tau, dt, horizon, q_traj, dq_traj, q_fin, dq_fin, B, ld, status, cost_w, cost, false, false, st);
 }
 cudaError_t n_rollout_tip(const void* param, const double* q0, const double* dq0, const double* tau, double dt, int horizon,
                           double* q_traj, double* dq_traj, double* q_fin, double* dq_fin, size_t B, size_t ld, int* status,
                           const double* cost_w, double* cost, cudaStream_t st) {
-    return n_rollout_any(param, q0, dq0, tau, dt, horizon, q_traj, dq_traj, q_fin, dq_fin, B, ld, status, cost_w, cost, true, st);
+    return n_rollout_any(param, q0, dq0, tau, dt, horizon, q_traj, dq_traj, q_fin, dq_fin, B, ld, status, cost_w, cost, true, false, st);
+}
+cudaError_t n_rollout_col(const void* param, const double* q0, const double* dq0, const double* tau, double dt, int horizon,
+                          double* q_traj, double* dq_traj, double* q_fin, double* dq_fin, size_t B, size_t ld, int* status,
+                          const double* cost_w, double* cost, cudaStream_t st) {
+    return n_rollout_any(param, q0, dq0, tau, dt, horizon, q_traj, dq_traj, q_fin, dq_fin, B, ld, status, cost_w, cost, true, true, st);
 }
 }  // namespace
 
@@ -514,7 +535,7 @@ const RbOps* rb_ops_generic_n() {
         RbOps o{};
         o.name = "generic-n"; o.param_bytes = sizeof(RbNParam); o.shared_scratch = true;
         o.rnea = &n_rnea; o.fd = &n_fd; o.crba = &n_crba; o.fwd_kin = &n_fk; o.jac = &n_jac; o.rollout = &n_rollout;
-        o.rollout_tip = &n_rollout_tip;
+        o.rollout_tip = &n_rollout_tip; o.rollout_col = &n_rollout_col;
         return o;
     }();
     return &ops;

@@ -39,5 +39,15 @@ enum : int { RB_GEN = 0, RB_ZERO = 1, RB_ONE = 2, RB_NEG1 = 3 };
 // running / terminal orientation weights.
 enum : int { RB_TW_OFFSET = 0, RB_TW_PREF = 3, RB_TW_WP = 6, RB_TW_WPF = 9, RB_TW_RREF = 12, RB_TW_WR = 21, RB_TW_WRF = 22, RB_TW_COUNT = 23 };
 
+// Collision-sphere cost terms (RbCollisionCost in rigidbody.h), packed by the host into the block behind the cost-weight
+// rows (doubles): margin, running / terminal weight, the numbers of sphere and half-space obstacles, per link l the first
+// sphere index (entry l; entry n = the sphere count), the obstacles (4 each: sphere ones first, then half-spaces with
+// unit normals), and the spheres grouped by link (4 each: centre in the link's engine frame, radius).
+#define RB_CL_MAX_SPHERES 256    // RB_MAX_SPHERES
+#define RB_CL_MAX_OBSTACLES 64   // RB_MAX_OBSTACLES
+enum : int { RB_CL_MARGIN = 0, RB_CL_W = 1, RB_CL_WF = 2, RB_CL_NOS = 3, RB_CL_NOH = 4, RB_CL_TAB = 5,
+             RB_CL_OBS = RB_CL_TAB + RB_MAX_N + 1, RB_CL_SPH = RB_CL_OBS + 4 * RB_CL_MAX_OBSTACLES,
+             RB_CL_COUNT = RB_CL_SPH + 4 * RB_CL_MAX_SPHERES };
+
 // Field selectors for the model policy accessors.
 enum : int { RB_F_R = 0, RB_F_T = 1, RB_F_M = 2, RB_F_H = 3, RB_F_I = 4 };

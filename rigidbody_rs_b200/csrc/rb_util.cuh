@@ -43,6 +43,7 @@ struct RbAdjointArgs {
     double *grad_tau, *grad_q0, *grad_dq0;
     double dt; int horizon;
     bool tip = false;                                    // with cost_w: add the tip-pose terms of its RB_CW_TIP row
+    bool col = false;                                    // with cost_w and tip: add the collision terms of its block at RB_CW_COL
 };
 cudaError_t rb_launch_rollout_adjoint(int n, const double* flat_model, const RbAdjointArgs& a, size_t B, size_t ld, int* status,
                                       cudaStream_t st);
@@ -59,6 +60,13 @@ struct RbIkParam {
 };
 cudaError_t rb_launch_tip_pose(const double* model, int n, const double* offset, const double* q, double* pose, size_t B,
                                size_t ld, cudaStream_t st);
+// Pose of every link in its descriptor frame (rb_kernels_ik.cu): [12 n][ld], per link P then R row-major; link_rot = device
+// [n][9] rotations Q_l^T taking each engine frame to the descriptor one.
+cudaError_t rb_launch_link_poses(const double* model, const double* link_rot, int n, const double* q, double* pose, size_t B,
+                                 size_t ld, cudaStream_t st);
+// min d and Phi (rb_col_link) per state: [2][ld]; col = the device collision block (RB_CL_* entries).
+cudaError_t rb_launch_sphere_distance(const double* model, int n, const double* col, const double* q, double* out, size_t B,
+                                      size_t ld, cudaStream_t st);
 // out: [n + 3][ld] = q, position error, rotation angle error, iterations (-1 = not converged).  Takes a stream-ordered
 // workspace of n doubles per thread of the grid (cudaMallocAsync on st).
 cudaError_t rb_launch_ik(const double* model, int n, const RbIkParam& P, const double* q_init, const double* p_target,

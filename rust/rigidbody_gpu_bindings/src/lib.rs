@@ -129,6 +129,18 @@ extern "C" {
                                     n_states: usize, ld: usize, layout: RbLayout, mem: RbMem, stream: *mut c_void) -> c_int;
     pub fn multibody_ik_batch(g: *mut RbGpu, q_init: *const f64, p_target: *const f64, r_target: *const f64, opt: *const RbIkOptions,
                               out: *mut f64, n_problems: usize, ld: usize, layout: RbLayout, mem: RbMem, stream: *mut c_void) -> c_int;
+    pub fn multibody_link_poses_batch(g: *mut RbGpu, q: *const f64, pose: *mut f64, n_states: usize, ld: usize, layout: RbLayout,
+                                      mem: RbMem, stream: *mut c_void) -> c_int;
+    pub fn multibody_sphere_distance_batch(g: *mut RbGpu, q: *const f64, col: *const RbCollisionCost, out: *mut f64, n_states: usize,
+                                           ld: usize, layout: RbLayout, mem: RbMem, stream: *mut c_void) -> c_int;
+    pub fn multibody_rollout_collision_cost(g: *mut RbGpu, q0: *const f64, dq0: *const f64, tau: *const f64, dt: f64, horizon: c_int,
+                                            w: *const RbQuadCost, tip: *const RbTipCost, col: *const RbCollisionCost, cost: *mut f64,
+                                            q_final: *mut f64, dq_final: *mut f64, n_traj: usize, ld: usize, layout: RbLayout, mem: RbMem,
+                                            stream: *mut c_void) -> c_int;
+    pub fn multibody_rollout_collision_cost_grad(g: *mut RbGpu, q0: *const f64, dq0: *const f64, tau: *const f64, dt: f64, horizon: c_int,
+                                                 w: *const RbQuadCost, tip: *const RbTipCost, col: *const RbCollisionCost, cost: *mut f64,
+                                                 grad_tau: *mut f64, grad_q0: *mut f64, grad_dq0: *mut f64, n_traj: usize, ld: usize,
+                                                 layout: RbLayout, mem: RbMem, stream: *mut c_void) -> c_int;
     // ---- device-side helpers
     pub fn multibody_gpu_fill(g: *mut RbGpu, dev_out: *mut f64, seed: u64, field: u32, lo: *const f64, hi: *const f64,
                               first_index: usize, count: usize, ld: usize, stream: *mut c_void) -> c_int;
@@ -167,6 +179,32 @@ pub struct RbTipCost {
     pub r_ref: *const f64,
     pub w_r: f64,
     pub w_r_final: f64,
+}
+
+/// Obstacle kinds of `RbCollisionCost` (include/rigidbody.h RbObstacleKind).
+#[repr(C)]
+#[derive(Clone, Copy, Debug, PartialEq, Eq)]
+pub enum RbObstacleKind {
+    Sphere = 0,
+    HalfSpace = 1,
+}
+
+/// Collision-sphere terms (include/rigidbody.h RbCollisionCost, where the penalty is stated): `n_spheres` spheres fixed to
+/// links (`link`, `center` 3 per sphere in the link's frame, `radius`) and `n_obstacles` obstacles (`kind`, `obstacle` 4
+/// each: centre and radius, or normal and offset).  `kind` points to `RbObstacleKind` values as 32-bit integers.
+#[repr(C)]
+#[derive(Clone, Copy)]
+pub struct RbCollisionCost {
+    pub n_spheres: i32,
+    pub link: *const i32,
+    pub center: *const f64,
+    pub radius: *const f64,
+    pub n_obstacles: i32,
+    pub kind: *const i32,
+    pub obstacle: *const f64,
+    pub margin: f64,
+    pub w: f64,
+    pub w_final: f64,
 }
 
 /// Options of `multibody_ik_batch` (include/rigidbody.h RbIkOptions, where the algorithm is stated): host arrays of 3
@@ -404,6 +442,28 @@ impl GpuMultibody {
         check(unsafe { multibody_rollout_tip_cost_grad(self.raw, q0.as_ptr(), dq0.as_ptr(), tau.as_ptr(), dt, horizon as c_int, w, tip,
                                                        cost.as_mut_ptr(), grad_tau.as_mut_ptr(), grad_q0.as_mut_ptr(), grad_dq0.as_mut_ptr(),
                                                        n_traj, 0, layout, RbMem::Host, ptr::null_mut()) })
+    }
+
+    /// Pose of every link's frame (multibody_link_poses_batch), host slices: `pose` 12 n values per state, per link P then
+    /// R row-major.
+    pub fn link_poses(&mut self, q: &[f64], pose: &mut [f64], n_states: usize, layout: RbLayout) -> Result<(), RbError> {
+        self.check_len("q", q.len(), self.n, n_states)?;
+        self.check_len("pose", pose.len(), 12 * self.n, n_states)?;
+        check(unsafe { multibody_link_poses_batch(self.raw, q.as_ptr(), pose.as_mut_ptr(), n_states, 0, layout, RbMem::Host, ptr::null_mut()) })
+    }
+
+    /// `rollout_tip_cost` with the collision-sphere terms of `col` added (multibody_rollout_collision_cost); host slices,
+    /// `cost` one value per trajectory.
+    #[allow(clippy::too_many_arguments)]
+    pub fn rollout_collision_cost(&mut self, q0: &[f64], dq0: &[f64], tau: &[f64], dt: f64, horizon: usize, w: &RbQuadCost, tip: &RbTipCost,
+                                  col: &RbCollisionCost, cost: &mut [f64], n_traj: usize, layout: RbLayout) -> Result<(), RbError> {
+        self.check_len("q0", q0.len(), self.n, n_traj)?;
+        self.check_len("dq0", dq0.len(), self.n, n_traj)?;
+        self.check_len("tau", tau.len(), self.n * horizon, n_traj)?;
+        self.check_len("cost", cost.len(), 1, n_traj)?;
+        check(unsafe { multibody_rollout_collision_cost(self.raw, q0.as_ptr(), dq0.as_ptr(), tau.as_ptr(), dt, horizon as c_int, w, tip, col,
+                                                        cost.as_mut_ptr(), ptr::null_mut(), ptr::null_mut(), n_traj, 0, layout, RbMem::Host,
+                                                        ptr::null_mut()) })
     }
 
     /// Inverse kinematics of the tip frame (multibody_ik_batch): one damped least-squares problem per entry, host slices.
