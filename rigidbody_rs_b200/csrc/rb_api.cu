@@ -124,7 +124,6 @@ struct RbGpu {
     // bound by bind_entries; the optional entries (rnea_aos, fd_aos, rnea_fd, rnea_f32, fd_f32) are the primary family's alone
     Bound<decltype(RbOps::rnea)> rnea; Bound<decltype(RbOps::fd)> fd; Bound<decltype(RbOps::crba)> crba;
     Bound<decltype(RbOps::fwd_kin)> fwd_kin; Bound<decltype(RbOps::jac)> jac; Bound<decltype(RbOps::rollout)> rollout;
-    Bound<decltype(RbOps::rollout_tip)> rollout_tip; Bound<decltype(RbOps::rollout_col)> rollout_col;
     size_t hpk_states = 0;
     RbJitParam jit{};                     // run-time compiled kernels (jit-specialised family); lib == nullptr if unused
     std::string family_note;              // why this family was chosen (e.g. the JIT fallback reason)
@@ -309,7 +308,7 @@ int pick_ops(RbGpu* g) {
     return setup_generic_n(g, &g->param);
 }
 
-// Binds rnea, fd, crba, fwd_kin, jac, rollout, rollout_tip and rollout_col once: to the primary family where it has the entry, otherwise to the
+// Binds rnea, fd, crba, fwd_kin, jac and rollout once: to the primary family where it has the entry, otherwise to the
 // fallback table, whose parameter block pick_ops set up for the families that need it.
 int bind_entries(RbGpu* g) {
     bool ok = true;
@@ -321,7 +320,6 @@ int bind_entries(RbGpu* g) {
     };
     bind(g->rnea, &RbOps::rnea); bind(g->fd, &RbOps::fd); bind(g->crba, &RbOps::crba);
     bind(g->fwd_kin, &RbOps::fwd_kin); bind(g->jac, &RbOps::jac); bind(g->rollout, &RbOps::rollout);
-    bind(g->rollout_tip, &RbOps::rollout_tip); bind(g->rollout_col, &RbOps::rollout_col);
     return ok ? RB_OK : fail(RB_ERR_ARG, std::string("internal: kernel family '") + g->ops->name + "' leaves an entry point unbound");
 }
 
@@ -1284,12 +1282,17 @@ int pack_cost_weights(int n, const RbQuadCost* w, double* cw) {
     return RB_OK;
 }
 
-// The whole cost-weight block of a cost call: the RB_CW_* rows, the RB_CW_TIP row when tip terms are on, and the
-// collision block (at RB_CW_COL) when collision terms are on.
+// The whole cost-weight block of a cost call and the terms it carries: the RB_CW_* rows, the RB_CW_TIP row with tip
+// terms, and the collision block (at RB_CW_COL) with collision terms.  bytes() = the part a call uploads.
 struct CostBlock {
     double w[RB_CW_DOUBLES_COL];
-    bool tip, col;
-    size_t bytes() const { return sizeof(double) * (col ? RB_CW_DOUBLES_COL : (tip ? RB_CW_ROWS_TIP : RB_CW_ROWS) * RB_MAX_N); }
+    RbCostTerms terms = RB_COST_QUAD;
+    size_t bytes() const {
+        const size_t doubles = terms == RB_COST_TIP_COL ? (size_t)RB_CW_DOUBLES_COL
+                             : terms == RB_COST_TIP     ? (size_t)RB_CW_ROWS_TIP * RB_MAX_N
+                                                        : (size_t)RB_CW_ROWS * RB_MAX_N;
+        return sizeof(double) * doubles;
+    }
 };
 
 // Checks the terms of an RbTipCost and packs them into row RB_CW_TIP (RB_TW_* entries).  `on` = some weight is not
@@ -1315,12 +1318,14 @@ int pack_tip_weights(const RbTipCost* t, double* row, bool* on) {
     return RB_OK;
 }
 
-// Checks and packs every part of a cost call's weights.  Collision terms run in the kernels that carry the tip terms
-// too: with collision terms on, the tip row is uploaded whatever its weights.
+// Checks and packs every part of a cost call's weights, and picks its terms from those that are on.  Collision terms run
+// in the kernels that carry the tip terms too: with collision terms on, the tip row is uploaded whatever its weights.
 int pack_cost_block(const RbHostModel& m, const RbQuadCost* w, const RbTipCost* tip, const RbCollisionCost* col, CostBlock& cb) {
+    bool tip_on = false, col_on = false;
     int rc = pack_cost_weights(m.n, w, cb.w);
-    if (rc == RB_OK) rc = pack_tip_weights(tip, cb.w + RB_CW_TIP * RB_MAX_N, &cb.tip);
-    if (rc == RB_OK) rc = pack_collision(m, col, cb.w + RB_CW_COL, &cb.col);
+    if (rc == RB_OK) rc = pack_tip_weights(tip, cb.w + RB_CW_TIP * RB_MAX_N, &tip_on);
+    if (rc == RB_OK) rc = pack_collision(m, col, cb.w + RB_CW_COL, &col_on);
+    cb.terms = col_on ? RB_COST_TIP_COL : tip_on ? RB_COST_TIP : RB_COST_QUAD;
     return rc;
 }
 
@@ -1355,41 +1360,37 @@ int rollout_impl(RbGpu* g, const double* q0, const double* dq0, const double* ta
     if (horizon == 0 && !q_final && !dq_final && !cost) return RB_OK;
     if (!q0 || !dq0 || (!tau && horizon > 0)) return fail(RB_ERR_NULL, "input pointer is NULL");
     if (layout == RB_LAYOUT_SOA) { if (ld == 0) ld = n_traj; if (ld < n_traj) return fail(RB_ERR_ARG, "ld < n_traj"); }
-    const int n = g->model.n;
     if (cost && !w) return fail(RB_ERR_NULL, "cost weights are NULL");
     DeviceGuard dg(g->device);
     if (!dg.ok) return fail(RB_ERR_CUDA, "cudaSetDevice failed");
     cudaStream_t st = mem == RB_MEM_DEVICE ? (cudaStream_t)stream : g->stream;
-    // cost weights -> the engine's device block (shared by all cost rollouts, hence ordered like scratch)
     CostBlock cb;
-    cb.tip = cb.col = false;
     if (cost) { const int rc = pack_cost_block(g->model, w, tip, col, cb); if (rc != RB_OK) return rc; }
-    const auto& ro = cb.col ? g->rollout_col : cb.tip ? g->rollout_tip : g->rollout;
-    const bool shared = cost != nullptr || ro.shared;
-    if (mem == RB_MEM_DEVICE && layout == RB_LAYOUT_SOA) {
-        ScratchOrder so(g, shared, st);
-        if (cost) RB_CUDA(cudaMemcpyAsync(g->cost_w.p, cb.w, cb.bytes(), cudaMemcpyHostToDevice, st));
-        cudaError_t e = ro.fn(ro.param, q0, dq0, tau, dt, horizon, q_traj, dq_traj, q_final, dq_final,
-                              n_traj, ld, g->d_status, cost ? g->cost_w.p : nullptr, cost, st);
-        g->launches += 1;
-        if (e != cudaSuccess) return fail_cuda(e, "rollout launch");
-        return RB_OK;
-    }
-    // Host pointers and/or AoS: stage everything on the device as SoA with ld = n_traj, run once, bring results back.
-    const size_t H = (size_t)horizon;
-    return run_staged(g, {{q0, 1}, {dq0, 1}, {tau, H}}, {{q_traj, H, false}, {dq_traj, H, false}, {q_final, 1, false}, {dq_final, 1, false}, {cost, 1, true}},
-                      n_traj, ld, layout, mem, aos_stride, st, [&](const double* const* in, double* const* out, int* d_stat) -> int {
+    // One rollout over device SoA arrays: in = (q0, dq0, tau), out = (q_traj, dq_traj, q_final, dq_final, cost).  The cost
+    // weights go to the engine's device block, shared by all cost rollouts and hence ordered like scratch.
+    auto run = [&](const double* const* in, double* const* out, size_t ldr, int* d_stat) -> int {
+        const auto& ro = g->rollout;
         cudaError_t e;
         {
-            ScratchOrder so(g, shared, st);
+            ScratchOrder so(g, cost != nullptr || ro.shared, st);
             if (cost) RB_CUDA(cudaMemcpyAsync(g->cost_w.p, cb.w, cb.bytes(), cudaMemcpyHostToDevice, st));
-            e = ro.fn(ro.param, in[0], in[1], in[2], dt, horizon, out[0], out[1], out[2], out[3], n_traj, n_traj, d_stat,
-                      cost ? g->cost_w.p : nullptr, out[4], st);
+            e = ro.fn(ro.param, in[0], in[1], in[2], dt, horizon, out[0], out[1], out[2], out[3], n_traj, ldr, d_stat,
+                      cost ? g->cost_w.p : nullptr, out[4], cb.terms, st);
         }
         g->launches += 1;
         if (e != cudaSuccess) return fail_cuda(e, "rollout launch");
         return RB_OK;
-    });
+    };
+    if (mem == RB_MEM_DEVICE && layout == RB_LAYOUT_SOA) {
+        const double* const in[] = {q0, dq0, tau};
+        double* const out[] = {q_traj, dq_traj, q_final, dq_final, cost};
+        return run(in, out, ld, g->d_status);
+    }
+    // Host pointers and/or AoS: stage everything on the device as SoA with ld = n_traj, run once, bring results back.
+    const size_t H = (size_t)horizon;
+    return run_staged(g, {{q0, 1}, {dq0, 1}, {tau, H}}, {{q_traj, H, false}, {dq_traj, H, false}, {q_final, 1, false}, {dq_final, 1, false}, {cost, 1, true}},
+                      n_traj, ld, layout, mem, aos_stride, st,
+                      [&](const double* const* in, double* const* out, int* d_stat) { return run(in, out, n_traj, d_stat); });
 }
 // Arguments of multibody_rollout_vjp (q_traj .. g_dqf) and multibody_rollout_cost_grad (w, cost).
 struct GradArgs {
@@ -1420,9 +1421,8 @@ int grad_device(RbGpu* g, const GradArgs& a, const CostBlock& cb, size_t B, size
     ScratchOrder so(g, true, st);
     RB_CUDA(cudaMemcpyAsync(g->cost_w.p, cb.w, cb.bytes(), cudaMemcpyHostToDevice, st));
     ad.cost_w = g->cost_w.p;
-    ad.tip = cb.tip || cb.col;
-    ad.col = cb.col;
-    const auto& ro = cb.col ? g->rollout_col : cb.tip ? g->rollout_tip : g->rollout;
+    ad.terms = cb.terms;
+    const auto& ro = g->rollout;
     const size_t H = (size_t)a.horizon, nn = (size_t)n;
     // A rollout writes its trajectory with the leading dimension of its inputs: a chunk whose inputs are not already a
     // dense [n][chunk] block (a cut batch, a padded ld) gets a dense copy of them next to its trajectory.
@@ -1449,7 +1449,7 @@ int grad_device(RbGpu* g, const GradArgs& a, const CostBlock& cb, size_t B, size
             if (e != cudaSuccess) { rc = fail_cuda(e, "cudaMemcpy2DAsync(gradient workspace)"); break; }
             rq0 = in; rdq0 = in + nn * cnt; rtau = in + 2 * nn * cnt;
         }
-        e = ro.fn(ro.param, rq0, rdq0, rtau, a.dt, a.horizon, qt, dqt, nullptr, nullptr, cnt, lw, d_stat, g->cost_w.p, a.cost + lo, st);
+        e = ro.fn(ro.param, rq0, rdq0, rtau, a.dt, a.horizon, qt, dqt, nullptr, nullptr, cnt, lw, d_stat, g->cost_w.p, a.cost + lo, cb.terms, st);
         g->launches += 1;
         if (e != cudaSuccess) { rc = fail_cuda(e, "rollout launch"); break; }
         RbAdjointArgs c = ad;
@@ -1500,7 +1500,6 @@ int grad_impl(RbGpu* g, const GradArgs& a, size_t n_traj, size_t ld, RbLayout la
     if (!a.q0 || !a.dq0 || (H > 0 && (!a.tau || (!cost && (!a.q_traj || !a.dq_traj))))) return fail(RB_ERR_NULL, "input pointer is NULL");
     if (layout == RB_LAYOUT_SOA) { if (ld == 0) ld = n_traj; if (ld < n_traj) return fail(RB_ERR_ARG, "ld < n_traj"); }
     CostBlock cb;
-    cb.tip = cb.col = false;
     if (cost) { const int rc = pack_cost_block(g->model, a.w, a.tip, a.col, cb); if (rc != RB_OK) return rc; }
     if (!cost && !a.grad_tau && !a.grad_q0 && !a.grad_dq0) return RB_OK;
     DeviceGuard dg(g->device);

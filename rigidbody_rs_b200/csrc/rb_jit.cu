@@ -307,21 +307,9 @@ cudaError_t j_jac(const void* p, const double* q, double* J, size_t B, size_t ld
 }
 cudaError_t j_rollout(const void* p, const double* q0, const double* dq0, const double* tau, double dt, int horizon,
                       double* q_traj, double* dq_traj, double* q_fin, double* dq_fin, size_t B, size_t ld, int* status,
-                      const double* cost_w, double* cost, cudaStream_t st) {
-    return jlaunch(p, RB_JK_ROLLOUT, RB_RO_BLOCK, 0, B, st, q0, dq0, tau, dt, horizon, q_traj, dq_traj, q_fin, dq_fin, B, ld,
-                   status, cost_w, cost);
-}
-cudaError_t j_rollout_tip(const void* p, const double* q0, const double* dq0, const double* tau, double dt, int horizon,
-                          double* q_traj, double* dq_traj, double* q_fin, double* dq_fin, size_t B, size_t ld, int* status,
-                          const double* cost_w, double* cost, cudaStream_t st) {
-    return jlaunch(p, RB_JK_ROLLOUT_TIP, RB_RO_BLOCK, 0, B, st, q0, dq0, tau, dt, horizon, q_traj, dq_traj, q_fin, dq_fin, B, ld,
-                   status, cost_w, cost);
-}
-cudaError_t j_rollout_col(const void* p, const double* q0, const double* dq0, const double* tau, double dt, int horizon,
-                          double* q_traj, double* dq_traj, double* q_fin, double* dq_fin, size_t B, size_t ld, int* status,
-                          const double* cost_w, double* cost, cudaStream_t st) {
-    return jlaunch(p, RB_JK_ROLLOUT_COL, RB_RO_BLOCK, 0, B, st, q0, dq0, tau, dt, horizon, q_traj, dq_traj, q_fin, dq_fin, B, ld,
-                   status, cost_w, cost);
+                      const double* cost_w, double* cost, RbCostTerms terms, cudaStream_t st) {
+    const int k = terms == RB_COST_TIP_COL ? RB_JK_ROLLOUT_COL : terms == RB_COST_TIP ? RB_JK_ROLLOUT_TIP : RB_JK_ROLLOUT;
+    return jlaunch(p, k, RB_RO_BLOCK, 0, B, st, q0, dq0, tau, dt, horizon, q_traj, dq_traj, q_fin, dq_fin, B, ld, status, cost_w, cost);
 }
 cudaError_t j_rnea_f32(const void* p, const float* q, const float* dq, const float* ddq, float* tau, size_t B, size_t ld, cudaStream_t st) {
     return jlaunch(p, RB_JK_RNEA_F32, RB_BLOCK, 0, B, st, q, dq, ddq, tau, B, ld);
@@ -350,7 +338,7 @@ const RbOps* rb_ops_jit() {
         RbOps o{};
         o.name = "jit-specialised"; o.param_bytes = sizeof(RbJitParam);
         o.rnea = &j_rnea; o.fd = &j_fd; o.rnea_aos = &j_rnea_aos; o.fd_aos = &j_fd_aos; o.crba = &j_crba; o.fwd_kin = &j_fk;
-        o.jac = &j_jac; o.rollout = &j_rollout; o.rollout_tip = &j_rollout_tip; o.rollout_col = &j_rollout_col; o.rnea_f32 = &j_rnea_f32; o.fd_f32 = &j_fd_f32; o.rnea_fd = &j_rnea_fd;
+        o.jac = &j_jac; o.rollout = &j_rollout; o.rnea_f32 = &j_rnea_f32; o.fd_f32 = &j_fd_f32; o.rnea_fd = &j_rnea_fd;
         return o;
     }();
     return &ops;

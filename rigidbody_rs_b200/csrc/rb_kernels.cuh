@@ -71,17 +71,12 @@ struct RbOps {
     cudaError_t (*crba)(const void* param, const double* q, double* H, size_t B, size_t ld, cudaStream_t st);
     cudaError_t (*fwd_kin)(const void* param, const double* q, double* xyz, size_t B, size_t ld, cudaStream_t st);
     cudaError_t (*jac)(const void* param, const double* q, double* J, size_t B, size_t ld, cudaStream_t st);
+    // `terms` picks the cost terms, and with them the kernel: RB_COST_TIP adds those of RbTipCost (cost_w carries the
+    // RB_CW_TIP row), RB_COST_TIP_COL those of RbCollisionCost as well (cost_w carries the tip row and the block at RB_CW_COL)
     cudaError_t (*rollout)(const void* param, const double* q0, const double* dq0, const double* tau, double dt,
                            int horizon, double* q_traj, double* dq_traj, double* q_fin, double* dq_fin,
-                           size_t B, size_t ld, int* status, const double* cost_w, double* cost, cudaStream_t st);
-    // the same rollout with the tip-pose terms of RbTipCost added to the cost (cost_w carries the RB_CW_TIP row)
-    cudaError_t (*rollout_tip)(const void* param, const double* q0, const double* dq0, const double* tau, double dt,
-                               int horizon, double* q_traj, double* dq_traj, double* q_fin, double* dq_fin,
-                               size_t B, size_t ld, int* status, const double* cost_w, double* cost, cudaStream_t st);
-    // ... with the collision-sphere terms of RbCollisionCost added as well (cost_w carries the tip row and the block at RB_CW_COL)
-    cudaError_t (*rollout_col)(const void* param, const double* q0, const double* dq0, const double* tau, double dt,
-                               int horizon, double* q_traj, double* dq_traj, double* q_fin, double* dq_fin,
-                               size_t B, size_t ld, int* status, const double* cost_w, double* cost, cudaStream_t st);
+                           size_t B, size_t ld, int* status, const double* cost_w, double* cost, RbCostTerms terms,
+                           cudaStream_t st);
     // optional fp32 mode (BASELINE.json: "an optional fp32 mode is held to a stated 1e-4 tolerance"): the same kernels
     // instantiated with Real = float, device-resident SoA batches only (null = family has no fp32 kernels)
     cudaError_t (*rnea_f32)(const void* param, const float* q, const float* dq, const float* ddq, float* tau,
@@ -320,7 +315,8 @@ rb_jac_kernel(const __grid_constant__ typename M::Param p, const RB_R* __restric
 // the pose of q_{t+1} right after the integration would pay a second sin/cos of every joint per step instead.
 // COL (with TIP) adds the collision-sphere terms of RbCollisionCost (the block at cost_w + RB_CW_COL, RB_CL_* entries) on
 // the same schedule: dt w Phi(q_t) at the top of step t >= 1 from that step's sin/cos, and dt w Phi(q_H) + w_final Phi(q_H)
-// after the last step.  Without collision terms the caller runs the TIP kernel (same bits as the tip-cost call).
+// after the last step.  RbLaunch::rollout maps the RbCostTerms value of the call to <M>, <M, TIP> or <M, TIP, COL>; a
+// call whose collision terms are inactive carries RB_COST_TIP and runs the TIP kernel (same bits as the tip-cost call).
 #ifndef RB_MINB_ROLLOUT
 #define RB_MINB_ROLLOUT 2   // measured on B200 (profiles/r1_kbench_rollout.jsonl): 255 regs, 2 blocks per SM is fastest
 #endif
@@ -501,35 +497,34 @@ struct RbLaunch {
     }
     static cudaError_t rollout(const void* param, const double* q0, const double* dq0, const double* tau, double dt,
                                int horizon, double* q_traj, double* dq_traj, double* q_fin, double* dq_fin,
-                               size_t B, size_t ld, int* status, const double* cost_w, double* cost, cudaStream_t st) {
+                               size_t B, size_t ld, int* status, const double* cost_w, double* cost, RbCostTerms terms,
+                               cudaStream_t st) {
         if (B == 0) return cudaSuccess;
 #if RB_ROLLOUT_WS
         if constexpr (M::N <= RB_RO2_MAX_N) {
-            if (rb_rollout_mode() == 2) {
+            if (terms == RB_COST_QUAD && rb_rollout_mode() == 2) {
                 rb_rollout_ws_kernel<M><<<(unsigned)((B + 63) / 64), 128, 0, st>>>(*(const P*)param, q0, dq0, tau, dt, horizon, q_traj, dq_traj,
                                                                                   q_fin, dq_fin, B, ld, status, cost_w, cost);
                 return cudaGetLastError();
             }
         }
 #endif
-        rb_rollout_kernel<M><<<(unsigned)((B + RB_RO_BLOCK - 1) / RB_RO_BLOCK), RB_RO_BLOCK, 0, st>>>(
-            *(const P*)param, q0, dq0, tau, dt, horizon, q_traj, dq_traj, q_fin, dq_fin, B, ld, status, cost_w, cost);
-        return cudaGetLastError();
-    }
-    static cudaError_t rollout_tip(const void* param, const double* q0, const double* dq0, const double* tau, double dt,
-                                   int horizon, double* q_traj, double* dq_traj, double* q_fin, double* dq_fin,
-                                   size_t B, size_t ld, int* status, const double* cost_w, double* cost, cudaStream_t st) {
-        if (B == 0) return cudaSuccess;
-        rb_rollout_kernel<M, true><<<(unsigned)((B + RB_RO_BLOCK - 1) / RB_RO_BLOCK), RB_RO_BLOCK, 0, st>>>(
-            *(const P*)param, q0, dq0, tau, dt, horizon, q_traj, dq_traj, q_fin, dq_fin, B, ld, status, cost_w, cost);
-        return cudaGetLastError();
-    }
-    static cudaError_t rollout_col(const void* param, const double* q0, const double* dq0, const double* tau, double dt,
-                                   int horizon, double* q_traj, double* dq_traj, double* q_fin, double* dq_fin,
-                                   size_t B, size_t ld, int* status, const double* cost_w, double* cost, cudaStream_t st) {
-        if (B == 0) return cudaSuccess;
-        rb_rollout_kernel<M, true, true><<<(unsigned)((B + RB_RO_BLOCK - 1) / RB_RO_BLOCK), RB_RO_BLOCK, 0, st>>>(
-            *(const P*)param, q0, dq0, tau, dt, horizon, q_traj, dq_traj, q_fin, dq_fin, B, ld, status, cost_w, cost);
+        const unsigned blocks = (unsigned)((B + RB_RO_BLOCK - 1) / RB_RO_BLOCK);
+        const P& p = *(const P*)param;
+        switch (terms) {
+            case RB_COST_QUAD:
+                rb_rollout_kernel<M><<<blocks, RB_RO_BLOCK, 0, st>>>(p, q0, dq0, tau, dt, horizon, q_traj, dq_traj, q_fin, dq_fin, B, ld,
+                                                                     status, cost_w, cost);
+                break;
+            case RB_COST_TIP:
+                rb_rollout_kernel<M, true><<<blocks, RB_RO_BLOCK, 0, st>>>(p, q0, dq0, tau, dt, horizon, q_traj, dq_traj, q_fin, dq_fin,
+                                                                           B, ld, status, cost_w, cost);
+                break;
+            case RB_COST_TIP_COL:
+                rb_rollout_kernel<M, true, true><<<blocks, RB_RO_BLOCK, 0, st>>>(p, q0, dq0, tau, dt, horizon, q_traj, dq_traj, q_fin,
+                                                                                 dq_fin, B, ld, status, cost_w, cost);
+                break;
+        }
         return cudaGetLastError();
     }
     // M32 = the same policy with Real = float (fp32 mode)
@@ -552,8 +547,7 @@ struct RbLaunch {
         RbOps o{};
         o.name = name; o.param_bytes = sizeof(P);
         o.rnea = &rnea; o.fd = &fd; o.rnea_aos = &rnea_aos; o.fd_aos = &fd_aos;
-        o.crba = &crba; o.fwd_kin = &fwd_kin; o.jac = &jac; o.rollout = &rollout; o.rollout_tip = &rollout_tip;
-        o.rollout_col = &rollout_col;
+        o.crba = &crba; o.fwd_kin = &fwd_kin; o.jac = &jac; o.rollout = &rollout;
         o.rnea_fd = &rnea_fd;
         if constexpr (!std::is_void<M32>::value) { o.rnea_f32 = &rnea_f32<M32>; o.fd_f32 = &fd_f32<M32>; }
         return o;

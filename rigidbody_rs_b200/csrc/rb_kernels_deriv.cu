@@ -228,27 +228,25 @@ cudaError_t launch_fd(const double* flat, const double* q, const double* dq, con
     rb_fd_deriv_kernel<N><<<dgrid(B), RB_BLOCK, 0, st>>>(p, q, dq, tau, out, B, ld, status);
     return cudaGetLastError();
 }
+// The cost instantiations (QUAD) form their upstream gradients from cost_w; the plain vector-Jacobian product reads g_*.
+template <int N, bool QUAD, bool TIP = false, bool COL = false>
+cudaError_t launch_adjoint_as(const RbModelK<N>& p, const RbAdjointArgs& a, size_t B, size_t ld, int* status, cudaStream_t st) {
+    rb_rollout_adjoint_kernel<N, QUAD, TIP, COL><<<dgrid(B), RB_BLOCK, 0, st>>>(
+        p, a.q0, a.dq0, a.tau, a.q_traj, a.dq_traj, a.ld_traj, QUAD ? nullptr : a.g_q, QUAD ? nullptr : a.g_dq,
+        QUAD ? nullptr : a.g_qf, QUAD ? nullptr : a.g_dqf, QUAD ? a.cost_w : nullptr, a.grad_tau, a.grad_q0, a.grad_dq0,
+        a.dt, a.horizon, B, ld, status);
+    return cudaGetLastError();
+}
 template <int N>
 cudaError_t launch_adjoint(const double* flat, const RbAdjointArgs& a, size_t B, size_t ld, int* status, cudaStream_t st) {
     RbModelK<N> p;
     memcpy(&p, flat, sizeof(p));
-    if (a.cost_w && a.col)
-        rb_rollout_adjoint_kernel<N, true, true, true><<<dgrid(B), RB_BLOCK, 0, st>>>(p, a.q0, a.dq0, a.tau, a.q_traj, a.dq_traj, a.ld_traj, nullptr,
-                                                                                      nullptr, nullptr, nullptr, a.cost_w, a.grad_tau, a.grad_q0,
-                                                                                      a.grad_dq0, a.dt, a.horizon, B, ld, status);
-    else if (a.cost_w && a.tip)
-        rb_rollout_adjoint_kernel<N, true, true><<<dgrid(B), RB_BLOCK, 0, st>>>(p, a.q0, a.dq0, a.tau, a.q_traj, a.dq_traj, a.ld_traj, nullptr, nullptr,
-                                                                                nullptr, nullptr, a.cost_w, a.grad_tau, a.grad_q0, a.grad_dq0,
-                                                                                a.dt, a.horizon, B, ld, status);
-    else if (a.cost_w)
-        rb_rollout_adjoint_kernel<N, true><<<dgrid(B), RB_BLOCK, 0, st>>>(p, a.q0, a.dq0, a.tau, a.q_traj, a.dq_traj, a.ld_traj, nullptr, nullptr,
-                                                                          nullptr, nullptr, a.cost_w, a.grad_tau, a.grad_q0, a.grad_dq0,
-                                                                          a.dt, a.horizon, B, ld, status);
-    else
-        rb_rollout_adjoint_kernel<N, false><<<dgrid(B), RB_BLOCK, 0, st>>>(p, a.q0, a.dq0, a.tau, a.q_traj, a.dq_traj, a.ld_traj, a.g_q, a.g_dq,
-                                                                           a.g_qf, a.g_dqf, nullptr, a.grad_tau, a.grad_q0, a.grad_dq0,
-                                                                           a.dt, a.horizon, B, ld, status);
-    return cudaGetLastError();
+    if (a.cost_w) switch (a.terms) {
+        case RB_COST_TIP_COL: return launch_adjoint_as<N, true, true, true>(p, a, B, ld, status, st);
+        case RB_COST_TIP: return launch_adjoint_as<N, true, true>(p, a, B, ld, status, st);
+        case RB_COST_QUAD: return launch_adjoint_as<N, true>(p, a, B, ld, status, st);
+    }
+    return launch_adjoint_as<N, false>(p, a, B, ld, status, st);
 }
 }  // namespace
 

@@ -474,11 +474,12 @@ cudaError_t n_jac(const void* param, const double* q, double* J, size_t B, size_
     rbn_fk_jac_kernel<<<ngrid(P, B), RB_BLOCK, 0, st>>>(*P, q, nullptr, J, B, ld);
     return cudaGetLastError();
 }
-cudaError_t n_rollout_any(const void* param, const double* q0, const double* dq0, const double* tau, double dt, int horizon,
-                          double* q_traj, double* dq_traj, double* q_fin, double* dq_fin, size_t B, size_t ld, int* status,
-                          const double* cost_w, double* cost, bool tip, bool col, cudaStream_t st) {
+cudaError_t n_rollout(const void* param, const double* q0, const double* dq0, const double* tau, double dt, int horizon,
+                      double* q_traj, double* dq_traj, double* q_fin, double* dq_fin, size_t B, size_t ld, int* status,
+                      const double* cost_w, double* cost, RbCostTerms terms, cudaStream_t st) {
     const RbNParam* P = (const RbNParam*)param;
     if (B == 0) return cudaSuccess;
+    const bool tip = terms != RB_COST_QUAD, col = terms == RB_COST_TIP_COL;
 #if RB_WARP_FD
     if (P->n <= 32 && !P->tree && horizon > 0) {
         const int n = P->n;
@@ -513,21 +514,6 @@ cudaError_t n_rollout_any(const void* param, const double* q0, const double* dq0
         *P, q0, dq0, tau, dt, horizon, q_traj, dq_traj, q_fin, dq_fin, B, ld, status, cost_w, cost, tip ? 1 : 0);
     return cudaGetLastError();
 }
-cudaError_t n_rollout(const void* param, const double* q0, const double* dq0, const double* tau, double dt, int horizon,
-                      double* q_traj, double* dq_traj, double* q_fin, double* dq_fin, size_t B, size_t ld, int* status,
-                      const double* cost_w, double* cost, cudaStream_t st) {
-    return n_rollout_any(param, q0, dq0, tau, dt, horizon, q_traj, dq_traj, q_fin, dq_fin, B, ld, status, cost_w, cost, false, false, st);
-}
-cudaError_t n_rollout_tip(const void* param, const double* q0, const double* dq0, const double* tau, double dt, int horizon,
-                          double* q_traj, double* dq_traj, double* q_fin, double* dq_fin, size_t B, size_t ld, int* status,
-                          const double* cost_w, double* cost, cudaStream_t st) {
-    return n_rollout_any(param, q0, dq0, tau, dt, horizon, q_traj, dq_traj, q_fin, dq_fin, B, ld, status, cost_w, cost, true, false, st);
-}
-cudaError_t n_rollout_col(const void* param, const double* q0, const double* dq0, const double* tau, double dt, int horizon,
-                          double* q_traj, double* dq_traj, double* q_fin, double* dq_fin, size_t B, size_t ld, int* status,
-                          const double* cost_w, double* cost, cudaStream_t st) {
-    return n_rollout_any(param, q0, dq0, tau, dt, horizon, q_traj, dq_traj, q_fin, dq_fin, B, ld, status, cost_w, cost, true, true, st);
-}
 }  // namespace
 
 const RbOps* rb_ops_generic_n() {
@@ -535,7 +521,6 @@ const RbOps* rb_ops_generic_n() {
         RbOps o{};
         o.name = "generic-n"; o.param_bytes = sizeof(RbNParam); o.shared_scratch = true;
         o.rnea = &n_rnea; o.fd = &n_fd; o.crba = &n_crba; o.fwd_kin = &n_fk; o.jac = &n_jac; o.rollout = &n_rollout;
-        o.rollout_tip = &n_rollout_tip; o.rollout_col = &n_rollout_col;
         return o;
     }();
     return &ops;

@@ -49,5 +49,10 @@ enum : int { RB_CL_MARGIN = 0, RB_CL_W = 1, RB_CL_WF = 2, RB_CL_NOS = 3, RB_CL_N
              RB_CL_OBS = RB_CL_TAB + RB_MAX_N + 1, RB_CL_SPH = RB_CL_OBS + 4 * RB_CL_MAX_OBSTACLES,
              RB_CL_COUNT = RB_CL_SPH + 4 * RB_CL_MAX_SPHERES };
 
+// The terms a rollout's cost carries, each served by one kernel instantiation: the quadratic terms of RbQuadCost only,
+// plus the tip-pose terms (RB_TW_* row), or plus the tip-pose and the collision-sphere terms (RB_CL_* block).  Collision
+// terms run in the kernels that carry the tip terms too.
+enum RbCostTerms : int { RB_COST_QUAD = 0, RB_COST_TIP = 1, RB_COST_TIP_COL = 2 };
+
 // Field selectors for the model policy accessors.
 enum : int { RB_F_R = 0, RB_F_T = 1, RB_F_M = 2, RB_F_H = 3, RB_F_I = 4 };

@@ -33,8 +33,8 @@ cudaError_t rb_launch_fd_deriv(int n, const double* flat_model, const double* q,
                                double* out, size_t B, size_t ld, int* status, cudaStream_t st);
 // Reverse-mode pass through a rollout (rb_kernels_deriv.cu, where the recursion is stated), serial chains of
 // n <= RB_DERIV_MAX_N joints.  Device pointers; q0 / dq0 / tau / g_* / grad_* use the leading dimension `ld` of the
-// launch, the stored trajectory its own.  cost_w != NULL selects the quadratic cost of that weight block (RB_CW_*
-// rows, and the RB_CW_TIP row if `tip`) as the upstream gradient, and g_* are ignored; otherwise a NULL g_* is zero.  A NULL grad_* is not written.
+// launch, the stored trajectory its own.  cost_w != NULL selects the cost of that weight block, with the terms of
+// `terms`, as the upstream gradient, and g_* are ignored; otherwise a NULL g_* is zero.  A NULL grad_* is not written.
 struct RbAdjointArgs {
     const double *q0, *dq0, *tau;                        // [n][ld], [n][ld], [horizon][n][ld]
     const double *q_traj, *dq_traj; size_t ld_traj;      // [horizon][n][ld_traj]: the states after each step
@@ -42,8 +42,7 @@ struct RbAdjointArgs {
     const double* cost_w;
     double *grad_tau, *grad_q0, *grad_dq0;
     double dt; int horizon;
-    bool tip = false;                                    // with cost_w: add the tip-pose terms of its RB_CW_TIP row
-    bool col = false;                                    // with cost_w and tip: add the collision terms of its block at RB_CW_COL
+    RbCostTerms terms = RB_COST_QUAD;                    // with cost_w: the terms of the block, as for RbOps::rollout
 };
 cudaError_t rb_launch_rollout_adjoint(int n, const double* flat_model, const RbAdjointArgs& a, size_t B, size_t ld, int* status,
                                       cudaStream_t st);
