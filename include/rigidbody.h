@@ -433,6 +433,50 @@ int multibody_rollout_collision_cost_grad(RbGpu* g, const double* q0, const doub
                                           double* grad_dq0, size_t n_traj, size_t ld, RbLayout layout, RbMem mem,
                                           void* stream);
 
+/* ---- one MPPI iteration (DESIGN.md 4.12) ------------------------------------------------------
+ * P = n_problems independent problems, each with its own start state (q0, dq0) and nominal torque sequence u_nom, all
+ * sharing the cost terms (weights, tip, col: checked and selected as in multibody_rollout_collision_cost; weights == NULL
+ * = no quadratic terms, a NULL or inactive tip / col = those terms off).  q0, dq0 are laid out like one state array and
+ * u_nom, u_new like tau of a rollout with n_traj = P (layout and ld refer to P).  With K = n_samples, H = horizon:
+ *   noise: sample s = p K + k (global over the batch), step t, joint i use the counter c = (s H + t) n + i and
+ *     z = splitmix64(seed + 0x9E3779B97F4A7C15 (c + 1))   (the mixer of multibody_gpu_fill),
+ *     u1 = ((z >> 32) + 0.5) 2^-32,  u2 = (z & 0xffffffff) 2^-32,  eps = sqrt(-2 ln u1) cospi(2 u2);
+ *     sample 0 of every problem has eps = 0 (it is the nominal sequence);
+ *   samples: tau_{p,k,t,i} = min(max(fma(sigma_i, eps, u_nom_{p,t,i}), lower_i), upper_i)  (a NaN passes through);
+ *   cost: c_{p,k} = what multibody_rollout_collision_cost returns for (q0_p, dq0_p, tau_{p,k}, dt, H) with these terms, bit
+ *     for bit on the same engine;
+ *   weights: m_p = min over the finite c_{p,k};  w_{p,k} = exp((m_p - c_{p,k}) / lambda) for a finite cost, else 0;
+ *     eta_p = sum_k w_{p,k};
+ *   update: u_new_{p,t,i} = (sum_k w_{p,k} tau_{p,k,t,i}) / eta_p, the weighted mean of the clamped samples (within the
+ *     bounds up to rounding).  A problem with no finite cost gets NaN in u_new and in its weights.
+ * Optional outputs (each may be NULL): cost [P K] (sample k of problem p at p K + k), sample_weights [P K] = w / eta, and
+ * samples = tau shaped like tau of a rollout with n_traj = P K (SOA dense [H][n][P K], leading dimension P K whatever ld
+ * is; AOS [H][P K][n]).  A sample that meets a non-SPD mass matrix sets the status as the rollout cost does (RB_ERR_NOT_SPD
+ * from host calls, the status word for device calls); its cost is NaN, its weight 0, and every output is still written.
+ * horizon == 0: every sample costs the terminal cost of q0 and the weights are uniform; u_nom is not read and u_new is not
+ * written.  RB_ERR_NULL for opt or sigma NULL, q0, dq0, u_nom or u_new NULL when H > 0, or q0 or dq0 NULL when H == 0 and
+ * cost or sample_weights is asked for; RB_ERR_ARG for n_samples < 1,
+ * a temperature that is not finite and > 0, a negative or non-finite sigma, a NaN bound or lower > upper, and whatever the
+ * cost calls reject.  The results depend on the inputs and the seed only: not on layout, memory kind, chunking or a
+ * multi-device handle (host calls slice the problems; a problem runs on one device), and every sum runs in an order fixed
+ * by (P, K, H, n), without atomics.  Every chain, tree and kernel family multibody_rollout_cost serves.  Every call takes a
+ * stream-ordered workspace on its stream of at most 1 GiB per chunk of whole problems, plus, when `samples` is given (the
+ * rollout then reads it in place), the broadcast start states: 16 n bytes per sample.  It comes from a pool the engine owns,
+ * which keeps up to 1 GiB of it between calls and gives that back when the engine is freed.  Host and AoS calls stage only
+ * the arguments passed: without `samples`, nothing of size H n P K is staged. */
+typedef struct RbMppiOptions {
+    const double* sigma;      /* [n] noise standard deviation per joint, finite, >= 0 (required) */
+    const double* lower;      /* [n] torque bounds, +-inf allowed; NULL = unbounded */
+    const double* upper;      /* [n] */
+    double temperature;       /* lambda > 0, finite */
+    int32_t n_samples;        /* K >= 1 samples per problem */
+    uint64_t seed;
+} RbMppiOptions;
+int multibody_mppi_step(RbGpu* g, const double* q0, const double* dq0, const double* u_nom, double dt, int horizon,
+                        const RbQuadCost* weights, const RbTipCost* tip, const RbCollisionCost* col,
+                        const RbMppiOptions* opt, double* u_new, double* cost, double* sample_weights, double* samples,
+                        size_t n_problems, size_t ld, RbLayout layout, RbMem mem, void* stream);
+
 /* ---- device-side helpers (bench / tests) --------------------------------------------------- */
 /* Fill a device SOA array [n][ld] with the counter-based sampler of SURVEY.md 8d:
  * value(joint i, state s) = fma(hi[i]-lo[i], u, lo[i]),  u = top 53 bits of

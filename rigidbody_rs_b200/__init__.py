@@ -500,6 +500,47 @@ class Multibody:
         `tip`, `collision` and the weights as for `rollout_cost`."""
         return _rollout_cost_function().apply(self, q0, dq0, tau, float(dt), tip, collision, weights)
 
+    def mppi_step(self, q0, dq0, u_nom, dt, sigma, n_samples, temperature, seed, limits=True, layout="soa", tip=None, collision=None,
+                  samples=False, **weights):
+        """One MPPI iteration for each of P problems (include/rigidbody.h multibody_mppi_step, where the sampler, the weights
+        and the update are stated): K = n_samples torque sequences around each nominal sequence, drawn on the device from
+        `seed` (sample 0 is the nominal one) and clamped to the bounds, costed with the fused rollout cost, and averaged with
+        softmin weights of temperature lambda.  The cost terms are `rollout_cost`'s: the weights (q_ref, w_q, ...), `tip`
+        and `collision`.  soa: q0, dq0 [n, P], u_nom [H, n, P];  aos: [P, n], [P, n], [H, P, n].  sigma: n values or one.
+        limits=True bounds the samples by +-limits()["effort"] (a joint with effort <= 0 is unbounded); None = unbounded; or
+        a (lower, upper) pair.  Returns (u_new shaped like u_nom, cost [P, K], sample_weights [P, K]), and with samples=True
+        also the samples [H, n, P K] (soa) or [H, P K, n] (aos), sample k of problem p at p K + k."""
+        a_q, a_dq, a_u, P, H, lay, new = self._rollout_args(q0, dq0, u_nom, layout, "mppi_step")
+        cuda = a_q.cuda
+        if cuda and a_q.device.index not in (None, self.device):
+            raise ValueError(f"tensors are on cuda:{a_q.device.index}, engine is on cuda:{self.device}")
+        n, K = self.n, int(n_samples)
+        vec = lambda v: np.ascontiguousarray(np.broadcast_to(np.asarray(v, dtype=np.float64), (n,)))
+        if limits is True:
+            eff = self.limits()["effort"]
+            lo, hi = np.where(eff > 0, -eff, -np.inf), np.where(eff > 0, eff, np.inf)
+        elif limits is None:
+            lo, hi = np.full(n, -np.inf), np.full(n, np.inf)
+        else:
+            lo, hi = (vec(v) for v in limits)
+        sg = vec(sigma)
+        dp = lambda a: a.ctypes.data_as(C.POINTER(C.c_double))
+        opt = _lib.RbMppiOptions(sigma=dp(sg), lower=dp(lo), upper=dp(hi), temperature=float(temperature), n_samples=K,
+                                 seed=int(seed) & 0xFFFFFFFFFFFFFFFF)
+        qc, keep = self._quad_cost(**weights)
+        tc, keep_tip = _tip_cost(tip or {}) if tip is not None or collision is not None else (None, None)
+        cc, keep_col = _collision_cost(collision) if collision is not None else (None, None)
+        Kp = max(K, 0)
+        u_new, cost, sw = new(a_u.shape), new((P, Kp)), new((P, Kp))
+        smp = new((H, n, P * Kp) if lay == RB_LAYOUT_SOA else (H, P * Kp, n)) if samples else None
+        ptr = lambda a: C.c_void_p(a.ptr) if a is not None else None
+        ref = lambda s: C.byref(s) if s is not None else None
+        check(lib.multibody_mppi_step(self._h, ptr(a_q), ptr(a_dq), ptr(a_u), float(dt), int(H), C.byref(qc), ref(tc), ref(cc), C.byref(opt),
+                                      ptr(u_new), ptr(cost), ptr(sw), ptr(smp), P, 0, lay, RB_MEM_DEVICE if cuda else RB_MEM_HOST,
+                                      self._stream(cuda, a_q)))
+        res = (u_new.arr, cost.arr, sw.arr)
+        return res + (smp.arr,) if samples else res
+
     def rollout_vjp(self, q0, dq0, tau, dt, q_traj, dq_traj, g_q_traj=None, g_dq_traj=None, g_q_final=None, g_dq_final=None,
                     layout="soa"):
         """Vector-Jacobian product of `rollout` (include/rigidbody.h multibody_rollout_vjp): given the trajectory `rollout`

@@ -48,6 +48,11 @@ class RbIkOptions(C.Structure):
                 ("tol_p", C.c_double), ("tol_R", C.c_double), ("damping", C.c_double)]
 
 
+class RbMppiOptions(C.Structure):
+    _fields_ = [("sigma", _dp), ("lower", _dp), ("upper", _dp), ("temperature", C.c_double), ("n_samples", C.c_int32),
+                ("seed", C.c_uint64)]
+
+
 class RbJointLimits(C.Structure):
     _fields_ = [(k, C.c_double * RB_MAX_JOINTS) for k in ("lower", "upper", "velocity", "effort")]
 
@@ -104,6 +109,8 @@ PROTOTYPES = {
                                               C.POINTER(RbCollisionCost), _vp, _vp, _vp, _sz, _sz, _i, _i, _vp]),
     "multibody_rollout_collision_cost_grad": (_i, [_vp, _vp, _vp, _vp, C.c_double, _i, C.POINTER(RbQuadCost), C.POINTER(RbTipCost),
                                                    C.POINTER(RbCollisionCost), _vp, _vp, _vp, _vp, _sz, _sz, _i, _i, _vp]),
+    "multibody_mppi_step": (_i, [_vp, _vp, _vp, _vp, C.c_double, _i, C.POINTER(RbQuadCost), C.POINTER(RbTipCost), C.POINTER(RbCollisionCost),
+                                 C.POINTER(RbMppiOptions), _vp, _vp, _vp, _vp, _sz, _sz, _i, _i, _vp]),
     "multibody_gpu_fill": (_i, [_vp, _vp, _u64, C.c_uint32, _dp, _dp, _sz, _sz, _sz, _vp]),
     "multibody_gpu_sync": (_i, [_vp]),
     "multibody_gpu_status": (_i, [_vp]),

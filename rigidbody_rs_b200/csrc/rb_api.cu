@@ -147,6 +147,9 @@ struct RbGpu {
     int sticky = RB_OK;
     std::atomic<uint64_t> launches{0};
     cudaEvent_t ev_scratch = nullptr;     // orders users of the engine-owned scratch (run-time-n / long-chain families) across streams
+    // stream-ordered pool of the MPPI workspace: keeps up to 1 GiB between calls (the device's default pool hands it back at
+    // every synchronisation, and mapping it again costs more than the step's kernels); released with the engine
+    cudaMemPool_t ws_pool = nullptr;
     std::mutex mu;                        // serialises host-batch calls that share the staging buffers
     std::mutex mu_scratch;                // guards ev_scratch
 };
@@ -355,6 +358,16 @@ int gpu_create(const RbHostModel& model, int device, RbGpu** out) {
         if ((e = cudaEventCreateWithFlags(&g->ev_d2h[k], cudaEventDisableTiming)) != cudaSuccess) return bail(fail_cuda(e, "cudaEventCreate"));
     }
     if ((e = cudaEventCreateWithFlags(&g->ev_scratch, cudaEventDisableTiming)) != cudaSuccess) return bail(fail_cuda(e, "cudaEventCreate"));
+    {
+        cudaMemPoolProps pp = {};
+        pp.allocType = cudaMemAllocationTypePinned;
+        pp.location.type = cudaMemLocationTypeDevice;
+        pp.location.id = device;
+        if ((e = cudaMemPoolCreate(&g->ws_pool, &pp)) != cudaSuccess) return bail(fail_cuda(e, "cudaMemPoolCreate"));
+        uint64_t keep = (uint64_t)1 << 30;            // what one chunk of an MPPI step may take (kGradWorkspace)
+        if ((e = cudaMemPoolSetAttribute(g->ws_pool, cudaMemPoolAttrReleaseThreshold, &keep)) != cudaSuccess)
+            return bail(fail_cuda(e, "cudaMemPoolSetAttribute"));
+    }
     if ((e = cudaMalloc((void**)&g->d_status, 2 * sizeof(int))) != cudaSuccess) return bail(fail_cuda(e, "cudaMalloc(status)"));
     if ((e = cudaMemset(g->d_status, 0, 2 * sizeof(int))) != cudaSuccess) return bail(fail_cuda(e, "cudaMemset(status)"));
     if ((e = cudaMallocHost((void**)&g->h_status, 2 * sizeof(int))) != cudaSuccess) return bail(fail_cuda(e, "cudaMallocHost(status)"));
@@ -742,6 +755,7 @@ extern "C" void multibody_gpu_free(RbGpu* g) {
     DeviceGuard dg(g->device);
     cudaDeviceSynchronize();              // device calls may still be running on caller streams and use our scratch
     if (g->ev_scratch) cudaEventDestroy(g->ev_scratch);
+    if (g->ws_pool) cudaMemPoolDestroy(g->ws_pool);
     for (int k = 0; k < kSlots; ++k) {
         g->in[k].release(); g->out[k].release(); g->tmp[k].release();
         if (g->ev_h2d[k]) cudaEventDestroy(g->ev_h2d[k]);
@@ -1159,17 +1173,19 @@ extern "C" int multibody_ik_batch(RbGpu* g, const double* q_init, const double* 
 namespace {
 // Host and/or AoS arguments of the rollout entries, moved through the engine's staging buffers as SoA with ld = n_traj.
 // An input or output is `arrays` consecutive state arrays (n doubles per trajectory each: q0 is one, tau `horizon`),
-// or, `plain`, one vector of n_traj doubles (the cost).  A NULL pointer is neither copied nor handed on.
+// or, `plain`, one vector of n_traj doubles (the cost).  An output may hold `mult` trajectories per trajectory of the call
+// (the samples of an MPPI step); the caller's SoA copy of such an array group is dense, with leading dimension mult times
+// the whole batch.  A NULL pointer is neither copied nor handed on.
 struct StagedIn { const double* p; size_t arrays; };
-struct StagedOut { double* p; size_t arrays; bool plain; };
+struct StagedOut { double* p; size_t arrays; bool plain; size_t mult = 1; };
 using StagedRun = std::function<int(const double* const* d_in, double* const* d_out, int* d_stat)>;
 
-// Brings `ins` in, calls run() on the staged copies (SoA, ld = n_traj; NULL where the caller passed NULL), brings `outs`
-// back, and drains the stream.  `aos_stride`: elements between consecutive steps of the caller's AoS arrays (0 = n_traj * n,
-// a dense [H][n_traj][n] array; a multi-device engine passes the stride of the whole batch when it hands out slices).
-// Takes g->mu; a host call owns status word 1 and reports it.
+// Brings `ins` in, calls run() on the staged copies (SoA, ld = n_traj, or mult n_traj; NULL where the caller passed NULL),
+// brings `outs` back, and drains the stream.  `batch`: trajectories of the whole batch the caller's arrays hold (0 = n_traj;
+// a multi-device engine passes it when it hands out slices): the distance between consecutive steps of the caller's AoS
+// arrays is batch n.  Takes g->mu; a host call owns status word 1 and reports it.
 int run_staged(RbGpu* g, const std::vector<StagedIn>& ins, const std::vector<StagedOut>& outs, size_t n_traj, size_t ld,
-               RbLayout layout, RbMem mem, size_t aos_stride, cudaStream_t st, const StagedRun& run) {
+               RbLayout layout, RbMem mem, size_t batch, cudaStream_t st, const StagedRun& run) {
     std::lock_guard<std::mutex> lk(g->mu);
     int* const d_stat = g->d_status + (mem == RB_MEM_HOST ? 1 : 0);
     if (mem == RB_MEM_HOST) RB_CUDA(cudaMemsetAsync(d_stat, 0, sizeof(int), st));
@@ -1177,10 +1193,12 @@ int run_staged(RbGpu* g, const std::vector<StagedIn>& ins, const std::vector<Sta
     const int n = g->model.n;
     const size_t B = n_traj, one = (size_t)n * B;
     const bool aos = layout == RB_LAYOUT_AOS, host = mem == RB_MEM_HOST;
-    const size_t src_step = aos ? (aos_stride ? aos_stride : one) : (size_t)n * ld;    // caller's distance between steps
+    if (batch == 0) batch = B;
+    const size_t src_step = aos ? (size_t)n * batch : (size_t)n * ld;    // caller's distance between steps
     size_t in_arrays = 0, out_arrays = 0, out_plain = 0;
-    for (const StagedIn& a : ins) in_arrays += a.arrays;
-    for (const StagedOut& a : outs) (a.plain ? out_plain : out_arrays) += a.arrays;
+    // only the arguments the caller passed take staging space
+    for (const StagedIn& a : ins) if (a.p) in_arrays += a.arrays;
+    for (const StagedOut& a : outs) if (a.p) (a.plain ? out_plain : out_arrays) += a.arrays * a.mult;
     // in[0]: the inputs in order      out[0]: the outputs in order      tmp[0]: AoS landing zone
     int rc = g->in[0].ensure(in_arrays * one * sizeof(double)); if (rc) return rc;
     rc = g->out[0].ensure((out_arrays * one + out_plain * B) * sizeof(double)); if (rc) return rc;
@@ -1212,30 +1230,34 @@ int run_staged(RbGpu* g, const std::vector<StagedIn>& ins, const std::vector<Sta
     double* d = g->in[0].p;
     for (size_t k = 0; k < ins.size(); ++k) {
         d_in[k] = ins[k].p ? d : nullptr;
-        if (ins[k].p) { rc = bring_in(ins[k].p, d, ins[k].arrays); if (rc) return rc; }
+        if (!ins[k].p) continue;
+        rc = bring_in(ins[k].p, d, ins[k].arrays); if (rc) return rc;
         d += ins[k].arrays * one;
     }
     std::vector<double*> d_out(outs.size());
     d = g->out[0].p;
     for (size_t k = 0; k < outs.size(); ++k) {
         d_out[k] = outs[k].p ? d : nullptr;
-        d += outs[k].arrays * (outs[k].plain ? B : one);
+        if (outs[k].p) d += outs[k].arrays * outs[k].mult * (outs[k].plain ? B : one);
     }
     rc = run(d_in.data(), d_out.data(), d_stat); if (rc) return rc;
-    auto bring_out = [&](const double* src, double* dst, size_t arrays) -> int {
+    auto bring_out = [&](const double* src, double* dst, size_t arrays, size_t mult) -> int {
         if (!dst) return RB_OK;
+        const size_t Bm = B * mult, one_m = one * mult;
+        const size_t ld_m = mult == 1 ? ld : mult * batch;                // caller's SoA leading dimension
+        const size_t step_m = aos ? mult * src_step : (size_t)n * ld_m;   // caller's distance between steps
         for (size_t a = 0; a < arrays; ++a) {
-            const double* s_a = src + a * one;
-            double* d_a = dst + a * src_step;
+            const double* s_a = src + a * one_m;
+            double* d_a = dst + a * step_m;
             if (!aos) {
-                RB_CUDA(cudaMemcpy2DAsync(d_a, ld * sizeof(double), s_a, B * sizeof(double), B * sizeof(double), (size_t)n,
+                RB_CUDA(cudaMemcpy2DAsync(d_a, ld_m * sizeof(double), s_a, Bm * sizeof(double), Bm * sizeof(double), (size_t)n,
                                           host ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice, st));
             } else {
-                double* a_dst = host ? d_tmp + a * one : d_a;
-                cudaError_t e2 = rb_launch_soa_to_aos(s_a, a_dst, n, B, B, st);
+                double* a_dst = host ? d_tmp + a * one_m : d_a;
+                cudaError_t e2 = rb_launch_soa_to_aos(s_a, a_dst, n, Bm, Bm, st);
                 g->launches += 1;
                 if (e2 != cudaSuccess) return fail_cuda(e2, "soa_to_aos launch");
-                if (host) RB_CUDA(cudaMemcpyAsync(d_a, a_dst, one * sizeof(double), cudaMemcpyDeviceToHost, st));
+                if (host) RB_CUDA(cudaMemcpyAsync(d_a, a_dst, one_m * sizeof(double), cudaMemcpyDeviceToHost, st));
             }
         }
         return RB_OK;
@@ -1244,16 +1266,17 @@ int run_staged(RbGpu* g, const std::vector<StagedIn>& ins, const std::vector<Sta
     bool first = true;
     for (size_t k = 0; k < outs.size(); ++k) {
         const StagedOut& o = outs[k];
+        if (!o.p) continue;
         if (o.plain) {
-            if (o.p) RB_CUDA(cudaMemcpyAsync(o.p, d, B * sizeof(double), host ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice, st));
-            d += o.arrays * B;
+            RB_CUDA(cudaMemcpyAsync(o.p, d, B * o.mult * sizeof(double), host ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice, st));
+            d += o.arrays * o.mult * B;
             continue;
         }
         // the AoS landing zone is reused per output array group, so drain between groups
         if (!first && aos && host) RB_CUDA(cudaStreamSynchronize(st));
         first = false;
-        rc = bring_out(d, o.p, o.arrays); if (rc) return rc;
-        d += o.arrays * one;
+        rc = bring_out(d, o.p, o.arrays, o.mult); if (rc) return rc;
+        d += o.arrays * o.mult * one;
     }
     // everything above went through engine-owned staging: drain before another call may reuse it
     RB_CUDA(cudaStreamSynchronize(st));
@@ -1332,7 +1355,7 @@ int pack_cost_block(const RbHostModel& m, const RbQuadCost* w, const RbTipCost* 
 int rollout_impl(RbGpu* g, const double* q0, const double* dq0, const double* tau, double dt, int horizon,
                  double* q_traj, double* dq_traj, double* q_final, double* dq_final, const RbQuadCost* w, const RbTipCost* tip,
                  const RbCollisionCost* col, double* cost, size_t n_traj, size_t ld, RbLayout layout, RbMem mem, void* stream,
-                 size_t aos_stride = 0) {
+                 size_t batch = 0) {
     if (!g) return fail(RB_ERR_NULL, "engine handle is NULL");
     if (!g->peers.empty()) {
         if (layout != RB_LAYOUT_SOA && layout != RB_LAYOUT_AOS) return fail(RB_ERR_ARG, "bad layout");
@@ -1348,7 +1371,7 @@ int rollout_impl(RbGpu* g, const double* q0, const double* dq0, const double* ta
             auto at = [&](const double* p) { return p ? p + o : nullptr; };
             auto atw = [&](double* p) { return p ? p + o : nullptr; };
             return rollout_impl(g->peers[i], at(q0), at(dq0), at(tau), dt, horizon, atw(q_traj), atw(dq_traj), atw(q_final), atw(dq_final),
-                                w, tip, col, cost ? cost + lo : nullptr, hi - lo, ld, layout, mem, nullptr, aos ? n_traj * n : 0);
+                                w, tip, col, cost ? cost + lo : nullptr, hi - lo, ld, layout, mem, nullptr, n_traj);
         });
     }
     if (layout != RB_LAYOUT_SOA && layout != RB_LAYOUT_AOS) return fail(RB_ERR_ARG, "bad layout");
@@ -1389,7 +1412,7 @@ int rollout_impl(RbGpu* g, const double* q0, const double* dq0, const double* ta
     // Host pointers and/or AoS: stage everything on the device as SoA with ld = n_traj, run once, bring results back.
     const size_t H = (size_t)horizon;
     return run_staged(g, {{q0, 1}, {dq0, 1}, {tau, H}}, {{q_traj, H, false}, {dq_traj, H, false}, {q_final, 1, false}, {dq_final, 1, false}, {cost, 1, true}},
-                      n_traj, ld, layout, mem, aos_stride, st,
+                      n_traj, ld, layout, mem, batch, st,
                       [&](const double* const* in, double* const* out, int* d_stat) { return run(in, out, n_traj, d_stat); });
 }
 // Arguments of multibody_rollout_vjp (q_traj .. g_dqf) and multibody_rollout_cost_grad (w, cost).
@@ -1466,7 +1489,7 @@ int grad_device(RbGpu* g, const GradArgs& a, const CostBlock& cb, size_t B, size
     return rc;
 }
 
-int grad_impl(RbGpu* g, const GradArgs& a, size_t n_traj, size_t ld, RbLayout layout, RbMem mem, void* stream, size_t aos_stride = 0) {
+int grad_impl(RbGpu* g, const GradArgs& a, size_t n_traj, size_t ld, RbLayout layout, RbMem mem, void* stream, size_t batch = 0) {
     if (!g) return fail(RB_ERR_NULL, "engine handle is NULL");
     if (g->model.n > RB_DERIV_MAX_N || !g->model.serial)
         return fail(RB_ERR_UNSUPPORTED, "rollout gradients use the forward-dynamics derivative kernels, which serve serial chains of at most 12 joints");
@@ -1488,7 +1511,7 @@ int grad_impl(RbGpu* g, const GradArgs& a, size_t n_traj, size_t ld, RbLayout la
             s.g_q = at(a.g_q); s.g_dq = at(a.g_dq); s.g_qf = at(a.g_qf); s.g_dqf = at(a.g_dqf);
             s.cost = a.cost ? a.cost + lo : nullptr;
             s.grad_tau = atw(a.grad_tau); s.grad_q0 = atw(a.grad_q0); s.grad_dq0 = atw(a.grad_dq0);
-            return grad_impl(g->peers[i], s, hi - lo, ld, layout, mem, nullptr, aos ? n_traj * n : 0);
+            return grad_impl(g->peers[i], s, hi - lo, ld, layout, mem, nullptr, n_traj);
         });
     }
     if (mem != RB_MEM_HOST && mem != RB_MEM_DEVICE) return fail(RB_ERR_ARG, "bad mem");
@@ -1509,9 +1532,147 @@ int grad_impl(RbGpu* g, const GradArgs& a, size_t n_traj, size_t ld, RbLayout la
     // Host pointers and/or AoS: staged like the rollout; the staged call then runs as a device SoA call with ld = n_traj.
     return run_staged(g, {{a.q0, 1}, {a.dq0, 1}, {a.tau, H}, {a.q_traj, H}, {a.dq_traj, H}, {a.g_q, H}, {a.g_dq, H}, {a.g_qf, 1}, {a.g_dqf, 1}},
                       {{a.grad_tau, H, false}, {a.grad_q0, 1, false}, {a.grad_dq0, 1, false}, {a.cost, 1, true}},
-                      n_traj, ld, layout, mem, aos_stride, st, [&](const double* const* in, double* const* out, int* d_stat) -> int {
+                      n_traj, ld, layout, mem, batch, st, [&](const double* const* in, double* const* out, int* d_stat) -> int {
         const GradArgs s{in[0], in[1], in[2], a.dt, a.horizon, in[3], in[4], in[5], in[6], in[7], in[8], a.w, out[3], out[0], out[1], out[2], a.tip, a.col};
         return grad_device(g, s, cb, n_traj, n_traj, st, d_stat);
+    });
+}
+// Arguments of multibody_mppi_step: q0, dq0, u_nom and u_new per problem; cost, sample weights and samples per sample.
+struct MppiArgs {
+    const double *q0, *dq0, *u_nom; double dt; int horizon;
+    double *u_new, *cost, *sw, *samples;
+};
+
+// Checks an RbMppiOptions and packs it into the kernels' parameter block.
+int pack_mppi(const RbHostModel& m, const RbMppiOptions* o, int horizon, RbMppiParam& P) {
+    if (!o || !o->sigma) return fail(RB_ERR_NULL, "MPPI options or sigma are NULL");
+    memset(&P, 0, sizeof(P));
+    if (o->n_samples < 1) return fail(RB_ERR_ARG, "MPPI n_samples < 1");
+    if (!std::isfinite(o->temperature) || !(o->temperature > 0.0)) return fail(RB_ERR_ARG, "MPPI temperature must be finite and positive");
+    for (int i = 0; i < m.n; ++i) {
+        P.sigma[i] = o->sigma[i];
+        P.lower[i] = o->lower ? o->lower[i] : -INFINITY;
+        P.upper[i] = o->upper ? o->upper[i] : INFINITY;
+        if (!std::isfinite(P.sigma[i]) || P.sigma[i] < 0.0) return fail(RB_ERR_ARG, "MPPI sigma must be finite and non-negative");
+        if (std::isnan(P.lower[i]) || std::isnan(P.upper[i]) || P.lower[i] > P.upper[i])
+            return fail(RB_ERR_ARG, "MPPI bounds must not be NaN and lower <= upper");
+    }
+    P.seed = o->seed; P.K = (size_t)o->n_samples; P.n = m.n; P.H = horizon;
+    return RB_OK;
+}
+
+// One MPPI step of P problems on device SoA arrays (q0, dq0, u_nom, u_new with leading dimension ld; cost and sw dense
+// [P K]; samples, when not NULL, dense [H][n][P K]), asynchronous on st.  Per chunk of whole problems: the sampler, the
+// engine's rollout launcher with the call's terms (so that each cost is multibody_rollout_collision_cost's, bit for bit),
+// the weights and the two update stages, in one ScratchOrder region with the weight upload.  The workspace comes from the
+// engine's stream-ordered pool, at most kGradWorkspace per chunk; with caller samples the rollout reads them in place, and
+// the broadcast start states then share their leading dimension P K.
+int mppi_device(RbGpu* g, const MppiArgs& a, const RbMppiParam& M, double lambda, const CostBlock& cb, size_t P, size_t ld,
+                size_t p_first, cudaStream_t st, int* d_stat) {
+    const size_t K = M.K, n = (size_t)M.n, H = (size_t)M.H, rows = H * n, nt = rb_mppi_tiles(K);
+    const bool direct = a.samples && H > 0;
+    // per problem: samples and start states (unless direct), cost, weights, eta, update partials
+    const size_t per_prob = K * ((direct ? 0 : rows + 2 * n) + 2) + 1 + nt * rows;
+    const size_t fixed = direct ? 2 * n * P * K : 0;
+    const size_t chunk = std::max<size_t>(1, std::min<size_t>({P, kGradWorkspace / (per_prob * sizeof(double)), 65535}));
+    ScratchOrder so(g, true, st);
+    RB_CUDA(cudaMemcpyAsync(g->cost_w.p, cb.w, cb.bytes(), cudaMemcpyHostToDevice, st));
+    double* ws = nullptr;
+    RB_CUDA(cudaMallocFromPoolAsync((void**)&ws, (fixed + chunk * per_prob) * sizeof(double), g->ws_pool, st));
+    const auto& ro = g->rollout;
+    int rc = RB_OK;
+    for (size_t lo = 0; lo < P && rc == RB_OK; lo += chunk) {
+        const size_t cnt = std::min(chunk, P - lo), J = cnt * K;
+        const size_t ldS = direct ? P * K : J;                 // leading dimension of the samples and the start states
+        double* at = ws + fixed;
+        double *tau = nullptr, *q0s, *dq0s;
+        if (direct) {
+            tau = a.samples + lo * K; q0s = ws + lo * K; dq0s = ws + n * P * K + lo * K;
+        } else {
+            if (rows) tau = at;
+            q0s = at + rows * J; dq0s = q0s + n * J;
+            at += (rows + 2 * n) * chunk * K;
+        }
+        double* cost = a.cost ? a.cost + lo * K : at;
+        double* w = at + chunk * K;
+        double* eta = w + chunk * K;
+        double* part = eta + chunk;
+        cudaError_t e = rb_launch_mppi_sample(M, a.q0 + lo, a.dq0 + lo, a.u_nom ? a.u_nom + lo : nullptr, ld, p_first + lo, cnt, tau,
+                                              q0s, dq0s, ldS, st);
+        g->launches += 1;
+        if (e != cudaSuccess) { rc = fail_cuda(e, "MPPI sampler launch"); break; }
+        e = ro.fn(ro.param, q0s, dq0s, tau, a.dt, a.horizon, nullptr, nullptr, nullptr, nullptr, J, ldS, d_stat, g->cost_w.p, cost,
+                  cb.terms, st);
+        g->launches += 1;
+        if (e != cudaSuccess) { rc = fail_cuda(e, "rollout launch"); break; }
+        e = rb_launch_mppi_weights(cost, K, lambda, cnt, w, eta, a.sw ? a.sw + lo * K : nullptr, st);
+        g->launches += 1;
+        if (e != cudaSuccess) { rc = fail_cuda(e, "MPPI weights launch"); break; }
+        if (rows) {
+            e = rb_launch_mppi_update(tau, ldS, K, (int)rows, w, eta, cnt, part, a.u_new + lo, ld, st);
+            g->launches += 2;
+            if (e != cudaSuccess) rc = fail_cuda(e, "MPPI update launch");
+        }
+    }
+    cudaError_t e = cudaFreeAsync(ws, st);
+    if (e != cudaSuccess && rc == RB_OK) rc = fail_cuda(e, "cudaFreeAsync(MPPI workspace)");
+    return rc;
+}
+
+// multibody_mppi_step.  p_first: global index of the first problem (the sample counter of a multi-device slice);
+// batch: problems of the whole batch the caller's arrays hold (0 = P), as for run_staged.
+int mppi_impl(RbGpu* g, const MppiArgs& a, const RbQuadCost* w, const RbTipCost* tip, const RbCollisionCost* col,
+              const RbMppiOptions* opt, size_t P, size_t ld, RbLayout layout, RbMem mem, void* stream, size_t p_first = 0,
+              size_t batch = 0) {
+    if (!g) return fail(RB_ERR_NULL, "engine handle is NULL");
+    RbMppiParam M;
+    int rc = pack_mppi(g->model, opt, a.horizon, M);
+    if (rc != RB_OK) return rc;
+    if (layout != RB_LAYOUT_SOA && layout != RB_LAYOUT_AOS) return fail(RB_ERR_ARG, "bad layout");
+    const size_t K = M.K;
+    if (!g->peers.empty()) {
+        if (mem != RB_MEM_HOST) return fail(mem == RB_MEM_DEVICE ? RB_ERR_UNSUPPORTED : RB_ERR_ARG, mem == RB_MEM_DEVICE ? kMultiDeviceOnly : "bad mem");
+        if (P == 0) return RB_OK;
+        const bool aos = layout == RB_LAYOUT_AOS;
+        const size_t n = (size_t)g->model.n;
+        if (!aos) { if (ld == 0) ld = P; if (ld < P) return fail(RB_ERR_ARG, "ld < n_problems"); }
+        return run_on_peers(g, [&](size_t i) -> int {
+            size_t lo, hi; slice_bounds(P, g->peers.size(), i, &lo, &hi);
+            if (hi == lo) return RB_OK;
+            const size_t o = lo * (aos ? n : 1);              // offset of problem lo inside one state array
+            auto at = [&](const double* p) { return p ? p + o : nullptr; };
+            auto atw = [&](double* p) { return p ? p + o : nullptr; };
+            auto per_sample = [&](double* p, size_t per) { return p ? p + lo * K * per : nullptr; };
+            MppiArgs s = a;
+            s.q0 = at(a.q0); s.dq0 = at(a.dq0); s.u_nom = at(a.u_nom); s.u_new = atw(a.u_new);
+            s.cost = per_sample(a.cost, 1); s.sw = per_sample(a.sw, 1); s.samples = per_sample(a.samples, aos ? n : 1);
+            return mppi_impl(g->peers[i], s, w, tip, col, opt, hi - lo, ld, layout, mem, nullptr, lo, P);
+        });
+    }
+    if (mem != RB_MEM_HOST && mem != RB_MEM_DEVICE) return fail(RB_ERR_ARG, "bad mem");
+    if (a.horizon < 0) return fail(RB_ERR_ARG, "horizon < 0");
+    if (!std::isfinite(a.dt)) return fail(RB_ERR_ARG, "dt must be finite");
+    const RbQuadCost none{};
+    CostBlock cb;
+    rc = pack_cost_block(g->model, w ? w : &none, tip, col, cb);
+    if (rc != RB_OK) return rc;
+    if (P == 0) return RB_OK;
+    const size_t H = (size_t)a.horizon;
+    // horizon == 0: u_nom is not read and u_new not written; the costs are the terminal cost of q0
+    if (H == 0 && !a.cost && !a.sw) return RB_OK;
+    if (!a.q0 || !a.dq0 || (H > 0 && (!a.u_nom || !a.u_new))) return fail(RB_ERR_NULL, "input or output pointer is NULL");
+    if (layout == RB_LAYOUT_SOA) { if (ld == 0) ld = P; if (ld < P) return fail(RB_ERR_ARG, "ld < n_problems"); }
+    DeviceGuard dg(g->device);
+    if (!dg.ok) return fail(RB_ERR_CUDA, "cudaSetDevice failed");
+    cudaStream_t st = mem == RB_MEM_DEVICE ? (cudaStream_t)stream : g->stream;
+    const double lambda = opt->temperature;
+    if (mem == RB_MEM_DEVICE && layout == RB_LAYOUT_SOA) return mppi_device(g, a, M, lambda, cb, P, ld, p_first, st, g->d_status);
+    // Host pointers and/or AoS: staged like the rollout (the per-sample outputs with K trajectories per problem), then run
+    // as a device SoA call with ld = P.
+    return run_staged(g, {{a.q0, 1}, {a.dq0, 1}, {a.u_nom, H}}, {{a.u_new, H, false}, {a.cost, 1, true, K}, {a.sw, 1, true, K}, {a.samples, H, false, K}},
+                      P, ld, layout, mem, batch, st, [&](const double* const* in, double* const* out, int* d_stat) -> int {
+        const MppiArgs s{in[0], in[1], in[2], a.dt, a.horizon, out[0], out[1], out[2], out[3]};
+        return mppi_device(g, s, M, lambda, cb, P, P, p_first, st, d_stat);
     });
 }
 }  // namespace
@@ -1591,6 +1752,14 @@ extern "C" int multibody_rollout_collision_cost_grad(RbGpu* g, const double* q0,
     const GradArgs a{q0, dq0, tau, dt, horizon, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, weights ? weights : &none, cost,
                      grad_tau, grad_q0, grad_dq0, tip, col};
     return grad_impl(g, a, n_traj, ld, layout, mem, stream);
+}
+
+extern "C" int multibody_mppi_step(RbGpu* g, const double* q0, const double* dq0, const double* u_nom, double dt, int horizon,
+                                  const RbQuadCost* weights, const RbTipCost* tip, const RbCollisionCost* col, const RbMppiOptions* opt,
+                                  double* u_new, double* cost, double* sample_weights, double* samples, size_t n_problems, size_t ld,
+                                  RbLayout layout, RbMem mem, void* stream) {
+    const MppiArgs a{q0, dq0, u_nom, dt, horizon, u_new, cost, sample_weights, samples};
+    return mppi_impl(g, a, weights, tip, col, opt, n_problems, ld, layout, mem, stream);
 }
 
 // ===================================================================== helpers

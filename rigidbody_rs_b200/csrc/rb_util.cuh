@@ -70,3 +70,22 @@ cudaError_t rb_launch_sphere_distance(const double* model, int n, const double* 
 // workspace of n doubles per thread of the grid (cudaMallocAsync on st).
 cudaError_t rb_launch_ik(const double* model, int n, const RbIkParam& P, const double* q_init, const double* p_target,
                          const double* R_target, double* out, size_t B, size_t ld, int sm_count, cudaStream_t st);
+// One MPPI step (rb_kernels_mppi.cu, multibody_mppi_step), on a chunk of `cnt` problems of K samples each, device SoA.
+struct RbMppiParam {
+    double sigma[RB_MAX_N], lower[RB_MAX_N], upper[RB_MAX_N];
+    uint64_t seed;
+    size_t K;                          // samples per problem
+    int n, H;
+};
+// Sampler: the start states q0s / dq0s [n][ldS] and tau [H][n][ldS] of sample j = p K + k of the chunk (column j), from
+// q0 / dq0 [n][ld] and u_nom [H][n][ld] (column p); p_first = the global index of the chunk's first problem.
+cudaError_t rb_launch_mppi_sample(const RbMppiParam& P, const double* q0, const double* dq0, const double* u_nom, size_t ld,
+                                  size_t p_first, size_t cnt, double* tau, double* q0s, double* dq0s, size_t ldS, cudaStream_t st);
+// Weights: from cost [cnt K], the unnormalised weights w [cnt K] and their sums eta [cnt]; sw [cnt K] = w / eta unless NULL.
+cudaError_t rb_launch_mppi_weights(const double* cost, size_t K, double lambda, size_t cnt, double* w, double* eta, double* sw,
+                                   cudaStream_t st);
+// Update, two launches: u_new [rows][ld] (column p) = sum_k w tau / eta over tau [rows][ldS], rows = H n.  `part` holds
+// cnt * rb_mppi_tiles(K) * rows doubles.
+size_t rb_mppi_tiles(size_t K);
+cudaError_t rb_launch_mppi_update(const double* tau, size_t ldS, size_t K, int rows, const double* w, const double* eta, size_t cnt,
+                                  double* part, double* u_new, size_t ld, cudaStream_t st);

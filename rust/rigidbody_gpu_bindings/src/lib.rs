@@ -141,6 +141,10 @@ extern "C" {
                                                  w: *const RbQuadCost, tip: *const RbTipCost, col: *const RbCollisionCost, cost: *mut f64,
                                                  grad_tau: *mut f64, grad_q0: *mut f64, grad_dq0: *mut f64, n_traj: usize, ld: usize,
                                                  layout: RbLayout, mem: RbMem, stream: *mut c_void) -> c_int;
+    pub fn multibody_mppi_step(g: *mut RbGpu, q0: *const f64, dq0: *const f64, u_nom: *const f64, dt: f64, horizon: c_int,
+                               w: *const RbQuadCost, tip: *const RbTipCost, col: *const RbCollisionCost, opt: *const RbMppiOptions,
+                               u_new: *mut f64, cost: *mut f64, sample_weights: *mut f64, samples: *mut f64, n_problems: usize, ld: usize,
+                               layout: RbLayout, mem: RbMem, stream: *mut c_void) -> c_int;
     // ---- device-side helpers
     pub fn multibody_gpu_fill(g: *mut RbGpu, dev_out: *mut f64, seed: u64, field: u32, lo: *const f64, hi: *const f64,
                               first_index: usize, count: usize, ld: usize, stream: *mut c_void) -> c_int;
@@ -222,6 +226,20 @@ pub struct RbIkOptions {
     pub tol_p: f64,
     pub tol_r: f64,
     pub damping: f64,
+}
+
+/// Options of `multibody_mppi_step` (include/rigidbody.h RbMppiOptions, where the sampler, the weights and the update are
+/// stated): host arrays of n values (`sigma` required; `lower`, `upper` null = unbounded), the temperature lambda > 0, the
+/// number of samples per problem and the seed of the sampler.
+#[repr(C)]
+#[derive(Clone, Copy)]
+pub struct RbMppiOptions {
+    pub sigma: *const f64,
+    pub lower: *const f64,
+    pub upper: *const f64,
+    pub temperature: f64,
+    pub n_samples: i32,
+    pub seed: u64,
 }
 
 #[derive(Debug)]
@@ -464,6 +482,25 @@ impl GpuMultibody {
         check(unsafe { multibody_rollout_collision_cost(self.raw, q0.as_ptr(), dq0.as_ptr(), tau.as_ptr(), dt, horizon as c_int, w, tip, col,
                                                         cost.as_mut_ptr(), ptr::null_mut(), ptr::null_mut(), n_traj, 0, layout, RbMem::Host,
                                                         ptr::null_mut()) })
+    }
+
+    /// One MPPI iteration per problem (multibody_mppi_step), host slices: `q0`, `dq0` n values per problem, `u_nom` and
+    /// `u_new` n per step and problem, `cost` and `sample_weights` `opt.n_samples` per problem (sample k of problem p at
+    /// p K + k).  The cost terms as for `rollout_collision_cost`.
+    #[allow(clippy::too_many_arguments)]
+    pub fn mppi_step(&mut self, q0: &[f64], dq0: &[f64], u_nom: &[f64], dt: f64, horizon: usize, w: &RbQuadCost, tip: &RbTipCost,
+                     col: &RbCollisionCost, opt: &RbMppiOptions, u_new: &mut [f64], cost: &mut [f64], sample_weights: &mut [f64],
+                     n_problems: usize, layout: RbLayout) -> Result<(), RbError> {
+        let k = opt.n_samples.max(0) as usize;
+        self.check_len("q0", q0.len(), self.n, n_problems)?;
+        self.check_len("dq0", dq0.len(), self.n, n_problems)?;
+        self.check_len("u_nom", u_nom.len(), self.n * horizon, n_problems)?;
+        self.check_len("u_new", u_new.len(), self.n * horizon, n_problems)?;
+        self.check_len("cost", cost.len(), k, n_problems)?;
+        self.check_len("sample_weights", sample_weights.len(), k, n_problems)?;
+        check(unsafe { multibody_mppi_step(self.raw, q0.as_ptr(), dq0.as_ptr(), u_nom.as_ptr(), dt, horizon as c_int, w, tip, col, opt,
+                                           u_new.as_mut_ptr(), cost.as_mut_ptr(), sample_weights.as_mut_ptr(), ptr::null_mut(), n_problems,
+                                           0, layout, RbMem::Host, ptr::null_mut()) })
     }
 
     /// Inverse kinematics of the tip frame (multibody_ik_batch): one damped least-squares problem per entry, host slices.
